@@ -2,6 +2,7 @@
 """bench.py -- ARK/DTB decrypt throughput on B200 (BASELINE.json metric), one JSON line.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg3|cfg2|cfg4]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Headline workload (config.workload = "cfg3", BASELINE.json configs[2], the north_star target): a
@@ -22,6 +23,10 @@ windows of the rank's own shard (both sides of every interior cut and part bound
 windows) are byte-compared with the CPU oracle -- the unmodified reference cipher (oracle/_ref) for
 windows that start a part, its closed-form restatement (pinned against it) for windows deep inside
 one.  `parity_bytes_checked` is the sum over ranks; any mismatch ends the run with rc != 0.
+
+--dump-outputs DIR writes, after the K timed steps of the headline workload, what they left in the output
+buffers (dump_outputs()).  Inputs are seeded, so two builds run with the same arguments can be compared file
+by file.
 
 At N == 1 the line also carries `extra.cfg2` (1 GiB / 10 000 entries, misaligned gather; BASELINE
 configs[1]) and `extra.cfg4` (1 000 000 entries of 1..64 KiB, one launch; configs[3]), each with its
@@ -47,6 +52,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (ROOT, os.path.join(ROOT, "tests")):
     if p not in sys.path:
         sys.path.insert(0, p)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree (which may be read-only)
 
 import synth  # noqa: E402  (synthetic inputs shared with the tests)
 
@@ -439,6 +445,37 @@ def timed_steps(c: Ctx, step, kernel, steps: int, warmup: int):
     return ms_total, kernel_ms, info, launches
 
 
+DUMP_WINDOWS = 1024       # over all ranks
+DUMP_WINDOW_BYTES = 4096  # 4 MiB of payload in all: 16 MiB as float32
+
+
+def dump_windows(descs: np.ndarray, world: int):
+    """(entry index, position in entry, length) arrays of the seeded windows dump_outputs() samples."""
+    rng = np.random.default_rng(2718)
+    idx = rng.integers(0, len(descs), size=max(1, DUMP_WINDOWS // world))
+    lens = descs["len"][idx].astype(np.int64)
+    width = np.minimum(lens, DUMP_WINDOW_BYTES)
+    return idx, rng.integers(0, lens - width + 1), width
+
+
+def dump_outputs(c: Ctx, out_dir: str, descs: np.ndarray, d_dst, d_hdr) -> None:
+    """Write what the last timed step left in this rank's output buffers, as float32 byte values:
+    `hdr.npy`, the whole HDR (rank 0), and `payload.npy`, a fixed sample of the payload -- the dump_windows()
+    of the entries, concatenated (bytes between extract slots are never written and stay out of it).  With
+    N > 1 ranks each rank writes `payload_rank<r>.npy` of its shard.  In-place workloads hold ciphertext or
+    plaintext depending on whether the passes so far (parity check, restore, warm-up, timed steps) are odd or
+    even in number: the cipher is an involution."""
+    torch = c.torch
+    idx, pos, width = dump_windows(descs, c.world)
+    start = descs["dst_off"][idx].astype(np.int64) + pos
+    at = np.concatenate([np.arange(s, s + n) for s, n in zip(start, width)])
+    os.makedirs(out_dir, exist_ok=True)
+    sample = d_dst[torch.from_numpy(at).to(c.dev)].cpu().numpy().astype(np.float32)
+    np.save(os.path.join(out_dir, f"payload_rank{c.rank}.npy" if c.world > 1 else "payload.npy"), sample)
+    if d_hdr is not None:
+        np.save(os.path.join(out_dir, "hdr.npy"), d_hdr.cpu().numpy().astype(np.float32))
+
+
 def sustained(c: Ctx, kernel, payload: int, kernel_ms: float, seconds: float = 3.0) -> dict:
     """>= `seconds` of back-to-back launches of the dominant kernel, with NVML samples."""
     torch = c.torch
@@ -494,9 +531,9 @@ def piece_count(descs: np.ndarray, group: int = 16 * MIB) -> int:
 
 
 def measure_workload(c: Ctx, args, workload: str, *, full: bool, cfg4_n: int = 1_000_000, sustain_s: float = 3.0,
-                     cooldown_s: float = 0.0) -> dict:
+                     cooldown_s: float = 0.0, dump_dir: str | None = None) -> dict:
     """Device-resident value, per-launch roofline, parity, the sustained run (`sustain_s` seconds of back-to-back
-    launches; 0 = skip) and, if `full`, e2e for one workload."""
+    launches; 0 = skip) and, if `full`, e2e for one workload.  `dump_dir`: see dump_outputs()."""
     torch, mb = c.torch, c.mb
     gdescs = global_descs(mb, workload, cfg4_n)
     shard = mb.shard_descs(gdescs, c.rank, c.world) if c.world > 1 else gdescs
@@ -543,6 +580,8 @@ def measure_workload(c: Ctx, args, workload: str, *, full: bool, cfg4_n: int = 1
         torch.cuda.synchronize()  # averaging window has forgotten it, so the burst figure is a burst figure
         time.sleep(cooldown_s)
     ms_total, kernel_ms, clock_info, launches = timed_steps(c, step, kernel, args.steps, args.warmup)
+    if dump_dir:  # before the sustained run, whose launch count depends on the measured kernel time
+        dump_outputs(c, dump_dir, descs, d_dst, d_hdr if do_hdr else None)
     total_payload = int(gdescs["len"].sum())
     value = (total_payload + (HDR_BYTES - 4)) * args.steps / (ms_total * 1e-3) / 1e9
     out = {"value": value, "ms_per_step": ms_total / args.steps, "kernel_ms": kernel_ms,
@@ -585,7 +624,7 @@ def measure_workload(c: Ctx, args, workload: str, *, full: bool, cfg4_n: int = 1
                 raise SystemExit(f"PARITY FAILURE (e2e {workload}): rank {c.rank} piece {i}")
             e2e_checked += n
         e2e_step()  # warm-up 2 (in-place sets: back to plaintext)
-        e2e_steps = max(2, min(args.steps, 4))
+        e2e_steps = args.steps
         c.barrier()
         t0 = time.perf_counter()
         for _ in range(e2e_steps):
@@ -764,7 +803,7 @@ def run_gpu_arm(args) -> None:
     if c.world != args.gpus and not (c.world == 1 and args.gpus == 1):
         if c.world == 1 and args.gpus > 1:
             raise SystemExit("launch with torch.distributed.run --nproc-per-node N for --gpus N")
-    main = measure_workload(c, args, args.workload, full=True)
+    main = measure_workload(c, args, args.workload, full=True, dump_dir=args.dump_outputs)
     extra = {}
     if not args.kernel_only and not args.no_extras:
         if c.world > 1 and args.workload == "cfg3":
@@ -850,7 +889,13 @@ def main() -> None:
     ap.add_argument("--kernel-only", action="store_true",
                     help="profiling aid: device-resident legs only (no sustained run, e2e, extras or CPU baseline)")
     ap.add_argument("--no-extras", action="store_true", help="skip the extra.cfg2 / extra.cfg4 / in-process blocks")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (float32, a seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload == "cfg5"):
+        ap.error("--dump-outputs needs the GPU arm and a cfg2 / cfg3 / cfg4 workload")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

@@ -19,6 +19,7 @@ Only ``tests/``, ``__graft_entry__.smoke()`` and ``bench.py``'s ``cpu_baseline``
 from __future__ import annotations
 
 import ctypes
+import hashlib
 import os
 import subprocess
 
@@ -51,9 +52,14 @@ PART_DTYPE = np.dtype([("off", "<u8"), ("len", "<u4"), ("key", "<i4")])
 
 def build(force: bool = False) -> None:
     """Compile liboracle.so and (when /root/reference is present) _ref/libcycle_ref.so."""
-    if force or not os.path.exists(_LIB) or \
-            os.path.getmtime(_LIB) < os.path.getmtime(os.path.join(_HERE, "cycle_oracle.c")):
-        subprocess.check_call(["make", "-C", _HERE, "liboracle.so"], stdout=subprocess.DEVNULL)
+    # staleness by content, not modification time: a copied tree keeps its build and is never written to
+    with open(os.path.join(_HERE, "cycle_oracle.c"), "rb") as f:
+        fp = hashlib.sha256(f.read()).hexdigest()
+    stamp = _LIB + ".stamp"
+    if force or not os.path.exists(_LIB) or not os.path.exists(stamp) or open(stamp).read().strip() != fp:
+        subprocess.check_call(["make", "-B", "-C", _HERE, "liboracle.so"], stdout=subprocess.DEVNULL)
+        with open(stamp, "w") as f:
+            f.write(fp)
     if os.path.exists("/root/reference/Modulate/CEncryptionCycler.cpp") and \
             (force or not os.path.exists(_REF)):
         subprocess.check_call(["make", "-C", _HERE, "ref"], stdout=subprocess.DEVNULL)

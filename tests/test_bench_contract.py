@@ -99,7 +99,7 @@ def test_gpu_arm_line():
     assert d["gpu_launches"] == 2 * d["steps"]          # HDR Cycle + one batched launch per step
     e = d["e2e"]
     assert e["h2d_bytes_per_step"] > d["config"]["payload_bytes"] and e["d2h_bytes_per_step"] > 0
-    assert 0 < e["value"] < d["value"] and e["parity_bytes_checked"] > 0
+    assert 0 < e["value"] < d["value"] and e["parity_bytes_checked"] > 0 and e["steps"] == d["steps"]
     cb = d["cpu_baseline"]
     assert cb["kind"] in ("reference", "port") and cb["cores"] >= 1 and cb["value"] > 0
     assert d["clocks"]["sm_max_mhz"] and isinstance(d["clocks"]["reasons"], list)
@@ -107,3 +107,31 @@ def test_gpu_arm_line():
         x = d["extra"][w]
         assert x["config"]["workload"] == w and x["config"]["entries"] == entries
         assert x["parity_bytes_checked"] > 0 and 0.3 < x["roofline"]["frac"] < 1.25
+
+
+@pytest.mark.gpu
+def test_dump_outputs_hold_what_the_timed_steps_wrote(tmp_path):
+    """--dump-outputs DIR: float32 files of at most 64 MB in all.  The gather workload (cfg2) writes a fresh
+    destination every step, so every sampled byte must be the oracle's cipher of its entry; the HDR is Cycled
+    in place 7 times (parity pass, restore, 3 warm-ups, 2 timed steps), so it holds ciphertext."""
+    import numpy as np
+
+    sys.path.insert(0, ROOT)
+    import bench
+    import modulate_b200 as mb
+    import oracle
+    import synth
+    run_bench("--workload", "cfg2", "--kernel-only", "--steps", "2", "--warmup", "0", "--dump-outputs", str(tmp_path))
+    assert sorted(p.name for p in tmp_path.iterdir()) == ["hdr.npy", "payload.npy"]
+    assert sum(p.stat().st_size for p in tmp_path.iterdir()) <= 64 << 20
+    got = np.load(tmp_path / "payload.npy")
+    descs = bench.global_descs(mb, "cfg2")
+    idx, pos, width = bench.dump_windows(descs, 1)
+    want = np.concatenate([oracle.cycle_at(synth.payload(int(descs[i]["src_off"]) + p, n), int(descs[i]["key"]), p)
+                           for i, p, n in zip(idx, pos, width)])
+    assert got.dtype == np.float32 and got.size == int(width.sum()) >= 1 << 20
+    assert np.array_equal(got, want.astype(np.float32))
+    hdr = np.load(tmp_path / "hdr.npy")
+    plain = synth.payload(1 << 40, bench.HDR_BYTES)
+    assert hdr.dtype == np.float32 and np.array_equal(hdr[:4], plain[:4].astype(np.float32))
+    assert np.array_equal(hdr[4:], oracle.cycle(plain[4:], synth.PS4_KEY).astype(np.float32))
