@@ -8,15 +8,8 @@
 #include <unistd.h>
 
 #include <algorithm>
-#include <atomic>
 #include <cctype>
-#include <chrono>
-#include <condition_variable>
-#include <cstdlib>
-#include <deque>
-#include <functional>
 #include <mutex>
-#include <thread>
 #include <unordered_map>
 #include <unordered_set>
 #include <cstdio>
@@ -24,33 +17,11 @@
 #include <iostream>
 
 #include "../../include/modulate_b200.h"
+#include "ArkPipeline.h"
 #include "CEncryptionCycler.h"
 #include "Settings.h"
 
 namespace {
-
-double NowSeconds()
-{
-    return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count();
-}
-
-bool TraceEnabled()
-{
-    const char* lpValue = std::getenv("MOD_TRACE");
-    return lpValue && *lpValue && *lpValue != '0';
-}
-
-// Tracing aid: reports a pipeline operation that took longer than 50 ms (MOD_TRACE=1).
-struct SlowOp {
-    const char* mpWhat;
-    double mdStart;
-    explicit SlowOp(const char* lpWhat) : mpWhat(lpWhat), mdStart(TraceEnabled() ? NowSeconds() : 0.0) {}
-    ~SlowOp()
-    {
-        if (mdStart > 0.0 && NowSeconds() - mdStart > 0.05)
-            std::fprintf(stderr, "[mod] slow: %s took %.3f s\n", mpWhat, NowSeconds() - mdStart);
-    }
-};
 
 bool ReadWholeFile(const std::string& lPath, std::vector<unsigned char>& lOut)
 {
@@ -177,262 +148,6 @@ bool MakeParentDirectoriesCached(const std::string& lFilePath, std::unordered_se
     lKnown.insert(lFilePath.substr(0, liLast));
     return true;
 }
-
-// A few worker threads draining a queue of closures: the reader and writer stages of the pipelines.
-class TaskPool
-{
-public:
-    explicit TaskPool(int liThreads)
-    {
-        for (int ii = 0; ii < liThreads; ++ii)
-            maThreads.emplace_back([this]() { Loop(); });
-    }
-    ~TaskPool() { Finish(); }
-    void Push(std::function<void()> lTask)
-    {
-        {
-            std::lock_guard<std::mutex> lLock(mMutex);
-            maTasks.push_back(std::move(lTask));
-        }
-        mSignal.notify_one();
-    }
-    void Finish()  // run what is queued, then stop
-    {
-        {
-            std::lock_guard<std::mutex> lLock(mMutex);
-            mbClosed = true;
-        }
-        mSignal.notify_all();
-        for (std::thread& lThread : maThreads)
-            if (lThread.joinable())
-                lThread.join();
-    }
-
-private:
-    void Loop()
-    {
-        for (;;) {
-            std::function<void()> lTask;
-            {
-                std::unique_lock<std::mutex> lLock(mMutex);
-                mSignal.wait(lLock, [this]() { return !maTasks.empty() || mbClosed; });
-                if (maTasks.empty())
-                    return;
-                lTask = std::move(maTasks.front());
-                maTasks.pop_front();
-            }
-            lTask();
-        }
-    }
-    std::mutex mMutex;
-    std::condition_variable mSignal;
-    std::deque<std::function<void()>> maTasks;
-    std::vector<std::thread> maThreads;
-    bool mbClosed = false;
-};
-
-int HostThreads()
-{
-    const unsigned int luCores = std::thread::hardware_concurrency();
-    return luCores ? (int)luCores : 4;
-}
-
-// Tuning aid: MOD_IO_<NAME>=<n> overrides a pipeline's thread / slot count (tools/unpack_timing.py sweeps them).
-int Tunable(const char* lpName, int liDefault)
-{
-    const char* lpValue = std::getenv(lpName);
-    const int liValue = lpValue && *lpValue ? std::atoi(lpValue) : 0;
-    return liValue > 0 ? liValue : liDefault;
-}
-
-// GPUs the facade spreads an archive over: every visible device (MOD_DEVICES = bit mask restricts
-// them) once the archive is large enough to be worth it, else only the calling thread's device.
-std::vector<int> FacadeDevices(uint64_t luBytes)
-{
-    std::vector<int> laDevices;
-    const int liCurrent = std::max(0, mod_current_device());
-    const int liCount = mod_device_count();
-    const char* lpMask = std::getenv("MOD_DEVICES");
-    const uint64_t luMask = lpMask && *lpMask ? std::strtoull(lpMask, nullptr, 0) : 0;
-    const uint64_t kuMultiGpuThreshold = 256ull << 20;
-    if (liCount > 1 && luBytes >= kuMultiGpuThreshold)
-        for (int ii = 0; ii < liCount && ii < 64; ++ii)
-            if (luMask == 0 || ((luMask >> ii) & 1ull))
-                laDevices.push_back(ii);
-    if (laDevices.empty())
-        laDevices.push_back(liCurrent);
-    return laDevices;
-}
-
-// One stage buffer set of the streaming pipelines: pinned host memory either side of the GPU, the
-// two HBM windows the batched kernel works on, and the stream that orders upload -> kernel -> download.
-struct Slot {
-    enum eState { eFree, eFilling, eFilled, eDraining };
-    int miDevice = 0;
-    unsigned char* mpHostIn = nullptr;   // what the readers fill (image range / input files)
-    unsigned char* mpHostOut = nullptr;  // what the writers drain (extracted files / ciphered image range)
-    void* mpDevIn = nullptr;
-    void* mpDevOut = nullptr;
-    void* mpStream = nullptr;
-    eState meState = eFree;
-    int miFillLeft = 0;
-    int miDrainLeft = 0;
-    bool mbUsedGpu = false;
-    uint64_t muInCapacity = 0, muOutCapacity = 0;
-};
-
-// Slots handed back by a finished pipeline, kept for the next one: page-locking memory costs more than
-// moving the data does (0.3-1 ms per MiB), and a repack runs an extract and a build back to back.  At
-// most kiMaxCached slots are kept; the cache is never destroyed (the CUDA context may be gone by the
-// time static destructors run), the OS reclaims it with the process.
-struct SlotCache {
-    std::mutex mMutex;
-    std::vector<Slot> maSlots;
-    static constexpr size_t kiMaxCached = 24;
-    static SlotCache& Get()
-    {
-        static SlotCache* lpCache = new SlotCache();
-        return *lpCache;
-    }
-    bool Take(int liDevice, uint64_t luIn, uint64_t luOut, bool lbNeedGpu, Slot& lOut)
-    {
-        std::lock_guard<std::mutex> lLock(mMutex);
-        for (size_t ii = 0; ii < maSlots.size(); ++ii) {
-            Slot& lSlot = maSlots[ii];
-            if (lSlot.muInCapacity >= luIn && lSlot.muOutCapacity >= luOut && (!lbNeedGpu || (lSlot.mpStream && lSlot.miDevice == liDevice))) {
-                lOut = lSlot;
-                maSlots.erase(maSlots.begin() + (long)ii);
-                return true;
-            }
-        }
-        return false;
-    }
-    bool Give(const Slot& lSlot)
-    {
-        std::lock_guard<std::mutex> lLock(mMutex);
-        if (maSlots.size() >= kiMaxCached)
-            return false;
-        maSlots.push_back(lSlot);
-        return true;
-    }
-};
-
-struct SlotRing {
-    std::vector<Slot> maSlots;
-    std::mutex mMutex;
-    std::condition_variable mSignal;
-    std::atomic<int> miError{(int)eError_NoError};
-
-    void Fail(eError leWhat)
-    {
-        int liExpected = (int)eError_NoError;
-        miError.compare_exchange_strong(liExpected, (int)leWhat);
-        mSignal.notify_all();
-    }
-    bool Failed() const { return miError.load() != (int)eError_NoError; }
-    void Set(Slot& lSlot, Slot::eState leState)
-    {
-        {
-            std::lock_guard<std::mutex> lLock(mMutex);
-            lSlot.meState = leState;
-        }
-        mSignal.notify_all();
-    }
-    // one unit of fill / drain work done; the last one flips the slot's state
-    void FillDone(Slot& lSlot)
-    {
-        bool lbLast = false;
-        {
-            std::lock_guard<std::mutex> lLock(mMutex);
-            lbLast = --lSlot.miFillLeft == 0;
-            if (lbLast)
-                lSlot.meState = Slot::eFilled;
-        }
-        if (lbLast)
-            mSignal.notify_all();
-    }
-    void DrainDone(Slot& lSlot)
-    {
-        bool lbLast = false;
-        {
-            std::lock_guard<std::mutex> lLock(mMutex);
-            lbLast = --lSlot.miDrainLeft == 0;
-            if (lbLast)
-                lSlot.meState = Slot::eFree;
-        }
-        if (lbLast)
-            mSignal.notify_all();
-    }
-    // Allocate liPerDevice slots on each device: pinned buffers of luInBytes / luOutBytes, HBM windows
-    // of the same sizes (+ slack for the 16-byte phase), one stream each.
-    bool Allocate(const std::vector<int>& laDevices, int liPerDevice, size_t liGroups, uint64_t luInBytes, uint64_t luOutBytes,
-                  bool lbNeedGpu)
-    {
-        const size_t liWanted = std::min(liGroups, (size_t)liPerDevice * laDevices.size());
-        maSlots.resize(std::max<size_t>(1, liWanted));
-        std::vector<size_t> laFresh;  // slots the cache could not supply
-        for (size_t ii = 0; ii < maSlots.size(); ++ii) {
-            Slot& lSlot = maSlots[ii];
-            const int liDevice = laDevices[ii % laDevices.size()];
-            if (SlotCache::Get().Take(liDevice, luInBytes + 32, luOutBytes + 32, lbNeedGpu, lSlot)) {
-                lSlot.meState = Slot::eFree;
-                lSlot.mbUsedGpu = false;
-                continue;
-            }
-            lSlot.miDevice = liDevice;
-            lSlot.muInCapacity = luInBytes + 32;
-            lSlot.muOutCapacity = luOutBytes + 32;
-            laFresh.push_back(ii);
-        }
-        // Page-locking dominates a cold start (0.3-1 ms per MiB, i.e. more than the whole pipeline of a 1 GiB
-        // archive): the fresh slots are therefore set up side by side, one thread each.
-        std::atomic<bool> lbOk{true};
-        auto lSetUp = [&](size_t ii) {
-            Slot& lSlot = maSlots[ii];
-            lSlot.mpHostIn = (unsigned char*)mod_host_alloc(lSlot.muInCapacity);
-            lSlot.mpHostOut = (unsigned char*)mod_host_alloc(lSlot.muOutCapacity);
-            bool lbGood = lSlot.mpHostIn && lSlot.mpHostOut;
-            if (lbGood && lbNeedGpu) {
-                lbGood = mod_init(lSlot.miDevice) == MOD_OK;
-                if (lbGood) {
-                    lSlot.mpDevIn = mod_device_alloc(lSlot.muInCapacity);
-                    lSlot.mpDevOut = mod_device_alloc(lSlot.muOutCapacity);
-                    lSlot.mpStream = mod_stream_create();
-                    lbGood = lSlot.mpDevIn && lSlot.mpDevOut && lSlot.mpStream;
-                }
-            }
-            if (!lbGood)
-                lbOk.store(false);
-        };
-        if (laFresh.size() <= 1 || Tunable("MOD_IO_SERIAL_SETUP", 0)) {
-            for (size_t ii : laFresh)
-                lSetUp(ii);
-        } else {
-            std::vector<std::thread> laThreads;
-            for (size_t ii : laFresh)
-                laThreads.emplace_back(lSetUp, ii);
-            for (std::thread& lThread : laThreads)
-                lThread.join();
-        }
-        return lbOk.load();
-    }
-    void Release()
-    {
-        for (Slot& lSlot : maSlots) {
-            if (lSlot.mpStream)
-                mod_stream_sync(lSlot.mpStream);
-            if (lSlot.mpHostIn && lSlot.mpHostOut && SlotCache::Get().Give(lSlot))
-                continue;
-            if (lSlot.mpStream)
-                mod_stream_destroy(lSlot.mpStream);
-            mod_device_free(lSlot.mpDevIn);
-            mod_device_free(lSlot.mpDevOut);
-            mod_host_free(lSlot.mpHostIn);
-            mod_host_free(lSlot.mpHostOut);
-        }
-        maSlots.clear();
-    }
-};
 
 // pread / pwrite the whole range (short transfers are retried; a short FILE reads as zeros).
 bool ReadFully(int liFd, unsigned char* lpDst, uint64_t luSize, uint64_t luOffset)
@@ -612,26 +327,17 @@ bool CArk::ReadImageRange(std::vector<int>& laFds, uint64_t luOffset, uint64_t l
     return luSize == 0;
 }
 
-// Extraction streams the archive through a ring of slots instead of the reference's one archive-sized
-// buffer (CArk.cpp:431, :738) and its serial one-file-at-a-time writes (:435-501):
-//   * the file table becomes ONE descriptor plan (mod_plan_create: one tile map for the whole archive,
-//     on every GPU in use), the entries ordered by image offset and cut into ~32 MiB groups;
-//   * reader threads pread the image range of a group from the part files into the slot's pinned buffer;
-//   * this thread only ENQUEUES, per group and never waiting: upload of the range, the batched kernel over
-//     the group's tile sub-range (mod_plan_run_window: gather + per-entry Cycle into a byte-packed
-//     staging window), download -- on the slot's own stream, slots (and GPUs) taking groups in turn;
-//   * writer threads wait for the slot's stream, create directories and write the group's files, then
-//     hand the slot back.
-// Disk reads, PCIe both ways, the kernel and disk writes all overlap; pinned memory and HBM are
-// O(slots), not O(archive).  Entries that share an output name are resolved up front to the one whose
-// bytes the reference's in-order loop would leave on disk.
+// Extraction streams the archive through the slot-ring pipeline (ArkPipeline.h) instead of the
+// reference's one archive-sized buffer (CArk.cpp:431, :738) and its serial one-file-at-a-time writes
+// (:435-501): the entries, ordered by image offset, are packed back to back into a staging space, and
+// the batched kernel gathers and deciphers each group of them there.  Entries that share an output name
+// are resolved up front to the one whose bytes the reference's in-order loop would leave on disk.
 eError CArk::ExtractFiles(int liFirstFileIndex, int liNumFiles, const char* lpTargetDirectory)
 {
     (void)liFirstFileIndex;  // the reference ignores both and walks the whole table (CArk.cpp:435)
     (void)liNumFiles;
     if (mHeader.maFiles.empty())
         return eError_NoData;
-    const double ldStart = NowSeconds();
     const std::string lTarget = lpTargetDirectory;
 
     uint64_t luImageSize = 0;
@@ -671,73 +377,31 @@ eError CArk::ExtractFiles(int liFirstFileIndex, int liNumFiles, const char* lpTa
         }
     }
 
-    // order by where the entries sit in the image, cut entries larger than a group into PIECES (a piece that
-    // starts p bytes into its entry continues the entry's keystream from the jumped key), then form groups of
-    // consecutive pieces (~32 MiB of payload each): a slot never has to hold more than about one group
+    // order by where the entries sit in the image
     std::vector<uint32_t> laOrder = laWinners;
     std::stable_sort(laOrder.begin(), laOrder.end(), [&](uint32_t a, uint32_t b) {
         return mHeader.maFiles[a].mi64Offset < mHeader.maFiles[b].mi64Offset;
     });
-    struct Piece {
-        uint32_t file;        // index into mHeader.maFiles
-        uint64_t fileOffset;  // where in the output file the piece goes
-        uint32_t size;
-        bool whole;           // the piece is the whole file
-    };
-    struct Group {
-        size_t first, last;     // positions in laPieces
-        uint64_t srcLo, srcHi;  // image range
-        uint64_t dstLo, dstHi;  // range of the byte-packed staging space
-    };
-    const uint64_t kuGroupBytes = (uint64_t)Tunable("MOD_IO_GROUP_MIB", 32) << 20;
-    std::vector<Piece> laPieces;
+    const uint64_t kuGroupBytes = arkpipe::GroupBytes();
+    std::vector<arkpipe::Piece> laPieces;
+    std::vector<mod_desc> laDescs;
     laPieces.reserve(laOrder.size());
+    laDescs.reserve(laOrder.size());
+    uint64_t luStaged = 0;
     for (uint32_t luFile : laOrder) {
-        const uint64_t luSize = (uint64_t)mHeader.maFiles[luFile].miSize;
-        if (luSize <= kuGroupBytes + kuGroupBytes / 2) {
-            laPieces.push_back(Piece{luFile, 0, (uint32_t)luSize, true});
-            continue;
-        }
-        for (uint64_t luAt = 0; luAt < luSize;) {
-            uint64_t luTake = std::min(kuGroupBytes, luSize - luAt);
-            if (luSize - luAt - luTake < kuGroupBytes / 2)
-                luTake = luSize - luAt;  // no short tail piece
-            laPieces.push_back(Piece{luFile, luAt, (uint32_t)luTake, false});
-            luAt += luTake;
-        }
+        const modark::FileDef& lFile = mHeader.maFiles[luFile];
+        arkpipe::CutEntry(luFile, (uint64_t)lFile.miSize, (uint64_t)lFile.mi64Offset, luStaged, EntryKey(luFile), kuGroupBytes,
+                          laPieces, laDescs);
+        luStaged += (uint64_t)lFile.miSize;
     }
-    std::vector<Group> laGroups;
-    std::vector<mod_desc> laDescs(laPieces.size());
-    uint64_t luMaxRange = 1, luMaxPayload = 1, luStaged = 0;
-    for (size_t liFirst = 0; liFirst < laPieces.size();) {
-        Group lGroup{liFirst, liFirst, UINT64_MAX, 0, luStaged, luStaged};
-        while (lGroup.last < laPieces.size() && (lGroup.dstHi - lGroup.dstLo < kuGroupBytes || lGroup.last == liFirst)) {
-            const Piece& lPiece = laPieces[lGroup.last];
-            const uint64_t luSource = (uint64_t)mHeader.maFiles[lPiece.file].mi64Offset + lPiece.fileOffset;
-            if (lPiece.size) {
-                lGroup.srcLo = std::min(lGroup.srcLo, luSource);
-                lGroup.srcHi = std::max(lGroup.srcHi, luSource + lPiece.size);
-            }
-            const int liKey = EntryKey(lPiece.file);
-            laDescs[lGroup.last] = mod_desc{luSource, lGroup.dstHi, lPiece.size,
-                                            lPiece.fileOffset ? mod_key_jump(liKey, lPiece.fileOffset) : liKey};
-            lGroup.dstHi += lPiece.size;
-            ++lGroup.last;
-        }
-        if (lGroup.srcLo == UINT64_MAX)
-            lGroup.srcLo = lGroup.srcHi = 0;
-        luStaged = lGroup.dstHi;
-        luMaxRange = std::max(luMaxRange, lGroup.srcHi - lGroup.srcLo);
-        luMaxPayload = std::max(luMaxPayload, lGroup.dstHi - lGroup.dstLo);
-        laGroups.push_back(lGroup);
-        liFirst = lGroup.last;
-    }
+    const std::vector<arkpipe::Group> laGroups = arkpipe::GroupPieces(laDescs, kuGroupBytes);
+    auto lInPieces = [&](const arkpipe::Piece& lPiece) { return lPiece.size != (uint32_t)mHeader.maFiles[lPiece.file].miSize; };
 
     // files that arrive in several pieces are created (and emptied) up front, so that the pieces -- written by
     // whichever threads get them, in any order -- only ever pwrite into an existing file
     std::vector<uint8_t> laSkipFile(liCount, 0);
-    for (const Piece& lPiece : laPieces) {
-        if (lPiece.whole || lPiece.fileOffset != 0)
+    for (const arkpipe::Piece& lPiece : laPieces) {
+        if (!lInPieces(lPiece) || lPiece.fileOffset != 0)
             continue;
         const modark::FileDef& lFile = mHeader.maFiles[lPiece.file];
         const std::string lOutputPath = lTarget + lFile.mName;
@@ -760,193 +424,76 @@ eError CArk::ExtractFiles(int liFirstFileIndex, int liNumFiles, const char* lpTa
         }
     }
 
-    // slots on every GPU in use, and the archive's plan on each of them
-    const int liOriginalDevice = mod_current_device();
-    const std::vector<int> laDevices = FacadeDevices(luStaged);
-    SlotRing lRing;
-    std::vector<mod_plan*> laPlans(laDevices.size(), nullptr);
-    auto lCleanup = [&]() {
-        const double ldT0 = NowSeconds();
-        lRing.Release();
-        const double ldT1 = NowSeconds();
-        for (mod_plan* lpPlan : laPlans)
-            mod_plan_destroy(lpPlan);
-        if (liOriginalDevice >= 0)
-            mod_init(liOriginalDevice);
-        if (TraceEnabled())
-            std::fprintf(stderr, "[mod] ExtractFiles cleanup: slots %.3f s, plans %.3f s\n", ldT1 - ldT0, NowSeconds() - ldT1);
-    };
-    const double ldPlanned = NowSeconds();
-    const int liSlotsPerDevice = Tunable("MOD_IO_SLOTS", std::max(3, 6 / (int)laDevices.size()));
-    bool lbReady = lRing.Allocate(laDevices, liSlotsPerDevice, laGroups.size(), luMaxRange, luMaxPayload, true);
-    const double ldSlots = NowSeconds();
-    for (size_t dd = 0; dd < laDevices.size() && lbReady; ++dd)
-        lbReady = mod_init(laDevices[dd]) == MOD_OK &&
-                  mod_plan_create(laDescs.data(), laDescs.size(), luImageSize, luStaged, 0, &laPlans[dd]) == MOD_OK;
-    if (!lbReady) {
-        std::cout << "GPU extract could not be set up: " << mod_last_error() << "\n";
-        lCleanup();
-        return eError_NoData;
-    }
-    const double ldAllocated = NowSeconds();
-    if (TraceEnabled())
-        std::fprintf(stderr, "[mod] ExtractFiles setup: table -> groups %.3f s, slots %.3f s, plans %.3f s\n", ldPlanned - ldStart,
-                     ldSlots - ldPlanned, ldAllocated - ldSlots);
-
-    const int liCores = HostThreads();
-    TaskPool lReaders(Tunable("MOD_IO_READERS", std::max(2, std::min(8, liCores / 4))));
-    TaskPool lWriters(Tunable("MOD_IO_WRITERS", std::max(4, std::min(16, liCores / 2))));
+    // fill: the image range of a group, 8 MiB per task
     std::vector<int> laPartFds(mHeader.maParts.size(), -1);
+    const uint64_t kuReadPiece = 8ull << 20;
+    const arkpipe::Stage lRead{
+        [&](size_t gg) { return (int)std::max<uint64_t>(1, (laGroups[gg].srcHi - laGroups[gg].srcLo + kuReadPiece - 1) / kuReadPiece); },
+        [&](size_t gg, int tt, unsigned char* lpRange) {
+            arkpipe::SlowOp lTimer("ExtractFiles read of an 8 MiB image piece");
+            const arkpipe::Group& lGroup = laGroups[gg];
+            const uint64_t luLo = (uint64_t)tt * kuReadPiece, luHi = std::min(lGroup.srcHi - lGroup.srcLo, luLo + kuReadPiece);
+            if (luHi > luLo && !ReadImageRange(laPartFds, lGroup.srcLo + luLo, luHi - luLo, lpRange + luLo))
+                return eError_FailedToOpenFile;
+            return eError_NoError;
+        }};
 
-    // stage 1 (reader threads): the image range of a group, in pieces
-    auto lStartFill = [&](size_t gg) {
-        const Group& lGroup = laGroups[gg];
-        Slot& lSlot = lRing.maSlots[gg % lRing.maSlots.size()];
-        const uint64_t kuPiece = 8ull << 20;
-        const uint64_t luRange = lGroup.srcHi - lGroup.srcLo;
-        const int liPieces = (int)std::max<uint64_t>(1, (luRange + kuPiece - 1) / kuPiece);
-        {
-            std::lock_guard<std::mutex> lLock(lRing.mMutex);
-            lSlot.meState = Slot::eFilling;
-            lSlot.miFillLeft = liPieces;
-        }
-        for (int pp = 0; pp < liPieces; ++pp) {
-            lReaders.Push([&, pp, luRange, kuPiece]() {
-                SlowOp lTimer("ExtractFiles read of an 8 MiB image piece");
-                const uint64_t luLo = (uint64_t)pp * kuPiece, luHi = std::min(luRange, luLo + kuPiece);
-                // the range keeps its (offset & 15) phase inside the pinned buffer, like on the device
-                if (!lRing.Failed() && luHi > luLo &&
-                    !ReadImageRange(laPartFds, lGroup.srcLo + luLo, luHi - luLo, lSlot.mpHostIn + (lGroup.srcLo & 15u) + luLo))
-                    lRing.Fail(eError_FailedToOpenFile);
-                lRing.FillDone(lSlot);
-            });
-        }
-    };
-
-    // stage 3 (writer threads): the files of a group, a few dozen per task
-    auto lWriteFiles = [&](size_t gg, size_t liFrom, size_t liTo) {
-        const Group& lGroup = laGroups[gg];
-        Slot& lSlot = lRing.maSlots[gg % lRing.maSlots.size()];
-        thread_local std::unordered_set<std::string> lKnownDirectories;
-        SlowOp lTimer("ExtractFiles writer task (stream sync + up to 48 files)");
-        if (!lRing.Failed() && lSlot.mbUsedGpu && [&]() { SlowOp lSync("ExtractFiles stream sync"); return mod_stream_sync(lSlot.mpStream); }() != MOD_OK) {
-            std::cout << "GPU extract failed: " << mod_last_error() << "\n";
-            lRing.Fail(eError_InvalidData);
-        }
-        for (size_t ii = liFrom; ii < liTo && !lRing.Failed(); ++ii) {
-            const Piece& lPiece = laPieces[ii];
-            const modark::FileDef& lFile = mHeader.maFiles[lPiece.file];
-            const std::string lOutputPath = lTarget + lFile.mName;
-            const unsigned char* lpBytes = lSlot.mpHostOut + (lGroup.dstLo & 15u) + (laDescs[ii].dst_off - lGroup.dstLo);
-            if (!lPiece.whole) {  // one piece of a big file that was created up front
-                if (laSkipFile[lPiece.file])
+    // drain: the files of a group, 48 per task
+    const size_t kiFilesPerTask = 48;
+    const arkpipe::Stage lWrite{
+        [&](size_t gg) { return (int)((laGroups[gg].last - laGroups[gg].first + kiFilesPerTask - 1) / kiFilesPerTask); },
+        [&](size_t gg, int tt, unsigned char* lpStaged) {
+            thread_local std::unordered_set<std::string> lKnownDirectories;
+            arkpipe::SlowOp lTimer("ExtractFiles writer task (up to 48 files)");
+            const arkpipe::Group& lGroup = laGroups[gg];
+            const size_t liFrom = lGroup.first + (size_t)tt * kiFilesPerTask, liTo = std::min(lGroup.last, liFrom + kiFilesPerTask);
+            for (size_t ii = liFrom; ii < liTo; ++ii) {
+                const arkpipe::Piece& lPiece = laPieces[ii];
+                const modark::FileDef& lFile = mHeader.maFiles[lPiece.file];
+                const std::string lOutputPath = lTarget + lFile.mName;
+                const unsigned char* lpBytes = lpStaged + (laDescs[ii].dst_off - lGroup.dstLo);
+                if (lInPieces(lPiece)) {  // one piece of a big file that was created up front
+                    if (laSkipFile[lPiece.file])
+                        continue;
+                    const int liFd = open(lOutputPath.c_str(), O_WRONLY);
+                    const bool lbOk = liFd >= 0 && WriteFully(liFd, lpBytes, lPiece.size, lPiece.fileOffset);
+                    if (liFd >= 0)
+                        close(liFd);
+                    if (!lbOk)
+                        return eError_FailedToWriteData;
                     continue;
-                const int liFd = open(lOutputPath.c_str(), O_WRONLY);
-                const bool lbOk = liFd >= 0 && WriteFully(liFd, lpBytes, lPiece.size, lPiece.fileOffset);
-                if (liFd >= 0)
-                    close(liFd);
-                if (!lbOk)
-                    lRing.Fail(eError_FailedToWriteData);
-                continue;
-            }
-            if (EscapesTarget(lFile.mName)) {
-                std::cout << "Refusing to write outside the target directory: " << lFile.mName.c_str() << "\n";
-                continue;
-            }
-            if (KeepExistingOutput(lOutputPath)) {
-                VERBOSE_OUT("Output file already exists, skipping: " << lOutputPath.c_str() << "\n");
-                continue;
-            }
-            if (!MakeParentDirectoriesCached(lOutputPath, lKnownDirectories)) {
-                lRing.Fail(eError_FailedToCreateDirectory);
-                break;
-            }
-            const int liFd = open(lOutputPath.c_str(), O_WRONLY | O_CREAT | O_TRUNC, 0666);
-            if (liFd < 0) {
-                std::cout << "Failed to create " << lOutputPath.c_str() << "\n";  // the reference carries on too (CArk.cpp:488-491)
-                continue;
-            }
-            const bool lbOk = lFile.miSize == 0 || WriteFully(liFd, lpBytes, (uint64_t)lFile.miSize, 0);
-            close(liFd);
-            if (!lbOk)
-                lRing.Fail(eError_FailedToWriteData);
-        }
-        lRing.DrainDone(lSlot);
-    };
-
-    // stage 2 (this thread): enqueue upload -> kernel -> download per group, never waiting for the GPU
-    size_t liNextFill = 0, liNextGpu = 0;
-    while (liNextGpu < laGroups.size() && !lRing.Failed()) {
-        {
-            std::unique_lock<std::mutex> lLock(lRing.mMutex);
-            lRing.mSignal.wait(lLock, [&]() {
-                const bool lbCanFill = liNextFill < laGroups.size() && liNextFill < liNextGpu + lRing.maSlots.size() &&
-                                       lRing.maSlots[liNextFill % lRing.maSlots.size()].meState == Slot::eFree;
-                const bool lbCanRun = lRing.maSlots[liNextGpu % lRing.maSlots.size()].meState == Slot::eFilled && liNextGpu < liNextFill;
-                return lbCanFill || lbCanRun || lRing.Failed();
-            });
-        }
-        if (lRing.Failed())
-            break;
-        while (liNextFill < laGroups.size() && liNextFill < liNextGpu + lRing.maSlots.size() &&
-               lRing.maSlots[liNextFill % lRing.maSlots.size()].meState == Slot::eFree)
-            lStartFill(liNextFill++);
-        while (liNextGpu < liNextFill && lRing.maSlots[liNextGpu % lRing.maSlots.size()].meState == Slot::eFilled) {
-            const size_t gg = liNextGpu++;
-            const Group& lGroup = laGroups[gg];
-            Slot& lSlot = lRing.maSlots[gg % lRing.maSlots.size()];
-            const uint64_t luRange = lGroup.srcHi - lGroup.srcLo, luPayload = lGroup.dstHi - lGroup.dstLo;
-            lSlot.mbUsedGpu = luPayload != 0;
-            if (luPayload) {
-                size_t liDeviceIndex = 0;
-                while (laDevices[liDeviceIndex] != lSlot.miDevice)
-                    ++liDeviceIndex;
-                uint64_t luTile0 = 0, luTile1 = 0;
-                SlowOp lTimer("ExtractFiles GPU enqueue of a group");
-                unsigned char* lpDevIn = (unsigned char*)lSlot.mpDevIn + (lGroup.srcLo & 15u);
-                unsigned char* lpDevOut = (unsigned char*)lSlot.mpDevOut + (lGroup.dstLo & 15u);
-                const bool lbOk =
-                    mod_init(lSlot.miDevice) == MOD_OK &&
-                    mod_plan_tile_range(laPlans[liDeviceIndex], lGroup.first, lGroup.last, &luTile0, &luTile1) == MOD_OK &&
-                    mod_memcpy_h2d(lpDevIn, lSlot.mpHostIn + (lGroup.srcLo & 15u), luRange, lSlot.mpStream) == MOD_OK &&
-                    mod_plan_run_window(laPlans[liDeviceIndex], luTile0, luTile1, lpDevIn, lGroup.srcLo, luRange, lpDevOut,
-                                        lGroup.dstLo, luPayload, lSlot.mpStream) == MOD_OK &&
-                    mod_memcpy_d2h(lSlot.mpHostOut + (lGroup.dstLo & 15u), lpDevOut, luPayload, lSlot.mpStream) == MOD_OK;
-                if (!lbOk) {
-                    std::cout << "GPU extract failed: " << mod_last_error() << "\n";
-                    lRing.Fail(eError_InvalidData);
-                    break;
                 }
+                if (EscapesTarget(lFile.mName)) {
+                    std::cout << "Refusing to write outside the target directory: " << lFile.mName.c_str() << "\n";
+                    continue;
+                }
+                if (KeepExistingOutput(lOutputPath)) {
+                    VERBOSE_OUT("Output file already exists, skipping: " << lOutputPath.c_str() << "\n");
+                    continue;
+                }
+                if (!MakeParentDirectoriesCached(lOutputPath, lKnownDirectories))
+                    return eError_FailedToCreateDirectory;
+                const int liFd = open(lOutputPath.c_str(), O_WRONLY | O_CREAT | O_TRUNC, 0666);
+                if (liFd < 0) {
+                    std::cout << "Failed to create " << lOutputPath.c_str() << "\n";  // the reference carries on too (CArk.cpp:488-491)
+                    continue;
+                }
+                const bool lbOk = lFile.miSize == 0 || WriteFully(liFd, lpBytes, (uint64_t)lFile.miSize, 0);
+                close(liFd);
+                if (!lbOk)
+                    return eError_FailedToWriteData;
             }
-            const size_t kiFilesPerTask = 48;
-            const size_t liFiles = lGroup.last - lGroup.first;
-            const int liTasks = (int)std::max<size_t>(1, (liFiles + kiFilesPerTask - 1) / kiFilesPerTask);
-            {
-                std::lock_guard<std::mutex> lLock(lRing.mMutex);
-                lSlot.meState = Slot::eDraining;
-                lSlot.miDrainLeft = liTasks;
-            }
-            for (int tt = 0; tt < liTasks; ++tt) {
-                const size_t liFrom = lGroup.first + (size_t)tt * kiFilesPerTask;
-                lWriters.Push([&, gg, liFrom, liTo = std::min(lGroup.last, liFrom + kiFilesPerTask)]() { lWriteFiles(gg, liFrom, liTo); });
-            }
-        }
-    }
-    const double ldEnqueued = NowSeconds();
-    lReaders.Finish();
-    lWriters.Finish();
-    const double ldWritten = NowSeconds();
+            return eError_NoError;
+        }};
+
+    const int liCores = arkpipe::HostThreads();
+    eError leError = arkpipe::RunPipeline("extract", laDescs, laGroups, luImageSize, luStaged, true, std::max(2, std::min(8, liCores / 4)),
+                                          std::max(4, std::min(16, liCores / 2)), lRead, lWrite);
     for (int liFd : laPartFds)
         if (liFd >= 0)
             close(liFd);
-    const size_t liSlotsUsed = lRing.maSlots.size();
-    lCleanup();
-    if (TraceEnabled())
-        std::fprintf(stderr, "[mod] ExtractFiles: %zu groups on %zu GPU(s), %zu slots; setup %.3f s, pipeline %.3f s, drain %.3f s, free %.3f s\n",
-                     laGroups.size(), laDevices.size(), liSlotsUsed,
-                     ldAllocated - ldStart, ldEnqueued - ldAllocated, ldWritten - ldEnqueued, NowSeconds() - ldWritten);
-
-    eError leError = (eError)lRing.miError.load();
+    if (leError == eError_NoData)  // the GPU could not be set up; RunPipeline has said why
+        return leError;
     SHOW_ERROR_AND_RETURN;
     return eError_NoError;
 }
@@ -1089,24 +636,16 @@ eError CArk::BuildArk(const char* lpInputDirectory, std::vector<SSongConfig> laS
     return eError_NoError;
 }
 
-// Stream the image BuildArk laid out into the part files: reader threads load the input files of a
-// ~32 MiB group into a pinned slot, entries that carry a key are ciphered on the GPU (upload, one
-// mod_plan_run_window over the group's tiles of the archive-wide plan, download -- enqueued on the
-// slot's stream, never waited for here), writer threads pwrite the group's byte range into the part
-// file(s) it falls in.  With all keys 0 (the reference never ciphers ARK bodies) the GPU is not
-// involved and the bytes go from the read buffer straight to the part files.
+// Stream the image BuildArk laid out into the part files through the slot-ring pipeline (ArkPipeline.h):
+// reader threads load the input files of a ~32 MiB group, entries that carry a key are ciphered on the
+// GPU, writer threads pwrite the group's byte range into the part file(s) it falls in.  With all keys 0
+// (the reference never ciphers ARK bodies) the GPU is not involved and the bytes go from the read buffer
+// straight to the part files.
 eError CArk::StreamBuiltImage(const std::vector<PartTarget>& laTargets) const
 {
-    const double ldStart = NowSeconds();
-    // non-empty entries in table order == image order; files larger than a group are read (and ciphered) in
-    // PIECES, each continuing the entry's keystream from the jumped key, so a slot stays about one group big
-    struct Piece {
-        uint32_t file;        // index into mHeader.maFiles
-        uint64_t fileOffset;  // where in the input file the piece starts
-        uint32_t size;
-    };
-    const uint64_t kuGroupBytes = (uint64_t)Tunable("MOD_IO_GROUP_MIB", 32) << 20;
-    std::vector<Piece> laPieces;
+    // non-empty entries in table order == image order, which is also where they go: destination == source
+    const uint64_t kuGroupBytes = arkpipe::GroupBytes();
+    std::vector<arkpipe::Piece> laPieces;
     std::vector<mod_desc> laDescs;
     bool lbAnyKey = false;
     for (size_t ii = 0; ii < mHeader.maFiles.size(); ++ii) {
@@ -1115,202 +654,73 @@ eError CArk::StreamBuiltImage(const std::vector<PartTarget>& laTargets) const
             continue;
         const int liKey = EntryKey(ii);
         lbAnyKey = lbAnyKey || (liKey % 0x7FFFFFFF) != 0;
-        const uint64_t luSize = (uint64_t)lFile.miSize;
-        for (uint64_t luAt = 0; luAt < luSize;) {
-            uint64_t luTake = luSize <= kuGroupBytes + kuGroupBytes / 2 ? luSize : std::min(kuGroupBytes, luSize - luAt);
-            if (luSize - luAt - luTake < kuGroupBytes / 2)
-                luTake = luSize - luAt;  // no short tail piece
-            const uint64_t luImage = (uint64_t)lFile.mi64Offset + luAt;
-            laPieces.push_back(Piece{(uint32_t)ii, luAt, (uint32_t)luTake});
-            laDescs.push_back(mod_desc{luImage, luImage, (uint32_t)luTake, luAt ? mod_key_jump(liKey, luAt) : liKey});
-            luAt += luTake;
-        }
+        arkpipe::CutEntry((uint32_t)ii, (uint64_t)lFile.miSize, (uint64_t)lFile.mi64Offset, (uint64_t)lFile.mi64Offset, liKey,
+                          kuGroupBytes, laPieces, laDescs);
     }
     if (laPieces.empty())
         return eError_NoError;
+    const std::vector<arkpipe::Group> laGroups = arkpipe::GroupPieces(laDescs, kuGroupBytes);
 
-    struct Group {
-        size_t first, last;  // positions in laPieces
-        uint64_t lo, hi;     // image range
+    // each group's range, cut into 4 MiB writes (several writer threads share a group) per part file that
+    // receives it; none when every part the group falls in was skipped (existing output kept)
+    struct Range {
+        size_t target;
+        uint64_t lo, hi;
     };
-    std::vector<Group> laGroups;
-    uint64_t luMaxRange = 1;
-    for (size_t liFirst = 0; liFirst < laPieces.size();) {
-        Group lGroup{liFirst, liFirst, laDescs[liFirst].src_off, laDescs[liFirst].src_off};
-        while (lGroup.last < laPieces.size() && (lGroup.hi - lGroup.lo < kuGroupBytes || lGroup.last == liFirst)) {
-            lGroup.hi = laDescs[lGroup.last].src_off + laDescs[lGroup.last].len;
-            ++lGroup.last;
-        }
-        luMaxRange = std::max(luMaxRange, lGroup.hi - lGroup.lo);
-        laGroups.push_back(lGroup);
-        liFirst = lGroup.last;
-    }
-
-    const int liOriginalDevice = lbAnyKey ? mod_current_device() : -1;
-    const std::vector<int> laDevices = lbAnyKey ? FacadeDevices(muBuiltImageSize) : std::vector<int>{0};
-    SlotRing lRing;
-    std::vector<mod_plan*> laPlans(laDevices.size(), nullptr);
-    auto lCleanup = [&]() {
-        lRing.Release();
-        for (mod_plan* lpPlan : laPlans)
-            mod_plan_destroy(lpPlan);
-        if (liOriginalDevice >= 0)
-            mod_init(liOriginalDevice);
-    };
-    const int liSlotsPerDevice = Tunable("MOD_IO_SLOTS", std::max(3, 6 / (int)laDevices.size()));
-    bool lbReady = lRing.Allocate(laDevices, liSlotsPerDevice, laGroups.size(), luMaxRange, lbAnyKey ? luMaxRange : 0, lbAnyKey);
-    for (size_t dd = 0; dd < laDevices.size() && lbReady && lbAnyKey; ++dd)
-        lbReady = mod_init(laDevices[dd]) == MOD_OK &&
-                  mod_plan_create(laDescs.data(), laDescs.size(), muBuiltImageSize, muBuiltImageSize, 0, &laPlans[dd]) == MOD_OK;
-    if (!lbReady) {
-        std::cout << "GPU build could not be set up: " << mod_last_error() << "\n";
-        lCleanup();
-        return eError_NoData;
-    }
-
-    const double ldReady = NowSeconds();
-    const int liCores = HostThreads();
-    TaskPool lReaders(Tunable("MOD_IO_READERS", std::max(2, std::min(12, liCores / 2))));
-    TaskPool lWriters(Tunable("MOD_IO_WRITERS", std::max(2, std::min(12, liCores / 2))));
-
-    // stage 1 (reader threads): the input files of a group, a few dozen per task (the reference's one
-    // fread per file, CArk.cpp:796-811 -- thousands of small files are latency-bound on any file system)
-    auto lReadFiles = [&](size_t gg, size_t liFrom, size_t liTo) {
-        const Group& lGroup = laGroups[gg];
-        Slot& lSlot = lRing.maSlots[gg % lRing.maSlots.size()];
-        SlowOp lTimer("SaveArk reader task (up to 48 input files)");
-        for (size_t ii = liFrom; ii < liTo && !lRing.Failed(); ++ii) {
-            const Piece& lPiece = laPieces[ii];
-            const modark::FileDef& lFile = mHeader.maFiles[lPiece.file];
-            const int liFd = open((mBuildInputDirectory + lFile.mName).c_str(), O_RDONLY);
-            if (liFd < 0) {
-                lRing.Fail(eError_FailedToOpenFile);
-                break;
-            }
-            unsigned char* lpDst = lSlot.mpHostIn + (lGroup.lo & 15u) + (laDescs[ii].src_off - lGroup.lo);
-            const bool lbOk = ReadFully(liFd, lpDst, lPiece.size, lPiece.fileOffset);  // a file that shrank reads as zeros
-            close(liFd);
-            if (!lbOk)
-                lRing.Fail(eError_FailedToOpenFile);
-        }
-        lRing.FillDone(lSlot);
-    };
-    auto lStartFill = [&](size_t gg) {
-        const Group& lGroup = laGroups[gg];
-        Slot& lSlot = lRing.maSlots[gg % lRing.maSlots.size()];
-        const size_t kiFilesPerTask = 48;
-        const int liTasks = (int)((lGroup.last - lGroup.first + kiFilesPerTask - 1) / kiFilesPerTask);
-        {
-            std::lock_guard<std::mutex> lLock(lRing.mMutex);
-            lSlot.meState = Slot::eFilling;
-            lSlot.miFillLeft = liTasks;
-        }
-        for (int tt = 0; tt < liTasks; ++tt) {
-            const size_t liFrom = lGroup.first + (size_t)tt * kiFilesPerTask;
-            lReaders.Push([&, gg, liFrom, liTo = std::min(lGroup.last, liFrom + kiFilesPerTask)]() { lReadFiles(gg, liFrom, liTo); });
-        }
-    };
-
-    // stage 3 (writer threads): the group's byte range, cut where it crosses into another part file
-    auto lWriteRange = [&](size_t gg, size_t liTarget, uint64_t luLo, uint64_t luHi) {
-        const Group& lGroup = laGroups[gg];
-        Slot& lSlot = lRing.maSlots[gg % lRing.maSlots.size()];
-        SlowOp lTimer("SaveArk writer task (stream sync + a 4 MiB range)");
-        if (!lRing.Failed() && lSlot.mbUsedGpu && [&]() { SlowOp lSync("SaveArk stream sync"); return mod_stream_sync(lSlot.mpStream); }() != MOD_OK) {
-            std::cout << "GPU build failed: " << mod_last_error() << "\n";
-            lRing.Fail(eError_InvalidData);
-        }
-        const unsigned char* lpBytes = (lSlot.mbUsedGpu ? lSlot.mpHostOut : lSlot.mpHostIn) + (lGroup.lo & 15u) + (luLo - lGroup.lo);
-        const PartTarget& lPart = laTargets[liTarget];
-        if (!lRing.Failed()) {
-            if (lPart.mpMap)  // pages of a mapped file are faulted in and filled by many threads at once
-                std::memcpy(lPart.mpMap + (luLo - lPart.muImageStart), lpBytes, (size_t)(luHi - luLo));
-            else if (!WriteFully(lPart.miFd, lpBytes, luHi - luLo, luLo - lPart.muImageStart))
-                lRing.Fail(eError_FailedToWriteData);
-        }
-        lRing.DrainDone(lSlot);
-    };
-
-    // stage 2 (this thread)
-    size_t liNextFill = 0, liNextGpu = 0;
-    while (liNextGpu < laGroups.size() && !lRing.Failed()) {
-        {
-            std::unique_lock<std::mutex> lLock(lRing.mMutex);
-            lRing.mSignal.wait(lLock, [&]() {
-                const bool lbCanFill = liNextFill < laGroups.size() && liNextFill < liNextGpu + lRing.maSlots.size() &&
-                                       lRing.maSlots[liNextFill % lRing.maSlots.size()].meState == Slot::eFree;
-                const bool lbCanRun = liNextGpu < liNextFill && lRing.maSlots[liNextGpu % lRing.maSlots.size()].meState == Slot::eFilled;
-                return lbCanFill || lbCanRun || lRing.Failed();
-            });
-        }
-        if (lRing.Failed())
-            break;
-        while (liNextFill < laGroups.size() && liNextFill < liNextGpu + lRing.maSlots.size() &&
-               lRing.maSlots[liNextFill % lRing.maSlots.size()].meState == Slot::eFree)
-            lStartFill(liNextFill++);
-        while (liNextGpu < liNextFill && lRing.maSlots[liNextGpu % lRing.maSlots.size()].meState == Slot::eFilled) {
-            const size_t gg = liNextGpu++;
-            const Group& lGroup = laGroups[gg];
-            Slot& lSlot = lRing.maSlots[gg % lRing.maSlots.size()];
-            const uint64_t luRange = lGroup.hi - lGroup.lo;
-            lSlot.mbUsedGpu = lbAnyKey;
-            if (lbAnyKey) {
-                size_t liDeviceIndex = 0;
-                while (laDevices[liDeviceIndex] != lSlot.miDevice)
-                    ++liDeviceIndex;
-                uint64_t luTile0 = 0, luTile1 = 0;
-                SlowOp lTimer("SaveArk GPU enqueue of a group");
-                unsigned char* lpDevIn = (unsigned char*)lSlot.mpDevIn + (lGroup.lo & 15u);
-                unsigned char* lpDevOut = (unsigned char*)lSlot.mpDevOut + (lGroup.lo & 15u);
-                const bool lbOk =
-                    mod_init(lSlot.miDevice) == MOD_OK &&
-                    mod_plan_tile_range(laPlans[liDeviceIndex], lGroup.first, lGroup.last, &luTile0, &luTile1) == MOD_OK &&
-                    mod_memcpy_h2d(lpDevIn, lSlot.mpHostIn + (lGroup.lo & 15u), luRange, lSlot.mpStream) == MOD_OK &&
-                    mod_plan_run_window(laPlans[liDeviceIndex], luTile0, luTile1, lpDevIn, lGroup.lo, luRange, lpDevOut, lGroup.lo,
-                                        luRange, lSlot.mpStream) == MOD_OK &&
-                    mod_memcpy_d2h(lSlot.mpHostOut + (lGroup.lo & 15u), lpDevOut, luRange, lSlot.mpStream) == MOD_OK;
-                if (!lbOk) {
-                    std::cout << "GPU build failed: " << mod_last_error() << "\n";
-                    lRing.Fail(eError_InvalidData);
-                    break;
-                }
-            }
-            // pieces of [lo, hi) per part file that receives them
-            struct Piece {
-                size_t target;
-                uint64_t lo, hi;
-            };
-            std::vector<Piece> laPieces;
-            const uint64_t kuWritePiece = 4ull << 20;  // several writer threads share a group
-            for (size_t tt = 0; tt < laTargets.size(); ++tt) {
-                const uint64_t luLo = std::max(lGroup.lo, laTargets[tt].muImageStart);
-                const uint64_t luHi = std::min(lGroup.hi, laTargets[tt].muImageStart + laTargets[tt].muSize);
-                if (laTargets[tt].miFd < 0)
-                    continue;
-                for (uint64_t luAt = luLo; luAt < luHi; luAt += kuWritePiece)
-                    laPieces.push_back(Piece{tt, luAt, std::min(luHi, luAt + kuWritePiece)});
-            }
-            if (laPieces.empty()) {  // every part this group falls in was skipped (existing output kept)
-                lRing.Set(lSlot, Slot::eFree);
+    std::vector<std::vector<Range>> laRanges(laGroups.size());
+    const uint64_t kuWritePiece = 4ull << 20;
+    for (size_t gg = 0; gg < laGroups.size(); ++gg)
+        for (size_t tt = 0; tt < laTargets.size(); ++tt) {
+            const uint64_t luLo = std::max(laGroups[gg].dstLo, laTargets[tt].muImageStart);
+            const uint64_t luHi = std::min(laGroups[gg].dstHi, laTargets[tt].muImageStart + laTargets[tt].muSize);
+            if (laTargets[tt].miFd < 0)
                 continue;
-            }
-            {
-                std::lock_guard<std::mutex> lLock(lRing.mMutex);
-                lSlot.meState = Slot::eDraining;
-                lSlot.miDrainLeft = (int)laPieces.size();
-            }
-            for (const Piece& lPiece : laPieces)
-                lWriters.Push([&, gg, lPiece]() { lWriteRange(gg, lPiece.target, lPiece.lo, lPiece.hi); });
+            for (uint64_t luAt = luLo; luAt < luHi; luAt += kuWritePiece)
+                laRanges[gg].push_back(Range{tt, luAt, std::min(luHi, luAt + kuWritePiece)});
         }
-    }
-    lReaders.Finish();
-    lWriters.Finish();
-    const double ldDone = NowSeconds();
-    lCleanup();
-    if (TraceEnabled())
-        std::fprintf(stderr, "[mod] SaveArk: streamed %zu groups (%s): setup %.3f s, pipeline %.3f s, free %.3f s\n", laGroups.size(),
-                     lbAnyKey ? "ciphered on the GPU" : "plain copy, no GPU", ldReady - ldStart, ldDone - ldReady, NowSeconds() - ldDone);
-    return (eError)lRing.miError.load();
+
+    // fill: the input files of a group, 48 per task (the reference's one fread per file, CArk.cpp:796-811 --
+    // thousands of small files are latency-bound on any file system)
+    const size_t kiFilesPerTask = 48;
+    const arkpipe::Stage lRead{
+        [&](size_t gg) { return (int)((laGroups[gg].last - laGroups[gg].first + kiFilesPerTask - 1) / kiFilesPerTask); },
+        [&](size_t gg, int tt, unsigned char* lpRange) {
+            arkpipe::SlowOp lTimer("SaveArk reader task (up to 48 input files)");
+            const arkpipe::Group& lGroup = laGroups[gg];
+            const size_t liFrom = lGroup.first + (size_t)tt * kiFilesPerTask, liTo = std::min(lGroup.last, liFrom + kiFilesPerTask);
+            for (size_t ii = liFrom; ii < liTo; ++ii) {
+                const arkpipe::Piece& lPiece = laPieces[ii];
+                const int liFd = open((mBuildInputDirectory + mHeader.maFiles[lPiece.file].mName).c_str(), O_RDONLY);
+                if (liFd < 0)
+                    return eError_FailedToOpenFile;
+                unsigned char* lpDst = lpRange + (laDescs[ii].src_off - lGroup.srcLo);
+                const bool lbOk = ReadFully(liFd, lpDst, lPiece.size, lPiece.fileOffset);  // a file that shrank reads as zeros
+                close(liFd);
+                if (!lbOk)
+                    return eError_FailedToOpenFile;
+            }
+            return eError_NoError;
+        }};
+
+    // drain: one 4 MiB range into its part file
+    const arkpipe::Stage lWrite{
+        [&](size_t gg) { return (int)laRanges[gg].size(); },
+        [&](size_t gg, int tt, unsigned char* lpImage) {
+            arkpipe::SlowOp lTimer("SaveArk writer task (a 4 MiB range)");
+            const Range& lRange = laRanges[gg][tt];
+            const PartTarget& lPart = laTargets[lRange.target];
+            const unsigned char* lpBytes = lpImage + (lRange.lo - laGroups[gg].dstLo);
+            if (lPart.mpMap) {  // pages of a mapped file are faulted in and filled by many threads at once
+                std::memcpy(lPart.mpMap + (lRange.lo - lPart.muImageStart), lpBytes, (size_t)(lRange.hi - lRange.lo));
+                return eError_NoError;
+            }
+            return WriteFully(lPart.miFd, lpBytes, lRange.hi - lRange.lo, lRange.lo - lPart.muImageStart) ? eError_NoError
+                                                                                                      : eError_FailedToWriteData;
+        }};
+
+    const int liThreads = std::max(2, std::min(12, arkpipe::HostThreads() / 2));
+    return arkpipe::RunPipeline("build", laDescs, laGroups, muBuiltImageSize, muBuiltImageSize, lbAnyKey, liThreads, liThreads, lRead,
+                                lWrite);
 }
 
 eError CArk::SaveArk(const char* lpOutputDirectory, const char* lpHeaderFilename) const

@@ -7,12 +7,13 @@
 //   LoadArkData           concatenates the .ark parts into one PINNED host image (CArk.cpp:723-758)
 //   ExtractFiles          turns the file table into ONE descriptor plan (mod_plan_create) and gathers
 //                         the entries through the batched kernel group by group (mod_plan_run_window;
-//                         CArk.cpp:494) in a reader -> GPU -> writer pipeline over a ring of slots on
-//                         every visible GPU: nothing is ever waited for on the thread that enqueues
+//                         CArk.cpp:494) in the reader -> GPU -> writer slot-ring pipeline of
+//                         ArkPipeline.h, over every visible GPU: nothing is ever waited for on the
+//                         thread that enqueues
 //   BuildArk              assigns byte-packed offsets and part sizes from the file sizes (CArk.cpp:760-828)
 //   SaveArk               serialises + enciphers the header (CArk.cpp:1135-1136) and STREAMS the payload
-//                         from the input files into the part files through the same kind of slot ring
-//                         (entries that carry a key are ciphered on the GPU on the way)
+//                         from the input files into the part files through the same pipeline (entries
+//                         that carry a key are ciphered on the GPU on the way)
 //
 // The reference never ciphers ARK bodies (SURVEY.md Finding 2): all entry keys default to 0, the
 // identity keystream, so the bytes produced are the reference's.  SetEntryKeys / SetUniformEntryKey

@@ -7,6 +7,11 @@
 // descriptor list plus the same first-tile prefix the real library computes (8 KiB tiles of one
 // entry each), so mod_plan_tile_range / mod_plan_run_window can be answered for whole-entry ranges --
 // the only kind the facade issues.
+//
+// MOD_MOCK_DEVICES=<n> (default 1) makes it report n devices.  Like the CUDA runtime, each thread is
+// bound to a device (mod_init, 0 until then); plans and streams remember the device they were created
+// on, and mod_plan_run_window refuses to run unless the caller, the plan and the stream agree (the real
+// library's plan_check_device; a stream of another device is a CUDA error there).
 #include <cstdlib>
 #include <cstring>
 #include <vector>
@@ -28,7 +33,21 @@ struct mod_plan {
     std::vector<mod_desc> descs;
     std::vector<uint64_t> first_tile;  // n + 1
     uint32_t dst_align = 0;
+    int device = 0;
 };
+
+struct mock_stream {
+    int device;
+};
+
+static thread_local int tl_device = 0;
+
+static int mock_device_count()
+{
+    const char* v = std::getenv("MOD_MOCK_DEVICES");
+    const int n = v && *v ? std::atoi(v) : 1;
+    return n > 0 ? n : 1;
+}
 
 static uint64_t tiles_for_entry(uint32_t h0, uint32_t len)
 {
@@ -41,9 +60,15 @@ static uint64_t tiles_for_entry(uint32_t h0, uint32_t len)
 extern "C" {
 
 int mod_abi_version(void) { return MOD_ABI_VERSION; }
-int mod_device_count(void) { return 1; }
-int mod_init(int) { return MOD_OK; }
-int mod_current_device(void) { return 0; }
+int mod_device_count(void) { return mock_device_count(); }
+int mod_init(int device)
+{
+    if (device < 0 || device >= mock_device_count())
+        return MOD_ERR_ARG;
+    tl_device = device;
+    return MOD_OK;
+}
+int mod_current_device(void) { return tl_device; }
 int mod_is_device_pointer(const void*) { return 0; }
 void mod_shutdown(void) {}
 const char* mod_last_error(void) { return "mock ABI (oracle-backed, tests only)"; }
@@ -71,10 +96,10 @@ int mod_memcpy_d2h(void* h, const void* d, uint64_t bytes, void*)
     return MOD_OK;
 }
 int mod_stream_sync(void*) { return MOD_OK; }
-void* mod_stream_create(void) { return std::malloc(1); }
+void* mod_stream_create(void) { return new mock_stream{tl_device}; }
 int mod_stream_destroy(void* s)
 {
-    std::free(s);
+    delete (mock_stream*)s;
     return MOD_OK;
 }
 int mod_cycle(void* data, uint64_t len, int32_t key)
@@ -102,6 +127,7 @@ int mod_plan_create(const mod_desc* descs, uint64_t n, uint64_t src_bytes, uint6
     mod_plan* p = new mod_plan();
     p->descs.assign(descs, descs + n);
     p->dst_align = dst_align;
+    p->device = tl_device;
     p->first_tile.resize(n + 1);
     uint64_t tiles = 0;
     for (uint64_t i = 0; i < n; ++i) {
@@ -126,8 +152,10 @@ int mod_plan_tile_range(const mod_plan* plan, uint64_t e0, uint64_t e1, uint64_t
     return MOD_OK;
 }
 int mod_plan_run_window(const mod_plan* plan, uint64_t t0, uint64_t t1, const void* src_win, uint64_t src_win_off,
-                        uint64_t src_win_bytes, void* dst_win, uint64_t dst_win_off, uint64_t dst_win_bytes, void*)
+                        uint64_t src_win_bytes, void* dst_win, uint64_t dst_win_off, uint64_t dst_win_bytes, void* stream)
 {
+    if (plan->device != tl_device || (stream && ((const mock_stream*)stream)->device != tl_device))
+        return MOD_ERR_ARG;
     if ((((uintptr_t)dst_win - dst_win_off) & 15u) != plan->dst_align)
         return MOD_ERR_ALIGN;
     for (size_t e = 0; e < plan->descs.size(); ++e) {

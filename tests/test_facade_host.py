@@ -210,6 +210,30 @@ def test_large_entries_travel_in_pieces(cli, tmp_path, monkeypatch):
         assert oracle.cycle(image[e.offset:e.offset + e.size], key).tobytes() == by_name[e.name], e.name
 
 
+def test_pipelines_deal_groups_to_two_devices(cli, tmp_path):
+    """An archive above the facade's 256 MiB multi-GPU threshold is spread over every device, in both
+    directions: each slot's group must run on the slot's device with that device's plan and stream (the
+    mock, like the real library, refuses a plan or stream of another device)."""
+    key = 0x1357BDF
+    sizes = [900_000] * 300
+    sizes[7] = sizes[150] = 0
+    sizes[100] = 60 << 20  # cut into pieces
+    hdr, payloads, _ = arkfixture.write_archive(str(tmp_path), n_files=len(sizes), n_parts=3, seed=31, body_key=key, sizes=sizes)
+    assert sum(sizes) > 256 << 20
+    env = dict(os.environ, MOD_MOCK_DEVICES="2", MOD_TRACE="1")
+
+    def run_env(cwd, *args):
+        out = subprocess.run([cli, "-bodykey", str(key), *args], cwd=cwd, capture_output=True, text=True, timeout=300, env=env)
+        assert out.returncode == 0, out.stdout + out.stderr
+        return out.stderr
+
+    assert "on 2 GPU(s)" in run_env(tmp_path, "-unpack", "out")
+    check_unpacked(tmp_path / "out", hdr, payloads)
+    assert "on 2 GPU(s)" in run_env(tmp_path, "-packall", "-pack_add", "out", "re")
+    assert "on 2 GPU(s)" in run_env(tmp_path / "re", "-unpack", "again")
+    check_unpacked(tmp_path / "re" / "again", hdr, payloads)
+
+
 def test_pack_fails_loudly_on_an_unreadable_file(cli, tmp_path):
     """BuildArk gives up on the first input it cannot open (reference CArk.cpp:799-804)."""
     if os.geteuid() == 0:
