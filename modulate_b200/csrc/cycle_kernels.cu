@@ -175,7 +175,7 @@ __device__ __forceinline__ uint32_t low8_canonical_fma(uint32_t s, uint32_t two)
 // before the chunk's first byte -- exact for every state.  Per byte: IMAD.WIDE + LEA.HI (step) and
 // a canonical low byte (LEA.HI on the ALU pipe or IMAD.HI on the FMA pipe, per MODK_CANON_FMA_MASK);
 // per word: three PRMTs pack four keystream bytes and one LOP3 applies them.  Out of line: used for
-// the ~1 chunk in 8 000 the speculative hot loop hands over, and by the byte-granular slow path.
+// the ~1 chunk in 14 000 the speculative hot loop hands over, and by the byte-granular slow path.
 __device__ __noinline__ uint4 cycle_chunk_exact(uint4 d, uint32_t s, const uint32_t two)
 {
     uint32_t w[4] = {d.x, d.y, d.z, d.w};
@@ -358,7 +358,7 @@ __device__ __forceinline__ void process_tile(const uint64_t src_tile, const uint
                 load_staged(u);
         }
 #endif
-        // some state of this thread's chunks needed a canonical subtract (~1 thread in 2 000): redo all four
+        // some state of this thread's chunks needed a canonical subtract (~1 thread in 3 600): redo all four
         // exactly, from start states recomputed here (nothing is kept live for this path)
 #pragma unroll 1
         for (int u = 0; u < U; ++u) {

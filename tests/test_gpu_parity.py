@@ -5,6 +5,7 @@ import hashlib
 import numpy as np
 import pytest
 
+import kernel_model
 import oracle
 import synth
 from gpuutil import DeviceBuffer, sync
@@ -337,7 +338,8 @@ def test_archive_10k_entries_extract(mb):
 
 def test_many_small_entries(mb):
     """BASELINE config 4 shape (1-64 KiB entries, per-entry keys, one launch) at 20k entries:
-    sampled entries against the oracle, every entry through the decrypt round trip."""
+    sampled entries, and every entry that holds a byte only the kernel's redo branch gets right
+    (tests/kernel_model.py), against the oracle; every entry through the decrypt round trip."""
     rng = np.random.default_rng(4)
     n = 20_000
     sizes = rng.integers(1 << 10, (64 << 10) + 1, size=n).astype(np.int64)
@@ -350,7 +352,10 @@ def test_many_small_entries(mb):
     plan = mb.Plan(descs, total, total)
     plan.run(buf.ptr, buf.ptr)
     sync()
-    for i in [0, 1, 2, 3, 4, n - 1] + [int(x) for x in rng.integers(0, n, size=40)]:
+    sampled = [0, 1, 2, 3, 4, n - 1] + [int(x) for x in rng.integers(0, n, size=40)]
+    redo = kernel_model.entries_with_trigger_bytes(list(zip(off.tolist(), off.tolist(), sizes.tolist(), keys.tolist())))
+    assert len(redo) > 1000
+    for i in sampled + [int(x) for x in redo]:
         o, l = int(off[i]), int(sizes[i])
         assert (buf.download(o, l) == oracle.cycle(synth.payload(o, l), int(keys[i]))).all(), i
     plan.run(buf.ptr, buf.ptr)
