@@ -6,6 +6,8 @@
  * modulate_b200/csrc/ (which forward the data-parallel half to the kernels behind
  * modulate_b200.h):
  *   mod_ark_unpack   Unpack   (reference Modulate.cpp:291-317: CArk::Load + CArk::ExtractFiles)
+ *   mod_ark_find     search every entry for a byte pattern (CArk::Load + CArk::FindInFiles; no
+ *                    reference counterpart)
  *   mod_ark_pack     Pack     (reference Modulate.cpp:380-450: song list from the DTA configs unless
  *                              pack_all, CArk::Load of the reference header, ConstructFromDirectory,
  *                              BuildArk, SaveArk)
@@ -28,6 +30,14 @@ extern "C" {
 /* `header_path`: the .hdr file; `part_dir`: directory of the .ark parts ("" = current directory);
  * `target_dir`: where the files go (created as needed; must end in '/'). */
 int mod_ark_unpack(const char* header_path, const char* part_dir, const char* target_dir, int32_t body_key);
+
+/* CArk::Load + CArk::FindInFiles: every position at which an entry's deciphered bytes (entry keys all
+ * `body_key`) hold the `len`-byte pattern (1..64).  *out_total gets the exact number of matches;
+ * out_file / out_offset (capacity max_matches each; may be NULL when max_matches is 0) get the first
+ * min(total, max_matches) of them, (file table index, offset in the entry), sorted -- see CArk.h for
+ * when a truncated list is not the first ones.  Returns an eError (0 = success). */
+int mod_ark_find(const char* header_path, const char* part_dir, const uint8_t* pattern, uint32_t len, int32_t body_key,
+                 uint64_t max_matches, uint32_t* out_file, uint32_t* out_offset, uint64_t* out_total);
 
 /* `input_dir` and `output_dir` must end in '/'; the header is written to output_dir + header_name. */
 int mod_ark_pack(const char* reference_header_path, const char* input_dir, const char* output_dir,

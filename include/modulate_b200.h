@@ -161,6 +161,43 @@ int mod_cycle_batch(const mod_desc* descs, uint64_t n, const void* src, uint64_t
 int mod_cycle_batch_sharded(const mod_desc* descs, uint64_t n, const void* src, uint64_t src_bytes,
                             void* dst, uint64_t dst_bytes, uint64_t dev_mask);
 
+/* ---- search: which entries contain a byte pattern ------------------------------------------ */
+
+/* One match: `pos` is where the pattern starts inside descriptor `desc`'s deciphered bytes. */
+typedef struct mod_match {
+    uint32_t desc;
+    uint32_t pos;
+} mod_match;
+
+/* Search every descriptor of `plan` for the `len`-byte pattern (1 <= len <= 64, else MOD_ERR_ARG).  A
+ * descriptor's bytes are src[src_off, +len) after Cycle(., len, key) -- what mod_plan_run would write for
+ * it -- and every start i with i + pattern_len <= len whose bytes equal the pattern is a match, overlapping
+ * matches included; a match never spans two descriptors.  The plan must have been built with dst_off ==
+ * src_off for every descriptor and dst_align == d_src & 15 (the chunk grid then lies on the source, and
+ * nothing is written but the results).  Results ACCUMULATE, so the caller zeroes them first:
+ * d_counts[i] += matches in descriptor i (uint32_t per descriptor of the plan); *d_total += all matches;
+ * each match takes slot (*d_total before it) of d_matches and is stored only if that slot is below `cap`.
+ * The list order is unspecified; the counts are exact however many matches the list drops.
+ * Asynchronous on `stream`; all four result pointers are device memory. */
+int mod_plan_find(const mod_plan* plan, const void* d_src, const uint8_t* pattern, uint32_t len, uint32_t* d_counts,
+                  mod_match* d_matches, uint64_t cap, uint64_t* d_total, void* stream);
+
+/* mod_plan_find over tiles [tile_begin, tile_end) with only a window of the source resident (bytes
+ * [src_win_off, +src_win_bytes) of the plan's source space at d_src_win; (d_src_win - src_win_off) & 15
+ * must equal the plan's dst_align).  Every byte the tiles read, the up to len - 1 bytes past a tile that a
+ * match starting in it may cover included, must lie inside the window (checked on the host).  This is the
+ * slot-ring form CArk::FindInFiles streams an archive through.  Asynchronous on `stream`. */
+int mod_plan_find_window(const mod_plan* plan, uint64_t tile_begin, uint64_t tile_end, const void* d_src_win,
+                         uint64_t src_win_off, uint64_t src_win_bytes, const uint8_t* pattern, uint32_t len,
+                         uint32_t* d_counts, mod_match* d_matches, uint64_t cap, uint64_t* d_total, void* stream);
+
+/* Plan + find + destroy, synchronous: `d_src` must be device memory (MOD_ERR_ARG otherwise).  The HOST
+ * outputs get the per-descriptor counts (n entries), the total, and min(total, cap) matches sorted by
+ * (desc, pos); which matches a truncated list keeps is unspecified.  Only src_off, len and key of the
+ * descriptors are used. */
+int mod_find_batch(const mod_desc* descs, uint64_t n, const void* d_src, uint64_t src_bytes, const uint8_t* pattern,
+                   uint32_t len, uint32_t* counts_out, mod_match* matches_out, uint64_t cap, uint64_t* total_out);
+
 /* ---- offset-range sharding (host logic, no GPU needed) -------------------------------------- */
 
 /* (No reference counterpart: the reference is single-threaded, SURVEY.md section 8(e).)

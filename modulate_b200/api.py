@@ -111,6 +111,18 @@ def make_descs(src_off, dst_off, length, key) -> np.ndarray:
     return d
 
 
+# numpy view of ``mod_match``: where a pattern starts inside a descriptor's deciphered bytes
+MATCH_DTYPE = np.dtype([("desc", "<u4"), ("pos", "<u4")])
+MAX_PATTERN = 64
+
+
+def _pattern(pattern: Any) -> bytes:
+    p = bytes(pattern.encode() if isinstance(pattern, str) else pattern)
+    if not 1 <= len(p) <= MAX_PATTERN:
+        raise ValueError(f"the pattern must be 1 to {MAX_PATTERN} bytes, not {len(p)}")
+    return p
+
+
 def _descs(descs: np.ndarray) -> np.ndarray:
     d = np.ascontiguousarray(descs, dtype=DESC_DTYPE)
     return d
@@ -156,6 +168,24 @@ class Plan:
                                                  int(src_win_off), int(src_win_bytes), d_addr, int(dst_win_off),
                                                  int(dst_win_bytes), stream or None))
 
+    def find(self, src: Any, pattern: Any, counts: Any, matches: Any, cap: int, total: Any, stream: int = 0) -> None:
+        """Asynchronous search (``mod_plan_find``) of every descriptor for `pattern`: `counts` (uint32 per
+        descriptor), `matches` (``MATCH_DTYPE`` slots, `cap` of them) and `total` (one uint64) are device buffers
+        the results ACCUMULATE into.  The plan must have dst_off == src_off and dst_align == src & 15."""
+        p = _pattern(pattern)
+        _abi.check(self._lib.mod_plan_find(self._handle, _buffer_info(src)[0], p, len(p), _buffer_info(counts)[0],
+                                           _buffer_info(matches)[0] if cap else None, int(cap), _buffer_info(total)[0],
+                                           stream or None))
+
+    def find_window(self, tile_begin: int, tile_end: int, src_win: Any, src_win_off: int, src_win_bytes: int,
+                    pattern: Any, counts: Any, matches: Any, cap: int, total: Any, stream: int = 0) -> None:
+        """``find`` over a tile sub-range with only a window of the source resident (slot-ring streaming)."""
+        p = _pattern(pattern)
+        _abi.check(self._lib.mod_plan_find_window(self._handle, int(tile_begin), int(tile_end), _buffer_info(src_win)[0],
+                                                  int(src_win_off), int(src_win_bytes), p, len(p), _buffer_info(counts)[0],
+                                                  _buffer_info(matches)[0] if cap else None, int(cap),
+                                                  _buffer_info(total)[0], stream or None))
+
     def close(self) -> None:
         if self._handle:
             self._lib.mod_plan_destroy(self._handle)
@@ -180,6 +210,26 @@ def cycle_batch(descs: np.ndarray, src: Any, dst: Any, src_bytes: Optional[int] 
         raise ValueError("buffer sizes are required with raw addresses")
     _abi.check(_abi.load().mod_cycle_batch(d.ctypes.data if len(d) else None, len(d), s_addr, int(src_bytes),
                                            d_addr, int(dst_bytes)))
+
+
+def find_batch(descs: np.ndarray, src: Any, pattern: Any, src_bytes: Optional[int] = None,
+               max_matches: int = 1 << 20) -> Tuple[np.ndarray, np.ndarray, int]:
+    """Search each descriptor's deciphered bytes (``src`` on the device: a raw address or a CUDA tensor) for
+    `pattern` (synchronous).  -> (counts uint32[n], matches ``MATCH_DTYPE`` sorted by (desc, pos), at most
+    `max_matches` of them, exact total)."""
+    d = _descs(descs)
+    p = _pattern(pattern)
+    s_addr, s_n, _ = _buffer_info(src)
+    src_bytes = s_n if src_bytes is None else src_bytes
+    if src_bytes < 0:
+        raise ValueError("src_bytes is required with a raw address")
+    counts = np.zeros(len(d), dtype=np.uint32)
+    matches = np.zeros(max(0, int(max_matches)), dtype=MATCH_DTYPE)
+    total = ctypes.c_uint64()
+    _abi.check(_abi.load().mod_find_batch(d.ctypes.data if len(d) else None, len(d), s_addr, int(src_bytes), p, len(p),
+                                          counts.ctypes.data if len(d) else None, matches.ctypes.data if len(matches) else None,
+                                          len(matches), ctypes.byref(total)))
+    return counts, matches[:min(total.value, len(matches))].copy(), int(total.value)
 
 
 def cycle_batch_sharded(descs: np.ndarray, src: Any, dst: Any, src_bytes: Optional[int] = None,
@@ -259,6 +309,22 @@ def ark_pack(reference_header_path: str, input_dir: str, output_dir: str, header
                                   header_name.encode(), int(ps4), int(pack_all), int(ignore_new_files), _i32(body_key))
     if rc:
         raise ArkError(rc, "mod_ark_pack")
+
+
+def ark_find(header_path: str, part_dir: str, pattern: Any, body_key: int = 0,
+             max_matches: int = 1 << 20) -> Tuple[list, int]:
+    """``CArk::Load`` + ``CArk::FindInFiles``: -> ([(file_index, offset), ...] sorted, exact total)."""
+    p = _pattern(pattern)
+    files = np.zeros(max(0, int(max_matches)), dtype=np.uint32)
+    offsets = np.zeros_like(files)
+    total = ctypes.c_uint64()
+    rc = _abi.load().mod_ark_find(header_path.encode(), _slash(part_dir) if part_dir else b"", p, len(p), _i32(body_key),
+                                  len(files), files.ctypes.data if len(files) else None,
+                                  offsets.ctypes.data if len(files) else None, ctypes.byref(total))
+    if rc:
+        raise ArkError(rc, "mod_ark_find")
+    k = min(total.value, len(files))
+    return [(int(f), int(o)) for f, o in zip(files[:k], offsets[:k])], int(total.value)
 
 
 def dta_set_int(dta_path: str, key: str, value: int) -> None:

@@ -287,15 +287,19 @@ int HostThreads()
 uint64_t GroupBytes() { return (uint64_t)Tunable("MOD_IO_GROUP_MIB", 32) << 20; }
 
 void CutEntry(uint32_t luFile, uint64_t luSize, uint64_t luSrc, uint64_t luDst, int32_t liKey, uint64_t luGroupBytes,
-              std::vector<Piece>& laPieces, std::vector<mod_desc>& laDescs)
+              uint32_t luOverlap, std::vector<Piece>& laPieces, std::vector<mod_desc>& laDescs)
 {
     uint64_t luAt = 0;
     do {
         uint64_t luTake = luSize <= luGroupBytes + luGroupBytes / 2 ? luSize : std::min(luGroupBytes, luSize - luAt);
         if (luSize - luAt - luTake < luGroupBytes / 2)
             luTake = luSize - luAt;  // no short tail piece
-        laPieces.push_back(Piece{luFile, luAt, (uint32_t)luTake});
-        laDescs.push_back(mod_desc{luSrc + luAt, luDst + luAt, (uint32_t)luTake, luAt ? mod_key_jump(liKey, luAt) : liKey});
+        // Search: piece k covers [a_k, min(a_{k+1} + L - 1, size)) with luOverlap = L - 1.  A match inside it starts
+        // at i with i + L <= a_{k+1} + L - 1, i.e. i < a_{k+1}: every match that starts in [a_k, a_{k+1}) is
+        // found in piece k and in no other piece, so nothing is counted twice and nothing needs deduplicating.
+        const uint64_t luCover = luTake + std::min<uint64_t>(luOverlap, luSize - luAt - luTake);
+        laPieces.push_back(Piece{luFile, luAt, (uint32_t)luCover});
+        laDescs.push_back(mod_desc{luSrc + luAt, luDst + luAt, (uint32_t)luCover, luAt ? mod_key_jump(liKey, luAt) : liKey});
         luAt += luTake;
     } while (luAt < luSize);
 }
@@ -321,9 +325,26 @@ std::vector<Group> GroupPieces(const std::vector<mod_desc>& laDescs, uint64_t lu
     return laGroups;
 }
 
+GpuStep CipherStep()
+{
+    GpuStep lStep;
+    lStep.mEnqueue = [](const Group& lGroup, const SlotView& lSlot) {
+        const uint64_t luRange = lGroup.srcHi - lGroup.srcLo, luPayload = lGroup.dstHi - lGroup.dstLo;
+        uint64_t luTile0 = 0, luTile1 = 0;
+        unsigned char* lpDevIn = (unsigned char*)lSlot.mpDevIn + (lGroup.srcLo & 15u);
+        unsigned char* lpDevOut = (unsigned char*)lSlot.mpDevOut + (lGroup.dstLo & 15u);
+        return mod_plan_tile_range(lSlot.mpPlan, lGroup.first, lGroup.last, &luTile0, &luTile1) == MOD_OK &&
+               mod_memcpy_h2d(lpDevIn, lSlot.mpHostIn + (lGroup.srcLo & 15u), luRange, lSlot.mpStream) == MOD_OK &&
+               mod_plan_run_window(lSlot.mpPlan, luTile0, luTile1, lpDevIn, lGroup.srcLo, luRange, lpDevOut, lGroup.dstLo,
+                                   luPayload, lSlot.mpStream) == MOD_OK &&
+               mod_memcpy_d2h(lSlot.mpHostOut + (lGroup.dstLo & 15u), lpDevOut, luPayload, lSlot.mpStream) == MOD_OK;
+    };
+    return lStep;
+}
+
 eError RunPipeline(const char* lpName, const std::vector<mod_desc>& laDescs, const std::vector<Group>& laGroups,
                    uint64_t luSrcBytes, uint64_t luDstBytes, bool lbUseGpu, int liReaders, int liWriters, const Stage& lFill,
-                   const Stage& lDrain)
+                   const GpuStep& lGpu, const Stage& lDrain)
 {
     const double ldStart = NowSeconds();
     uint64_t luMaxRange = 1, luMaxPayload = 1;
@@ -338,7 +359,8 @@ eError RunPipeline(const char* lpName, const std::vector<mod_desc>& laDescs, con
     SlotRing lRing;
     std::vector<mod_plan*> laPlans(laDevices.size(), nullptr);
     const int liSlotsPerDevice = Tunable("MOD_IO_SLOTS", std::max(3, 6 / (int)laDevices.size()));
-    bool lbReady = lRing.Allocate(laDevices, liSlotsPerDevice, laGroups.size(), luMaxRange, lbUseGpu ? luMaxPayload : 0, lbUseGpu);
+    const uint64_t luOutBytes = !lbUseGpu ? 0 : lGpu.muOutBytes ? lGpu.muOutBytes : luMaxPayload;
+    bool lbReady = lRing.Allocate(laDevices, liSlotsPerDevice, laGroups.size(), luMaxRange, luOutBytes, lbUseGpu);
     for (size_t dd = 0; dd < laDevices.size() && lbReady && lbUseGpu; ++dd)
         lbReady = mod_init(laDevices[dd]) == MOD_OK &&
                   mod_plan_create(laDescs.data(), laDescs.size(), luSrcBytes, luDstBytes, 0, &laPlans[dd]) == MOD_OK;
@@ -373,20 +395,13 @@ eError RunPipeline(const char* lpName, const std::vector<mod_desc>& laDescs, con
                 });
             }
         };
-        // upload -> kernel over the group's tiles -> download on the slot's stream, on the slot's device
+        // the GPU step of the group on the slot's stream, on the slot's device
         auto lEnqueue = [&](const Group& lGroup, Slot& lSlot) {
-            const uint64_t luRange = lGroup.srcHi - lGroup.srcLo, luPayload = lGroup.dstHi - lGroup.dstLo;
             const size_t liDeviceIndex = (size_t)(std::find(laDevices.begin(), laDevices.end(), lSlot.miDevice) - laDevices.begin());
-            uint64_t luTile0 = 0, luTile1 = 0;
             SlowOp lTimer(lEnqueueWhat.c_str());
-            unsigned char* lpDevIn = (unsigned char*)lSlot.mpDevIn + (lGroup.srcLo & 15u);
-            unsigned char* lpDevOut = (unsigned char*)lSlot.mpDevOut + (lGroup.dstLo & 15u);
-            return mod_init(lSlot.miDevice) == MOD_OK &&
-                   mod_plan_tile_range(laPlans[liDeviceIndex], lGroup.first, lGroup.last, &luTile0, &luTile1) == MOD_OK &&
-                   mod_memcpy_h2d(lpDevIn, lSlot.mpHostIn + (lGroup.srcLo & 15u), luRange, lSlot.mpStream) == MOD_OK &&
-                   mod_plan_run_window(laPlans[liDeviceIndex], luTile0, luTile1, lpDevIn, lGroup.srcLo, luRange, lpDevOut,
-                                       lGroup.dstLo, luPayload, lSlot.mpStream) == MOD_OK &&
-                   mod_memcpy_d2h(lSlot.mpHostOut + (lGroup.dstLo & 15u), lpDevOut, luPayload, lSlot.mpStream) == MOD_OK;
+            const SlotView lView{liDeviceIndex, laPlans[liDeviceIndex], lSlot.mpHostIn, lSlot.mpHostOut, lSlot.mpDevIn, lSlot.mpDevOut,
+                                 lSlot.mpStream};
+            return mod_init(lSlot.miDevice) == MOD_OK && lGpu.mEnqueue(lGroup, lView);
         };
 
         // this thread: start fills while slots are free, enqueue each filled group in turn, never waiting for the GPU

@@ -21,6 +21,11 @@
 #include "CEncryptionCycler.h"
 #include "Settings.h"
 
+// The search entry points are an addition to version 2 of the C ABI: they are referenced weakly, so the
+// facade still links against an implementation of the ABI that predates them, and FindInFiles reports that
+// the library lacks the search instead of the program failing to load.
+#pragma weak mod_plan_find_window
+
 namespace {
 
 bool ReadWholeFile(const std::string& lPath, std::vector<unsigned char>& lOut)
@@ -327,6 +332,38 @@ bool CArk::ReadImageRange(std::vector<int>& laFds, uint64_t luOffset, uint64_t l
     return luSize == 0;
 }
 
+// Fill stage of the pipelines that read the archive: the image range of a group, 8 MiB per task (laPartFds
+// caches the part files' descriptors; the caller closes them).
+arkpipe::Stage CArk::ReadGroupsStage(const std::vector<arkpipe::Group>& laGroups, std::vector<int>& laPartFds) const
+{
+    const uint64_t kuReadPiece = 8ull << 20;
+    return arkpipe::Stage{
+        [&laGroups, kuReadPiece](size_t gg) {
+            return (int)std::max<uint64_t>(1, (laGroups[gg].srcHi - laGroups[gg].srcLo + kuReadPiece - 1) / kuReadPiece);
+        },
+        [this, &laGroups, &laPartFds, kuReadPiece](size_t gg, int tt, unsigned char* lpRange) {
+            arkpipe::SlowOp lTimer("ExtractFiles read of an 8 MiB image piece");
+            const arkpipe::Group& lGroup = laGroups[gg];
+            const uint64_t luLo = (uint64_t)tt * kuReadPiece, luHi = std::min(lGroup.srcHi - lGroup.srcLo, luLo + kuReadPiece);
+            if (luHi > luLo && !ReadImageRange(laPartFds, lGroup.srcLo + luLo, luHi - luLo, lpRange + luLo))
+                return eError_FailedToOpenFile;
+            return eError_NoError;
+        }};
+}
+
+// Entries that lie (partly) outside the image of luImageSize bytes are refused, whatever reads the archive.
+eError CArk::CheckEntriesInImage(uint64_t luImageSize) const
+{
+    for (const modark::FileDef& lFile : mHeader.maFiles) {
+        if ((uint64_t)lFile.mi64Offset > luImageSize || (uint64_t)lFile.miSize > luImageSize - (uint64_t)lFile.mi64Offset) {
+            std::cout << "Entry " << lFile.mName.c_str() << " lies outside the archive data\n";
+            eError leError = eError_InvalidData;
+            SHOW_ERROR_AND_RETURN;
+        }
+    }
+    return eError_NoError;
+}
+
 // Extraction streams the archive through the slot-ring pipeline (ArkPipeline.h) instead of the
 // reference's one archive-sized buffer (CArk.cpp:431, :738) and its serial one-file-at-a-time writes
 // (:435-501): the entries, ordered by image offset, are packed back to back into a staging space, and
@@ -345,14 +382,8 @@ eError CArk::ExtractFiles(int liFirstFileIndex, int liNumFiles, const char* lpTa
         luImageSize += lPart.muSize;
 
     const size_t liCount = mHeader.maFiles.size();
-    for (size_t ii = 0; ii < liCount; ++ii) {
-        const modark::FileDef& lFile = mHeader.maFiles[ii];
-        if ((uint64_t)lFile.mi64Offset > luImageSize || (uint64_t)lFile.miSize > luImageSize - (uint64_t)lFile.mi64Offset) {
-            std::cout << "Entry " << lFile.mName.c_str() << " lies outside the archive data\n";
-            eError leError = eError_InvalidData;
-            SHOW_ERROR_AND_RETURN;
-        }
-    }
+    eError leError = CheckEntriesInImage(luImageSize);
+    ERROR_RETURN;
 
     // Duplicate output names.  The reference writes in table order, one file at a time (CArk.cpp:435-501):
     // with overwriting on (the default) the LAST entry of a name is what stays on disk; with it off a
@@ -390,7 +421,7 @@ eError CArk::ExtractFiles(int liFirstFileIndex, int liNumFiles, const char* lpTa
     uint64_t luStaged = 0;
     for (uint32_t luFile : laOrder) {
         const modark::FileDef& lFile = mHeader.maFiles[luFile];
-        arkpipe::CutEntry(luFile, (uint64_t)lFile.miSize, (uint64_t)lFile.mi64Offset, luStaged, EntryKey(luFile), kuGroupBytes,
+        arkpipe::CutEntry(luFile, (uint64_t)lFile.miSize, (uint64_t)lFile.mi64Offset, luStaged, EntryKey(luFile), kuGroupBytes, 0,
                           laPieces, laDescs);
         luStaged += (uint64_t)lFile.miSize;
     }
@@ -424,19 +455,8 @@ eError CArk::ExtractFiles(int liFirstFileIndex, int liNumFiles, const char* lpTa
         }
     }
 
-    // fill: the image range of a group, 8 MiB per task
     std::vector<int> laPartFds(mHeader.maParts.size(), -1);
-    const uint64_t kuReadPiece = 8ull << 20;
-    const arkpipe::Stage lRead{
-        [&](size_t gg) { return (int)std::max<uint64_t>(1, (laGroups[gg].srcHi - laGroups[gg].srcLo + kuReadPiece - 1) / kuReadPiece); },
-        [&](size_t gg, int tt, unsigned char* lpRange) {
-            arkpipe::SlowOp lTimer("ExtractFiles read of an 8 MiB image piece");
-            const arkpipe::Group& lGroup = laGroups[gg];
-            const uint64_t luLo = (uint64_t)tt * kuReadPiece, luHi = std::min(lGroup.srcHi - lGroup.srcLo, luLo + kuReadPiece);
-            if (luHi > luLo && !ReadImageRange(laPartFds, lGroup.srcLo + luLo, luHi - luLo, lpRange + luLo))
-                return eError_FailedToOpenFile;
-            return eError_NoError;
-        }};
+    const arkpipe::Stage lRead = ReadGroupsStage(laGroups, laPartFds);
 
     // drain: the files of a group, 48 per task
     const size_t kiFilesPerTask = 48;
@@ -487,14 +507,150 @@ eError CArk::ExtractFiles(int liFirstFileIndex, int liNumFiles, const char* lpTa
         }};
 
     const int liCores = arkpipe::HostThreads();
-    eError leError = arkpipe::RunPipeline("extract", laDescs, laGroups, luImageSize, luStaged, true, std::max(2, std::min(8, liCores / 4)),
-                                          std::max(4, std::min(16, liCores / 2)), lRead, lWrite);
+    leError = arkpipe::RunPipeline("extract", laDescs, laGroups, luImageSize, luStaged, true, std::max(2, std::min(8, liCores / 4)),
+                                          std::max(4, std::min(16, liCores / 2)), lRead, arkpipe::CipherStep(), lWrite);
     for (int liFd : laPartFds)
         if (liFd >= 0)
             close(liFd);
     if (leError == eError_NoData)  // the GPU could not be set up; RunPipeline has said why
         return leError;
     SHOW_ERROR_AND_RETURN;
+    return eError_NoError;
+}
+
+// The search reads the parts like ExtractFiles, but the GPU step deciphers and matches instead of storing: only
+// each group's short match list comes back over PCIe, and nothing is written.  Entries are searched in image
+// order, pieces of big entries overlapping by luLen - 1 bytes (CutEntry), and every entry is searched, also
+// when another one has the same name.
+eError CArk::FindInFiles(const unsigned char* lpPattern, uint32_t luLen, uint64_t luMaxMatches, std::vector<SFileMatch>& laMatches,
+                         uint64_t* lpTotal, std::vector<uint64_t>* lpFileCounts)
+{
+    laMatches.clear();
+    if (!lpPattern || luLen == 0 || luLen > 64 || !lpTotal)
+        return eError_InvalidParameter;
+    *lpTotal = 0;
+    if (!mod_plan_find_window) {
+        std::cout << "The GPU library in use has no search (mod_plan_find_window)\n";
+        return eError_NoData;
+    }
+    if (mHeader.maFiles.empty())
+        return eError_NoData;
+    uint64_t luImageSize = 0;
+    for (const modark::PartDef& lPart : mHeader.maParts)
+        luImageSize += lPart.muSize;
+    eError leError = CheckEntriesInImage(luImageSize);
+    ERROR_RETURN;
+
+    const size_t liCount = mHeader.maFiles.size();
+    std::vector<uint32_t> laOrder(liCount);
+    for (size_t ii = 0; ii < liCount; ++ii)
+        laOrder[ii] = (uint32_t)ii;
+    std::stable_sort(laOrder.begin(), laOrder.end(), [&](uint32_t a, uint32_t b) {
+        return mHeader.maFiles[a].mi64Offset < mHeader.maFiles[b].mi64Offset;
+    });
+    const uint64_t kuGroupBytes = arkpipe::GroupBytes();
+    std::vector<arkpipe::Piece> laPieces;
+    std::vector<mod_desc> laDescs;  // dst_off == src_off: the plan's chunk grid lies on the image
+    for (uint32_t luFile : laOrder) {
+        const modark::FileDef& lFile = mHeader.maFiles[luFile];
+        arkpipe::CutEntry(luFile, (uint64_t)lFile.miSize, (uint64_t)lFile.mi64Offset, (uint64_t)lFile.mi64Offset, EntryKey(luFile),
+                          kuGroupBytes, luLen - 1, laPieces, laDescs);
+    }
+    const std::vector<arkpipe::Group> laGroups = arkpipe::GroupPieces(laDescs, kuGroupBytes);
+    uint64_t luCap = 0;  // list slots per group: a group cannot hold more matches than it has bytes
+    for (const arkpipe::Group& lGroup : laGroups)
+        luCap = std::max(luCap, std::min<uint64_t>(luMaxMatches, lGroup.dstHi - lGroup.dstLo));
+    const uint64_t luListBytes = 16 + 8 * luCap;  // total (8 bytes), 8 spare, the list
+
+    // GPU step: zero the slot's total, upload, search the group's tiles, download the total and the list.  The
+    // per-descriptor counts live in one array per device, zeroed on the device's first group.
+    struct DeviceCounts {
+        int miDevice = -1;
+        uint32_t* mpCounts = nullptr;
+    };
+    std::vector<DeviceCounts> laCounts(64);
+    const std::vector<uint32_t> laZeros(laDescs.size(), 0);
+    arkpipe::GpuStep lFind;
+    lFind.muOutBytes = luListBytes;
+    lFind.mEnqueue = [&](const arkpipe::Group& lGroup, const arkpipe::SlotView& lSlot) {
+        DeviceCounts& lCounts = laCounts[lSlot.miDeviceIndex];
+        if (!lCounts.mpCounts) {
+            lCounts.miDevice = mod_current_device();
+            lCounts.mpCounts = (uint32_t*)mod_device_alloc(4 * laDescs.size());
+            if (!lCounts.mpCounts || mod_memcpy_h2d(lCounts.mpCounts, laZeros.data(), 4 * laDescs.size(), lSlot.mpStream) != MOD_OK ||
+                mod_stream_sync(lSlot.mpStream) != MOD_OK)
+                return false;
+        }
+        const uint64_t luRange = lGroup.srcHi - lGroup.srcLo;
+        unsigned char* lpDevIn = (unsigned char*)lSlot.mpDevIn + (lGroup.srcLo & 15u);
+        unsigned char* lpList = lSlot.mpHostOut + (lGroup.dstLo & 15u);
+        std::memset(lpList, 0, 16);
+        uint64_t luTile0 = 0, luTile1 = 0;
+        return mod_plan_tile_range(lSlot.mpPlan, lGroup.first, lGroup.last, &luTile0, &luTile1) == MOD_OK &&
+               mod_memcpy_h2d(lSlot.mpDevOut, lpList, 16, lSlot.mpStream) == MOD_OK &&
+               mod_memcpy_h2d(lpDevIn, lSlot.mpHostIn + (lGroup.srcLo & 15u), luRange, lSlot.mpStream) == MOD_OK &&
+               mod_plan_find_window(lSlot.mpPlan, luTile0, luTile1, lpDevIn, lGroup.srcLo, luRange, lpPattern, luLen, lCounts.mpCounts,
+                                    (mod_match*)((unsigned char*)lSlot.mpDevOut + 16), luCap, (uint64_t*)lSlot.mpDevOut,
+                                    lSlot.mpStream) == MOD_OK &&
+               mod_memcpy_d2h(lpList, lSlot.mpDevOut, luListBytes, lSlot.mpStream) == MOD_OK;
+    };
+
+    // drain: the group's list, as (file, offset in the entry)
+    std::mutex lMutex;
+    const arkpipe::Stage lCollect{
+        [&](size_t gg) { return laGroups[gg].dstHi > laGroups[gg].dstLo ? 1 : 0; },
+        [&](size_t, int, unsigned char* lpList) {
+            uint64_t luTotal = 0;
+            std::memcpy(&luTotal, lpList, 8);
+            const uint64_t luKept = std::min(luTotal, luCap);
+            std::lock_guard<std::mutex> lLock(lMutex);
+            for (uint64_t kk = 0; kk < luKept; ++kk) {
+                mod_match lMatch;
+                std::memcpy(&lMatch, lpList + 16 + 8 * kk, sizeof(lMatch));
+                const arkpipe::Piece& lPiece = laPieces[lMatch.desc];
+                laMatches.push_back(SFileMatch{(int)lPiece.file, (uint32_t)(lPiece.fileOffset + lMatch.pos)});
+            }
+            return eError_NoError;
+        }};
+
+    std::vector<int> laPartFds(mHeader.maParts.size(), -1);
+    const int liOriginalDevice = mod_current_device();
+    const int liCores = arkpipe::HostThreads();
+    leError = arkpipe::RunPipeline("find", laDescs, laGroups, luImageSize, luImageSize, true, std::max(2, std::min(8, liCores / 4)), 2,
+                                   ReadGroupsStage(laGroups, laPartFds), lFind, lCollect);
+    for (int liFd : laPartFds)
+        if (liFd >= 0)
+            close(liFd);
+
+    // exact counts: the devices' arrays, summed per entry
+    std::vector<uint64_t> laFileCounts(liCount, 0);
+    std::vector<uint32_t> laDescCounts(laDescs.size());
+    for (DeviceCounts& lCounts : laCounts) {
+        if (!lCounts.mpCounts)
+            continue;
+        if (leError == eError_NoError &&
+            (mod_init(lCounts.miDevice) != MOD_OK || mod_memcpy_d2h(laDescCounts.data(), lCounts.mpCounts, 4 * laDescs.size(), nullptr) != MOD_OK ||
+             mod_stream_sync(nullptr) != MOD_OK)) {
+            std::cout << "GPU find failed: " << mod_last_error() << "\n";
+            leError = eError_InvalidData;
+        }
+        for (size_t ii = 0; ii < laDescs.size() && leError == eError_NoError; ++ii)
+            laFileCounts[laPieces[ii].file] += laDescCounts[ii];
+        mod_device_free(lCounts.mpCounts);
+    }
+    if (liOriginalDevice >= 0)
+        mod_init(liOriginalDevice);
+    if (leError == eError_NoData)  // the GPU could not be set up; RunPipeline has said why
+        return leError;
+    SHOW_ERROR_AND_RETURN;
+    for (uint64_t luCount : laFileCounts)
+        *lpTotal += luCount;
+    std::sort(laMatches.begin(), laMatches.end(),
+              [](const SFileMatch& a, const SFileMatch& b) { return a.file != b.file ? a.file < b.file : a.offset < b.offset; });
+    if (laMatches.size() > luMaxMatches)
+        laMatches.resize((size_t)luMaxMatches);
+    if (lpFileCounts)
+        *lpFileCounts = std::move(laFileCounts);
     return eError_NoError;
 }
 
@@ -655,7 +811,7 @@ eError CArk::StreamBuiltImage(const std::vector<PartTarget>& laTargets) const
         const int liKey = EntryKey(ii);
         lbAnyKey = lbAnyKey || (liKey % 0x7FFFFFFF) != 0;
         arkpipe::CutEntry((uint32_t)ii, (uint64_t)lFile.miSize, (uint64_t)lFile.mi64Offset, (uint64_t)lFile.mi64Offset, liKey,
-                          kuGroupBytes, laPieces, laDescs);
+                          kuGroupBytes, 0, laPieces, laDescs);
     }
     if (laPieces.empty())
         return eError_NoError;
@@ -720,7 +876,7 @@ eError CArk::StreamBuiltImage(const std::vector<PartTarget>& laTargets) const
 
     const int liThreads = std::max(2, std::min(12, arkpipe::HostThreads() / 2));
     return arkpipe::RunPipeline("build", laDescs, laGroups, muBuiltImageSize, muBuiltImageSize, lbAnyKey, liThreads, liThreads, lRead,
-                                lWrite);
+                                arkpipe::CipherStep(), lWrite);
 }
 
 eError CArk::SaveArk(const char* lpOutputDirectory, const char* lpHeaderFilename) const

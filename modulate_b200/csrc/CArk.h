@@ -10,6 +10,8 @@
 //                         CArk.cpp:494) in the reader -> GPU -> writer slot-ring pipeline of
 //                         ArkPipeline.h, over every visible GPU: nothing is ever waited for on the
 //                         thread that enqueues
+//   FindInFiles           searches every entry for a byte pattern through the same pipeline, reading
+//                         the parts like ExtractFiles and keeping only the match lists (mod_plan_find_window)
 //   BuildArk              assigns byte-packed offsets and part sizes from the file sizes (CArk.cpp:760-828)
 //   SaveArk               serialises + enciphers the header (CArk.cpp:1135-1136) and STREAMS the payload
 //                         from the input files into the part files through the same pipeline (entries
@@ -28,6 +30,17 @@
 #include "ArkHeader.h"
 #include "CDtaFile.h"  // SSongConfig, like the reference (CArk.h:6)
 #include "Error.h"
+
+namespace arkpipe {
+struct Group;
+struct Stage;
+}
+
+// One match of CArk::FindInFiles: entry `file` (index into the file table) holds the pattern at `offset`.
+struct SFileMatch {
+    int file;
+    uint32_t offset;
+};
 
 class CArk
 {
@@ -54,6 +67,15 @@ public:
     void SetUniformEntryKey(int liKey);                  // every entry ciphered with liKey, stream restarting per entry
     void SetEntryKeys(const std::vector<int>& laKeys);   // one key per entry, in table order
     void SetPartDirectory(const char* lpDirectory);      // where LoadArkData looks for the part files ("" = cwd)
+    // Every position at which an entry's deciphered bytes hold the luLen-byte pattern (1..64), overlapping
+    // ones included, found on the GPU in one pass over the part files that writes nothing.  Entries that
+    // share a name are each searched and reported (ExtractFiles keeps only one of them).  *lpTotal gets the
+    // exact number of matches and lpFileCounts, when given, the exact number per entry in table order;
+    // laMatches gets min(total, luMaxMatches) of them sorted by (file, offset) -- all of them, and so the
+    // first luMaxMatches, unless more than luMaxMatches fall into one pipeline group (MOD_IO_GROUP_MIB of the
+    // image), in which case which ones that group keeps is unspecified.
+    eError FindInFiles(const unsigned char* lpPattern, uint32_t luLen, uint64_t luMaxMatches, std::vector<SFileMatch>& laMatches,
+                       uint64_t* lpTotal, std::vector<uint64_t>* lpFileCounts = nullptr);
     const modark::HeaderImage& Header() const { return mHeader; }
 
 private:
@@ -61,6 +83,8 @@ private:
     eError AllocateArkData();
     eError ReadParts();
     bool ReadImageRange(std::vector<int>& laFds, uint64_t luOffset, uint64_t luSize, unsigned char* lpDst) const;
+    arkpipe::Stage ReadGroupsStage(const std::vector<arkpipe::Group>& laGroups, std::vector<int>& laPartFds) const;
+    eError CheckEntriesInImage(uint64_t luImageSize) const;
     struct PartTarget {
         int miFd = -1;             // part file open for writing
         unsigned char* mpMap = nullptr;  // its mapping, when it could be mapped

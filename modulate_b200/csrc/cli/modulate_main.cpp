@@ -5,7 +5,10 @@
 // reference are host-side tooling outside the hot path and are not provided.
 //
 // Extensions: -bodykey K (cipher every entry body with key K, stream restarting per entry -- the
-// synthetic per-entry-key configurations), -device N (bind GPU N).
+// synthetic per-entry-key configurations), -device N (bind GPU N), -find TEXT / -findhex HEX (which
+// entries hold a byte pattern, searched on the GPU without unpacking).
+#include <algorithm>
+#include <cctype>
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
@@ -107,6 +110,63 @@ eError Unpack(std::deque<std::string>& laParams)
         std::fprintf(stderr, "[mod] Unpack: Load (CUDA init + header Cycle + parse) %.3f s, ExtractFiles %.3f s\n",
                      ldLoaded - ldStart, lNow() - ldLoaded);
     return eError_NoError;
+}
+
+// -find / -findhex: one line "<name>\t<offset>" per match in table order, then by offset, at most
+// kiMaxLines of them, and always the exact "<total> matches in <files> files".
+eError FindPattern(const std::string& lPattern)
+{
+    constexpr uint64_t kiMaxLines = 10000;
+    if (lPattern.empty() || lPattern.size() > 64) {
+        std::cout << "The pattern must be 1 to 64 bytes long\n";
+        return eError_InvalidParameter;
+    }
+    std::cout << "Searching " << HeaderName() << " for " << lPattern.size() << " bytes\n";
+    CArk lArkHeader;
+    lArkHeader.SetUniformEntryKey(giBodyKey);
+    eError leError = lArkHeader.Load(HeaderName().c_str());
+    SHOW_ERROR_AND_RETURN;
+    std::vector<SFileMatch> laMatches;
+    std::vector<uint64_t> laFileCounts;
+    uint64_t luTotal = 0;
+    leError = lArkHeader.FindInFiles((const unsigned char*)lPattern.data(), (uint32_t)lPattern.size(), kiMaxLines, laMatches,
+                                     &luTotal, &laFileCounts);
+    SHOW_ERROR_AND_RETURN;
+    for (const SFileMatch& lMatch : laMatches)
+        std::cout << lArkHeader.Header().maFiles[(size_t)lMatch.file].mName << "\t" << lMatch.offset << "\n";
+    if (luTotal > laMatches.size())
+        std::cout << "... " << luTotal - laMatches.size() << " more\n";
+    const size_t liFiles = (size_t)std::count_if(laFileCounts.begin(), laFileCounts.end(), [](uint64_t n) { return n != 0; });
+    std::cout << luTotal << " matches in " << liFiles << " files\n";
+    return eError_NoError;
+}
+
+eError Find(std::deque<std::string>& laParams)
+{
+    if (laParams.empty())
+        return eError_InvalidParameter;
+    const std::string lText = laParams.front();
+    laParams.pop_front();
+    return FindPattern(lText);
+}
+
+eError FindHex(std::deque<std::string>& laParams)
+{
+    if (laParams.empty())
+        return eError_InvalidParameter;
+    std::string lDigits;
+    for (char c : laParams.front())
+        if (!std::isspace((unsigned char)c))
+            lDigits += c;
+    laParams.pop_front();
+    if (lDigits.size() % 2 != 0 || lDigits.find_first_not_of("0123456789abcdefABCDEF") != std::string::npos) {
+        std::cout << "-findhex takes pairs of hex digits\n";
+        return eError_InvalidParameter;
+    }
+    std::string lBytes;
+    for (size_t ii = 0; ii < lDigits.size(); ii += 2)
+        lBytes += (char)std::stoi(lDigits.substr(ii, 2), nullptr, 16);
+    return FindPattern(lBytes);
 }
 
 eError PackImpl(std::deque<std::string>& laParams)
@@ -282,6 +342,8 @@ void PrintUsage()
               << "  -pack <in_dir> <out_dir>    Repack the files the reference header knows\n"
               << "  -pack_add <in_dir> <out_dir> Repack, also adding new files\n"
               << "  -decode                     Write the deciphered header to main_<platform>.hdr.dec\n"
+              << "  -find <text>                List the entries (and offsets) whose bytes contain <text>\n"
+              << "  -findhex <hex>              Same for a pattern given as hex bytes, e.g. 00ff1a\n"
               << "  -listsongs <dir>            List the songs the DTA configs under <dir> define\n"
               << "  -dtaset <file> <key> <val>  Patch the value following symbol <key> in a binary DTA file\n"
               << "  -dtacopy <in> <out>         Load and re-save a binary DTA file\n";
@@ -311,7 +373,7 @@ int main(int argc, char* argv[])
         {"-ps3", PS3},       {"-verbose", EnableVerbose}, {"-force", EnableForceWrite}, {"-packall", EnablePackAll},
         {"-bodykey", BodyKey}, {"-device", Device},       {"-unpack", Unpack},          {"-pack", Pack},
         {"-pack_add", AddPack}, {"-decode", Decode},   {"-dtaset", DtaSet},          {"-dtacopy", DtaCopy},
-        {"-listsongs", ListSongs},
+        {"-listsongs", ListSongs}, {"-find", Find},     {"-findhex", FindHex},
     };
 
     std::deque<std::string> laParams;

@@ -502,7 +502,7 @@ __device__ __forceinline__ TileRec make_tile_rec(uint64_t src_off, uint64_t dst_
     r.state = tile_start_state(n0, h0, tin);
     r.geom = pack_geom(n_valid, tin == 0u ? h0 : 0u, last ? (((uint32_t)span - 1u) & 15u) + 1u : 16u);
     r.entry = entry;
-    r.pad = 0u;
+    r.rest = last ? 0u : (uint32_t)(span - 16ull * (c_begin + n_valid));
     return r;
 }
 
@@ -605,11 +605,165 @@ __global__ void build_tiles_kernel(const DevDesc* __restrict__ descs, uint32_t n
     tiles[t] = make_tile_rec(d.src_off, d.dst_off, d.len, d.neg_state, t - d.first_tile, dst_align, lo);
 }
 
+// ---- search: decipher a tile into shared memory, match a pattern there, store nothing -------------------
+//
+// One CTA per tile of a plan whose chunk grid is co-aligned with the source, so every chunk is one LDG.128.
+// The keystream is the batched kernel's: lazy states, speculative packing, and the thread's chunks redone
+// exactly when one of their states had bit 31 set (the redo reloads its source: ~1 thread in 3 600).
+// A match may start in the tile and end in the next L - 1 bytes of its entry, so a tile whose entry
+// continues also deciphers that HALO (at most kHaloChunks chunks, exact, a constant jump from the tile
+// state).  Every start position inside the tile is tested: a 2-byte SWAR filter, then a 4-byte masked word
+// compare, then the remaining pattern bytes.  Matches are rare, so the atomics that count
+// and list them are off the common path.
+#ifndef MODK_MIN_CTAS_FIND
+#define MODK_MIN_CTAS_FIND 10
+#endif
+
+__constant__ uint32_t c_halo_pow2[kHaloChunks];  // 2 * a^(16 * (kChunksPerTile + k)): halo chunk k's jump
+
+__device__ __noinline__ void find_record(const FindArgs& f, uint32_t entry, int64_t src_rel, uint32_t p)
+{
+    const uint64_t src_off = __ldg(&f.descs[entry].src_off);
+    atomicAdd(&f.counts[entry], 1u);
+    const unsigned long long slot = atomicAdd(f.total, 1ull);
+    if (slot < f.cap)
+        f.matches[slot] = make_uint2(entry, (uint32_t)((uint64_t)(src_rel + (int64_t)p) - src_off));
+}
+
+// Bytes [lo, hi) of the 16 at `addr`, the others zero: for chunks whose granule may leave the source buffer.
+__device__ __noinline__ uint4 load_bytes(uint64_t addr, uint32_t lo, uint32_t hi)
+{
+    uint32_t w[4] = {0u, 0u, 0u, 0u};
+#pragma unroll
+    for (uint32_t b = 0; b < 16; ++b) {
+        if (b >= lo && b < hi) {
+            uint32_t byte;
+            asm volatile("ld.global.u8 %0, [%1];" : "=r"(byte) : "l"(addr + b));
+            w[b >> 2] |= byte << (8u * (b & 3u));
+        }
+    }
+    return make_uint4(w[0], w[1], w[2], w[3]);
+}
+
+__global__ void __launch_bounds__(kThreadsPerCta, MODK_MIN_CTAS_FIND) find_batch_kernel(const __grid_constant__ FindArgs f)
+{
+    constexpr int U = kUnroll;
+    constexpr uint32_t T = (uint32_t)kThreadsPerCta;
+    // the tile, its halo, and one word of slack for the filter's second word
+    __shared__ __align__(16) uint32_t s_w[(kTileBytes + 16u * kHaloChunks) / 4u + 4u];
+    const uint32_t tid = threadIdx.x;
+    uint32_t pw[U];
+    load_chunk_pows<U>(pw, tid);
+    const uint4* rp = reinterpret_cast<const uint4*>(f.tiles + blockIdx.x);
+    const uint4 lo = __ldg(rp);
+    const uint4 hi = __ldg(rp + 1);
+    const int64_t src_rel = (int64_t)((uint64_t)lo.x | ((uint64_t)lo.y << 32));
+    const uint32_t st = hi.x, geom = hi.y, entry = hi.z;
+    const uint32_t n_valid = geom & 0xFFFu, head = (geom >> 12) & 15u, tail = (geom >> 16) & 31u;
+    const uint32_t end = 16u * (n_valid - 1u) + tail;  // tile-local end of the entry's bytes
+    const uint32_t halo = min(hi.w, f.len - 1u);       // entry bytes past the tile a match can reach
+    const uint64_t src_tile = (uint64_t)f.src + (uint64_t)src_rel;
+    const bool whole = src_tile >= f.src_lo16 && src_tile + 16ull * n_valid <= f.src_hi16;  // CTA-uniform
+
+    auto load_chunk = [&](uint32_t idx) {
+        return whole ? ldg128(src_tile + 16ull * idx)
+                     : load_bytes(src_tile + 16ull * idx, idx == 0u ? head : 0u, idx + 1u == n_valid ? tail : 16u);
+    };
+    uint4 d[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+        const uint32_t idx = tid + (uint32_t)u * T;
+        d[u] = make_uint4(0u, 0u, 0u, 0u);
+        if (idx < n_valid)
+            d[u] = load_chunk(idx);
+    }
+    // the halo: exact keystream, byte loads (it ends inside the entry, wherever the granule does)
+    if (tid < (uint32_t)kHaloChunks && 16u * tid < halo) {
+        const uint4 h = load_bytes(src_tile + 16ull * (n_valid + tid), 0u, min(16u, halo - 16u * tid));
+        const uint4 o = cycle_chunk_exact(h, jump_lazy(st, c_halo_pow2[tid]), f.two);
+        reinterpret_cast<uint4*>(s_w)[n_valid + tid] = o;
+    }
+
+    uint32_t s[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u)
+        s[u] = jump_lazy(st, pw[u]);
+    uint32_t any = 0u;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+#pragma unroll
+        for (int u = 0; u < U; ++u) {
+            const uint32_t b0 = step_lazy(s[u]);
+            const uint32_t b1 = step_lazy(b0);
+            const uint32_t b2 = step_lazy(b1);
+            const uint32_t b3 = step_lazy(b2);
+            s[u] = b3;
+            const uint32_t l = __byte_perm(b0, b1, 0x7340);
+            const uint32_t h = __byte_perm(b2, b3, 0x7340);
+            any |= l | h;
+            const uint32_t ks = __byte_perm(l, h, 0x5410);
+            if (j == 0) d[u].x ^= ks;
+            if (j == 1) d[u].y ^= ks;
+            if (j == 2) d[u].z ^= ks;
+            if (j == 3) d[u].w ^= ks;
+        }
+    }
+    if (__builtin_expect((any & 0x80800000u) != 0u, 0)) {
+        // some state needed a canonical subtract: redo this thread's chunks exactly from their source
+#pragma unroll 1
+        for (int u = 0; u < U; ++u) {
+            const uint32_t idx = tid + (uint32_t)u * T;
+            if (idx < n_valid)
+                reinterpret_cast<uint4*>(s_w)[idx] =
+                    cycle_chunk_exact(load_chunk(idx), jump_lazy(st, __ldg(&g_chunk_pow2[idx])), f.two);
+        }
+    } else {
+#pragma unroll
+        for (int u = 0; u < U; ++u) {
+            const uint32_t idx = tid + (uint32_t)u * T;
+            if (idx < n_valid)
+                reinterpret_cast<uint4*>(s_w)[idx] = d[u];
+        }
+    }
+    __syncthreads();
+
+    // start positions [head, p_end): inside the tile's part of the entry, with room for the whole pattern
+    const int32_t reach = (int32_t)(end + halo) - (int32_t)f.len + 1;
+    const uint32_t p_end = (uint32_t)max(0, min((int32_t)end, reach));
+    // Filter, 4 starts per word: a SWAR zero-byte test of (bytes ^ pattern[0]) AND-ed with the same test of the
+    // next bytes ^ pattern[1] (L >= 2).  It flags every start whose first two bytes match (false positives only
+    // above a matching byte), about 2 instructions per byte; the flagged starts are then compared exactly.
+    const uint8_t* sb = reinterpret_cast<const uint8_t*>(s_w);
+    const bool two_bytes = f.len > 1u;
+    for (uint32_t w = (head >> 2) + tid; 4u * w < p_end; w += T) {
+        const uint32_t x = s_w[w], y = s_w[w + 1u];
+        const uint32_t v0 = x ^ f.rep0;
+        uint32_t m = (v0 - 0x01010101u) & ~v0;
+        if (two_bytes) {
+            const uint32_t v1 = __funnelshift_r(x, y, 8u) ^ f.rep1;
+            m &= (v1 - 0x01010101u) & ~v1;
+        }
+        if (__builtin_expect((m & 0x80808080u) == 0u, 1))
+            continue;
+#pragma unroll 1
+        for (uint32_t o = 0; o < 4u; ++o) {
+            const uint32_t p = 4u * w + o;
+            if (((__funnelshift_r(x, y, 8u * o) ^ f.head_word) & f.head_mask) != 0u || p < head || p >= p_end)
+                continue;
+            bool hit = true;
+            for (uint32_t k = 4u; k < f.len && hit; ++k)
+                hit = sb[p + k] == f.pattern[k];
+            if (hit)
+                find_record(f, entry, src_rel, p);
+        }
+    }
+}
+
 // ---- host side --------------------------------------------------------------------------------------
 
 cudaError_t upload_tables()
 {
-    static uint32_t h_tw0[kTw0Size], h_tw1[kTw1Size], h_ainv[16], h_chunk[kChunksPerTile];
+    static uint32_t h_tw0[kTw0Size], h_tw1[kTw1Size], h_ainv[16], h_chunk[kChunksPerTile], h_halo[kHaloChunks];
     static const bool built = []() {
         for (int j = 0; j < kTw0Size; ++j)
             h_tw0[j] = modlcg::pow_a((uint64_t)kTileBytes * (uint64_t)j);
@@ -619,6 +773,8 @@ cudaError_t upload_tables()
             h_ainv[h] = modlcg::pow_a_inv((uint64_t)h);
         for (int j = 0; j < kChunksPerTile; ++j)
             h_chunk[j] = 2u * modlcg::pow_a(16ull * (uint64_t)j);
+        for (int k = 0; k < kHaloChunks; ++k)
+            h_halo[k] = 2u * modlcg::pow_a(16ull * (uint64_t)(kChunksPerTile + k));
         return true;
     }();  // thread-safe: several device workers may call this at once
     (void)built;
@@ -627,6 +783,7 @@ cudaError_t upload_tables()
     if ((err = cudaMemcpyToSymbol(c_tw1, h_tw1, sizeof(h_tw1))) != cudaSuccess) return err;
     if ((err = cudaMemcpyToSymbol(c_ainv, h_ainv, sizeof(h_ainv))) != cudaSuccess) return err;
     if ((err = cudaMemcpyToSymbol(g_chunk_pow2, h_chunk, sizeof(h_chunk))) != cudaSuccess) return err;
+    if ((err = cudaMemcpyToSymbol(c_halo_pow2, h_halo, sizeof(h_halo))) != cudaSuccess) return err;
     return cudaSuccess;
 }
 
@@ -669,6 +826,22 @@ cudaError_t launch_batch_inline(const BatchArgs& args, const InlineDescs& descs,
     else
         cycle_inline_kernel<true><<<args.n_tiles, kThreadsPerCta, 0, stream>>>(args, descs);
     return cudaGetLastError();
+}
+
+cudaError_t launch_find(const FindArgs& args, cudaStream_t stream)
+{
+    for (uint32_t t0 = 0; t0 < args.n_tiles;) {
+        const uint32_t n = args.n_tiles - t0 < kMaxGrid ? args.n_tiles - t0 : kMaxGrid;
+        FindArgs a = args;
+        a.tiles = args.tiles + t0;
+        a.n_tiles = n;
+        find_batch_kernel<<<n, kThreadsPerCta, 0, stream>>>(a);
+        const cudaError_t err = cudaGetLastError();
+        if (err != cudaSuccess)
+            return err;
+        t0 += n;
+    }
+    return cudaSuccess;
 }
 
 cudaError_t launch_build_tiles(const DevDesc* descs, uint32_t n_descs, uint32_t dst_align, TileRec* tiles,

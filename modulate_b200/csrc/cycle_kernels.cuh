@@ -40,8 +40,8 @@ struct __align__(16) TileRec {
     int64_t dst_rel;   // destination byte (relative to the dst base) of chunk 0; base + dst_rel is 16-byte aligned
     uint32_t state;    // negated LCG state just before byte 0 of chunk 0
     uint32_t geom;     // bits 0-11: chunks in the tile; 12-15: first valid byte of chunk 0; 16-20: valid bytes of the last chunk
-    uint32_t entry;    // descriptor index (diagnostics)
-    uint32_t pad;
+    uint32_t entry;    // descriptor index (the search kernel's counts and matches)
+    uint32_t rest;     // bytes of the entry after this tile: bounds the search kernel's halo
 };
 
 __host__ __device__ inline uint32_t pack_geom(uint32_t n_valid, uint32_t head, uint32_t tail)
@@ -68,6 +68,28 @@ struct BatchArgs {
     int32_t uniform_delta = -1;
 };
 
+// Search launch (find_batch_kernel): one CTA per tile of a plan whose chunk grid is co-aligned with the
+// source (built with dst_off == src_off and dst_align == source address & 15), nothing stored.
+constexpr uint32_t kMaxPattern = 64;
+constexpr int kHaloChunks = (int)((kMaxPattern - 1 + 15) / 16);  // chunks past a tile a match may reach into
+struct FindArgs {
+    const uint8_t* src;    // virtual base: src + TileRec::src_rel is 16-byte aligned
+    const TileRec* tiles;
+    const DevDesc* descs;  // the plan's descriptors: a match's position is relative to its entry's src_off
+    uint32_t n_tiles;
+    uint64_t src_lo16, src_hi16;  // as in BatchArgs
+    uint32_t* counts;             // per descriptor, accumulated
+    uint2* matches;               // {descriptor, position}: slots [0, cap) of the list
+    unsigned long long* total;    // accumulated; also hands out list slots
+    uint64_t cap;
+    uint32_t len;        // pattern bytes, 1..kMaxPattern
+    uint32_t head_word;  // first min(4, len) pattern bytes, little-endian
+    uint32_t head_mask;  // which bytes of head_word take part
+    uint32_t rep0, rep1; // pattern[0] and pattern[1] (0 if len == 1) in every byte: the search filter
+    uint32_t two = 2;
+    uint8_t pattern[kMaxPattern];
+};
+
 // Number of tiles an entry of `len` bytes occupies when its first destination byte sits at
 // (address & 15) == h0.
 __host__ __device__ inline uint32_t tiles_for_entry(uint32_t h0, uint32_t len)
@@ -81,6 +103,7 @@ __host__ __device__ inline uint32_t tiles_for_entry(uint32_t h0, uint32_t len)
 cudaError_t upload_tables();  // jump tables -> __constant__ / global memory of the current device
 cudaError_t launch_batch(const BatchArgs& args, cudaStream_t stream);
 cudaError_t launch_batch_inline(const BatchArgs& args, const InlineDescs& descs, cudaStream_t stream);
+cudaError_t launch_find(const FindArgs& args, cudaStream_t stream);
 // Plan kernel: expands descriptors into per-tile records (binary search + jump-ahead per tile).
 cudaError_t launch_build_tiles(const DevDesc* descs, uint32_t n_descs, uint32_t dst_align, TileRec* tiles,
                                uint32_t n_tiles, cudaStream_t stream);

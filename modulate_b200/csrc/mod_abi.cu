@@ -843,6 +843,8 @@ struct mod_plan {
     int32_t uniform_delta = -1;  // (src_off - dst_off) & 15 if all entries agree: selects the co-aligned kernel
     modk::TileRec* d_tiles = nullptr;
     uint64_t d_tiles_bytes = 0;         // size of the pool block behind d_tiles
+    modk::DevDesc* d_descs = nullptr;   // the descriptors in HBM: the search kernel reads a match's src_off there
+    uint64_t d_descs_bytes = 0;
     std::vector<mod_desc> descs;        // host copy: window validation, tile ranges
     std::vector<uint32_t> first_tile;   // n + 1 entries
 };
@@ -1095,10 +1097,8 @@ int mod_plan_create(const mod_desc* descs, uint64_t n, uint64_t src_bytes, uint6
     p->payload = payload;
     p->n_tiles = (uint32_t)tiles;
     p->uniform_delta = uniform_delta_of(descs, n);
-    modk::DevDesc* d_descs = nullptr;  // only needed while the tile records are built
-    uint64_t d_descs_bytes = 0;
     auto cleanup = [&]() {
-        pool_free(*c, d_descs, d_descs_bytes);
+        pool_free(*c, p->d_descs, p->d_descs_bytes);
         pool_free(*c, p->d_tiles, p->d_tiles_bytes);
         delete p;
     };
@@ -1113,7 +1113,7 @@ int mod_plan_create(const mod_desc* descs, uint64_t n, uint64_t src_bytes, uint6
         throw;
     }
     if (n && tiles) {
-        cudaError_t e = pool_alloc(*c, n * sizeof(modk::DevDesc), (void**)&d_descs, &d_descs_bytes);
+        cudaError_t e = pool_alloc(*c, n * sizeof(modk::DevDesc), (void**)&p->d_descs, &p->d_descs_bytes);
         if (e == cudaSuccess)
             e = pool_alloc(*c, tiles * sizeof(modk::TileRec), (void**)&p->d_tiles, &p->d_tiles_bytes);
         if (e != cudaSuccess) {
@@ -1121,9 +1121,9 @@ int mod_plan_create(const mod_desc* descs, uint64_t n, uint64_t src_bytes, uint6
             cleanup();
             return fail(MOD_ERR_NOMEM, "mod_plan_create: cudaMalloc failed: %s", cudaGetErrorString(e));
         }
-        e = cudaMemcpy(d_descs, host.data(), n * sizeof(modk::DevDesc), cudaMemcpyHostToDevice);
+        e = cudaMemcpy(p->d_descs, host.data(), n * sizeof(modk::DevDesc), cudaMemcpyHostToDevice);
         if (e == cudaSuccess) {
-            e = modk::launch_build_tiles(d_descs, (uint32_t)n, dst_align, p->d_tiles, p->n_tiles, nullptr);
+            e = modk::launch_build_tiles(p->d_descs, (uint32_t)n, dst_align, p->d_tiles, p->n_tiles, nullptr);
             g_launches.fetch_add(1, std::memory_order_relaxed);
         }
         if (e == cudaSuccess)
@@ -1132,8 +1132,6 @@ int mod_plan_create(const mod_desc* descs, uint64_t n, uint64_t src_bytes, uint6
             cleanup();
             return fail(MOD_ERR_CUDA, "mod_plan_create: %s", cudaGetErrorString(e));
         }
-        pool_free(*c, d_descs, d_descs_bytes);
-        d_descs = nullptr;
     }
     *out = p;
     return MOD_OK;
@@ -1144,14 +1142,16 @@ int mod_plan_destroy(mod_plan* plan)
 {
     if (!plan)
         return MOD_OK;
-    if (plan->d_tiles) {
+    if (plan->d_tiles || plan->d_descs) {
         DeviceGuard guard;
         guard.enter(plan->device);
         cudaDeviceSynchronize();  // launches that still read the records finish first (what cudaFree used to guarantee)
-        if (plan->device >= 0 && plan->device < kMaxDevices)
-            pool_free(g_dev[plan->device], plan->d_tiles, plan->d_tiles_bytes);  // back to the device's block pool
-        else
-            cudaFree(plan->d_tiles);
+        for (auto blk : {std::make_pair((void*)plan->d_tiles, plan->d_tiles_bytes), std::make_pair((void*)plan->d_descs, plan->d_descs_bytes)}) {
+            if (plan->device >= 0 && plan->device < kMaxDevices)
+                pool_free(g_dev[plan->device], blk.first, blk.second);  // back to the device's block pool
+            else if (blk.first)
+                cudaFree(blk.first);
+        }
     }
     delete plan;
     return MOD_OK;
@@ -1258,6 +1258,156 @@ int mod_plan_run_window(const mod_plan* plan, uint64_t tile_begin, uint64_t tile
     CUDA_TRY(modk::launch_batch(args, (cudaStream_t)stream));
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return MOD_OK;
+}
+
+// Argument checks and the launch shared by mod_plan_find and mod_plan_find_window; `src_base` is the virtual
+// base (source byte 0 of the plan's space) and [lo16, hi16) the granules that may be loaded whole.
+static int plan_find_launch(const char* who, const mod_plan* plan, uint64_t tile_begin, uint64_t tile_end,
+                            const uint8_t* src_base, uint64_t lo16, uint64_t hi16, const uint8_t* pattern, uint32_t len,
+                            uint32_t* d_counts, mod_match* d_matches, uint64_t cap, uint64_t* d_total, void* stream)
+{
+    if (!pattern || len == 0 || len > modk::kMaxPattern)
+        return fail(MOD_ERR_ARG, "%s: the pattern must be 1 to %u bytes", who, modk::kMaxPattern);
+    if (tile_begin == tile_end)
+        return MOD_OK;
+    if (!d_counts || !d_total || (cap && !d_matches))
+        return fail(MOD_ERR_ARG, "%s: null result buffer", who);
+    // the search kernel needs the chunk grid on the source: src_off - dst_off == delta for every entry and
+    // base + delta - dst_align == 0 (mod 16)
+    if (plan->uniform_delta < 0 || (((uintptr_t)src_base + (uintptr_t)plan->uniform_delta - plan->dst_align) & 15u) != 0u)
+        return fail(MOD_ERR_ALIGN, "%s: the plan's chunk grid does not lie on the source (build it with dst_off == src_off "
+                    "and dst_align == source address & 15)", who);
+    int rc = plan_check_device(plan, who);
+    if (rc != MOD_OK)
+        return rc;
+    modk::FindArgs f;
+    f.src = src_base;
+    f.tiles = plan->d_tiles + tile_begin;
+    f.descs = plan->d_descs;
+    f.n_tiles = (uint32_t)(tile_end - tile_begin);
+    f.src_lo16 = lo16;
+    f.src_hi16 = hi16;
+    f.counts = d_counts;
+    f.matches = (uint2*)d_matches;
+    f.total = (unsigned long long*)d_total;
+    f.cap = cap;
+    f.len = len;
+    f.head_word = 0;
+    f.head_mask = 0;
+    for (uint32_t k = 0; k < 4 && k < len; ++k) {
+        f.head_word |= (uint32_t)pattern[k] << (8 * k);
+        f.head_mask |= 0xFFu << (8 * k);
+    }
+    f.rep0 = 0x01010101u * pattern[0];
+    f.rep1 = len > 1 ? 0x01010101u * pattern[1] : 0u;
+    std::memset(f.pattern, 0, sizeof(f.pattern));
+    std::memcpy(f.pattern, pattern, len);
+    CUDA_TRY(modk::launch_find(f, (cudaStream_t)stream));
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    return MOD_OK;
+}
+
+int mod_plan_find(const mod_plan* plan, const void* d_src, const uint8_t* pattern, uint32_t len, uint32_t* d_counts,
+                  mod_match* d_matches, uint64_t cap, uint64_t* d_total, void* stream)
+{
+    if (!plan)
+        return fail(MOD_ERR_ARG, "mod_plan_find: null plan");
+    if (!d_src && plan->n_tiles)
+        return fail(MOD_ERR_ARG, "mod_plan_find: null buffer");
+    return plan_find_launch("mod_plan_find", plan, 0, plan->n_tiles, (const uint8_t*)d_src,
+                            ((uint64_t)(uintptr_t)d_src + 15u) & ~15ull, ((uint64_t)(uintptr_t)d_src + plan->src_bytes) & ~15ull,
+                            pattern, len, d_counts, d_matches, cap, d_total, stream);
+}
+
+int mod_plan_find_window(const mod_plan* plan, uint64_t tile_begin, uint64_t tile_end, const void* d_src_win,
+                         uint64_t src_win_off, uint64_t src_win_bytes, const uint8_t* pattern, uint32_t len,
+                         uint32_t* d_counts, mod_match* d_matches, uint64_t cap, uint64_t* d_total, void* stream)
+{
+    if (!plan)
+        return fail(MOD_ERR_ARG, "mod_plan_find_window: null plan");
+    if (tile_begin > tile_end || tile_end > plan->n_tiles)
+        return fail(MOD_ERR_ARG, "mod_plan_find_window: tiles [%llu, %llu) outside the plan's %u",
+                    (unsigned long long)tile_begin, (unsigned long long)tile_end, plan->n_tiles);
+    if (!pattern || len == 0 || len > modk::kMaxPattern)
+        return fail(MOD_ERR_ARG, "mod_plan_find_window: the pattern must be 1 to %u bytes", modk::kMaxPattern);
+    if (tile_begin < tile_end && !d_src_win)
+        return fail(MOD_ERR_ARG, "mod_plan_find_window: null buffer");
+    // every byte the tile range reads, halos included, must lie inside the window
+    const uint32_t* ft = plan->first_tile.data();
+    uint64_t e = tile_begin < tile_end ? (uint64_t)(std::upper_bound(ft, ft + plan->n + 1, (uint32_t)tile_begin) - ft) - 1 : plan->n;
+    for (; e < plan->n && ft[e] < tile_end; ++e) {
+        const mod_desc& d = plan->descs[e];
+        if (ft[e + 1] == ft[e])
+            continue;  // empty entry
+        const uint32_t h0 = (uint32_t)((plan->dst_align + d.dst_off) & 15u);
+        const uint64_t ta = std::max<uint64_t>(tile_begin, ft[e]) - ft[e], tb = std::min<uint64_t>(tile_end, ft[e + 1]) - ft[e];
+        const uint64_t b0 = ta == 0 ? 0 : ta * modk::kTileBytes - h0;
+        const uint64_t b1 = std::min<uint64_t>(d.len, tb * modk::kTileBytes - h0 + (len - 1));
+        if (d.src_off + b0 < src_win_off || d.src_off + b1 > src_win_off + src_win_bytes)
+            return fail(MOD_ERR_ARG, "mod_plan_find_window: entry %llu reads outside the source window", (unsigned long long)e);
+    }
+    return plan_find_launch("mod_plan_find_window", plan, tile_begin, tile_end, (const uint8_t*)d_src_win - src_win_off,
+                            ((uint64_t)(uintptr_t)d_src_win + 15u) & ~15ull,
+                            ((uint64_t)(uintptr_t)d_src_win + src_win_bytes) & ~15ull, pattern, len, d_counts, d_matches,
+                            cap, d_total, stream);
+}
+
+int mod_find_batch(const mod_desc* descs, uint64_t n, const void* d_src, uint64_t src_bytes, const uint8_t* pattern,
+                   uint32_t len, uint32_t* counts_out, mod_match* matches_out, uint64_t cap, uint64_t* total_out)
+{
+    MOD_ABI_BEGIN
+    if (!pattern || len == 0 || len > modk::kMaxPattern)
+        return fail(MOD_ERR_ARG, "mod_find_batch: the pattern must be 1 to %u bytes", modk::kMaxPattern);
+    if ((n && (!descs || !counts_out)) || !total_out || (cap && !matches_out))
+        return fail(MOD_ERR_ARG, "mod_find_batch: null argument");
+    int src_dev = -1;
+    if (!d_src || !pointer_device(d_src, &src_dev))
+        return fail(MOD_ERR_ARG, "mod_find_batch: d_src must be device memory (stream host data with CArk::FindInFiles)");
+    DeviceGuard guard;
+    int rc = guard.enter(src_dev);
+    if (rc != MOD_OK)
+        return rc;
+    std::vector<mod_desc> own(descs, descs + n);
+    for (mod_desc& d : own)
+        d.dst_off = d.src_off;
+    mod_plan* plan = nullptr;
+    if ((rc = mod_plan_create(own.data(), n, src_bytes, src_bytes, (uint32_t)((uintptr_t)d_src & 15u), &plan)) != MOD_OK)
+        return rc;
+    // one allocation: total, counts, list
+    const uint64_t counts_at = 16, list_at = (counts_at + 4 * n + 15) & ~15ull, bytes = list_at + 8 * cap;
+    uint8_t* d_out = nullptr;
+    cudaError_t e = cudaMalloc((void**)&d_out, bytes);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        mod_plan_destroy(plan);
+        return fail(MOD_ERR_NOMEM, "mod_find_batch: cudaMalloc(%llu): %s", (unsigned long long)bytes, cudaGetErrorString(e));
+    }
+    e = cudaMemsetAsync(d_out, 0, list_at, nullptr);
+    if (e == cudaSuccess)
+        rc = mod_plan_find(plan, d_src, pattern, len, (uint32_t*)(d_out + counts_at), (mod_match*)(d_out + list_at), cap,
+                           (uint64_t*)d_out, nullptr);
+    uint64_t total = 0;
+    if (e == cudaSuccess && rc == MOD_OK)
+        e = cudaMemcpyAsync(&total, d_out, 8, cudaMemcpyDeviceToHost, nullptr);
+    if (e == cudaSuccess && rc == MOD_OK && n)
+        e = cudaMemcpyAsync(counts_out, d_out + counts_at, 4 * n, cudaMemcpyDeviceToHost, nullptr);
+    if (e == cudaSuccess && rc == MOD_OK)
+        e = cudaStreamSynchronize(nullptr);
+    const uint64_t kept = std::min(total, cap);
+    if (e == cudaSuccess && rc == MOD_OK && kept)
+        e = cudaMemcpyAsync(matches_out, d_out + list_at, 8 * kept, cudaMemcpyDeviceToHost, nullptr);
+    if (e == cudaSuccess && rc == MOD_OK)
+        e = cudaStreamSynchronize(nullptr);
+    cudaFree(d_out);
+    mod_plan_destroy(plan);
+    if (rc != MOD_OK)
+        return rc;
+    CUDA_TRY(e);
+    std::sort(matches_out, matches_out + kept,
+              [](const mod_match& a, const mod_match& b) { return a.desc != b.desc ? a.desc < b.desc : a.pos < b.pos; });
+    *total_out = total;
+    return MOD_OK;
+    MOD_ABI_END("mod_find_batch")
 }
 
 int mod_cycle_batch(const mod_desc* descs, uint64_t n, const void* src, uint64_t src_bytes, void* dst,
