@@ -65,7 +65,14 @@ def pow_a_inv(e: int) -> int:
     return pow_a((M - 1) - e % (M - 1))
 
 
-CHUNK_POW2 = np.array([2 * pow_a(16 * j) for j in range(CHUNKS)], dtype=np.uint64)  # g_chunk_pow2
+MAX_PATTERN = _parse("cycle_kernels.cuh", r"kMaxPattern = (\d+);")  # the search's longest pattern
+if not re.search(r"kHaloChunks = \(int\)\(\(kMaxPattern - 1 \+ 15\) / 16\);",
+                 open(os.path.join(_CSRC, "cycle_kernels.cuh")).read()):
+    raise RuntimeError("kHaloChunks changed in cycle_kernels.cuh: the kernel model no longer matches the kernel")
+HALO_CHUNKS = (MAX_PATTERN - 1 + 15) // 16  # kHaloChunks: chunks past a tile a match may reach into
+
+# g_chunk_pow2, then c_halo_pow2: halo chunk k of a tile is stream chunk CHUNKS + k of the tile state
+CHUNK_POW2 = np.array([2 * pow_a(16 * j) for j in range(CHUNKS + HALO_CHUNKS)], dtype=np.uint64)
 
 
 def i32(key: int) -> int:
@@ -724,3 +731,603 @@ def entries_with_trigger_bytes(descs, dst_align: int = 0, tiles_per_pass: int = 
                     hit[r.entry] = True
                     break
     return np.nonzero(hit)[0]
+
+
+# ==== search: find_batch_kernel ===========================================================================
+# One CTA per tile of a plan whose chunk grid lies on the source (dst_off == src_off, dst_align == source
+# address & 15).  The CTA loads its chunks (whole granules when the tile lies inside the source bounds, else byte
+# loads that zero-fill every byte that is not the entry's), deciphers them with the speculative keystream (exact
+# for a thread that takes the redo: any of its 4 rounds' states had bit 31 set), deciphers the halo -- the next
+# min(rest, L - 1) bytes of the entry -- exactly with byte loads, and tests the starts [head, p_end).  The model
+# restates that per tile; emulate_find_tile replays the shared-memory tile in numpy, with switches that drop
+# one guard at a time.  tests/test_gpu_find_paths.py runs one case per (kind, load path, cell) on the GPU.
+
+def tile_rest(r: TileRec) -> int:
+    """make_tile_rec's `rest`: bytes of the entry after the tile (0 for its last tile)."""
+    span = r.h0 + r.length
+    c_end = r.tin * CHUNKS + r.n_valid
+    return 0 if c_end == (span + 15) >> 4 else span - 16 * c_end
+
+
+@dataclass
+class FindLaunch:
+    src: int    # FindArgs::src, the virtual base: a window's address minus its offset
+    lo16: int
+    hi16: int
+    tiles: List[TileRec]
+
+
+def _grid_descs(descs):
+    return [(so, so, ln, key) for so, ln, key in descs]
+
+
+def find_batch_launch(descs, src: int, src_bytes: int) -> FindLaunch:
+    """mod_find_batch on (src_off, len, key) descriptors: dst_off = src_off, dst_align = src & 15, and the
+    whole source buffer bounds the whole-granule loads."""
+    return FindLaunch(src, (src + 15) & ~15, (src + src_bytes) & ~15, plan_tiles(_grid_descs(descs), src & 15))
+
+
+def find_window_launch(descs, dst_align: int, t0: int, t1: int, win: int, win_off: int, win_bytes: int) -> FindLaunch:
+    """mod_plan_find_window: tiles [t0, t1) of the plan, the window bounds the loads."""
+    return FindLaunch(win - win_off, (win + 15) & ~15, (win + win_bytes) & ~15,
+                      plan_tiles(_grid_descs(descs), dst_align)[t0:t1])
+
+
+def find_window_ok(descs, dst_align: int, t0: int, t1: int, win_off: int, win_bytes: int, L: int) -> bool:
+    """mod_plan_find_window's host check: every entry byte the tiles read, halos included, lies in the window."""
+    ft = plan_first_tiles(_grid_descs(descs), dst_align)
+    for e, (so, ln, _) in enumerate(descs):
+        if ft[e + 1] == ft[e] or ft[e + 1] <= t0 or ft[e] >= t1:
+            continue
+        h0 = (dst_align + so) & 15
+        ta, tb = max(t0, ft[e]) - ft[e], min(t1, ft[e + 1]) - ft[e]
+        b0 = 0 if ta == 0 else ta * TILE_BYTES - h0
+        b1 = min(ln, tb * TILE_BYTES - h0 + L - 1)
+        if so + b0 < win_off or so + b1 > win_off + win_bytes:
+            return False
+    return True
+
+
+GUARDS = ("head", "reach", "halo", "tile")
+
+
+def scan_bounds(r: TileRec, L: int, guards=GUARDS) -> Tuple[int, int, int]:
+    """(halo, first start, p_end) of the kernel, with the guards not in `guards` dropped:
+    head  -- `p < head`: without it the scan starts at the word that holds `head`;
+    reach -- p_end <= end + halo - L + 1: without it p_end = end;
+    halo  -- halo = min(rest, L - 1): without it the halo is L - 1 bytes whether or not the entry has them;
+    tile  -- p_end <= end, with the halo at most L - 1: without it the halo holds what it can of the entry
+             (up to HALO_CHUNKS chunks) and the tile also takes the starts that fit in it."""
+    rest = tile_rest(r)
+    end = 16 * (r.n_valid - 1) + r.tail
+    if "tile" not in guards:
+        halo = min(rest, 16 * HALO_CHUNKS)
+    else:
+        halo = min(rest, L - 1) if "halo" in guards else L - 1
+    reach = end + halo - L + 1
+    if "reach" not in guards:
+        p_end = end
+    elif "tile" not in guards:
+        p_end = max(0, reach)
+    else:
+        p_end = max(0, min(end, reach))
+    return halo, (r.head if "head" in guards else r.head & ~3), p_end
+
+
+@dataclass
+class FindTile:
+    """One tile of a search launch as the kernel runs it, for a pattern of L bytes."""
+    rec: TileRec
+    L: int
+    whole: bool            # CTA-uniform: the chunks are loaded as whole granules
+    rest: int
+    halo: int
+    end: int               # tile-local end of the entry's bytes
+    p_end: int
+    trig: np.ndarray = field(repr=False)       # [UNROLL, THREADS, 16]: bit 31 set (all four rounds count)
+    redo: np.ndarray = field(repr=False)       # [THREADS]
+    halo_trig: np.ndarray = field(repr=False)  # [HALO_CHUNKS, 16]
+
+    @property
+    def path(self) -> str:
+        return "whole" if self.whole else "bytes"
+
+    def halo_loaded(self) -> List[Tuple[int, int]]:
+        """(halo chunk, bytes loaded from the source; the rest of the chunk is zero-filled) of every written
+        halo chunk.  Chunks past the halo are never written: they hold stale shared memory."""
+        return [(k, min(16, self.halo - 16 * k)) for k in range(HALO_CHUNKS) if 16 * k < self.halo]
+
+    def compared(self, idx: int) -> Tuple[int, int]:
+        """Bytes [lo, hi) of tile chunk `idx` that some start's window covers (lo == hi: none)."""
+        a = self.rec.head
+        b = min(self.end, self.p_end + self.L - 1) if self.p_end > a else a
+        lo, hi = max(a, 16 * idx) - 16 * idx, min(b, 16 * idx + 16) - 16 * idx
+        return (lo, hi) if hi > lo else (0, 0)
+
+    def cells(self) -> Set[str]:
+        """The redo and halo cells this tile hits with its key (see FIND_CELLS)."""
+        out = set() if self.redo.any() else {"none"}
+        n, T = self.rec.n_valid, THREADS
+        compared_threads = set()
+        for u, t, b in zip(*np.nonzero(self.trig)):
+            u, t, b = int(u), int(t), int(b)
+            idx = u * T + t
+            lo, hi = self.compared(idx)
+            if lo <= b < hi:
+                compared_threads.add(t)
+                if idx == 0 and self.rec.head:
+                    out.add("head")
+                if idx + 1 == n and self.rec.tail < 16:
+                    out.add("tail")
+                if (lo, hi) == (0, 16):
+                    out.add("interior")
+                if u == UNROLL - 1:
+                    out.add("last-round")
+            elif idx >= n and t < n:
+                out.add("ghost")
+        if len(compared_threads) >= 2:
+            out.add("double")
+        for k, nb in self.halo_loaded():
+            if self.halo_trig[k, :nb].any():
+                out.add(f"halo{k}")
+        return out
+
+
+def model_find_tile(launch: FindLaunch, r: TileRec, L: int, keyed: bool = True) -> FindTile:
+    """keyed=False: geometry only (no trigger is computed)."""
+    src_tile = launch.src + r.src_rel
+    assert src_tile % 16 == 0, "the plan's chunk grid is not on the source"
+    whole = src_tile >= launch.lo16 and src_tile + 16 * r.n_valid <= launch.hi16
+    halo, _, p_end = scan_bounds(r, L)
+    if keyed:
+        trig = triggers(chunk_states(np.uint64(r.state), np.arange(CHUNKS + HALO_CHUNKS)))
+    else:
+        trig = np.zeros((CHUNKS + HALO_CHUNKS, 16), bool)
+    main = trig[:CHUNKS].reshape(UNROLL, THREADS, 16)
+    return FindTile(r, L, whole, tile_rest(r), halo, 16 * (r.n_valid - 1) + r.tail, p_end, main,
+                    main.any(axis=(0, 2)), trig[CHUNKS:])
+
+
+def find_keystream(r: TileRec) -> Tuple[np.ndarray, np.ndarray]:
+    """(speculative, exact) keystream bytes [CHUNKS + HALO_CHUNKS, 16] of every chunk the CTA may decipher, the
+    chunk-0 bytes before `head`, the last chunk's bytes after `tail` and the halo chunks included."""
+    s = chunk_states(np.uint64(r.state), np.arange(CHUNKS + HALO_CHUNKS))
+    return speculative_bytes(s), canonical_bytes(s)
+
+
+def _read(mem: np.ndarray, a: int, n: int) -> np.ndarray:
+    out = np.zeros(n, np.uint8)
+    lo, hi = max(a, 0), min(a + n, mem.size)
+    if hi > lo:
+        out[lo - a:hi - a] = mem[lo:hi]
+    return out
+
+
+def find_tile_bytes(launch: FindLaunch, r: TileRec, mem: np.ndarray, L: int, guards=GUARDS,
+                    redo: str = "exact") -> np.ndarray:
+    """The CTA's shared-memory tile (int16, -1 where never written) for source bytes `mem` (launch addresses
+    index it; bytes outside it read as zero, which only a dropped halo guard can load).  redo: "exact" (the
+    kernel), "off" (never redo) or "round0" (a redone chunk starts from round 0's state: g_chunk_pow2[tid])."""
+    ft = model_find_tile(launch, r, L)
+    halo = scan_bounds(r, L, guards)[0]
+    spec, exact = find_keystream(r)
+    tile = np.full(16 * (CHUNKS + HALO_CHUNKS) + 16, -1, np.int16)
+    src_tile = launch.src + r.src_rel
+    for idx in range(r.n_valid):
+        if ft.whole:
+            data = _read(mem, src_tile + 16 * idx, 16)
+        else:
+            lo, hi = r.stored(idx)
+            data = np.zeros(16, np.uint8)
+            data[lo:hi] = _read(mem, src_tile + 16 * idx + lo, hi - lo)
+        t = idx % THREADS
+        ks = spec[idx] if not ft.redo[t] or redo == "off" else exact[t if redo == "round0" else idx]
+        tile[16 * idx:16 * idx + 16] = data ^ ks
+    for k in range(HALO_CHUNKS):
+        if 16 * k < halo:
+            data = np.zeros(16, np.uint8)
+            nb = min(16, halo - 16 * k)
+            data[:nb] = _read(mem, src_tile + 16 * (r.n_valid + k), nb)
+            tile[16 * (r.n_valid + k):16 * (r.n_valid + k + 1)] = data ^ exact[CHUNKS + k]
+    return tile
+
+
+def emulate_find_tile(launch: FindLaunch, r: TileRec, mem: np.ndarray, pattern: bytes, guards=GUARDS,
+                      redo: str = "exact") -> List[int]:
+    """Tile-local starts the CTA reports.  With every guard on, no compared byte is stale (asserted)."""
+    L = len(pattern)
+    tile = find_tile_bytes(launch, r, mem, L, guards, redo)
+    _, lo, p_end = scan_bounds(r, L, guards)
+    if p_end <= lo:
+        return []
+    win = np.lib.stride_tricks.sliding_window_view(tile[lo:p_end + L - 1], L)
+    if set(guards) == set(GUARDS):
+        assert (win >= 0).all(), "a compared byte was never written"
+    return [lo + int(p) for p in np.nonzero((win == np.frombuffer(pattern, np.uint8)).all(axis=1))[0]]
+
+
+# ---- the search's cell matrix ------------------------------------------------------------------------------
+
+FIND_KINDS = ("batch", "window")
+FIND_PATHS = ("whole", "bytes")
+HALO_CELLS = tuple(f"halo{k}" for k in range(HALO_CHUNKS))
+GUARD_CELLS = ("before-head", "after-end", "past-rest", "across-tile")
+FIND_CELLS = TRIGGERS + HALO_CELLS + GUARD_CELLS
+GUARD_OF = {"before-head": "head", "after-end": "reach", "past-rest": "halo", "across-tile": "tile"}
+FIND_LENGTHS = (1, 2, 17, 64)
+
+
+def all_find_cells() -> List[Tuple[str, str, str]]:
+    return [(k, p, c) for k in FIND_KINDS for p in FIND_PATHS for c in FIND_CELLS]
+
+
+def find_unreachable_reason(kind: str, path: str, cell: str) -> Optional[str]:
+    """Why a search cell cannot occur, or None.  test_kernel_model checks every reason against the sweep."""
+    if cell.startswith("halo") and 16 * int(cell[4:]) >= MAX_PATTERN - 1:
+        return "the halo is at most kMaxPattern - 1 bytes"
+    return None
+
+
+def reachable_find_cells() -> Set[Tuple[str, str, str]]:
+    return {c for c in all_find_cells() if find_unreachable_reason(*c) is None}
+
+
+def _decoy_start(ft: FindTile, cell: str) -> Optional[int]:
+    """Tile-local start of the decoy a guard cell plants, or None if the geometry has no room for one."""
+    r, L = ft.rec, ft.L
+    if cell == "before-head":
+        p = r.head & ~3
+        return p if r.head & 3 and p < ft.p_end else None
+    if cell == "after-end":
+        p = max(r.head, ft.end - L + 1)
+        return p if ft.rest == 0 and L >= 2 and p < ft.end and p + L <= 16 * r.n_valid else None
+    if cell == "past-rest":
+        p = ft.end + ft.rest + 1 - L
+        return p if 0 < ft.rest < L - 1 and ft.rest % 16 and p >= r.head else None
+    if cell == "across-tile":  # the match [end - L + 1, end] ends in halo chunk 0; the decoy follows it
+        return ft.end + 1 if L >= 2 and ft.rest >= L + 1 and L + 1 <= 16 * HALO_CHUNKS else None
+    raise ValueError(cell)
+
+
+def find_geometric_cells(ft: FindTile) -> Set[str]:
+    """Cells some key (redo, halo) or decoy (guards) could reach in this tile: the geometry alone decides."""
+    r, n, T = ft.rec, ft.rec.n_valid, THREADS
+    out = {"none"}
+    lo = r.head
+    hi = min(ft.end, ft.p_end + ft.L - 1) if ft.p_end > lo else lo  # compared bytes [lo, hi), as FindTile.compared
+    if hi > lo:
+        c0, c1 = lo // 16, (hi - 1) // 16  # compared chunks c0..c1
+        if r.head and c0 == 0:
+            out.add("head")
+        if r.tail < 16 and c1 == n - 1:
+            out.add("tail")
+        if any(ft.compared(i) == (0, 16) for i in (c0, c0 + 1, c1 - 1, c1) if c0 <= i <= c1):
+            out.add("interior")
+        if c1 >= (UNROLL - 1) * T:
+            out.add("last-round")
+        if c1 > c0 and (c1 - c0 >= T or c0 % T != c1 % T):
+            out.add("double")
+        if n < CHUNKS and bool((np.arange(n, CHUNKS) % T < n).any()):
+            out.add("ghost")
+    out |= {f"halo{k}" for k, _ in ft.halo_loaded()}
+    out |= {c for c in GUARD_CELLS if _decoy_start(ft, c) is not None}
+    return out
+
+
+@dataclass
+class FindCase:
+    """One search launch over three entries (src_off, len, key) of a source image.  batch: the image sits
+    `src_ptr` bytes into a 16-byte aligned buffer.  window: tiles [t0, t1) of a plan with `dst_align` run over
+    image bytes [win_off, win_off + win_bytes), held `win_ptr` bytes into a buffer of their own."""
+    cell: Tuple[str, str, str]
+    kind: str
+    descs: List[Tuple[int, int, int]]
+    target: int
+    tin: int            # the target's tile the cell is built in
+    L: int
+    src_ptr: int
+    image_bytes: int
+    win: Optional[Tuple[int, int, int, int, int]] = None  # t0, t1, win_ptr, win_off, win_bytes
+    pattern: bytes = b""
+    image: Optional[np.ndarray] = field(default=None, repr=False)  # cipher bytes, built by make_find_case
+    decoys: List[int] = field(default_factory=list)               # tile-local starts of guard decoys
+
+    @property
+    def dst_align(self) -> int:
+        return (self.win[2] - self.win[3]) & 15 if self.win else self.src_ptr & 15
+
+    def launch(self) -> FindLaunch:
+        if self.win:
+            t0, t1, wp, wo, wb = self.win
+            return find_window_launch(self.descs, self.dst_align, t0, t1, wp, wo, wb)
+        return find_batch_launch(self.descs, self.src_ptr, self.image_bytes)
+
+    def memory(self) -> np.ndarray:
+        """The source allocation the kernel reads."""
+        if self.win:
+            _, _, wp, wo, wb = self.win
+            return np.concatenate([np.zeros(wp, np.uint8), self.image[wo:wo + wb]])
+        return np.concatenate([np.zeros(self.src_ptr, np.uint8), self.image])
+
+    def target_tile(self) -> Tuple[FindLaunch, TileRec]:
+        la = self.launch()
+        return la, next(r for r in la.tiles if r.entry == self.target and r.tin == self.tin)
+
+    def cells(self) -> Set[Tuple[str, str, str]]:
+        """Cells the case reaches in its target tile: the key's redo and halo cells, and each guard cell whose
+        decoy the case planted."""
+        la, r = self.target_tile()
+        ft = model_find_tile(la, r, self.L)
+        got = ft.cells()
+        if self.decoys:
+            got.add(self.cell[2])
+        return {(self.kind, ft.path, c) for c in got}
+
+    def entry_starts(self) -> Tuple[int, int]:
+        """Entry positions [lo, hi) of the starts the launch's tiles of the target own."""
+        la = self.launch()
+        so, ln, _ = self.descs[self.target]
+        tins = [r.tin for r in la.tiles if r.entry == self.target]
+        h0 = (self.dst_align + so) & 15
+        return max(0, TILE_BYTES * min(tins) - h0), min(ln - self.L + 1, TILE_BYTES * (max(tins) + 1) - h0)
+
+
+_FIND_NEIGHBOURS = (37, 23)
+
+
+def _find_layout(kind: str, h0: int, length: int, place: str, L: int, sub: str) -> Optional[FindCase]:
+    """Entries [n0, target, n1] in a source image, the target at chunk-grid offset h0.  batch: place 'start' /
+    'end' puts the target against the start / end of the source buffer, 'mid' leaves room.  window: the image
+    always has room; `sub` picks the tile range ('all', or the target's 'first', 'last' or 'mid' tile) and
+    `place` puts the window's start ('start') or end ('end') exactly on the bytes the range reads."""
+    d0, d1 = _FIND_NEIGHBOURS
+    if kind == "batch" and place == "start":
+        src_ptr, tgt = h0, 0
+        s1 = length + 5
+        s0 = s1 + d1 + 3
+        image_bytes = s0 + d0 + 11
+    else:
+        src_ptr = (5 * h0 + length + 3 * L) & 15
+        s0 = 0
+        tgt = d0 + 4 + ((h0 - src_ptr - d0 - 4) & 15)
+        s1 = tgt + length
+        image_bytes = s1 + d1 + 29
+        if kind == "batch" and place == "end":
+            s1 = d0 + 2
+            tgt = s1 + d1 + ((h0 - src_ptr - s1 - d1) & 15)
+            image_bytes = tgt + length
+    descs = [(s0, d0, None), (tgt, length, None), (s1, d1, None)]
+    case = FindCase((kind, "", ""), kind, descs, 1, 0, L, src_ptr, image_bytes)
+    if kind == "batch":
+        return case
+    dst_align = (h0 - tgt) & 15
+    ft = plan_first_tiles(_grid_descs(descs), dst_align)
+    nt = ft[2] - ft[1]
+    ta, tb = {"all": (0, nt), "first": (0, 1), "last": (nt - 1, nt), "mid": (1, nt - 1)}[sub]
+    if tb <= ta or (sub != "all" and nt < 2) or (sub == "mid" and nt < 3):
+        return None
+    b0 = tgt + (0 if ta == 0 else ta * TILE_BYTES - h0)
+    b1 = tgt + min(length, tb * TILE_BYTES - h0 + L - 1)
+    lo = b0 if place == "start" else max(0, b0 - 19)
+    hi = b1 if place == "end" else min(image_bytes, b1 + 21)
+    case.win = (ft[1] + ta, ft[1] + tb, (lo + dst_align) & 15, lo, hi - lo)
+    case.src_ptr = 0
+    assert find_window_ok(descs, dst_align, ft[1] + ta, ft[1] + tb, lo, hi - lo, L)
+    return case
+
+
+def _find_lengths(h0: int, L: int) -> List[int]:
+    out = set(range(1, 40)) | {3000, 5000, 7000}
+    for b in (TILE_BYTES, 2 * TILE_BYTES):
+        for d in (-L, 1 - L, 2 - L, -17, -16, -15, -2, -1, 0, 1, 2, 15, 16, 17, L - 2, L - 1, L, L + 1, 200):
+            out.add(b - h0 + d)
+    return sorted(x for x in out if x > 0)
+
+
+def _find_geometries(kind: str):
+    subs = ("all", "first", "last", "mid") if kind == "window" else ("all",)
+    for L in FIND_LENGTHS:
+        for h0 in range(16):
+            for length in _find_lengths(h0, L):
+                for place in ("mid", "start", "end"):
+                    for sub in subs:
+                        yield h0, length, place, L, sub
+
+
+@functools.lru_cache(maxsize=None)
+def _find_sweep(kind: str):
+    """(geometries, {cell: [(geometry index, target tile index)]}) of every geometry of `kind`."""
+    geoms, hits = [], {}
+    for g in _find_geometries(kind):
+        case = _find_layout(kind, *g)
+        if case is None:
+            continue
+        gi = len(geoms)
+        geoms.append(g)
+        la = case.launch()
+        for r in la.tiles:
+            if r.entry != case.target:
+                continue
+            ft = model_find_tile(la, r, g[3], keyed=False)
+            for c in find_geometric_cells(ft):
+                hits.setdefault((kind, ft.path, c), []).append((gi, r.tin))
+    return geoms, hits
+
+
+def enumerate_reachable_find(kind: str) -> Set[Tuple[str, str, str]]:
+    """Every search cell some geometry of `kind` makes possible: h0 0..15, lengths around every tile boundary
+    +- (L - 1), the entry against the start or end of its buffer (or window) or with room, L in FIND_LENGTHS, and
+    window ranges that start and end inside the entry."""
+    return set(_find_sweep(kind)[1])
+
+
+def _find_target_chunks(cell: str, ft: FindTile) -> List[Tuple[int, int, int]]:
+    """(chunk, byte_lo, byte_hi) to make trigger for a redo or halo cell: the redone thread should own a valid
+    chunk in a round > 0, so that a redo from round 0's state changes a compared byte."""
+    n, T = ft.rec.n_valid, THREADS
+    if cell.startswith("halo"):
+        k = int(cell[4:])
+        return [(CHUNKS + k, 0, dict(ft.halo_loaded())[k])]
+
+    def later(i):
+        return i % T + T < n
+
+    comp = [i for i in range(n) if ft.compared(i) != (0, 0)]
+    if cell == "ghost":
+        cand = sorted((c for c in range(n, CHUNKS) if c % T < n), key=lambda c: not later(c))
+        return [(c, 0, 16) for c in cand[:1]]
+    if cell in ("interior", "double", "none"):
+        cand = sorted((i for i in comp if ft.compared(i) == (0, 16)), key=lambda i: (not later(i), i // T != 1))
+    elif cell == "last-round":
+        cand = sorted((i for i in comp if i >= (UNROLL - 1) * T), key=lambda i: ft.compared(i) != (0, 16))
+    elif cell == "head":
+        cand = [0]
+    else:  # tail
+        cand = [n - 1]
+    return [(i, *ft.compared(i)) for i in cand[:1] if ft.compared(i) != (0, 0)]
+
+
+def _find_key(case: FindCase, rng) -> int:
+    kind, path, cell = case.cell
+    la, r = case.target_tile()
+    if cell in GUARD_CELLS or cell == "none":  # a quiet key: no redo, no halo trigger
+        for _ in range(1000):
+            key = int(rng.integers(1, M))
+            ft = model_find_tile(la, dataclasses.replace(r, state=tile_start_state(key_to_neg_state(key), r.h0, r.tin)), case.L)
+            if ft.cells() == {"none"}:
+                return key
+        raise AssertionError("no quiet key")
+    ft0 = model_find_tile(la, r, case.L, keyed=False)
+    for chunk, lo, hi in _find_target_chunks(cell, ft0):
+        for _ in range(64):
+            for st in find_tile_state(chunk, lo, hi, rng):
+                if cell in model_find_tile(la, dataclasses.replace(r, state=int(st)), case.L).cells():
+                    return key_for_state(int(st), r.h0, r.tin)
+    raise AssertionError(f"no key found for {case.cell}")
+
+
+def _fill_find_case(case: FindCase, rng) -> None:
+    """Pattern, plaintext plants, decoys and the enciphered image of a case whose keys are set."""
+    import oracle
+    L, cell = case.L, case.cell[2]
+    la, r = case.target_tile()
+    ft = model_find_tile(la, r, L)
+    spec, exact = (a.reshape(-1) for a in find_keystream(r))
+    used = np.where(np.repeat(ft.redo[np.arange(CHUNKS + HALO_CHUNKS) % THREADS], 16)
+                    & (np.arange(16 * (CHUNKS + HALO_CHUNKS)) < 16 * CHUNKS), exact, spec)
+    used[16 * CHUNKS:] = exact[16 * CHUNKS:]  # tile byte x -> keystream byte x (the halo follows a full tile)
+    pat = rng.integers(1, 256, size=L, dtype=np.uint8)
+    so_t, ln_t, _ = case.descs[case.target]
+
+    def epos(x):  # entry position of tile-local byte x
+        return TILE_BYTES * r.tin + x - r.h0
+
+    plants: Dict[int, int] = {}  # target entry position -> plain byte
+    image_sets: Dict[int, int] = {}  # image position -> cipher byte
+    taken: List[Tuple[int, int]] = []
+
+    def free(p):
+        return all(p + L <= a or b <= p for a, b in taken)
+
+    def plant(p, override=None):
+        taken.append((p, p + L))
+        for j in range(L):
+            plants[epos(p + j)] = int(pat[j]) if override is None or j != override[0] else override[1]
+
+    case.decoys = []
+    if cell in GUARD_CELLS:
+        p = _decoy_start(ft, cell)
+        if cell == "across-tile":
+            plant(ft.end - L + 1)  # a true match that ends in halo chunk 0
+        for j in range(L):
+            x, e = p + j, epos(p + j)
+            if 0 <= e < ln_t:
+                continue
+            if cell == "past-rest":  # zero-filled halo bytes: the tile holds the exact keystream
+                pat[j] = exact[x]
+                image_sets[so_t + e] = 0
+            elif ft.whole:
+                image_sets[so_t + e] = int(pat[j] ^ used[x])
+            else:  # zero-filled by the byte loads: the tile holds the keystream itself
+                pat[j] = used[x]
+        for j in range(L):
+            if 0 <= epos(p + j) < ln_t:
+                plants[epos(p + j)] = int(pat[j])
+        case.decoys = [p]
+    elif cell != "none":
+        trig = [16 * (u * THREADS + t) + b for u, t, b in zip(*np.nonzero(ft.trig))
+                if ft.compared(u * THREADS + t)[0] <= b < ft.compared(u * THREADS + t)[1]]
+        trig += [16 * (r.n_valid + k) + int(b) for k, nb in ft.halo_loaded() for b in np.nonzero(ft.halo_trig[k, :nb])[0]]
+        lo_p, hi_p = r.head, ft.p_end - 1
+
+        def start_over(x):
+            for p in range(max(lo_p, x - L + 1), min(hi_p, x) + 1):
+                if free(p):
+                    return p
+            return None
+
+        if trig:  # a match over a triggering byte: a skipped redo (or a speculative halo) misses it
+            p = start_over(trig[0])
+            if p is not None:
+                plant(p)
+        for x in trig[1:2]:  # a false match: plain byte = pattern ^ exact ^ speculative there
+            q = start_over(x)
+            if q is not None:
+                plant(q, (x - q, int(pat[x - q] ^ exact[x] ^ spec[x])))
+        for t in np.nonzero(ft.redo)[0]:  # a match in each redone thread's last valid round
+            idx = max(i for i in range(int(t), r.n_valid, THREADS)) if t < r.n_valid else None
+            if idx is not None and ft.compared(idx) != (0, 0):
+                p = start_over(16 * idx + ft.compared(idx)[0])
+                if p is not None:
+                    plant(p)
+    case.pattern = pat.tobytes()
+    image = rng.integers(0, 256, size=case.image_bytes, dtype=np.uint8)
+    for e, (so, ln, key) in enumerate(case.descs):
+        plain = rng.integers(0, 256, size=ln, dtype=np.uint8)
+        if e == case.target:
+            for pos, v in plants.items():
+                plain[pos] = v
+        image[so:so + ln] = oracle.cycle(plain, key)
+    for pos, v in image_sets.items():
+        if 0 <= pos < image.size:
+            image[pos] = v
+    case.image = image
+
+
+def make_find_case(cell: Tuple[str, str, str]) -> FindCase:
+    """A launch that reaches `cell` in its target's tile: a geometry from the sweep (picked by a hash of the cell,
+    preferring a redone thread with a valid chunk in a round > 0), a key, then plants and decoys."""
+    kind, path, c = cell
+    geoms, hits = _find_sweep(kind)
+    seed = zlib.crc32(repr(cell).encode())
+    rng = np.random.default_rng(seed)
+    cand = list(hits[cell])
+    order = rng.permutation(len(cand))
+    pick = None
+    for i in order[:200]:
+        gi, tin = cand[int(i)]
+        case = _find_layout(kind, *geoms[gi])
+        r = next(r for r in case.launch().tiles if r.entry == case.target and r.tin == tin)
+        if pick is None:
+            pick = (gi, tin)
+        n = r.n_valid
+        if c in ("interior", "double", "head", "tail", "last-round") and n <= THREADS + 1:
+            continue
+        if c == "ghost" and not THREADS < n < CHUNKS:
+            continue
+        pick = (gi, tin)
+        break
+    gi, tin = pick
+    case = _find_layout(kind, *geoms[gi])
+    case.cell, case.tin = cell, tin
+    keys = [int(k) for k in rng.integers(1, M, size=len(case.descs))]
+    case.descs = [(so, ln, k) for (so, ln, _), k in zip(case.descs, keys)]
+    so, ln, _ = case.descs[case.target]
+    case.descs[case.target] = (so, ln, 0)
+    case.descs[case.target] = (so, ln, _find_key(case, rng))
+    _fill_find_case(case, rng)
+    return case
+
+
+def find_cases() -> List[FindCase]:
+    return [make_find_case(c) for c in sorted(reachable_find_cells())]

@@ -157,11 +157,14 @@ def test_ps3_archive(cli, tmp_path):
     check(cli, tmp_path, "ps3", pat)
 
 
-@pytest.mark.parametrize("L", [1, 2, 17, 64])
-def test_matches_across_every_piece_cut(cli, tmp_path, L):
-    """MOD_IO_GROUP_MIB=1 cuts the big entries into 1 MiB pieces that overlap by L - 1 bytes: a match planted
-    across every cut is found exactly once, and so is one at each piece's first and last possible start."""
-    G = 1 << 20
+PIECE_GROUP = 1 << 20  # MOD_IO_GROUP_MIB=1
+
+
+def piece_cut_archive(root, L):
+    """An archive whose big entries a 1 MiB group cuts into pieces that overlap by L - 1 bytes, with an L-byte
+    pattern planted across every cut, at each piece's first and last possible start and at each entry's end.
+    -> (pattern, body key)."""
+    G = PIECE_GROUP
     key = 0x2468ACE
     sizes = [3_500_000, 10, 0, 2_200_001, 70_000, 1_572_864, 5] + [30_000] * 6
     rng = np.random.default_rng(L)
@@ -176,7 +179,15 @@ def test_matches_across_every_piece_cut(cli, tmp_path, L):
         if s >= L:
             blob[s - L:] = pat
         contents[i] = bytes(blob)
-    arkfixture.write_archive(str(tmp_path), n_files=len(sizes), n_parts=2, seed=29, body_key=key, sizes=sizes, contents=contents)
+    arkfixture.write_archive(str(root), n_files=len(sizes), n_parts=2, seed=29, body_key=key, sizes=sizes, contents=contents)
+    return pat, key
+
+
+@pytest.mark.parametrize("L", [1, 2, 17, 64])
+def test_matches_across_every_piece_cut(cli, tmp_path, L):
+    """MOD_IO_GROUP_MIB=1 cuts the big entries into 1 MiB pieces that overlap by L - 1 bytes: a match planted
+    across every cut is found exactly once, and so is one at each piece's first and last possible start."""
+    pat, key = piece_cut_archive(tmp_path, L)
     env = dict(os.environ, MOD_IO_GROUP_MIB="1")
     _, total, _, _ = check(cli, tmp_path, "ps4", pat, key=key, env=env)
     assert total >= 8

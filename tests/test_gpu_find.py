@@ -13,7 +13,7 @@ import synth
 import arkfixture
 import modulate_b200 as mb
 from gpuutil import DeviceBuffer, sync
-from test_find_host import oracle_find, SUMMARY
+from test_find_host import check, oracle_find, piece_cut_archive, SUMMARY
 
 pytestmark = pytest.mark.gpu
 
@@ -250,3 +250,16 @@ def test_facade_find_on_a_ciphered_1gib_archive(tmp_path):
                 assert "on 2 GPU(s)" in out.stderr.decode()
     finally:
         shutil.rmtree(root, ignore_errors=True)
+
+
+@pytest.mark.parametrize("L", [1, 2, 17, 64])
+def test_facade_find_across_every_piece_cut(tmp_path, L):
+    """The archive of test_find_host's piece-cut case through the CLI on the CUDA library: with 1 MiB groups the
+    big entries travel as pieces that overlap by L - 1 bytes, and every match is still found exactly once."""
+    if not os.path.exists(CLI):
+        from modulate_b200 import build as _build
+        _build.build()
+    pat, key = piece_cut_archive(tmp_path, L)
+    _, total, _, _ = check(CLI, tmp_path, "ps4", pat, key=key, env=dict(os.environ, MOD_IO_GROUP_MIB="1"))
+    assert total >= 8
+    check(CLI, tmp_path, "ps4", pat, key=key)

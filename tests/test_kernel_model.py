@@ -1,6 +1,8 @@
 """CPU checks of tests/kernel_model.py, the host model of the cipher kernels' dispatch: its keystream
 math against the oracle, its redo predicate against the bytes it would spoil, and the cell matrix that
 tests/test_gpu_kernel_paths.py runs on the GPU."""
+import functools
+
 import numpy as np
 import pytest
 
@@ -132,3 +134,99 @@ def test_entries_with_trigger_bytes_equals_byte_compare():
         if (spec != oracle.keystream(key, ln)).any():
             want.add(e)
     assert flagged == want and len(want) > 0
+
+
+# ---- the search kernel (find_batch_kernel) ---------------------------------------------------------------
+
+def test_search_geometry_is_parsed_from_the_kernel_header():
+    assert km.MAX_PATTERN == 64 and km.HALO_CHUNKS == (km.MAX_PATTERN - 1 + 15) // 16
+    assert km.CHUNK_POW2.size == km.CHUNKS + km.HALO_CHUNKS  # g_chunk_pow2, then c_halo_pow2
+
+
+@pytest.mark.parametrize("L", [1, 2, 3, 4, 5, 16, 17, 63, 64])
+def test_tile_start_ranges_partition_the_entry(L):
+    """The tiles' start ranges [head, p_end), in entry positions, are exactly [0, len - L + 1): no start is lost
+    at a tile end or the entry end, none is taken by two tiles."""
+    for h0 in range(16):
+        lengths = set(range(1, 3 * L + 3))
+        for b in (km.TILE_BYTES, 2 * km.TILE_BYTES, 3 * km.TILE_BYTES):
+            lengths |= {b - h0 + d for d in range(-L - 1, L + 2)}
+        for length in sorted(x for x in lengths if x > 0):
+            seen = np.zeros(length, np.int8)
+            for r in km.plan_tiles([(h0, h0, length, None)], 0):
+                _, lo, p_end = km.scan_bounds(r, L)
+                base = km.TILE_BYTES * r.tin - h0
+                if p_end > lo:
+                    seen[base + lo:base + p_end] += 1
+            assert (seen[:max(0, length - L + 1)] == 1).all() and not seen[max(0, length - L + 1):].any(), (L, h0, length)
+
+
+@pytest.mark.parametrize("key", synth.EDGE_KEYS + [0x12345678, 0x9E3779B9])
+def test_halo_keystream_equals_oracle(key):
+    """c_halo_pow2: halo chunk k of tile t is the stream's chunk 512 k later, exactly as the oracle has it."""
+    n0 = km.key_to_neg_state(key)
+    halo = np.arange(km.CHUNKS, km.CHUNKS + km.HALO_CHUNKS)
+    for tin in (0, 1, 1023, (1 << 19) - 1):
+        for h0 in range(16):
+            st = km.tile_start_state(n0, h0, tin)
+            got = km.canonical_bytes(km.chunk_states(np.uint64(st), halo)).reshape(-1)
+            want = oracle.cycle_at(np.zeros(got.size, np.uint8), key, km.TILE_BYTES * (tin + 1) - h0)
+            assert (got == want).all(), (hex(key), tin, h0)
+
+
+@functools.lru_cache(maxsize=None)
+def _find_cases():
+    return km.find_cases()
+
+
+def _tile_oracle(case):
+    """Entry positions of the target's true matches whose start the target tile owns."""
+    la, r = case.target_tile()
+    so, ln, key = case.descs[case.target]
+    plain = oracle.cycle(case.image[so:so + ln], key)
+    L = len(case.pattern)
+    lo, hi = max(0, km.TILE_BYTES * r.tin - r.h0), min(ln - L + 1, km.TILE_BYTES * (r.tin + 1) - r.h0)
+    if hi <= lo:
+        return []
+    win = np.lib.stride_tricks.sliding_window_view(plain[lo:hi + L - 1], L)
+    return [lo + int(p) for p in np.nonzero((win == np.frombuffer(case.pattern, np.uint8)).all(axis=1))[0]]
+
+
+def test_find_emulation_equals_oracle_and_every_guard_and_redo_matters():
+    """For every GPU case: the emulated tile with every guard on finds exactly the oracle's matches; with the
+    case's guard dropped its decoy is counted as well; without the redo (or with the redo from round 0's state,
+    for a ghost cell) the count changes."""
+    for case in _find_cases():
+        la, r = case.target_tile()
+        mem = case.memory()
+        base = km.TILE_BYTES * r.tin - r.h0
+        got = [base + p for p in km.emulate_find_tile(la, r, mem, case.pattern)]
+        assert got == _tile_oracle(case), case.cell
+        kind, path, cell = case.cell
+        if cell in km.GUARD_CELLS:
+            off = tuple(g for g in km.GUARDS if g != km.GUARD_OF[cell])
+            bad = km.emulate_find_tile(la, r, mem, case.pattern, guards=off)
+            assert set(case.decoys) <= set(bad) - {p - base for p in got}, case.cell
+        elif cell.startswith("halo"):
+            continue  # the halo is always exact; the GPU cases plant a match over its triggering byte
+        elif cell != "none":
+            mode = "round0" if cell == "ghost" else "off"
+            assert km.emulate_find_tile(la, r, mem, case.pattern, redo=mode) != [p - base for p in got], case.cell
+
+
+def test_find_cells_match_the_sweep_and_the_cases_cover_them():
+    declared = km.reachable_find_cells()
+    for kind in km.FIND_KINDS:
+        got = km.enumerate_reachable_find(kind)
+        assert got == {c for c in declared if c[0] == kind}, (kind, sorted(got ^ {c for c in declared if c[0] == kind}))
+    covered = set()
+    for case in _find_cases():
+        cells = case.cells()
+        assert case.cell in cells, case.cell
+        covered |= cells
+    assert covered >= declared
+    print("\nsearch cell matrix (x: GPU case, -: unreachable)")
+    print(f"{'':16}" + " ".join(f"{c:>11}" for c in km.FIND_CELLS))
+    for k in km.FIND_KINDS:
+        for p in km.FIND_PATHS:
+            print(f"{k + ' ' + p:16}" + " ".join(f"{'x' if (k, p, c) in covered else '-':>11}" for c in km.FIND_CELLS))
