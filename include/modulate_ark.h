@@ -8,6 +8,7 @@
  *   mod_ark_unpack   Unpack   (reference Modulate.cpp:291-317: CArk::Load + CArk::ExtractFiles)
  *   mod_ark_find     search every entry for a byte pattern (CArk::Load + CArk::FindInFiles; no
  *                    reference counterpart)
+ *   mod_ark_find_set the same for a set of patterns in one pass (CArk::FindSetInFiles)
  *   mod_ark_pack     Pack     (reference Modulate.cpp:380-450: song list from the DTA configs unless
  *                              pack_all, CArk::Load of the reference header, ConstructFromDirectory,
  *                              BuildArk, SaveArk)
@@ -38,6 +39,15 @@ int mod_ark_unpack(const char* header_path, const char* part_dir, const char* ta
  * when a truncated list is not the first ones.  Returns an eError (0 = success). */
 int mod_ark_find(const char* header_path, const char* part_dir, const uint8_t* pattern, uint32_t len, int32_t body_key,
                  uint64_t max_matches, uint32_t* out_file, uint32_t* out_offset, uint64_t* out_total);
+
+/* CArk::Load + CArk::FindSetInFiles: mod_ark_find for the `n` patterns (1..256, distinct, 1..64 bytes each) given
+ * as `lens` bytes each of `bytes`, concatenated in list order, searched in one pass.  out_file / out_offset /
+ * out_pattern (capacity max_matches each; may be NULL when max_matches is 0) get the first min(total, max_matches)
+ * matches sorted by (file, offset, pattern); out_pattern_counts (n entries, may be NULL) the exact matches per
+ * pattern.  Returns an eError (0 = success). */
+int mod_ark_find_set(const char* header_path, const char* part_dir, const uint8_t* bytes, const uint32_t* lens, uint32_t n,
+                     int32_t body_key, uint64_t max_matches, uint32_t* out_file, uint32_t* out_offset, uint32_t* out_pattern,
+                     uint64_t* out_total, uint64_t* out_pattern_counts);
 
 /* `input_dir` and `output_dir` must end in '/'; the header is written to output_dir + header_name. */
 int mod_ark_pack(const char* reference_header_path, const char* input_dir, const char* output_dir,

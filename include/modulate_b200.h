@@ -198,6 +198,52 @@ int mod_plan_find_window(const mod_plan* plan, uint64_t tile_begin, uint64_t til
 int mod_find_batch(const mod_desc* descs, uint64_t n, const void* d_src, uint64_t src_bytes, const uint8_t* pattern,
                    uint32_t len, uint32_t* counts_out, mod_match* matches_out, uint64_t cap, uint64_t* total_out);
 
+/* ---- search for a set of patterns in one pass ------------------------------------------------ */
+
+typedef struct mod_pattern_set mod_pattern_set; /* opaque: the set's filter and index, resident in HBM */
+
+/* One match of a set: pattern `pattern` (its position in the list the set was created from) starts at `pos`
+ * inside descriptor `desc`'s deciphered bytes. */
+typedef struct mod_set_match {
+    uint32_t desc;
+    uint32_t pos;
+    uint32_t pattern;
+} mod_set_match;
+
+/* Build a set of `n` patterns (1 <= n <= 256) on the calling thread's current device: pattern j is lens[j] bytes
+ * (1..64) of `bytes`, the patterns concatenated in list order.  Lengths may differ; the same pattern twice is
+ * refused.  Every invalid input is MOD_ERR_ARG, checked on the host.  Synchronous. */
+int mod_pattern_set_create(const uint8_t* bytes, const uint32_t* lens, uint32_t n, mod_pattern_set** out);
+int mod_pattern_set_destroy(mod_pattern_set* set);
+
+/* mod_plan_find for every pattern of `set` in one pass over the source.  A match is a pair (pattern j, start p)
+ * with p + len_j <= len whose bytes equal pattern j: overlapping matches count, and so do matches of different
+ * patterns at one start.  `d_owned` (device, one uint32 per descriptor, or NULL): starts p >= d_owned[i] of
+ * descriptor i are not reported -- what lets pieces of one entry overlap by Lmax - 1 bytes and still report each
+ * match once.  Results ACCUMULATE into caller-zeroed device memory: d_counts[i] (uint32) += matches in descriptor
+ * i; d_pattern_counts[j] (uint64) += matches of pattern j; *d_total += all matches; each match takes slot
+ * (*d_total before it) of d_matches and is stored only if that slot is below `cap`.  The list order is
+ * unspecified; the counts are exact however many matches the list drops.  The set must live on the plan's
+ * device (MOD_ERR_ARG otherwise); the plan must lie on the source grid as for mod_plan_find (MOD_ERR_ALIGN).
+ * Asynchronous on `stream`. */
+int mod_plan_find_set(const mod_plan* plan, const void* d_src, const mod_pattern_set* set, const uint32_t* d_owned,
+                      uint32_t* d_counts, uint64_t* d_pattern_counts, mod_set_match* d_matches, uint64_t cap,
+                      uint64_t* d_total, void* stream);
+
+/* mod_plan_find_set over tiles [tile_begin, tile_end) with only a window of the source resident, as
+ * mod_plan_find_window with Lmax (the set's longest pattern) in place of the pattern length. */
+int mod_plan_find_set_window(const mod_plan* plan, uint64_t tile_begin, uint64_t tile_end, const void* d_src_win,
+                             uint64_t src_win_off, uint64_t src_win_bytes, const mod_pattern_set* set,
+                             const uint32_t* d_owned, uint32_t* d_counts, uint64_t* d_pattern_counts,
+                             mod_set_match* d_matches, uint64_t cap, uint64_t* d_total, void* stream);
+
+/* Set + plan + find + destroy, synchronous: `d_src` must be device memory.  The HOST outputs get the counts per
+ * descriptor (n) and per pattern (n_patterns), the total, and min(total, cap) matches sorted by
+ * (desc, pos, pattern). */
+int mod_find_set_batch(const mod_desc* descs, uint64_t n, const void* d_src, uint64_t src_bytes, const uint8_t* bytes,
+                       const uint32_t* lens, uint32_t n_patterns, uint32_t* counts_out, uint64_t* pattern_counts_out,
+                       mod_set_match* matches_out, uint64_t cap, uint64_t* total_out);
+
 /* ---- offset-range sharding (host logic, no GPU needed) -------------------------------------- */
 
 /* (No reference counterpart: the reference is single-threaded, SURVEY.md section 8(e).)

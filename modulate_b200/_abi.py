@@ -71,12 +71,25 @@ SIGNATURES = {
                                             ctypes.c_void_p]),
     "mod_find_batch": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_uint64, ctypes.c_void_p, ctypes.c_uint64, ctypes.c_void_p,
                                       ctypes.c_uint32, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint64, ctypes.c_void_p]),
+    "mod_pattern_set_create": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint32, ctypes.POINTER(ctypes.c_void_p)]),
+    "mod_pattern_set_destroy": (ctypes.c_int, [ctypes.c_void_p]),
+    "mod_plan_find_set": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
+                                         ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint64, ctypes.c_void_p, ctypes.c_void_p]),
+    "mod_plan_find_set_window": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_uint64, ctypes.c_uint64, ctypes.c_void_p, ctypes.c_uint64,
+                                                ctypes.c_uint64, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
+                                                ctypes.c_void_p, ctypes.c_uint64, ctypes.c_void_p, ctypes.c_void_p]),
+    "mod_find_set_batch": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_uint64, ctypes.c_void_p, ctypes.c_uint64, ctypes.c_void_p,
+                                          ctypes.c_void_p, ctypes.c_uint32, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
+                                          ctypes.c_uint64, ctypes.c_void_p]),
     # include/modulate_ark.h: C binding of the archive-level facade
     "mod_ark_unpack": (ctypes.c_int, [ctypes.c_char_p, ctypes.c_char_p, ctypes.c_char_p, ctypes.c_int32]),
     "mod_ark_pack": (ctypes.c_int, [ctypes.c_char_p, ctypes.c_char_p, ctypes.c_char_p, ctypes.c_char_p, ctypes.c_int,
                                     ctypes.c_int, ctypes.c_int, ctypes.c_int32]),
     "mod_ark_find": (ctypes.c_int, [ctypes.c_char_p, ctypes.c_char_p, ctypes.c_char_p, ctypes.c_uint32, ctypes.c_int32,
                                     ctypes.c_uint64, ctypes.c_void_p, ctypes.c_void_p, ctypes.POINTER(ctypes.c_uint64)]),
+    "mod_ark_find_set": (ctypes.c_int, [ctypes.c_char_p, ctypes.c_char_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint32,
+                                        ctypes.c_int32, ctypes.c_uint64, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
+                                        ctypes.POINTER(ctypes.c_uint64), ctypes.c_void_p]),
     "mod_dta_set_int": (ctypes.c_int, [ctypes.c_char_p, ctypes.c_char_p, ctypes.c_int32]),
     "mod_shard_range": (ctypes.c_int, [ctypes.c_uint64, ctypes.c_int, ctypes.c_int,
                                        ctypes.POINTER(ctypes.c_uint64), ctypes.POINTER(ctypes.c_uint64)]),

@@ -123,6 +123,45 @@ def _pattern(pattern: Any) -> bytes:
     return p
 
 
+# numpy view of ``mod_set_match``: pattern `pattern` of a set starts at `pos` inside descriptor `desc`
+SET_MATCH_DTYPE = np.dtype([("desc", "<u4"), ("pos", "<u4"), ("pattern", "<u4")])
+MAX_SET_PATTERNS = 256
+
+
+def _pattern_list(patterns: Any) -> Tuple[np.ndarray, np.ndarray]:
+    """-> (concatenated bytes, uint32 lengths) of 1 to 256 distinct patterns of 1 to 64 bytes."""
+    ps = [_pattern(p) for p in patterns]
+    if not 1 <= len(ps) <= MAX_SET_PATTERNS:
+        raise ValueError(f"a set holds 1 to {MAX_SET_PATTERNS} patterns, not {len(ps)}")
+    if len(set(ps)) != len(ps):
+        raise ValueError("the set holds the same pattern twice")
+    return np.frombuffer(b"".join(ps), np.uint8).copy(), np.array([len(p) for p in ps], np.uint32)
+
+
+class PatternSet:
+    """A set of 1 to 256 distinct byte patterns (1 to 64 bytes each, lengths mixed) resident on the current
+    device, for ``Plan.find_set``: its filter and index are the library's business."""
+
+    def __init__(self, patterns: Any):
+        data, lens = _pattern_list(patterns)
+        self._lib = _abi.load()
+        self._handle = ctypes.c_void_p()
+        _abi.check(self._lib.mod_pattern_set_create(data.ctypes.data, lens.ctypes.data, len(lens), ctypes.byref(self._handle)))
+        self.n = len(lens)
+        self.lengths = lens
+
+    def close(self) -> None:
+        if self._handle:
+            self._lib.mod_pattern_set_destroy(self._handle)
+            self._handle = ctypes.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 def _descs(descs: np.ndarray) -> np.ndarray:
     d = np.ascontiguousarray(descs, dtype=DESC_DTYPE)
     return d
@@ -186,6 +225,28 @@ class Plan:
                                                   _buffer_info(matches)[0] if cap else None, int(cap),
                                                   _buffer_info(total)[0], stream or None))
 
+    def find_set(self, src: Any, pattern_set: PatternSet, counts: Any, pattern_counts: Any, matches: Any, cap: int, total: Any,
+                 owned: Any = None, stream: int = 0) -> None:
+        """Asynchronous search (``mod_plan_find_set``) of every descriptor for every pattern of `pattern_set` in one
+        pass: `counts` (uint32 per descriptor), `pattern_counts` (uint64 per pattern), `matches` (``SET_MATCH_DTYPE``
+        slots, `cap` of them) and `total` (one uint64) are device buffers the results ACCUMULATE into; `owned`
+        (device, uint32 per descriptor, or None) bounds the starts reported per descriptor."""
+        _abi.check(self._lib.mod_plan_find_set(self._handle, _buffer_info(src)[0], pattern_set._handle,
+                                               _buffer_info(owned)[0] if owned is not None else None, _buffer_info(counts)[0],
+                                               _buffer_info(pattern_counts)[0], _buffer_info(matches)[0] if cap else None,
+                                               int(cap), _buffer_info(total)[0], stream or None))
+
+    def find_set_window(self, tile_begin: int, tile_end: int, src_win: Any, src_win_off: int, src_win_bytes: int,
+                        pattern_set: PatternSet, counts: Any, pattern_counts: Any, matches: Any, cap: int, total: Any,
+                        owned: Any = None, stream: int = 0) -> None:
+        """``find_set`` over a tile sub-range with only a window of the source resident (slot-ring streaming)."""
+        _abi.check(self._lib.mod_plan_find_set_window(self._handle, int(tile_begin), int(tile_end), _buffer_info(src_win)[0],
+                                                      int(src_win_off), int(src_win_bytes), pattern_set._handle,
+                                                      _buffer_info(owned)[0] if owned is not None else None,
+                                                      _buffer_info(counts)[0], _buffer_info(pattern_counts)[0],
+                                                      _buffer_info(matches)[0] if cap else None, int(cap),
+                                                      _buffer_info(total)[0], stream or None))
+
     def close(self) -> None:
         if self._handle:
             self._lib.mod_plan_destroy(self._handle)
@@ -230,6 +291,28 @@ def find_batch(descs: np.ndarray, src: Any, pattern: Any, src_bytes: Optional[in
                                           counts.ctypes.data if len(d) else None, matches.ctypes.data if len(matches) else None,
                                           len(matches), ctypes.byref(total)))
     return counts, matches[:min(total.value, len(matches))].copy(), int(total.value)
+
+
+def find_set_batch(descs: np.ndarray, src: Any, patterns: Any, src_bytes: Optional[int] = None,
+                   max_matches: int = 1 << 20) -> Tuple[np.ndarray, np.ndarray, np.ndarray, int]:
+    """``find_batch`` for a list of 1 to 256 distinct patterns in one pass (synchronous).  -> (counts uint32[n],
+    pattern counts uint64[len(patterns)], matches ``SET_MATCH_DTYPE`` sorted by (desc, pos, pattern), at most
+    `max_matches` of them, exact total)."""
+    d = _descs(descs)
+    data, lens = _pattern_list(patterns)
+    s_addr, s_n, _ = _buffer_info(src)
+    src_bytes = s_n if src_bytes is None else src_bytes
+    if src_bytes < 0:
+        raise ValueError("src_bytes is required with a raw address")
+    counts = np.zeros(len(d), dtype=np.uint32)
+    pattern_counts = np.zeros(len(lens), dtype=np.uint64)
+    matches = np.zeros(max(0, int(max_matches)), dtype=SET_MATCH_DTYPE)
+    total = ctypes.c_uint64()
+    _abi.check(_abi.load().mod_find_set_batch(d.ctypes.data if len(d) else None, len(d), s_addr, int(src_bytes), data.ctypes.data,
+                                              lens.ctypes.data, len(lens), counts.ctypes.data if len(d) else None,
+                                              pattern_counts.ctypes.data, matches.ctypes.data if len(matches) else None,
+                                              len(matches), ctypes.byref(total)))
+    return counts, pattern_counts, matches[:min(total.value, len(matches))].copy(), int(total.value)
 
 
 def cycle_batch_sharded(descs: np.ndarray, src: Any, dst: Any, src_bytes: Optional[int] = None,
@@ -325,6 +408,25 @@ def ark_find(header_path: str, part_dir: str, pattern: Any, body_key: int = 0,
         raise ArkError(rc, "mod_ark_find")
     k = min(total.value, len(files))
     return [(int(f), int(o)) for f, o in zip(files[:k], offsets[:k])], int(total.value)
+
+
+def ark_find_set(header_path: str, part_dir: str, patterns: Any, body_key: int = 0,
+                 max_matches: int = 1 << 20) -> Tuple[list, np.ndarray, int]:
+    """``CArk::Load`` + ``CArk::FindSetInFiles``: -> ([(file_index, offset, pattern), ...] sorted, pattern counts, exact
+    total)."""
+    data, lens = _pattern_list(patterns)
+    files = np.zeros(max(0, int(max_matches)), dtype=np.uint32)
+    offsets, which = np.zeros_like(files), np.zeros_like(files)
+    pattern_counts = np.zeros(len(lens), dtype=np.uint64)
+    total = ctypes.c_uint64()
+    rc = _abi.load().mod_ark_find_set(header_path.encode(), _slash(part_dir) if part_dir else b"", data.ctypes.data,
+                                      lens.ctypes.data, len(lens), _i32(body_key), len(files),
+                                      files.ctypes.data if len(files) else None, offsets.ctypes.data if len(files) else None,
+                                      which.ctypes.data if len(files) else None, ctypes.byref(total), pattern_counts.ctypes.data)
+    if rc:
+        raise ArkError(rc, "mod_ark_find_set")
+    k = min(total.value, len(files))
+    return [(int(f), int(o), int(w)) for f, o, w in zip(files[:k], offsets[:k], which[:k])], pattern_counts, int(total.value)
 
 
 def dta_set_int(dta_path: str, key: str, value: int) -> None:

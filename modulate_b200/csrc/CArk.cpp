@@ -14,6 +14,7 @@
 #include <unordered_set>
 #include <cstdio>
 #include <cstring>
+#include <functional>
 #include <iostream>
 
 #include "../../include/modulate_b200.h"
@@ -22,9 +23,12 @@
 #include "Settings.h"
 
 // The search entry points are an addition to version 2 of the C ABI: they are referenced weakly, so the
-// facade still links against an implementation of the ABI that predates them, and FindInFiles reports that
-// the library lacks the search instead of the program failing to load.
+// facade still links against an implementation of the ABI that predates them, and FindInFiles /
+// FindSetInFiles report that the library lacks the search instead of the program failing to load.
 #pragma weak mod_plan_find_window
+#pragma weak mod_plan_find_set_window
+#pragma weak mod_pattern_set_create
+#pragma weak mod_pattern_set_destroy
 
 namespace {
 
@@ -518,21 +522,41 @@ eError CArk::ExtractFiles(int liFirstFileIndex, int liNumFiles, const char* lpTa
     return eError_NoError;
 }
 
+// What a search launch gets for one group: the slot's plan, stream and device buffers, the group's tiles and
+// source window, and the device's result arrays.
+struct CArk::SearchSlot {
+    size_t miDeviceIndex;
+    mod_plan* mpPlan;
+    uint64_t muTile0, muTile1;
+    const void* mpDevIn;       // the group's source range
+    uint64_t muSrcLo, muRange;
+    uint32_t* mpCounts;        // per descriptor
+    const uint32_t* mpOwned;   // per descriptor: starts the piece owns
+    uint64_t* mpPatternCounts;
+    void* mpList;              // muCap records
+    uint64_t muCap;
+    uint64_t* mpTotal;
+    void* mpStream;
+};
+
+// One search over the parts: pieces of big entries overlap by muOverlap bytes; each group's list holds records of
+// muRecordBytes, the first 8 bytes {descriptor, position}; mLaunch enqueues the kernel for one group.
+struct CArk::SearchPass {
+    uint32_t muOverlap;
+    size_t miPatterns;  // per-pattern counts kept (0: none)
+    uint64_t muMaxMatches;
+    uint64_t muRecordBytes;
+    std::function<bool(const SearchSlot&)> mLaunch;
+    std::function<void(uint32_t luFile, uint32_t luOffset, const unsigned char* lpRecord)> mCollect;  // under a lock
+};
+
 // The search reads the parts like ExtractFiles, but the GPU step deciphers and matches instead of storing: only
 // each group's short match list comes back over PCIe, and nothing is written.  Entries are searched in image
-// order, pieces of big entries overlapping by luLen - 1 bytes (CutEntry), and every entry is searched, also
-// when another one has the same name.
-eError CArk::FindInFiles(const unsigned char* lpPattern, uint32_t luLen, uint64_t luMaxMatches, std::vector<SFileMatch>& laMatches,
-                         uint64_t* lpTotal, std::vector<uint64_t>* lpFileCounts)
+// order, pieces of big entries overlapping by Lmax - 1 bytes (CutEntry), and every entry is searched, also
+// when another one has the same name.  Each piece but an entry's last owns the starts before the next piece's
+// first byte (the owned-start bounds): a pattern shorter than Lmax that starts in the overlap is the next piece's.
+eError CArk::SearchParts(const SearchPass& lPass, std::vector<uint64_t>& laFileCounts, std::vector<uint64_t>& laPatternCounts)
 {
-    laMatches.clear();
-    if (!lpPattern || luLen == 0 || luLen > 64 || !lpTotal)
-        return eError_InvalidParameter;
-    *lpTotal = 0;
-    if (!mod_plan_find_window) {
-        std::cout << "The GPU library in use has no search (mod_plan_find_window)\n";
-        return eError_NoData;
-    }
     if (mHeader.maFiles.empty())
         return eError_NoData;
     uint64_t luImageSize = 0;
@@ -554,30 +578,35 @@ eError CArk::FindInFiles(const unsigned char* lpPattern, uint32_t luLen, uint64_
     for (uint32_t luFile : laOrder) {
         const modark::FileDef& lFile = mHeader.maFiles[luFile];
         arkpipe::CutEntry(luFile, (uint64_t)lFile.miSize, (uint64_t)lFile.mi64Offset, (uint64_t)lFile.mi64Offset, EntryKey(luFile),
-                          kuGroupBytes, luLen - 1, laPieces, laDescs);
+                          kuGroupBytes, lPass.muOverlap, laPieces, laDescs);
     }
     const std::vector<arkpipe::Group> laGroups = arkpipe::GroupPieces(laDescs, kuGroupBytes);
     uint64_t luCap = 0;  // list slots per group: a group cannot hold more matches than it has bytes
     for (const arkpipe::Group& lGroup : laGroups)
-        luCap = std::max(luCap, std::min<uint64_t>(luMaxMatches, lGroup.dstHi - lGroup.dstLo));
-    const uint64_t luListBytes = 16 + 8 * luCap;  // total (8 bytes), 8 spare, the list
+        luCap = std::max(luCap, std::min<uint64_t>(lPass.muMaxMatches, lGroup.dstHi - lGroup.dstLo));
+    const uint64_t luListBytes = 16 + lPass.muRecordBytes * luCap;  // total (8 bytes), 8 spare, the list
 
-    // GPU step: zero the slot's total, upload, search the group's tiles, download the total and the list.  The
-    // per-descriptor counts live in one array per device, zeroed on the device's first group.
+    // Per device, one array of [counts per descriptor | owned starts per descriptor | counts per pattern], set up on
+    // the device's first group from laInit.
+    const size_t liDescs = laDescs.size();
+    std::vector<uint32_t> laInit(2 * liDescs + 2 * lPass.miPatterns, 0);
+    for (size_t ii = 0; ii < liDescs; ++ii) {
+        const bool lbNext = ii + 1 < liDescs && laPieces[ii + 1].file == laPieces[ii].file && laPieces[ii + 1].fileOffset != 0;
+        laInit[liDescs + ii] = lbNext ? (uint32_t)(laPieces[ii + 1].fileOffset - laPieces[ii].fileOffset) : laPieces[ii].size;
+    }
     struct DeviceCounts {
         int miDevice = -1;
         uint32_t* mpCounts = nullptr;
     };
     std::vector<DeviceCounts> laCounts(64);
-    const std::vector<uint32_t> laZeros(laDescs.size(), 0);
     arkpipe::GpuStep lFind;
     lFind.muOutBytes = luListBytes;
     lFind.mEnqueue = [&](const arkpipe::Group& lGroup, const arkpipe::SlotView& lSlot) {
         DeviceCounts& lCounts = laCounts[lSlot.miDeviceIndex];
         if (!lCounts.mpCounts) {
             lCounts.miDevice = mod_current_device();
-            lCounts.mpCounts = (uint32_t*)mod_device_alloc(4 * laDescs.size());
-            if (!lCounts.mpCounts || mod_memcpy_h2d(lCounts.mpCounts, laZeros.data(), 4 * laDescs.size(), lSlot.mpStream) != MOD_OK ||
+            lCounts.mpCounts = (uint32_t*)mod_device_alloc(4 * laInit.size());
+            if (!lCounts.mpCounts || mod_memcpy_h2d(lCounts.mpCounts, laInit.data(), 4 * laInit.size(), lSlot.mpStream) != MOD_OK ||
                 mod_stream_sync(lSlot.mpStream) != MOD_OK)
                 return false;
         }
@@ -585,14 +614,13 @@ eError CArk::FindInFiles(const unsigned char* lpPattern, uint32_t luLen, uint64_
         unsigned char* lpDevIn = (unsigned char*)lSlot.mpDevIn + (lGroup.srcLo & 15u);
         unsigned char* lpList = lSlot.mpHostOut + (lGroup.dstLo & 15u);
         std::memset(lpList, 0, 16);
-        uint64_t luTile0 = 0, luTile1 = 0;
-        return mod_plan_tile_range(lSlot.mpPlan, lGroup.first, lGroup.last, &luTile0, &luTile1) == MOD_OK &&
+        SearchSlot lSearch{lSlot.miDeviceIndex, lSlot.mpPlan, 0, 0, lpDevIn, lGroup.srcLo, luRange, lCounts.mpCounts,
+                           lCounts.mpCounts + liDescs, (uint64_t*)(lCounts.mpCounts + 2 * liDescs),
+                           (unsigned char*)lSlot.mpDevOut + 16, luCap, (uint64_t*)lSlot.mpDevOut, lSlot.mpStream};
+        return mod_plan_tile_range(lSlot.mpPlan, lGroup.first, lGroup.last, &lSearch.muTile0, &lSearch.muTile1) == MOD_OK &&
                mod_memcpy_h2d(lSlot.mpDevOut, lpList, 16, lSlot.mpStream) == MOD_OK &&
                mod_memcpy_h2d(lpDevIn, lSlot.mpHostIn + (lGroup.srcLo & 15u), luRange, lSlot.mpStream) == MOD_OK &&
-               mod_plan_find_window(lSlot.mpPlan, luTile0, luTile1, lpDevIn, lGroup.srcLo, luRange, lpPattern, luLen, lCounts.mpCounts,
-                                    (mod_match*)((unsigned char*)lSlot.mpDevOut + 16), luCap, (uint64_t*)lSlot.mpDevOut,
-                                    lSlot.mpStream) == MOD_OK &&
-               mod_memcpy_d2h(lpList, lSlot.mpDevOut, luListBytes, lSlot.mpStream) == MOD_OK;
+               lPass.mLaunch(lSearch) && mod_memcpy_d2h(lpList, lSlot.mpDevOut, luListBytes, lSlot.mpStream) == MOD_OK;
     };
 
     // drain: the group's list, as (file, offset in the entry)
@@ -605,10 +633,11 @@ eError CArk::FindInFiles(const unsigned char* lpPattern, uint32_t luLen, uint64_
             const uint64_t luKept = std::min(luTotal, luCap);
             std::lock_guard<std::mutex> lLock(lMutex);
             for (uint64_t kk = 0; kk < luKept; ++kk) {
+                const unsigned char* lpRecord = lpList + 16 + lPass.muRecordBytes * kk;
                 mod_match lMatch;
-                std::memcpy(&lMatch, lpList + 16 + 8 * kk, sizeof(lMatch));
+                std::memcpy(&lMatch, lpRecord, sizeof(lMatch));
                 const arkpipe::Piece& lPiece = laPieces[lMatch.desc];
-                laMatches.push_back(SFileMatch{(int)lPiece.file, (uint32_t)(lPiece.fileOffset + lMatch.pos)});
+                lPass.mCollect(lPiece.file, (uint32_t)(lPiece.fileOffset + lMatch.pos), lpRecord);
             }
             return eError_NoError;
         }};
@@ -622,20 +651,25 @@ eError CArk::FindInFiles(const unsigned char* lpPattern, uint32_t luLen, uint64_
         if (liFd >= 0)
             close(liFd);
 
-    // exact counts: the devices' arrays, summed per entry
-    std::vector<uint64_t> laFileCounts(liCount, 0);
-    std::vector<uint32_t> laDescCounts(laDescs.size());
+    // exact counts: the devices' arrays, summed per entry and per pattern
+    laFileCounts.assign(liCount, 0);
+    laPatternCounts.assign(lPass.miPatterns, 0);
+    std::vector<uint32_t> laDescCounts(liDescs);
+    std::vector<uint64_t> laDevicePatternCounts(lPass.miPatterns);
     for (DeviceCounts& lCounts : laCounts) {
         if (!lCounts.mpCounts)
             continue;
         if (leError == eError_NoError &&
-            (mod_init(lCounts.miDevice) != MOD_OK || mod_memcpy_d2h(laDescCounts.data(), lCounts.mpCounts, 4 * laDescs.size(), nullptr) != MOD_OK ||
+            (mod_init(lCounts.miDevice) != MOD_OK || mod_memcpy_d2h(laDescCounts.data(), lCounts.mpCounts, 4 * liDescs, nullptr) != MOD_OK ||
+             mod_memcpy_d2h(laDevicePatternCounts.data(), lCounts.mpCounts + 2 * liDescs, 8 * lPass.miPatterns, nullptr) != MOD_OK ||
              mod_stream_sync(nullptr) != MOD_OK)) {
             std::cout << "GPU find failed: " << mod_last_error() << "\n";
             leError = eError_InvalidData;
         }
-        for (size_t ii = 0; ii < laDescs.size() && leError == eError_NoError; ++ii)
+        for (size_t ii = 0; ii < liDescs && leError == eError_NoError; ++ii)
             laFileCounts[laPieces[ii].file] += laDescCounts[ii];
+        for (size_t jj = 0; jj < lPass.miPatterns && leError == eError_NoError; ++jj)
+            laPatternCounts[jj] += laDevicePatternCounts[jj];
         mod_device_free(lCounts.mpCounts);
     }
     if (liOriginalDevice >= 0)
@@ -643,6 +677,36 @@ eError CArk::FindInFiles(const unsigned char* lpPattern, uint32_t luLen, uint64_
     if (leError == eError_NoData)  // the GPU could not be set up; RunPipeline has said why
         return leError;
     SHOW_ERROR_AND_RETURN;
+    return eError_NoError;
+}
+
+eError CArk::FindInFiles(const unsigned char* lpPattern, uint32_t luLen, uint64_t luMaxMatches, std::vector<SFileMatch>& laMatches,
+                         uint64_t* lpTotal, std::vector<uint64_t>* lpFileCounts)
+{
+    laMatches.clear();
+    if (!lpPattern || luLen == 0 || luLen > 64 || !lpTotal)
+        return eError_InvalidParameter;
+    *lpTotal = 0;
+    if (!mod_plan_find_window) {
+        std::cout << "The GPU library in use has no search (mod_plan_find_window)\n";
+        return eError_NoData;
+    }
+    SearchPass lPass;
+    lPass.muOverlap = luLen - 1;
+    lPass.miPatterns = 0;
+    lPass.muMaxMatches = luMaxMatches;
+    lPass.muRecordBytes = sizeof(mod_match);
+    lPass.mLaunch = [&](const SearchSlot& lSlot) {
+        return mod_plan_find_window(lSlot.mpPlan, lSlot.muTile0, lSlot.muTile1, lSlot.mpDevIn, lSlot.muSrcLo, lSlot.muRange, lpPattern,
+                                    luLen, lSlot.mpCounts, (mod_match*)lSlot.mpList, lSlot.muCap, lSlot.mpTotal, lSlot.mpStream) == MOD_OK;
+    };
+    lPass.mCollect = [&](uint32_t luFile, uint32_t luOffset, const unsigned char*) {
+        laMatches.push_back(SFileMatch{(int)luFile, luOffset});
+    };
+    std::vector<uint64_t> laFileCounts, laPatternCounts;
+    const eError leError = SearchParts(lPass, laFileCounts, laPatternCounts);
+    if (leError != eError_NoError)
+        return leError;
     for (uint64_t luCount : laFileCounts)
         *lpTotal += luCount;
     std::sort(laMatches.begin(), laMatches.end(),
@@ -651,6 +715,68 @@ eError CArk::FindInFiles(const unsigned char* lpPattern, uint32_t luLen, uint64_
         laMatches.resize((size_t)luMaxMatches);
     if (lpFileCounts)
         *lpFileCounts = std::move(laFileCounts);
+    return eError_NoError;
+}
+
+eError CArk::FindSetInFiles(const std::vector<std::string>& laPatterns, uint64_t luMaxMatches, std::vector<SFileSetMatch>& laMatches,
+                            uint64_t* lpTotal, std::vector<uint64_t>* lpFileCounts, std::vector<uint64_t>* lpPatternCounts)
+{
+    laMatches.clear();
+    if (laPatterns.empty() || laPatterns.size() > 256 || !lpTotal)
+        return eError_InvalidParameter;
+    std::string lBytes;
+    std::vector<uint32_t> laLens;
+    uint32_t luMax = 0;
+    for (const std::string& lPattern : laPatterns) {
+        if (lPattern.empty() || lPattern.size() > 64)
+            return eError_InvalidParameter;
+        lBytes += lPattern;
+        laLens.push_back((uint32_t)lPattern.size());
+        luMax = std::max(luMax, (uint32_t)lPattern.size());
+    }
+    if (std::unordered_set<std::string>(laPatterns.begin(), laPatterns.end()).size() != laPatterns.size())
+        return eError_InvalidParameter;
+    *lpTotal = 0;
+    if (!mod_plan_find_set_window || !mod_pattern_set_create || !mod_pattern_set_destroy) {
+        std::cout << "The GPU library in use has no set search (mod_plan_find_set_window)\n";
+        return eError_NoData;
+    }
+    std::vector<mod_pattern_set*> laSets(64, nullptr);  // one per device, created on its first group
+    SearchPass lPass;
+    lPass.muOverlap = luMax - 1;
+    lPass.miPatterns = laPatterns.size();
+    lPass.muMaxMatches = luMaxMatches;
+    lPass.muRecordBytes = sizeof(mod_set_match);
+    lPass.mLaunch = [&](const SearchSlot& lSlot) {
+        mod_pattern_set*& lpSet = laSets[lSlot.miDeviceIndex];
+        if (!lpSet && mod_pattern_set_create((const uint8_t*)lBytes.data(), laLens.data(), (uint32_t)laLens.size(), &lpSet) != MOD_OK)
+            return false;
+        return mod_plan_find_set_window(lSlot.mpPlan, lSlot.muTile0, lSlot.muTile1, lSlot.mpDevIn, lSlot.muSrcLo, lSlot.muRange, lpSet,
+                                        lSlot.mpOwned, lSlot.mpCounts, lSlot.mpPatternCounts, (mod_set_match*)lSlot.mpList, lSlot.muCap,
+                                        lSlot.mpTotal, lSlot.mpStream) == MOD_OK;
+    };
+    lPass.mCollect = [&](uint32_t luFile, uint32_t luOffset, const unsigned char* lpRecord) {
+        mod_set_match lMatch;
+        std::memcpy(&lMatch, lpRecord, sizeof(lMatch));
+        laMatches.push_back(SFileSetMatch{(int)luFile, luOffset, lMatch.pattern});
+    };
+    std::vector<uint64_t> laFileCounts, laPatternCounts;
+    const eError leError = SearchParts(lPass, laFileCounts, laPatternCounts);
+    for (mod_pattern_set* lpSet : laSets)
+        mod_pattern_set_destroy(lpSet);
+    if (leError != eError_NoError)
+        return leError;
+    for (uint64_t luCount : laFileCounts)
+        *lpTotal += luCount;
+    std::sort(laMatches.begin(), laMatches.end(), [](const SFileSetMatch& a, const SFileSetMatch& b) {
+        return a.file != b.file ? a.file < b.file : a.offset != b.offset ? a.offset < b.offset : a.pattern < b.pattern;
+    });
+    if (laMatches.size() > luMaxMatches)
+        laMatches.resize((size_t)luMaxMatches);
+    if (lpFileCounts)
+        *lpFileCounts = std::move(laFileCounts);
+    if (lpPatternCounts)
+        *lpPatternCounts = std::move(laPatternCounts);
     return eError_NoError;
 }
 

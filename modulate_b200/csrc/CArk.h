@@ -42,6 +42,13 @@ struct SFileMatch {
     uint32_t offset;
 };
 
+// One match of CArk::FindSetInFiles: entry `file` holds pattern `pattern` (its index in the list) at `offset`.
+struct SFileSetMatch {
+    int file;
+    uint32_t offset;
+    uint32_t pattern;
+};
+
 class CArk
 {
 public:
@@ -76,6 +83,13 @@ public:
     // image), in which case which ones that group keeps is unspecified.
     eError FindInFiles(const unsigned char* lpPattern, uint32_t luLen, uint64_t luMaxMatches, std::vector<SFileMatch>& laMatches,
                        uint64_t* lpTotal, std::vector<uint64_t>* lpFileCounts = nullptr);
+    // FindInFiles for a set of 1 to 256 distinct patterns of 1 to 64 bytes each, lengths mixed, in one pass: every
+    // (pattern, position) at which an entry holds a pattern, overlapping matches and matches of different patterns
+    // at one position included.  laMatches is sorted by (file, offset, pattern) and truncated like FindInFiles';
+    // lpFileCounts gets the exact matches per entry and lpPatternCounts the exact matches per pattern, in list order.
+    eError FindSetInFiles(const std::vector<std::string>& laPatterns, uint64_t luMaxMatches, std::vector<SFileSetMatch>& laMatches,
+                          uint64_t* lpTotal, std::vector<uint64_t>* lpFileCounts = nullptr,
+                          std::vector<uint64_t>* lpPatternCounts = nullptr);
     const modark::HeaderImage& Header() const { return mHeader; }
 
 private:
@@ -85,6 +99,9 @@ private:
     bool ReadImageRange(std::vector<int>& laFds, uint64_t luOffset, uint64_t luSize, unsigned char* lpDst) const;
     arkpipe::Stage ReadGroupsStage(const std::vector<arkpipe::Group>& laGroups, std::vector<int>& laPartFds) const;
     eError CheckEntriesInImage(uint64_t luImageSize) const;
+    struct SearchSlot;
+    struct SearchPass;
+    eError SearchParts(const SearchPass& lPass, std::vector<uint64_t>& laFileCounts, std::vector<uint64_t>& laPatternCounts);
     struct PartTarget {
         int miFd = -1;             // part file open for writing
         unsigned char* mpMap = nullptr;  // its mapping, when it could be mapped

@@ -2,6 +2,7 @@
 // command bodies (Modulate.cpp:291-317, :380-450) and the archive search on the facade classes.
 #include "../../include/modulate_ark.h"
 
+#include <algorithm>
 #include <exception>
 #include <iostream>
 #include <string>
@@ -66,6 +67,39 @@ int mod_ark_find(const char* header_path, const char* part_dir, const uint8_t* p
             out_file[ii] = (uint32_t)laMatches[ii].file;
             out_offset[ii] = laMatches[ii].offset;
         }
+        return eError_NoError;
+    });
+}
+
+int mod_ark_find_set(const char* header_path, const char* part_dir, const uint8_t* bytes, const uint32_t* lens, uint32_t n,
+                     int32_t body_key, uint64_t max_matches, uint32_t* out_file, uint32_t* out_offset, uint32_t* out_pattern,
+                     uint64_t* out_total, uint64_t* out_pattern_counts)
+{
+    return Guarded([&]() -> eError {
+        if (!header_path || !bytes || !lens || !out_total || (max_matches && (!out_file || !out_offset || !out_pattern)))
+            return eError_InvalidParameter;
+        std::vector<std::string> laPatterns;
+        uint64_t luAt = 0;
+        for (uint32_t jj = 0; jj < n; ++jj) {
+            laPatterns.emplace_back((const char*)bytes + luAt, lens[jj]);
+            luAt += lens[jj];
+        }
+        CArk lArkHeader;
+        lArkHeader.SetUniformEntryKey(body_key);
+        lArkHeader.SetPartDirectory(part_dir ? part_dir : "");
+        eError leError = lArkHeader.Load(header_path);
+        SHOW_ERROR_AND_RETURN;
+        std::vector<SFileSetMatch> laMatches;
+        std::vector<uint64_t> laPatternCounts;
+        leError = lArkHeader.FindSetInFiles(laPatterns, max_matches, laMatches, out_total, nullptr, &laPatternCounts);
+        SHOW_ERROR_AND_RETURN;
+        for (size_t ii = 0; ii < laMatches.size(); ++ii) {
+            out_file[ii] = (uint32_t)laMatches[ii].file;
+            out_offset[ii] = laMatches[ii].offset;
+            out_pattern[ii] = laMatches[ii].pattern;
+        }
+        if (out_pattern_counts)
+            std::copy(laPatternCounts.begin(), laPatternCounts.end(), out_pattern_counts);
         return eError_NoError;
     });
 }

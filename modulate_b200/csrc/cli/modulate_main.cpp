@@ -6,7 +6,8 @@
 //
 // Extensions: -bodykey K (cipher every entry body with key K, stream restarting per entry -- the
 // synthetic per-entry-key configurations), -device N (bind GPU N), -find TEXT / -findhex HEX (which
-// entries hold a byte pattern, searched on the GPU without unpacking).
+// entries hold a byte pattern, searched on the GPU without unpacking), -findlist FILE / -findhexlist FILE
+// (the same for a list of patterns, all found in one pass).
 #include <algorithm>
 #include <cctype>
 #include <chrono>
@@ -14,10 +15,12 @@
 #include <cstdlib>
 #include <cstring>
 #include <deque>
+#include <fstream>
 #include <functional>
 #include <iostream>
 #include <string>
 #include <strings.h>
+#include <unordered_map>
 #include <vector>
 
 #include "../../../include/modulate_b200.h"
@@ -150,24 +153,112 @@ eError Find(std::deque<std::string>& laParams)
     return FindPattern(lText);
 }
 
+// Hex digit pairs, whitespace ignored (the -findhex syntax) -> lBytes; lpShown, when given, gets the digits
+// lowercased and without spaces.
+bool ParseHex(const std::string& lText, std::string& lBytes, std::string* lpShown)
+{
+    std::string lDigits;
+    for (char c : lText)
+        if (!std::isspace((unsigned char)c))
+            lDigits += (char)std::tolower((unsigned char)c);
+    if (lDigits.size() % 2 != 0 || lDigits.find_first_not_of("0123456789abcdef") != std::string::npos)
+        return false;
+    lBytes.clear();
+    for (size_t ii = 0; ii < lDigits.size(); ii += 2)
+        lBytes += (char)std::stoi(lDigits.substr(ii, 2), nullptr, 16);
+    if (lpShown)
+        *lpShown = lDigits;
+    return true;
+}
+
 eError FindHex(std::deque<std::string>& laParams)
 {
     if (laParams.empty())
         return eError_InvalidParameter;
-    std::string lDigits;
-    for (char c : laParams.front())
-        if (!std::isspace((unsigned char)c))
-            lDigits += c;
+    std::string lBytes;
+    const bool lbHex = ParseHex(laParams.front(), lBytes, nullptr);
     laParams.pop_front();
-    if (lDigits.size() % 2 != 0 || lDigits.find_first_not_of("0123456789abcdefABCDEF") != std::string::npos) {
+    if (!lbHex) {
         std::cout << "-findhex takes pairs of hex digits\n";
         return eError_InvalidParameter;
     }
-    std::string lBytes;
-    for (size_t ii = 0; ii < lDigits.size(); ii += 2)
-        lBytes += (char)std::stoi(lDigits.substr(ii, 2), nullptr, 16);
     return FindPattern(lBytes);
 }
+
+// -findlist / -findhexlist: one pattern per line (a trailing '\r' stripped, empty lines skipped), all searched in one
+// pass.  One line "<name>\t<offset>\t<pattern>" per match in table order, then by offset, then list order, at most
+// kiMaxLines of them; then "<count>\t<pattern>" per pattern in list order, and the "<total> matches in <files>
+// files" of -find.  A hex pattern is shown as given, lowercased and without spaces.
+eError FindList(std::deque<std::string>& laParams, bool lbHex)
+{
+    constexpr uint64_t kiMaxLines = 10000;
+    const char* lpWhat = lbHex ? "-findhexlist" : "-findlist";
+    if (laParams.empty())
+        return eError_InvalidParameter;
+    const std::string lListPath = laParams.front();
+    laParams.pop_front();
+    std::ifstream lList(lListPath, std::ios::binary);
+    if (!lList) {
+        std::cout << lpWhat << ": cannot read " << lListPath << "\n";
+        return eError_FailedToOpenFile;
+    }
+    std::vector<std::string> laPatterns, laShown;
+    std::unordered_map<std::string, size_t> lLineOf;
+    std::string lLine;
+    for (size_t liLine = 1; std::getline(lList, lLine); ++liLine) {
+        if (!lLine.empty() && lLine.back() == '\r')
+            lLine.pop_back();
+        if (lLine.empty())
+            continue;
+        std::string lBytes = lLine, lShown = lLine;
+        if (lbHex && !ParseHex(lLine, lBytes, &lShown)) {
+            std::cout << lpWhat << ": line " << liLine << " is not pairs of hex digits\n";
+            return eError_InvalidParameter;
+        }
+        if (lBytes.empty() || lBytes.size() > 64) {
+            std::cout << lpWhat << ": line " << liLine << ": the pattern must be 1 to 64 bytes long\n";
+            return eError_InvalidParameter;
+        }
+        const auto lSeen = lLineOf.emplace(lBytes, liLine);
+        if (!lSeen.second) {
+            std::cout << lpWhat << ": line " << liLine << " repeats the pattern of line " << lSeen.first->second << "\n";
+            return eError_InvalidParameter;
+        }
+        if (laPatterns.size() == 256) {
+            std::cout << lpWhat << ": line " << liLine << ": a list holds at most 256 patterns\n";
+            return eError_InvalidParameter;
+        }
+        laPatterns.push_back(lBytes);
+        laShown.push_back(lShown);
+    }
+    if (laPatterns.empty()) {
+        std::cout << lpWhat << ": " << lListPath << " holds no pattern\n";
+        return eError_InvalidParameter;
+    }
+    std::cout << "Searching " << HeaderName() << " for " << laPatterns.size() << " patterns\n";
+    CArk lArkHeader;
+    lArkHeader.SetUniformEntryKey(giBodyKey);
+    eError leError = lArkHeader.Load(HeaderName().c_str());
+    SHOW_ERROR_AND_RETURN;
+    std::vector<SFileSetMatch> laMatches;
+    std::vector<uint64_t> laFileCounts, laPatternCounts;
+    uint64_t luTotal = 0;
+    leError = lArkHeader.FindSetInFiles(laPatterns, kiMaxLines, laMatches, &luTotal, &laFileCounts, &laPatternCounts);
+    SHOW_ERROR_AND_RETURN;
+    for (const SFileSetMatch& lMatch : laMatches)
+        std::cout << lArkHeader.Header().maFiles[(size_t)lMatch.file].mName << "\t" << lMatch.offset << "\t" << laShown[lMatch.pattern]
+                  << "\n";
+    if (luTotal > laMatches.size())
+        std::cout << "... " << luTotal - laMatches.size() << " more\n";
+    for (size_t jj = 0; jj < laPatterns.size(); ++jj)
+        std::cout << laPatternCounts[jj] << "\t" << laShown[jj] << "\n";
+    const size_t liFiles = (size_t)std::count_if(laFileCounts.begin(), laFileCounts.end(), [](uint64_t n) { return n != 0; });
+    std::cout << luTotal << " matches in " << liFiles << " files\n";
+    return eError_NoError;
+}
+
+eError FindListText(std::deque<std::string>& laParams) { return FindList(laParams, false); }
+eError FindListHex(std::deque<std::string>& laParams) { return FindList(laParams, true); }
 
 eError PackImpl(std::deque<std::string>& laParams)
 {
@@ -344,6 +435,8 @@ void PrintUsage()
               << "  -decode                     Write the deciphered header to main_<platform>.hdr.dec\n"
               << "  -find <text>                List the entries (and offsets) whose bytes contain <text>\n"
               << "  -findhex <hex>              Same for a pattern given as hex bytes, e.g. 00ff1a\n"
+              << "  -findlist <file>            Same for every pattern of <file> (one per line, up to 256), in one pass\n"
+              << "  -findhexlist <file>         Same for a file of hex patterns, one per line\n"
               << "  -listsongs <dir>            List the songs the DTA configs under <dir> define\n"
               << "  -dtaset <file> <key> <val>  Patch the value following symbol <key> in a binary DTA file\n"
               << "  -dtacopy <in> <out>         Load and re-save a binary DTA file\n";
@@ -374,6 +467,7 @@ int main(int argc, char* argv[])
         {"-bodykey", BodyKey}, {"-device", Device},       {"-unpack", Unpack},          {"-pack", Pack},
         {"-pack_add", AddPack}, {"-decode", Decode},   {"-dtaset", DtaSet},          {"-dtacopy", DtaCopy},
         {"-listsongs", ListSongs}, {"-find", Find},     {"-findhex", FindHex},
+        {"-findlist", FindListText}, {"-findhexlist", FindListHex},
     };
 
     std::deque<std::string> laParams;

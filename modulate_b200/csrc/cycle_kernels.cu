@@ -36,6 +36,7 @@
 #include "cycle_kernels.cuh"
 #include "lcg.h"
 
+#include <algorithm>
 #include <cstdlib>
 
 namespace modk {
@@ -645,25 +646,36 @@ __device__ __noinline__ uint4 load_bytes(uint64_t addr, uint32_t lo, uint32_t hi
     return make_uint4(w[0], w[1], w[2], w[3]);
 }
 
-__global__ void __launch_bounds__(kThreadsPerCta, MODK_MIN_CTAS_FIND) find_batch_kernel(const __grid_constant__ FindArgs f)
+// What a CTA knows about the tile it has deciphered: where the tile lies and which of its bytes are the entry's.
+struct TileView {
+    int64_t src_rel;   // the tile record's src_rel
+    uint32_t entry;    // descriptor index
+    uint32_t head;     // tile-local first byte of the entry
+    uint32_t end;      // tile-local end of the entry's bytes in the tile
+    uint32_t halo;     // entry bytes past the tile that were deciphered too
+};
+
+// The decipher stage of both search kernels: tile `rec` of a plan whose chunk grid lies on the source, deciphered
+// into s_w (one LDG.128 per chunk, lazy states, speculative packing, the thread's chunks redone exactly from their
+// source when one of their states had bit 31 set), plus up to `halo_max` entry bytes past the tile (exact, a
+// constant jump from the tile state).  `pw` are the thread's chunk jump factors.  The caller synchronises the CTA
+// before it reads s_w.
+__device__ __forceinline__ TileView decipher_tile(const TileRec* rec, const uint8_t* src, uint64_t src_lo16, uint64_t src_hi16,
+                                                  uint32_t halo_max, uint32_t two, const uint32_t (&pw)[kUnroll], uint32_t* s_w)
 {
     constexpr int U = kUnroll;
     constexpr uint32_t T = (uint32_t)kThreadsPerCta;
-    // the tile, its halo, and one word of slack for the filter's second word
-    __shared__ __align__(16) uint32_t s_w[(kTileBytes + 16u * kHaloChunks) / 4u + 4u];
     const uint32_t tid = threadIdx.x;
-    uint32_t pw[U];
-    load_chunk_pows<U>(pw, tid);
-    const uint4* rp = reinterpret_cast<const uint4*>(f.tiles + blockIdx.x);
+    const uint4* rp = reinterpret_cast<const uint4*>(rec);
     const uint4 lo = __ldg(rp);
     const uint4 hi = __ldg(rp + 1);
     const int64_t src_rel = (int64_t)((uint64_t)lo.x | ((uint64_t)lo.y << 32));
     const uint32_t st = hi.x, geom = hi.y, entry = hi.z;
     const uint32_t n_valid = geom & 0xFFFu, head = (geom >> 12) & 15u, tail = (geom >> 16) & 31u;
     const uint32_t end = 16u * (n_valid - 1u) + tail;  // tile-local end of the entry's bytes
-    const uint32_t halo = min(hi.w, f.len - 1u);       // entry bytes past the tile a match can reach
-    const uint64_t src_tile = (uint64_t)f.src + (uint64_t)src_rel;
-    const bool whole = src_tile >= f.src_lo16 && src_tile + 16ull * n_valid <= f.src_hi16;  // CTA-uniform
+    const uint32_t halo = min(hi.w, halo_max);         // entry bytes past the tile a match can reach
+    const uint64_t src_tile = (uint64_t)src + (uint64_t)src_rel;
+    const bool whole = src_tile >= src_lo16 && src_tile + 16ull * n_valid <= src_hi16;  // CTA-uniform
 
     auto load_chunk = [&](uint32_t idx) {
         return whole ? ldg128(src_tile + 16ull * idx)
@@ -680,7 +692,7 @@ __global__ void __launch_bounds__(kThreadsPerCta, MODK_MIN_CTAS_FIND) find_batch
     // the halo: exact keystream, byte loads (it ends inside the entry, wherever the granule does)
     if (tid < (uint32_t)kHaloChunks && 16u * tid < halo) {
         const uint4 h = load_bytes(src_tile + 16ull * (n_valid + tid), 0u, min(16u, halo - 16u * tid));
-        const uint4 o = cycle_chunk_exact(h, jump_lazy(st, c_halo_pow2[tid]), f.two);
+        const uint4 o = cycle_chunk_exact(h, jump_lazy(st, c_halo_pow2[tid]), two);
         reinterpret_cast<uint4*>(s_w)[n_valid + tid] = o;
     }
 
@@ -715,7 +727,7 @@ __global__ void __launch_bounds__(kThreadsPerCta, MODK_MIN_CTAS_FIND) find_batch
             const uint32_t idx = tid + (uint32_t)u * T;
             if (idx < n_valid)
                 reinterpret_cast<uint4*>(s_w)[idx] =
-                    cycle_chunk_exact(load_chunk(idx), jump_lazy(st, __ldg(&g_chunk_pow2[idx])), f.two);
+                    cycle_chunk_exact(load_chunk(idx), jump_lazy(st, __ldg(&g_chunk_pow2[idx])), two);
         }
     } else {
 #pragma unroll
@@ -725,6 +737,20 @@ __global__ void __launch_bounds__(kThreadsPerCta, MODK_MIN_CTAS_FIND) find_batch
                 reinterpret_cast<uint4*>(s_w)[idx] = d[u];
         }
     }
+    return TileView{src_rel, entry, head, end, halo};
+}
+
+__global__ void __launch_bounds__(kThreadsPerCta, MODK_MIN_CTAS_FIND) find_batch_kernel(const __grid_constant__ FindArgs f)
+{
+    constexpr uint32_t T = (uint32_t)kThreadsPerCta;
+    // the tile, its halo, and one word of slack for the filter's second word
+    __shared__ __align__(16) uint32_t s_w[(kTileBytes + 16u * kHaloChunks) / 4u + 4u];
+    const uint32_t tid = threadIdx.x;
+    uint32_t pw[kUnroll];
+    load_chunk_pows<kUnroll>(pw, tid);
+    const TileView v = decipher_tile(f.tiles + blockIdx.x, f.src, f.src_lo16, f.src_hi16, f.len - 1u, f.two, pw, s_w);
+    const int64_t src_rel = v.src_rel;
+    const uint32_t entry = v.entry, head = v.head, end = v.end, halo = v.halo;
     __syncthreads();
 
     // start positions [head, p_end): inside the tile's part of the entry, with room for the whole pattern
@@ -756,6 +782,107 @@ __global__ void __launch_bounds__(kThreadsPerCta, MODK_MIN_CTAS_FIND) find_batch
             if (hit)
                 find_record(f, entry, src_rel, p);
         }
+    }
+}
+
+// ---- pattern-set search: the same decipher stage, an exact 2-byte filter, the set verified in HBM -----------------
+//
+// A persistent grid (every resident CTA slot of the device, each looping over tiles) so that the 8 KiB filter
+// bitmap is loaded into shared memory once per CTA rather than once per 8 KiB tile.  Per tile the CTA deciphers
+// the tile plus min(rest, Lmax - 1) halo bytes, then tests every start in [head, p_end) -- p_end from Lmin, the
+// owned-start bound and the tile end -- against the bitmap bit of its first two bytes.  A start that passes is a
+// candidate, and find_set_verify (out of line) checks each pattern that can start there, its end against the
+// entry's.
+#ifndef MODK_MIN_CTAS_FIND_SET
+#define MODK_MIN_CTAS_FIND_SET 10
+#endif
+
+// Every pattern of the set that starts at tile-local p, whose first two bytes passed the filter: the length-1
+// pattern of the first byte, then the patterns of the 2-byte key (binary search over the distinct keys), each
+// checked against `lim` (where the deciphered entry bytes end), its head word and then its remaining bytes.
+// `pos0` is the entry position of tile-local byte 0.
+__device__ __noinline__ void find_set_verify(const FindSetArgs& f, const uint8_t* sb, const uint16_t* s_keys, uint32_t p,
+                                             uint32_t lim, uint32_t entry, int64_t pos0)
+{
+    auto record = [&](uint32_t id) {
+        atomicAdd(&f.counts[entry], 1u);
+        atomicAdd(&f.pattern_counts[id], 1ull);
+        const unsigned long long slot = atomicAdd(f.total, 1ull);
+        if (slot < f.cap) {
+            uint32_t* m = f.matches + 3ull * slot;
+            m[0] = entry;
+            m[1] = (uint32_t)(pos0 + (int64_t)p);
+            m[2] = id;
+        }
+    };
+    const uint32_t b0 = sb[p], key = b0 | ((uint32_t)sb[p + 1] << 8);
+    const uint32_t one = __ldg(&f.set->one[b0]);
+    if (one)
+        record(one - 1u);
+    uint32_t lo = 0, hi = f.n_keys;
+    while (lo < hi) {
+        const uint32_t mid = (lo + hi) >> 1;
+        if (s_keys[mid] < key)
+            lo = mid + 1u;
+        else
+            hi = mid;
+    }
+    if (lo == f.n_keys || s_keys[lo] != key)
+        return;
+    const uint32_t word = b0 | ((uint32_t)sb[p + 1] << 8) | ((uint32_t)sb[p + 2] << 16) | ((uint32_t)sb[p + 3] << 24);
+    const uint32_t r1 = __ldg(&f.set->group[lo + 1u]);
+    for (uint32_t r = __ldg(&f.set->group[lo]); r < r1; ++r) {
+        const uint4 sp = __ldg(reinterpret_cast<const uint4*>(&f.set->pat[r]));  // {id, len, head, mask}
+        if (p + sp.y > lim || ((word ^ sp.z) & sp.w) != 0u)
+            continue;
+        bool hit = true;
+        for (uint32_t k = 4u; k < sp.y && hit; ++k)
+            hit = sb[p + k] == __ldg(&f.set->bytes[r][k]);
+        if (hit)
+            record(sp.x);
+    }
+}
+
+__global__ void __launch_bounds__(kThreadsPerCta, MODK_MIN_CTAS_FIND_SET) find_set_kernel(const __grid_constant__ FindSetArgs f)
+{
+    constexpr uint32_t T = (uint32_t)kThreadsPerCta;
+    __shared__ __align__(16) uint32_t s_w[(kTileBytes + 16u * kHaloChunks) / 4u + 4u];
+    __shared__ __align__(16) uint32_t s_bm[65536u / 32u];
+    __shared__ uint16_t s_keys[kMaxSetPatterns];
+    const uint32_t tid = threadIdx.x;
+    for (uint32_t i = tid; i < 65536u / 128u; i += T)
+        reinterpret_cast<uint4*>(s_bm)[i] = __ldg(reinterpret_cast<const uint4*>(f.set->bitmap) + i);
+    for (uint32_t i = tid; i < f.n_keys; i += T)
+        s_keys[i] = __ldg(&f.set->keys[i]);
+    uint32_t pw[kUnroll];
+    load_chunk_pows<kUnroll>(pw, tid);
+    const uint8_t* sb = reinterpret_cast<const uint8_t*>(s_w);
+    for (uint32_t t = blockIdx.x; t < f.n_tiles; t += gridDim.x) {
+        const TileView v = decipher_tile(f.tiles + t, f.src, f.src_lo16, f.src_hi16, f.lmax - 1u, f.two, pw, s_w);
+        const int64_t pos0 = v.src_rel - (int64_t)__ldg(&f.descs[v.entry].src_off);
+        const uint32_t lim = v.end + v.halo;  // every pattern must end here: the entry ends, or Lmax - 1 bytes on
+        // starts [head, p_end): inside the tile, with room for the shortest pattern, below the owned bound
+        int64_t p_end = min((int32_t)v.end, (int32_t)lim - (int32_t)f.lmin + 1);
+        if (f.owned)
+            p_end = min(p_end, (int64_t)__ldg(&f.owned[v.entry]) - pos0);
+        const uint32_t pe = (uint32_t)max(p_end, (int64_t)0);
+        __syncthreads();  // the tile (and, before the first, the bitmap and keys) are in shared memory
+        for (uint32_t w = (v.head >> 2) + tid; 4u * w < pe; w += T) {
+            const uint32_t x = s_w[w], y = s_w[w + 1u];
+            auto bit = [&](uint32_t o) {  // the filter bit of start 4w + o, in bit 0
+                const uint32_t key = __byte_perm(x, y, (o + 1u) << 4 | o) & 0xFFFFu;  // bytes p and p + 1
+                return s_bm[key >> 5] >> (key & 31u);
+            };
+            if (__builtin_expect(((bit(0) | bit(1) | bit(2) | bit(3)) & 1u) == 0u, 1))
+                continue;
+#pragma unroll 1
+            for (uint32_t o = 0; o < 4u; ++o) {
+                const uint32_t p = 4u * w + o;
+                if ((bit(o) & 1u) != 0u && p >= v.head && p < pe)
+                    find_set_verify(f, sb, s_keys, p, lim, v.entry, pos0);
+            }
+        }
+        __syncthreads();  // the tile is no longer read: the next one may overwrite it
     }
 }
 
@@ -842,6 +969,23 @@ cudaError_t launch_find(const FindArgs& args, cudaStream_t stream)
         t0 += n;
     }
     return cudaSuccess;
+}
+
+cudaError_t launch_find_set(const FindSetArgs& args, cudaStream_t stream)
+{
+    if (args.n_tiles == 0)
+        return cudaSuccess;
+    int dev = 0, sms = 0, per_sm = 0;
+    cudaError_t err = cudaGetDevice(&dev);
+    if (err == cudaSuccess)
+        err = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    if (err == cudaSuccess)
+        err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, find_set_kernel, kThreadsPerCta, 0);
+    if (err != cudaSuccess)
+        return err;
+    const uint32_t grid = (uint32_t)std::max(1, sms * per_sm);
+    find_set_kernel<<<std::min(grid, args.n_tiles), kThreadsPerCta, 0, stream>>>(args);
+    return cudaGetLastError();
 }
 
 cudaError_t launch_build_tiles(const DevDesc* descs, uint32_t n_descs, uint32_t dst_align, TileRec* tiles,

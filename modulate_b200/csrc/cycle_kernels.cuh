@@ -2,6 +2,7 @@
 #pragma once
 
 #include <cuda_runtime.h>
+#include <stddef.h>
 #include <stdint.h>
 
 namespace modk {
@@ -90,6 +91,43 @@ struct FindArgs {
     uint8_t pattern[kMaxPattern];
 };
 
+// Pattern-set search (find_set_kernel): the decipher stage of find_batch_kernel, then every start tested against
+// an exact 2-byte filter and the candidates verified against the set.  The index is built on the host
+// (mod_pattern_set_create) and lives in HBM; callers never see it.
+constexpr uint32_t kMaxSetPatterns = 256;
+struct __align__(16) SetPattern {  // read as one 16-byte load
+    uint32_t id;    // position in the caller's list
+    uint32_t len;
+    uint32_t head;  // first min(4, len) bytes, little-endian
+    uint32_t mask;  // which bytes of head take part
+};
+struct SetIndex {  // ~30 KB, one cudaMalloc
+    uint32_t bitmap[65536 / 32];          // bit b0 | b1 << 8: some pattern starts with (b0, b1); length 1 sets (b0, *)
+    uint16_t keys[kMaxSetPatterns];       // distinct 2-byte keys of the patterns of length >= 2, ascending
+    uint16_t one[256];                    // 1 + id of the length-1 pattern b0, or 0
+    uint16_t group[kMaxSetPatterns + 1];  // CSR: patterns [group[g], group[g + 1]) have keys[g]
+    SetPattern pat[kMaxSetPatterns];      // patterns of length >= 2, sorted by key
+    uint8_t bytes[kMaxSetPatterns][kMaxPattern];  // pat[r]'s bytes
+};
+static_assert(offsetof(SetIndex, pat) % 16 == 0 && offsetof(SetIndex, bitmap) == 0, "SetIndex: 16-byte loads");
+struct FindSetArgs {
+    const uint8_t* src;
+    const TileRec* tiles;
+    const DevDesc* descs;
+    uint32_t n_tiles;
+    uint64_t src_lo16, src_hi16;
+    const SetIndex* set;
+    uint32_t n_keys;                   // distinct keys of length >= 2
+    uint32_t lmin, lmax;
+    const uint32_t* owned;             // per descriptor: starts >= owned[i] are not reported (nullptr: all are)
+    uint32_t* counts;                  // per descriptor, accumulated
+    unsigned long long* pattern_counts;  // per pattern, accumulated
+    uint32_t* matches;                 // {descriptor, position, pattern}: slots [0, cap) of the list
+    unsigned long long* total;
+    uint64_t cap;
+    uint32_t two = 2;
+};
+
 // Number of tiles an entry of `len` bytes occupies when its first destination byte sits at
 // (address & 15) == h0.
 __host__ __device__ inline uint32_t tiles_for_entry(uint32_t h0, uint32_t len)
@@ -104,6 +142,7 @@ cudaError_t upload_tables();  // jump tables -> __constant__ / global memory of 
 cudaError_t launch_batch(const BatchArgs& args, cudaStream_t stream);
 cudaError_t launch_batch_inline(const BatchArgs& args, const InlineDescs& descs, cudaStream_t stream);
 cudaError_t launch_find(const FindArgs& args, cudaStream_t stream);
+cudaError_t launch_find_set(const FindSetArgs& args, cudaStream_t stream);
 // Plan kernel: expands descriptors into per-tile records (binary search + jump-ahead per tile).
 cudaError_t launch_build_tiles(const DevDesc* descs, uint32_t n_descs, uint32_t dst_align, TileRec* tiles,
                                uint32_t n_tiles, cudaStream_t stream);

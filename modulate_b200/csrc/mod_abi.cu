@@ -16,6 +16,7 @@
 #include <cstring>
 #include <exception>
 #include <mutex>
+#include <memory>
 #include <new>
 #include <string>
 #include <thread>
@@ -849,6 +850,14 @@ struct mod_plan {
     std::vector<uint32_t> first_tile;   // n + 1 entries
 };
 
+struct mod_pattern_set {
+    int device = -1;
+    modk::SetIndex* d_index = nullptr;  // filter bitmap and index, built on the host
+    uint32_t n = 0;
+    uint32_t n_keys = 0;  // distinct 2-byte keys of the patterns of length >= 2
+    uint32_t lmin = 0, lmax = 0;
+};
+
 extern "C" {
 
 int mod_abi_version(void) { return MOD_ABI_VERSION; }
@@ -1260,8 +1269,48 @@ int mod_plan_run_window(const mod_plan* plan, uint64_t tile_begin, uint64_t tile
     return MOD_OK;
 }
 
-// Argument checks and the launch shared by mod_plan_find and mod_plan_find_window; `src_base` is the virtual
-// base (source byte 0 of the plan's space) and [lo16, hi16) the granules that may be loaded whole.
+// Checks shared by every search launch: the result buffers, the chunk grid on the source, the device.  `src_base`
+// is the virtual base (source byte 0 of the plan's space).
+static int find_check(const char* who, const mod_plan* plan, const uint8_t* src_base, const void* d_counts, const void* d_total,
+                      uint64_t cap, const void* d_matches)
+{
+    if (!d_counts || !d_total || (cap && !d_matches))
+        return fail(MOD_ERR_ARG, "%s: null result buffer", who);
+    // the search kernels need the chunk grid on the source: src_off - dst_off == delta for every entry and
+    // base + delta - dst_align == 0 (mod 16)
+    if (plan->uniform_delta < 0 || (((uintptr_t)src_base + (uintptr_t)plan->uniform_delta - plan->dst_align) & 15u) != 0u)
+        return fail(MOD_ERR_ALIGN, "%s: the plan's chunk grid does not lie on the source (build it with dst_off == src_off "
+                    "and dst_align == source address & 15)", who);
+    return plan_check_device(plan, who);
+}
+
+// Checks shared by the windowed searches: the tile range, the buffer, and that every byte the tiles read -- the up
+// to `halo` bytes past a tile that a match starting in it may cover included -- lies inside the window.
+static int find_window_check(const char* who, const mod_plan* plan, uint64_t tile_begin, uint64_t tile_end, const void* d_src_win,
+                             uint64_t src_win_off, uint64_t src_win_bytes, uint32_t halo)
+{
+    if (tile_begin > tile_end || tile_end > plan->n_tiles)
+        return fail(MOD_ERR_ARG, "%s: tiles [%llu, %llu) outside the plan's %u", who, (unsigned long long)tile_begin,
+                    (unsigned long long)tile_end, plan->n_tiles);
+    if (tile_begin < tile_end && !d_src_win)
+        return fail(MOD_ERR_ARG, "%s: null buffer", who);
+    const uint32_t* ft = plan->first_tile.data();
+    uint64_t e = tile_begin < tile_end ? (uint64_t)(std::upper_bound(ft, ft + plan->n + 1, (uint32_t)tile_begin) - ft) - 1 : plan->n;
+    for (; e < plan->n && ft[e] < tile_end; ++e) {
+        const mod_desc& d = plan->descs[e];
+        if (ft[e + 1] == ft[e])
+            continue;  // empty entry
+        const uint32_t h0 = (uint32_t)((plan->dst_align + d.dst_off) & 15u);
+        const uint64_t ta = std::max<uint64_t>(tile_begin, ft[e]) - ft[e], tb = std::min<uint64_t>(tile_end, ft[e + 1]) - ft[e];
+        const uint64_t b0 = ta == 0 ? 0 : ta * modk::kTileBytes - h0;
+        const uint64_t b1 = std::min<uint64_t>(d.len, tb * modk::kTileBytes - h0 + halo);
+        if (d.src_off + b0 < src_win_off || d.src_off + b1 > src_win_off + src_win_bytes)
+            return fail(MOD_ERR_ARG, "%s: entry %llu reads outside the source window", who, (unsigned long long)e);
+    }
+    return MOD_OK;
+}
+
+// The launch shared by mod_plan_find and mod_plan_find_window; [lo16, hi16) are the granules that may be loaded whole.
 static int plan_find_launch(const char* who, const mod_plan* plan, uint64_t tile_begin, uint64_t tile_end,
                             const uint8_t* src_base, uint64_t lo16, uint64_t hi16, const uint8_t* pattern, uint32_t len,
                             uint32_t* d_counts, mod_match* d_matches, uint64_t cap, uint64_t* d_total, void* stream)
@@ -1270,14 +1319,7 @@ static int plan_find_launch(const char* who, const mod_plan* plan, uint64_t tile
         return fail(MOD_ERR_ARG, "%s: the pattern must be 1 to %u bytes", who, modk::kMaxPattern);
     if (tile_begin == tile_end)
         return MOD_OK;
-    if (!d_counts || !d_total || (cap && !d_matches))
-        return fail(MOD_ERR_ARG, "%s: null result buffer", who);
-    // the search kernel needs the chunk grid on the source: src_off - dst_off == delta for every entry and
-    // base + delta - dst_align == 0 (mod 16)
-    if (plan->uniform_delta < 0 || (((uintptr_t)src_base + (uintptr_t)plan->uniform_delta - plan->dst_align) & 15u) != 0u)
-        return fail(MOD_ERR_ALIGN, "%s: the plan's chunk grid does not lie on the source (build it with dst_off == src_off "
-                    "and dst_align == source address & 15)", who);
-    int rc = plan_check_device(plan, who);
+    int rc = find_check(who, plan, src_base, d_counts, d_total, cap, d_matches);
     if (rc != MOD_OK)
         return rc;
     modk::FindArgs f;
@@ -1325,44 +1367,32 @@ int mod_plan_find_window(const mod_plan* plan, uint64_t tile_begin, uint64_t til
 {
     if (!plan)
         return fail(MOD_ERR_ARG, "mod_plan_find_window: null plan");
-    if (tile_begin > tile_end || tile_end > plan->n_tiles)
-        return fail(MOD_ERR_ARG, "mod_plan_find_window: tiles [%llu, %llu) outside the plan's %u",
-                    (unsigned long long)tile_begin, (unsigned long long)tile_end, plan->n_tiles);
     if (!pattern || len == 0 || len > modk::kMaxPattern)
         return fail(MOD_ERR_ARG, "mod_plan_find_window: the pattern must be 1 to %u bytes", modk::kMaxPattern);
-    if (tile_begin < tile_end && !d_src_win)
-        return fail(MOD_ERR_ARG, "mod_plan_find_window: null buffer");
-    // every byte the tile range reads, halos included, must lie inside the window
-    const uint32_t* ft = plan->first_tile.data();
-    uint64_t e = tile_begin < tile_end ? (uint64_t)(std::upper_bound(ft, ft + plan->n + 1, (uint32_t)tile_begin) - ft) - 1 : plan->n;
-    for (; e < plan->n && ft[e] < tile_end; ++e) {
-        const mod_desc& d = plan->descs[e];
-        if (ft[e + 1] == ft[e])
-            continue;  // empty entry
-        const uint32_t h0 = (uint32_t)((plan->dst_align + d.dst_off) & 15u);
-        const uint64_t ta = std::max<uint64_t>(tile_begin, ft[e]) - ft[e], tb = std::min<uint64_t>(tile_end, ft[e + 1]) - ft[e];
-        const uint64_t b0 = ta == 0 ? 0 : ta * modk::kTileBytes - h0;
-        const uint64_t b1 = std::min<uint64_t>(d.len, tb * modk::kTileBytes - h0 + (len - 1));
-        if (d.src_off + b0 < src_win_off || d.src_off + b1 > src_win_off + src_win_bytes)
-            return fail(MOD_ERR_ARG, "mod_plan_find_window: entry %llu reads outside the source window", (unsigned long long)e);
-    }
+    int rc = find_window_check("mod_plan_find_window", plan, tile_begin, tile_end, d_src_win, src_win_off, src_win_bytes, len - 1);
+    if (rc != MOD_OK)
+        return rc;
     return plan_find_launch("mod_plan_find_window", plan, tile_begin, tile_end, (const uint8_t*)d_src_win - src_win_off,
                             ((uint64_t)(uintptr_t)d_src_win + 15u) & ~15ull,
                             ((uint64_t)(uintptr_t)d_src_win + src_win_bytes) & ~15ull, pattern, len, d_counts, d_matches,
                             cap, d_total, stream);
 }
 
-int mod_find_batch(const mod_desc* descs, uint64_t n, const void* d_src, uint64_t src_bytes, const uint8_t* pattern,
-                   uint32_t len, uint32_t* counts_out, mod_match* matches_out, uint64_t cap, uint64_t* total_out)
+// Plan + one search launch + destroy, synchronous: the body of mod_find_batch and mod_find_set_batch.  One device
+// allocation holds the total, the counts per descriptor, `aux_bytes` of counts per pattern and a list of `cap`
+// records of `rec` bytes; `launch(plan, d_counts, d_aux, d_list, d_total)` enqueues the search on the legacy
+// stream.  Everything comes back but the list order, which the caller sorts.
+extern "C++" {  // a template cannot have C linkage
+template <class Launch>
+static int find_batch_run(const char* who, const mod_desc* descs, uint64_t n, const void* d_src, uint64_t src_bytes,
+                          uint32_t* counts_out, void* aux_out, uint64_t aux_bytes, void* matches_out, uint64_t rec,
+                          uint64_t cap, uint64_t* total_out, Launch launch)
 {
-    MOD_ABI_BEGIN
-    if (!pattern || len == 0 || len > modk::kMaxPattern)
-        return fail(MOD_ERR_ARG, "mod_find_batch: the pattern must be 1 to %u bytes", modk::kMaxPattern);
-    if ((n && (!descs || !counts_out)) || !total_out || (cap && !matches_out))
-        return fail(MOD_ERR_ARG, "mod_find_batch: null argument");
+    if ((n && (!descs || !counts_out)) || !total_out || (cap && !matches_out) || (aux_bytes && !aux_out))
+        return fail(MOD_ERR_ARG, "%s: null argument", who);
     int src_dev = -1;
     if (!d_src || !pointer_device(d_src, &src_dev))
-        return fail(MOD_ERR_ARG, "mod_find_batch: d_src must be device memory (stream host data with CArk::FindInFiles)");
+        return fail(MOD_ERR_ARG, "%s: d_src must be device memory (stream host data with CArk::FindInFiles)", who);
     DeviceGuard guard;
     int rc = guard.enter(src_dev);
     if (rc != MOD_OK)
@@ -1373,29 +1403,31 @@ int mod_find_batch(const mod_desc* descs, uint64_t n, const void* d_src, uint64_
     mod_plan* plan = nullptr;
     if ((rc = mod_plan_create(own.data(), n, src_bytes, src_bytes, (uint32_t)((uintptr_t)d_src & 15u), &plan)) != MOD_OK)
         return rc;
-    // one allocation: total, counts, list
-    const uint64_t counts_at = 16, list_at = (counts_at + 4 * n + 15) & ~15ull, bytes = list_at + 8 * cap;
+    // one allocation: total, counts, counts per pattern, list
+    const uint64_t counts_at = 16, aux_at = (counts_at + 4 * n + 15) & ~15ull, list_at = (aux_at + aux_bytes + 15) & ~15ull,
+                   bytes = list_at + rec * cap;
     uint8_t* d_out = nullptr;
     cudaError_t e = cudaMalloc((void**)&d_out, bytes);
     if (e != cudaSuccess) {
         cudaGetLastError();
         mod_plan_destroy(plan);
-        return fail(MOD_ERR_NOMEM, "mod_find_batch: cudaMalloc(%llu): %s", (unsigned long long)bytes, cudaGetErrorString(e));
+        return fail(MOD_ERR_NOMEM, "%s: cudaMalloc(%llu): %s", who, (unsigned long long)bytes, cudaGetErrorString(e));
     }
     e = cudaMemsetAsync(d_out, 0, list_at, nullptr);
     if (e == cudaSuccess)
-        rc = mod_plan_find(plan, d_src, pattern, len, (uint32_t*)(d_out + counts_at), (mod_match*)(d_out + list_at), cap,
-                           (uint64_t*)d_out, nullptr);
+        rc = launch(plan, (uint32_t*)(d_out + counts_at), d_out + aux_at, d_out + list_at, (uint64_t*)d_out);
     uint64_t total = 0;
     if (e == cudaSuccess && rc == MOD_OK)
         e = cudaMemcpyAsync(&total, d_out, 8, cudaMemcpyDeviceToHost, nullptr);
     if (e == cudaSuccess && rc == MOD_OK && n)
         e = cudaMemcpyAsync(counts_out, d_out + counts_at, 4 * n, cudaMemcpyDeviceToHost, nullptr);
+    if (e == cudaSuccess && rc == MOD_OK && aux_bytes)
+        e = cudaMemcpyAsync(aux_out, d_out + aux_at, aux_bytes, cudaMemcpyDeviceToHost, nullptr);
     if (e == cudaSuccess && rc == MOD_OK)
         e = cudaStreamSynchronize(nullptr);
     const uint64_t kept = std::min(total, cap);
     if (e == cudaSuccess && rc == MOD_OK && kept)
-        e = cudaMemcpyAsync(matches_out, d_out + list_at, 8 * kept, cudaMemcpyDeviceToHost, nullptr);
+        e = cudaMemcpyAsync(matches_out, d_out + list_at, rec * kept, cudaMemcpyDeviceToHost, nullptr);
     if (e == cudaSuccess && rc == MOD_OK)
         e = cudaStreamSynchronize(nullptr);
     cudaFree(d_out);
@@ -1403,11 +1435,224 @@ int mod_find_batch(const mod_desc* descs, uint64_t n, const void* d_src, uint64_
     if (rc != MOD_OK)
         return rc;
     CUDA_TRY(e);
-    std::sort(matches_out, matches_out + kept,
-              [](const mod_match& a, const mod_match& b) { return a.desc != b.desc ? a.desc < b.desc : a.pos < b.pos; });
     *total_out = total;
     return MOD_OK;
+}
+}
+
+int mod_find_batch(const mod_desc* descs, uint64_t n, const void* d_src, uint64_t src_bytes, const uint8_t* pattern,
+                   uint32_t len, uint32_t* counts_out, mod_match* matches_out, uint64_t cap, uint64_t* total_out)
+{
+    MOD_ABI_BEGIN
+    if (!pattern || len == 0 || len > modk::kMaxPattern)
+        return fail(MOD_ERR_ARG, "mod_find_batch: the pattern must be 1 to %u bytes", modk::kMaxPattern);
+    const int rc = find_batch_run("mod_find_batch", descs, n, d_src, src_bytes, counts_out, nullptr, 0, matches_out, 8, cap,
+                                  total_out, [&](mod_plan* plan, uint32_t* d_counts, uint8_t*, uint8_t* d_list, uint64_t* d_total) {
+                                      return mod_plan_find(plan, d_src, pattern, len, d_counts, (mod_match*)d_list, cap, d_total,
+                                                           nullptr);
+                                  });
+    if (rc != MOD_OK)
+        return rc;
+    std::sort(matches_out, matches_out + std::min(*total_out, cap),
+              [](const mod_match& a, const mod_match& b) { return a.desc != b.desc ? a.desc < b.desc : a.pos < b.pos; });
+    return MOD_OK;
     MOD_ABI_END("mod_find_batch")
+}
+
+/* ---- pattern sets ------------------------------------------------------------------------------ */
+
+int mod_pattern_set_create(const uint8_t* bytes, const uint32_t* lens, uint32_t n, mod_pattern_set** out)
+{
+    MOD_ABI_BEGIN
+    if (!out)
+        return fail(MOD_ERR_ARG, "mod_pattern_set_create: out is null");
+    *out = nullptr;
+    if (!bytes || !lens || n == 0 || n > modk::kMaxSetPatterns)
+        return fail(MOD_ERR_ARG, "mod_pattern_set_create: a set holds 1 to %u patterns", modk::kMaxSetPatterns);
+    std::vector<std::string> pats(n);
+    uint64_t at = 0;
+    for (uint32_t j = 0; j < n; ++j) {
+        if (lens[j] == 0 || lens[j] > modk::kMaxPattern)
+            return fail(MOD_ERR_ARG, "mod_pattern_set_create: pattern %u is %u bytes, not 1 to %u", j, lens[j], modk::kMaxPattern);
+        pats[j].assign((const char*)bytes + at, lens[j]);
+        at += lens[j];
+    }
+    std::vector<uint32_t> order(n);
+    for (uint32_t j = 0; j < n; ++j)
+        order[j] = j;
+    std::sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return pats[a] != pats[b] ? pats[a] < pats[b] : a < b; });
+    for (uint32_t j = 1; j < n; ++j)
+        if (pats[order[j]] == pats[order[j - 1]])
+            return fail(MOD_ERR_ARG, "mod_pattern_set_create: patterns %u and %u are the same", order[j - 1], order[j]);
+
+    // the index: filter bits, the length-1 table, and the longer patterns sorted by their 2-byte key
+    std::unique_ptr<modk::SetIndex> idx(new modk::SetIndex());
+    std::memset(idx.get(), 0, sizeof(modk::SetIndex));
+    auto key_of = [&](uint32_t j) { return (uint32_t)(uint8_t)pats[j][0] | ((uint32_t)(uint8_t)pats[j][1] << 8); };
+    std::vector<uint32_t> longer;
+    uint32_t lmin = modk::kMaxPattern, lmax = 1;
+    for (uint32_t j = 0; j < n; ++j) {
+        lmin = std::min(lmin, lens[j]);
+        lmax = std::max(lmax, lens[j]);
+        const uint32_t b0 = (uint8_t)pats[j][0];
+        if (lens[j] == 1) {
+            idx->one[b0] = (uint16_t)(j + 1);
+            for (uint32_t b1 = 0; b1 < 256; ++b1)
+                idx->bitmap[(b0 | b1 << 8) >> 5] |= 1u << ((b0 | b1 << 8) & 31u);
+        } else {
+            idx->bitmap[key_of(j) >> 5] |= 1u << (key_of(j) & 31u);
+            longer.push_back(j);
+        }
+    }
+    std::sort(longer.begin(), longer.end(), [&](uint32_t a, uint32_t b) { return key_of(a) != key_of(b) ? key_of(a) < key_of(b) : a < b; });
+    uint32_t n_keys = 0;
+    for (uint32_t r = 0; r < longer.size(); ++r) {
+        const uint32_t j = longer[r];
+        if (r == 0 || key_of(j) != key_of(longer[r - 1])) {
+            idx->keys[n_keys] = (uint16_t)key_of(j);
+            idx->group[n_keys++] = (uint16_t)r;
+        }
+        modk::SetPattern& sp = idx->pat[r];
+        sp.id = j;
+        sp.len = lens[j];
+        for (uint32_t k = 0; k < 4 && k < lens[j]; ++k) {
+            sp.head |= (uint32_t)(uint8_t)pats[j][k] << (8 * k);
+            sp.mask |= 0xFFu << (8 * k);
+        }
+        std::memcpy(idx->bytes[r], pats[j].data(), lens[j]);
+    }
+    idx->group[n_keys] = (uint16_t)longer.size();
+
+    DeviceCtx* c = nullptr;
+    int rc = acquire(-1, &c);
+    if (rc != MOD_OK)
+        return rc;
+    modk::SetIndex* d_idx = nullptr;
+    CUDA_TRY(cudaMalloc((void**)&d_idx, sizeof(modk::SetIndex)));
+    cudaError_t e = cudaMemcpyAsync(d_idx, idx.get(), sizeof(modk::SetIndex), cudaMemcpyHostToDevice, nullptr);
+    if (e == cudaSuccess)
+        e = cudaStreamSynchronize(nullptr);
+    if (e != cudaSuccess) {
+        cudaFree(d_idx);
+        return fail(MOD_ERR_CUDA, "mod_pattern_set_create: %s", cudaGetErrorString(e));
+    }
+    mod_pattern_set* set = new mod_pattern_set();
+    set->device = c->device;
+    set->d_index = d_idx;
+    set->n = n;
+    set->n_keys = n_keys;
+    set->lmin = lmin;
+    set->lmax = lmax;
+    *out = set;
+    return MOD_OK;
+    MOD_ABI_END("mod_pattern_set_create")
+}
+
+int mod_pattern_set_destroy(mod_pattern_set* set)
+{
+    if (!set)
+        return MOD_OK;
+    if (set->d_index) {
+        DeviceGuard guard;
+        guard.enter(set->device);
+        cudaDeviceSynchronize();  // launches that still read the index finish first
+        cudaFree(set->d_index);
+    }
+    delete set;
+    return MOD_OK;
+}
+
+// The launch shared by mod_plan_find_set and mod_plan_find_set_window.
+static int plan_find_set_launch(const char* who, const mod_plan* plan, uint64_t tile_begin, uint64_t tile_end,
+                                const uint8_t* src_base, uint64_t lo16, uint64_t hi16, const mod_pattern_set* set,
+                                const uint32_t* d_owned, uint32_t* d_counts, uint64_t* d_pattern_counts,
+                                mod_set_match* d_matches, uint64_t cap, uint64_t* d_total, void* stream)
+{
+    if (tile_begin == tile_end)
+        return MOD_OK;
+    if (!d_pattern_counts)
+        return fail(MOD_ERR_ARG, "%s: null result buffer", who);
+    int rc = find_check(who, plan, src_base, d_counts, d_total, cap, d_matches);
+    if (rc != MOD_OK)
+        return rc;
+    if (set->device != plan->device)
+        return fail(MOD_ERR_ARG, "%s: the pattern set lives on device %d but the plan on device %d", who, set->device, plan->device);
+    modk::FindSetArgs f;
+    f.src = src_base;
+    f.tiles = plan->d_tiles + tile_begin;
+    f.descs = plan->d_descs;
+    f.n_tiles = (uint32_t)(tile_end - tile_begin);
+    f.src_lo16 = lo16;
+    f.src_hi16 = hi16;
+    f.set = set->d_index;
+    f.n_keys = set->n_keys;
+    f.lmin = set->lmin;
+    f.lmax = set->lmax;
+    f.owned = d_owned;
+    f.counts = d_counts;
+    f.pattern_counts = (unsigned long long*)d_pattern_counts;
+    f.matches = (uint32_t*)d_matches;
+    f.total = (unsigned long long*)d_total;
+    f.cap = cap;
+    CUDA_TRY(modk::launch_find_set(f, (cudaStream_t)stream));
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    return MOD_OK;
+}
+
+int mod_plan_find_set(const mod_plan* plan, const void* d_src, const mod_pattern_set* set, const uint32_t* d_owned,
+                      uint32_t* d_counts, uint64_t* d_pattern_counts, mod_set_match* d_matches, uint64_t cap,
+                      uint64_t* d_total, void* stream)
+{
+    if (!plan || !set)
+        return fail(MOD_ERR_ARG, "mod_plan_find_set: null plan or pattern set");
+    if (!d_src && plan->n_tiles)
+        return fail(MOD_ERR_ARG, "mod_plan_find_set: null buffer");
+    return plan_find_set_launch("mod_plan_find_set", plan, 0, plan->n_tiles, (const uint8_t*)d_src,
+                                ((uint64_t)(uintptr_t)d_src + 15u) & ~15ull,
+                                ((uint64_t)(uintptr_t)d_src + plan->src_bytes) & ~15ull, set, d_owned, d_counts,
+                                d_pattern_counts, d_matches, cap, d_total, stream);
+}
+
+int mod_plan_find_set_window(const mod_plan* plan, uint64_t tile_begin, uint64_t tile_end, const void* d_src_win,
+                             uint64_t src_win_off, uint64_t src_win_bytes, const mod_pattern_set* set,
+                             const uint32_t* d_owned, uint32_t* d_counts, uint64_t* d_pattern_counts,
+                             mod_set_match* d_matches, uint64_t cap, uint64_t* d_total, void* stream)
+{
+    if (!plan || !set)
+        return fail(MOD_ERR_ARG, "mod_plan_find_set_window: null plan or pattern set");
+    int rc = find_window_check("mod_plan_find_set_window", plan, tile_begin, tile_end, d_src_win, src_win_off, src_win_bytes,
+                               set->lmax - 1);
+    if (rc != MOD_OK)
+        return rc;
+    return plan_find_set_launch("mod_plan_find_set_window", plan, tile_begin, tile_end, (const uint8_t*)d_src_win - src_win_off,
+                                ((uint64_t)(uintptr_t)d_src_win + 15u) & ~15ull,
+                                ((uint64_t)(uintptr_t)d_src_win + src_win_bytes) & ~15ull, set, d_owned, d_counts,
+                                d_pattern_counts, d_matches, cap, d_total, stream);
+}
+
+int mod_find_set_batch(const mod_desc* descs, uint64_t n, const void* d_src, uint64_t src_bytes, const uint8_t* bytes,
+                       const uint32_t* lens, uint32_t n_patterns, uint32_t* counts_out, uint64_t* pattern_counts_out,
+                       mod_set_match* matches_out, uint64_t cap, uint64_t* total_out)
+{
+    MOD_ABI_BEGIN
+    if (!pattern_counts_out)
+        return fail(MOD_ERR_ARG, "mod_find_set_batch: null argument");
+    mod_pattern_set* set = nullptr;
+    int rc = find_batch_run("mod_find_set_batch", descs, n, d_src, src_bytes, counts_out, pattern_counts_out,
+                            8ull * n_patterns, matches_out, sizeof(mod_set_match), cap, total_out,
+                            [&](mod_plan* plan, uint32_t* d_counts, uint8_t* d_aux, uint8_t* d_list, uint64_t* d_total) {
+                                const int r = mod_pattern_set_create(bytes, lens, n_patterns, &set);
+                                return r != MOD_OK ? r : mod_plan_find_set(plan, d_src, set, nullptr, d_counts, (uint64_t*)d_aux,
+                                                                           (mod_set_match*)d_list, cap, d_total, nullptr);
+                            });
+    mod_pattern_set_destroy(set);
+    if (rc != MOD_OK)
+        return rc;
+    std::sort(matches_out, matches_out + std::min(*total_out, cap), [](const mod_set_match& a, const mod_set_match& b) {
+        return a.desc != b.desc ? a.desc < b.desc : a.pos != b.pos ? a.pos < b.pos : a.pattern < b.pattern;
+    });
+    return MOD_OK;
+    MOD_ABI_END("mod_find_set_batch")
 }
 
 int mod_cycle_batch(const mod_desc* descs, uint64_t n, const void* src, uint64_t src_bytes, void* dst,
