@@ -9,6 +9,7 @@
  *   mod_ark_find     search every entry for a byte pattern (CArk::Load + CArk::FindInFiles; no
  *                    reference counterpart)
  *   mod_ark_find_set the same for a set of patterns in one pass (CArk::FindSetInFiles)
+ *   mod_ark_find_masked / mod_ark_find_set_nocase  wildcard and case-insensitive forms of the two
  *   mod_ark_pack     Pack     (reference Modulate.cpp:380-450: song list from the DTA configs unless
  *                              pack_all, CArk::Load of the reference header, ConstructFromDirectory,
  *                              BuildArk, SaveArk)
@@ -48,6 +49,17 @@ int mod_ark_find(const char* header_path, const char* part_dir, const uint8_t* p
 int mod_ark_find_set(const char* header_path, const char* part_dir, const uint8_t* bytes, const uint32_t* lens, uint32_t n,
                      int32_t body_key, uint64_t max_matches, uint32_t* out_file, uint32_t* out_offset, uint32_t* out_pattern,
                      uint64_t* out_total, uint64_t* out_pattern_counts);
+
+/* mod_ark_find with a mask byte per pattern byte (CArk::FindMaskedInFiles): an entry byte t matches pattern byte k
+ * when ((t ^ pattern[k]) & mask[k]) == 0 -- 0x00 is any byte, 0xDF on an upper-case letter either case.  A null or
+ * all-zero mask is eError_InvalidParameter. */
+int mod_ark_find_masked(const char* header_path, const char* part_dir, const uint8_t* pattern, const uint8_t* mask, uint32_t len,
+                        int32_t body_key, uint64_t max_matches, uint32_t* out_file, uint32_t* out_offset, uint64_t* out_total);
+
+/* mod_ark_find_set ignoring ASCII case (mod_pattern_set_create_nocase): the patterns must differ ignoring case. */
+int mod_ark_find_set_nocase(const char* header_path, const char* part_dir, const uint8_t* bytes, const uint32_t* lens, uint32_t n,
+                            int32_t body_key, uint64_t max_matches, uint32_t* out_file, uint32_t* out_offset,
+                            uint32_t* out_pattern, uint64_t* out_total, uint64_t* out_pattern_counts);
 
 /* `input_dir` and `output_dir` must end in '/'; the header is written to output_dir + header_name. */
 int mod_ark_pack(const char* reference_header_path, const char* input_dir, const char* output_dir,

@@ -198,6 +198,27 @@ int mod_plan_find_window(const mod_plan* plan, uint64_t tile_begin, uint64_t til
 int mod_find_batch(const mod_desc* descs, uint64_t n, const void* d_src, uint64_t src_bytes, const uint8_t* pattern,
                    uint32_t len, uint32_t* counts_out, mod_match* matches_out, uint64_t cap, uint64_t* total_out);
 
+/* ---- masked search: wildcard bytes and nibbles, ASCII case folding --------------------------- */
+
+/* mod_plan_find with a mask byte per pattern byte: byte t matches pattern byte k when
+ * ((t ^ pattern[k]) & mask[k]) == 0.  mask 0xFF is an exact byte, 0x00 any byte, 0xF0 / 0x0F leave one nibble
+ * free, and 0xDF with pattern[k] in 'A'..'Z' matches that letter in either case.  The results, their accumulation
+ * and the cap are mod_plan_find's.  MOD_ERR_ARG for a null mask, len outside 1..64 and an all-zero mask.  An
+ * all-0xFF mask runs the exact search.  Asynchronous on `stream`. */
+int mod_plan_find_masked(const mod_plan* plan, const void* d_src, const uint8_t* pattern, const uint8_t* mask, uint32_t len,
+                         uint32_t* d_counts, mod_match* d_matches, uint64_t cap, uint64_t* d_total, void* stream);
+
+/* mod_plan_find_window with a mask, as mod_plan_find_masked. */
+int mod_plan_find_masked_window(const mod_plan* plan, uint64_t tile_begin, uint64_t tile_end, const void* d_src_win,
+                                uint64_t src_win_off, uint64_t src_win_bytes, const uint8_t* pattern, const uint8_t* mask,
+                                uint32_t len, uint32_t* d_counts, mod_match* d_matches, uint64_t cap, uint64_t* d_total,
+                                void* stream);
+
+/* mod_find_batch with a mask, as mod_plan_find_masked. */
+int mod_find_masked_batch(const mod_desc* descs, uint64_t n, const void* d_src, uint64_t src_bytes, const uint8_t* pattern,
+                          const uint8_t* mask, uint32_t len, uint32_t* counts_out, mod_match* matches_out, uint64_t cap,
+                          uint64_t* total_out);
+
 /* ---- search for a set of patterns in one pass ------------------------------------------------ */
 
 typedef struct mod_pattern_set mod_pattern_set; /* opaque: the set's filter and index, resident in HBM */
@@ -215,6 +236,11 @@ typedef struct mod_set_match {
  * refused.  Every invalid input is MOD_ERR_ARG, checked on the host.  Synchronous. */
 int mod_pattern_set_create(const uint8_t* bytes, const uint32_t* lens, uint32_t n, mod_pattern_set** out);
 int mod_pattern_set_destroy(mod_pattern_set* set);
+
+/* mod_pattern_set_create for a case-insensitive search: ASCII letters 'A'..'Z' match 'a'..'z' and back, every other
+ * byte only itself.  Two patterns that are equal ignoring case are refused.  The set is searched with
+ * mod_plan_find_set / _window like any other. */
+int mod_pattern_set_create_nocase(const uint8_t* bytes, const uint32_t* lens, uint32_t n, mod_pattern_set** out);
 
 /* mod_plan_find for every pattern of `set` in one pass over the source.  A match is a pair (pattern j, start p)
  * with p + len_j <= len whose bytes equal pattern j: overlapping matches count, and so do matches of different

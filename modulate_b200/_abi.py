@@ -71,7 +71,18 @@ SIGNATURES = {
                                             ctypes.c_void_p]),
     "mod_find_batch": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_uint64, ctypes.c_void_p, ctypes.c_uint64, ctypes.c_void_p,
                                       ctypes.c_uint32, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint64, ctypes.c_void_p]),
+    "mod_plan_find_masked": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint32,
+                                            ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint64, ctypes.c_void_p, ctypes.c_void_p]),
+    "mod_plan_find_masked_window": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_uint64, ctypes.c_uint64, ctypes.c_void_p,
+                                                   ctypes.c_uint64, ctypes.c_uint64, ctypes.c_void_p, ctypes.c_void_p,
+                                                   ctypes.c_uint32, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint64,
+                                                   ctypes.c_void_p, ctypes.c_void_p]),
+    "mod_find_masked_batch": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_uint64, ctypes.c_void_p, ctypes.c_uint64, ctypes.c_void_p,
+                                             ctypes.c_void_p, ctypes.c_uint32, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint64,
+                                             ctypes.c_void_p]),
     "mod_pattern_set_create": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint32, ctypes.POINTER(ctypes.c_void_p)]),
+    "mod_pattern_set_create_nocase": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint32,
+                                                     ctypes.POINTER(ctypes.c_void_p)]),
     "mod_pattern_set_destroy": (ctypes.c_int, [ctypes.c_void_p]),
     "mod_plan_find_set": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
                                          ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint64, ctypes.c_void_p, ctypes.c_void_p]),
@@ -90,6 +101,12 @@ SIGNATURES = {
     "mod_ark_find_set": (ctypes.c_int, [ctypes.c_char_p, ctypes.c_char_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint32,
                                         ctypes.c_int32, ctypes.c_uint64, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
                                         ctypes.POINTER(ctypes.c_uint64), ctypes.c_void_p]),
+    "mod_ark_find_masked": (ctypes.c_int, [ctypes.c_char_p, ctypes.c_char_p, ctypes.c_char_p, ctypes.c_char_p, ctypes.c_uint32,
+                                           ctypes.c_int32, ctypes.c_uint64, ctypes.c_void_p, ctypes.c_void_p,
+                                           ctypes.POINTER(ctypes.c_uint64)]),
+    "mod_ark_find_set_nocase": (ctypes.c_int, [ctypes.c_char_p, ctypes.c_char_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint32,
+                                               ctypes.c_int32, ctypes.c_uint64, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
+                                               ctypes.POINTER(ctypes.c_uint64), ctypes.c_void_p]),
     "mod_dta_set_int": (ctypes.c_int, [ctypes.c_char_p, ctypes.c_char_p, ctypes.c_int32]),
     "mod_shard_range": (ctypes.c_int, [ctypes.c_uint64, ctypes.c_int, ctypes.c_int,
                                        ctypes.POINTER(ctypes.c_uint64), ctypes.POINTER(ctypes.c_uint64)]),

@@ -123,32 +123,70 @@ def _pattern(pattern: Any) -> bytes:
     return p
 
 
+def _mask(mask: Any, n: int) -> bytes:
+    m = bytes(mask)
+    if len(m) != n:
+        raise ValueError(f"the mask must have one byte per pattern byte ({n}), not {len(m)}")
+    return m
+
+
+def _fold(p: bytes) -> bytes:
+    """ASCII upper case: b'a'..b'z' -> b'A'..b'Z', every other byte itself."""
+    return bytes(b - 0x20 if 0x61 <= b <= 0x7A else b for b in p)
+
+
+def wildcard_pattern(hex_text: str) -> Tuple[bytes, bytes]:
+    """(pattern, mask) of hex digit pairs in which any digit may be ``?`` (any nibble; ``??`` any byte), whitespace
+    ignored -- the ``-findwild`` syntax.  ``wildcard_pattern("0a ?? 4?")`` -> (b"\x0a\x00\x40", b"\xff\x00\xf0")."""
+    digits = "".join(hex_text.split()).lower()
+    if len(digits) % 2 or any(c not in "0123456789abcdef?" for c in digits):
+        raise ValueError(f"not pairs of hex digits or ?: {hex_text!r}")
+    if not 1 <= len(digits) // 2 <= MAX_PATTERN:
+        raise ValueError(f"the pattern must be 1 to {MAX_PATTERN} bytes, not {len(digits) // 2}")
+    if set(digits) == {"?"}:
+        raise ValueError("the pattern has no hex digit that is not ?")
+    value = bytes(int(digits[i:i + 2].replace("?", "0"), 16) for i in range(0, len(digits), 2))
+    mask = bytes((0 if digits[i] == "?" else 0xF0) | (0 if digits[i + 1] == "?" else 0x0F) for i in range(0, len(digits), 2))
+    return value, mask
+
+
+def ignore_case_pattern(text: Any) -> Tuple[bytes, bytes]:
+    """(pattern, mask) that matches `text` with every ASCII letter in either case: letters upper-cased with mask 0xDF,
+    every other byte exact (0xFF)."""
+    p = _fold(_pattern(text))
+    return p, bytes(0xDF if 0x41 <= b <= 0x5A else 0xFF for b in p)
+
+
 # numpy view of ``mod_set_match``: pattern `pattern` of a set starts at `pos` inside descriptor `desc`
 SET_MATCH_DTYPE = np.dtype([("desc", "<u4"), ("pos", "<u4"), ("pattern", "<u4")])
 MAX_SET_PATTERNS = 256
 
 
-def _pattern_list(patterns: Any) -> Tuple[np.ndarray, np.ndarray]:
-    """-> (concatenated bytes, uint32 lengths) of 1 to 256 distinct patterns of 1 to 64 bytes."""
+def _pattern_list(patterns: Any, ignore_case: bool = False) -> Tuple[np.ndarray, np.ndarray]:
+    """-> (concatenated bytes, uint32 lengths) of 1 to 256 distinct patterns of 1 to 64 bytes (distinct ignoring ASCII
+    case with `ignore_case`)."""
     ps = [_pattern(p) for p in patterns]
     if not 1 <= len(ps) <= MAX_SET_PATTERNS:
         raise ValueError(f"a set holds 1 to {MAX_SET_PATTERNS} patterns, not {len(ps)}")
-    if len(set(ps)) != len(ps):
-        raise ValueError("the set holds the same pattern twice")
+    if len(set(_fold(p) if ignore_case else p for p in ps)) != len(ps):
+        raise ValueError("the set holds the same pattern twice" + (" ignoring case" if ignore_case else ""))
     return np.frombuffer(b"".join(ps), np.uint8).copy(), np.array([len(p) for p in ps], np.uint32)
 
 
 class PatternSet:
     """A set of 1 to 256 distinct byte patterns (1 to 64 bytes each, lengths mixed) resident on the current
-    device, for ``Plan.find_set``: its filter and index are the library's business."""
+    device, for ``Plan.find_set``: its filter and index are the library's business.  With `ignore_case` ASCII letters
+    match either case (``mod_pattern_set_create_nocase``), and the patterns must differ ignoring case."""
 
-    def __init__(self, patterns: Any):
-        data, lens = _pattern_list(patterns)
+    def __init__(self, patterns: Any, ignore_case: bool = False):
+        data, lens = _pattern_list(patterns, ignore_case)
         self._lib = _abi.load()
         self._handle = ctypes.c_void_p()
-        _abi.check(self._lib.mod_pattern_set_create(data.ctypes.data, lens.ctypes.data, len(lens), ctypes.byref(self._handle)))
+        create = self._lib.mod_pattern_set_create_nocase if ignore_case else self._lib.mod_pattern_set_create
+        _abi.check(create(data.ctypes.data, lens.ctypes.data, len(lens), ctypes.byref(self._handle)))
         self.n = len(lens)
         self.lengths = lens
+        self.ignore_case = bool(ignore_case)
 
     def close(self) -> None:
         if self._handle:
@@ -207,23 +245,30 @@ class Plan:
                                                  int(src_win_off), int(src_win_bytes), d_addr, int(dst_win_off),
                                                  int(dst_win_bytes), stream or None))
 
-    def find(self, src: Any, pattern: Any, counts: Any, matches: Any, cap: int, total: Any, stream: int = 0) -> None:
+    def find(self, src: Any, pattern: Any, counts: Any, matches: Any, cap: int, total: Any, stream: int = 0,
+             mask: Any = None) -> None:
         """Asynchronous search (``mod_plan_find``) of every descriptor for `pattern`: `counts` (uint32 per
         descriptor), `matches` (``MATCH_DTYPE`` slots, `cap` of them) and `total` (one uint64) are device buffers
-        the results ACCUMULATE into.  The plan must have dst_off == src_off and dst_align == src & 15."""
+        the results ACCUMULATE into.  The plan must have dst_off == src_off and dst_align == src & 15.  `mask` (one
+        byte per pattern byte; ``mod_plan_find_masked``): byte t matches pattern byte k when
+        ``(t ^ pattern[k]) & mask[k] == 0`` -- see ``wildcard_pattern`` and ``ignore_case_pattern``."""
         p = _pattern(pattern)
-        _abi.check(self._lib.mod_plan_find(self._handle, _buffer_info(src)[0], p, len(p), _buffer_info(counts)[0],
-                                           _buffer_info(matches)[0] if cap else None, int(cap), _buffer_info(total)[0],
-                                           stream or None))
+        args = (_buffer_info(counts)[0], _buffer_info(matches)[0] if cap else None, int(cap), _buffer_info(total)[0], stream or None)
+        if mask is None:
+            _abi.check(self._lib.mod_plan_find(self._handle, _buffer_info(src)[0], p, len(p), *args))
+        else:
+            _abi.check(self._lib.mod_plan_find_masked(self._handle, _buffer_info(src)[0], p, _mask(mask, len(p)), len(p), *args))
 
     def find_window(self, tile_begin: int, tile_end: int, src_win: Any, src_win_off: int, src_win_bytes: int,
-                    pattern: Any, counts: Any, matches: Any, cap: int, total: Any, stream: int = 0) -> None:
+                    pattern: Any, counts: Any, matches: Any, cap: int, total: Any, stream: int = 0, mask: Any = None) -> None:
         """``find`` over a tile sub-range with only a window of the source resident (slot-ring streaming)."""
         p = _pattern(pattern)
-        _abi.check(self._lib.mod_plan_find_window(self._handle, int(tile_begin), int(tile_end), _buffer_info(src_win)[0],
-                                                  int(src_win_off), int(src_win_bytes), p, len(p), _buffer_info(counts)[0],
-                                                  _buffer_info(matches)[0] if cap else None, int(cap),
-                                                  _buffer_info(total)[0], stream or None))
+        win = (self._handle, int(tile_begin), int(tile_end), _buffer_info(src_win)[0], int(src_win_off), int(src_win_bytes))
+        args = (_buffer_info(counts)[0], _buffer_info(matches)[0] if cap else None, int(cap), _buffer_info(total)[0], stream or None)
+        if mask is None:
+            _abi.check(self._lib.mod_plan_find_window(*win, p, len(p), *args))
+        else:
+            _abi.check(self._lib.mod_plan_find_masked_window(*win, p, _mask(mask, len(p)), len(p), *args))
 
     def find_set(self, src: Any, pattern_set: PatternSet, counts: Any, pattern_counts: Any, matches: Any, cap: int, total: Any,
                  owned: Any = None, stream: int = 0) -> None:
@@ -274,10 +319,10 @@ def cycle_batch(descs: np.ndarray, src: Any, dst: Any, src_bytes: Optional[int] 
 
 
 def find_batch(descs: np.ndarray, src: Any, pattern: Any, src_bytes: Optional[int] = None,
-               max_matches: int = 1 << 20) -> Tuple[np.ndarray, np.ndarray, int]:
+               max_matches: int = 1 << 20, mask: Any = None) -> Tuple[np.ndarray, np.ndarray, int]:
     """Search each descriptor's deciphered bytes (``src`` on the device: a raw address or a CUDA tensor) for
     `pattern` (synchronous).  -> (counts uint32[n], matches ``MATCH_DTYPE`` sorted by (desc, pos), at most
-    `max_matches` of them, exact total)."""
+    `max_matches` of them, exact total).  `mask`: as for ``Plan.find`` (``mod_find_masked_batch``)."""
     d = _descs(descs)
     p = _pattern(pattern)
     s_addr, s_n, _ = _buffer_info(src)
@@ -287,9 +332,12 @@ def find_batch(descs: np.ndarray, src: Any, pattern: Any, src_bytes: Optional[in
     counts = np.zeros(len(d), dtype=np.uint32)
     matches = np.zeros(max(0, int(max_matches)), dtype=MATCH_DTYPE)
     total = ctypes.c_uint64()
-    _abi.check(_abi.load().mod_find_batch(d.ctypes.data if len(d) else None, len(d), s_addr, int(src_bytes), p, len(p),
-                                          counts.ctypes.data if len(d) else None, matches.ctypes.data if len(matches) else None,
-                                          len(matches), ctypes.byref(total)))
+    out = (counts.ctypes.data if len(d) else None, matches.ctypes.data if len(matches) else None, len(matches), ctypes.byref(total))
+    if mask is None:
+        _abi.check(_abi.load().mod_find_batch(d.ctypes.data if len(d) else None, len(d), s_addr, int(src_bytes), p, len(p), *out))
+    else:
+        _abi.check(_abi.load().mod_find_masked_batch(d.ctypes.data if len(d) else None, len(d), s_addr, int(src_bytes), p,
+                                                     _mask(mask, len(p)), len(p), *out))
     return counts, matches[:min(total.value, len(matches))].copy(), int(total.value)
 
 
@@ -395,36 +443,42 @@ def ark_pack(reference_header_path: str, input_dir: str, output_dir: str, header
 
 
 def ark_find(header_path: str, part_dir: str, pattern: Any, body_key: int = 0,
-             max_matches: int = 1 << 20) -> Tuple[list, int]:
-    """``CArk::Load`` + ``CArk::FindInFiles``: -> ([(file_index, offset), ...] sorted, exact total)."""
+             max_matches: int = 1 << 20, mask: Any = None) -> Tuple[list, int]:
+    """``CArk::Load`` + ``CArk::FindInFiles``: -> ([(file_index, offset), ...] sorted, exact total).  `mask`: as for
+    ``Plan.find`` (``CArk::FindMaskedInFiles``)."""
     p = _pattern(pattern)
     files = np.zeros(max(0, int(max_matches)), dtype=np.uint32)
     offsets = np.zeros_like(files)
     total = ctypes.c_uint64()
-    rc = _abi.load().mod_ark_find(header_path.encode(), _slash(part_dir) if part_dir else b"", p, len(p), _i32(body_key),
-                                  len(files), files.ctypes.data if len(files) else None,
-                                  offsets.ctypes.data if len(files) else None, ctypes.byref(total))
+    lib, where = _abi.load(), (header_path.encode(), _slash(part_dir) if part_dir else b"")
+    out = (_i32(body_key), len(files), files.ctypes.data if len(files) else None, offsets.ctypes.data if len(files) else None,
+           ctypes.byref(total))
+    if mask is None:
+        rc, name = lib.mod_ark_find(*where, p, len(p), *out), "mod_ark_find"
+    else:
+        rc, name = lib.mod_ark_find_masked(*where, p, _mask(mask, len(p)), len(p), *out), "mod_ark_find_masked"
     if rc:
-        raise ArkError(rc, "mod_ark_find")
+        raise ArkError(rc, name)
     k = min(total.value, len(files))
     return [(int(f), int(o)) for f, o in zip(files[:k], offsets[:k])], int(total.value)
 
 
 def ark_find_set(header_path: str, part_dir: str, patterns: Any, body_key: int = 0,
-                 max_matches: int = 1 << 20) -> Tuple[list, np.ndarray, int]:
+                 max_matches: int = 1 << 20, ignore_case: bool = False) -> Tuple[list, np.ndarray, int]:
     """``CArk::Load`` + ``CArk::FindSetInFiles``: -> ([(file_index, offset, pattern), ...] sorted, pattern counts, exact
-    total)."""
-    data, lens = _pattern_list(patterns)
+    total).  `ignore_case`: ASCII letters match either case (``mod_ark_find_set_nocase``)."""
+    data, lens = _pattern_list(patterns, ignore_case)
+    name = "mod_ark_find_set_nocase" if ignore_case else "mod_ark_find_set"
     files = np.zeros(max(0, int(max_matches)), dtype=np.uint32)
     offsets, which = np.zeros_like(files), np.zeros_like(files)
     pattern_counts = np.zeros(len(lens), dtype=np.uint64)
     total = ctypes.c_uint64()
-    rc = _abi.load().mod_ark_find_set(header_path.encode(), _slash(part_dir) if part_dir else b"", data.ctypes.data,
+    rc = getattr(_abi.load(), name)(header_path.encode(), _slash(part_dir) if part_dir else b"", data.ctypes.data,
                                       lens.ctypes.data, len(lens), _i32(body_key), len(files),
                                       files.ctypes.data if len(files) else None, offsets.ctypes.data if len(files) else None,
                                       which.ctypes.data if len(files) else None, ctypes.byref(total), pattern_counts.ctypes.data)
     if rc:
-        raise ArkError(rc, "mod_ark_find_set")
+        raise ArkError(rc, name)
     k = min(total.value, len(files))
     return [(int(f), int(o), int(w)) for f, o, w in zip(files[:k], offsets[:k], which[:k])], pattern_counts, int(total.value)
 

@@ -29,6 +29,8 @@
 #pragma weak mod_plan_find_set_window
 #pragma weak mod_pattern_set_create
 #pragma weak mod_pattern_set_destroy
+#pragma weak mod_plan_find_masked_window
+#pragma weak mod_pattern_set_create_nocase
 
 namespace {
 
@@ -683,6 +685,21 @@ eError CArk::SearchParts(const SearchPass& lPass, std::vector<uint64_t>& laFileC
 eError CArk::FindInFiles(const unsigned char* lpPattern, uint32_t luLen, uint64_t luMaxMatches, std::vector<SFileMatch>& laMatches,
                          uint64_t* lpTotal, std::vector<uint64_t>* lpFileCounts)
 {
+    return FindOneInFiles(lpPattern, nullptr, luLen, luMaxMatches, laMatches, lpTotal, lpFileCounts);
+}
+
+eError CArk::FindMaskedInFiles(const unsigned char* lpPattern, const unsigned char* lpMask, uint32_t luLen, uint64_t luMaxMatches,
+                               std::vector<SFileMatch>& laMatches, uint64_t* lpTotal, std::vector<uint64_t>* lpFileCounts)
+{
+    laMatches.clear();
+    if (!lpMask || std::all_of(lpMask, lpMask + std::min<uint32_t>(luLen, 64), [](unsigned char c) { return c == 0; }))
+        return eError_InvalidParameter;
+    return FindOneInFiles(lpPattern, lpMask, luLen, luMaxMatches, laMatches, lpTotal, lpFileCounts);
+}
+
+eError CArk::FindOneInFiles(const unsigned char* lpPattern, const unsigned char* lpMask, uint32_t luLen, uint64_t luMaxMatches,
+                            std::vector<SFileMatch>& laMatches, uint64_t* lpTotal, std::vector<uint64_t>* lpFileCounts)
+{
     laMatches.clear();
     if (!lpPattern || luLen == 0 || luLen > 64 || !lpTotal)
         return eError_InvalidParameter;
@@ -691,12 +708,20 @@ eError CArk::FindInFiles(const unsigned char* lpPattern, uint32_t luLen, uint64_
         std::cout << "The GPU library in use has no search (mod_plan_find_window)\n";
         return eError_NoData;
     }
+    if (lpMask && !mod_plan_find_masked_window) {
+        std::cout << "The GPU library in use has no masked search (mod_plan_find_masked_window)\n";
+        return eError_NoData;
+    }
     SearchPass lPass;
     lPass.muOverlap = luLen - 1;
     lPass.miPatterns = 0;
     lPass.muMaxMatches = luMaxMatches;
     lPass.muRecordBytes = sizeof(mod_match);
     lPass.mLaunch = [&](const SearchSlot& lSlot) {
+        if (lpMask)
+            return mod_plan_find_masked_window(lSlot.mpPlan, lSlot.muTile0, lSlot.muTile1, lSlot.mpDevIn, lSlot.muSrcLo, lSlot.muRange,
+                                               lpPattern, lpMask, luLen, lSlot.mpCounts, (mod_match*)lSlot.mpList, lSlot.muCap,
+                                               lSlot.mpTotal, lSlot.mpStream) == MOD_OK;
         return mod_plan_find_window(lSlot.mpPlan, lSlot.muTile0, lSlot.muTile1, lSlot.mpDevIn, lSlot.muSrcLo, lSlot.muRange, lpPattern,
                                     luLen, lSlot.mpCounts, (mod_match*)lSlot.mpList, lSlot.muCap, lSlot.mpTotal, lSlot.mpStream) == MOD_OK;
     };
@@ -719,7 +744,8 @@ eError CArk::FindInFiles(const unsigned char* lpPattern, uint32_t luLen, uint64_
 }
 
 eError CArk::FindSetInFiles(const std::vector<std::string>& laPatterns, uint64_t luMaxMatches, std::vector<SFileSetMatch>& laMatches,
-                            uint64_t* lpTotal, std::vector<uint64_t>* lpFileCounts, std::vector<uint64_t>* lpPatternCounts)
+                            uint64_t* lpTotal, std::vector<uint64_t>* lpFileCounts, std::vector<uint64_t>* lpPatternCounts,
+                            bool lbIgnoreCase)
 {
     laMatches.clear();
     if (laPatterns.empty() || laPatterns.size() > 256 || !lpTotal)
@@ -734,13 +760,25 @@ eError CArk::FindSetInFiles(const std::vector<std::string>& laPatterns, uint64_t
         laLens.push_back((uint32_t)lPattern.size());
         luMax = std::max(luMax, (uint32_t)lPattern.size());
     }
-    if (std::unordered_set<std::string>(laPatterns.begin(), laPatterns.end()).size() != laPatterns.size())
+    std::unordered_set<std::string> lDistinct;
+    for (std::string lPattern : laPatterns) {
+        if (lbIgnoreCase)
+            for (char& c : lPattern)
+                c = (char)(c >= 'a' && c <= 'z' ? c - 0x20 : c);
+        lDistinct.insert(std::move(lPattern));
+    }
+    if (lDistinct.size() != laPatterns.size())
         return eError_InvalidParameter;
     *lpTotal = 0;
     if (!mod_plan_find_set_window || !mod_pattern_set_create || !mod_pattern_set_destroy) {
         std::cout << "The GPU library in use has no set search (mod_plan_find_set_window)\n";
         return eError_NoData;
     }
+    if (lbIgnoreCase && !mod_pattern_set_create_nocase) {
+        std::cout << "The GPU library in use has no case-insensitive set search (mod_pattern_set_create_nocase)\n";
+        return eError_NoData;
+    }
+    const auto lCreate = lbIgnoreCase ? mod_pattern_set_create_nocase : mod_pattern_set_create;
     std::vector<mod_pattern_set*> laSets(64, nullptr);  // one per device, created on its first group
     SearchPass lPass;
     lPass.muOverlap = luMax - 1;
@@ -749,7 +787,7 @@ eError CArk::FindSetInFiles(const std::vector<std::string>& laPatterns, uint64_t
     lPass.muRecordBytes = sizeof(mod_set_match);
     lPass.mLaunch = [&](const SearchSlot& lSlot) {
         mod_pattern_set*& lpSet = laSets[lSlot.miDeviceIndex];
-        if (!lpSet && mod_pattern_set_create((const uint8_t*)lBytes.data(), laLens.data(), (uint32_t)laLens.size(), &lpSet) != MOD_OK)
+        if (!lpSet && lCreate((const uint8_t*)lBytes.data(), laLens.data(), (uint32_t)laLens.size(), &lpSet) != MOD_OK)
             return false;
         return mod_plan_find_set_window(lSlot.mpPlan, lSlot.muTile0, lSlot.muTile1, lSlot.mpDevIn, lSlot.muSrcLo, lSlot.muRange, lpSet,
                                         lSlot.mpOwned, lSlot.mpCounts, lSlot.mpPatternCounts, (mod_set_match*)lSlot.mpList, lSlot.muCap,

@@ -89,7 +89,14 @@ public:
     // lpFileCounts gets the exact matches per entry and lpPatternCounts the exact matches per pattern, in list order.
     eError FindSetInFiles(const std::vector<std::string>& laPatterns, uint64_t luMaxMatches, std::vector<SFileSetMatch>& laMatches,
                           uint64_t* lpTotal, std::vector<uint64_t>* lpFileCounts = nullptr,
-                          std::vector<uint64_t>* lpPatternCounts = nullptr);
+                          std::vector<uint64_t>* lpPatternCounts = nullptr, bool lbIgnoreCase = false);
+    // lbIgnoreCase: ASCII letters match either case (mod_pattern_set_create_nocase), and patterns equal ignoring case
+    // are refused.
+    // FindInFiles with a mask byte per pattern byte: an entry byte t matches pattern byte k when
+    // ((t ^ lpPattern[k]) & lpMask[k]) == 0 (0x00 any byte, 0xDF on a letter either case; mod_plan_find_masked).  An
+    // all-zero mask is eError_InvalidParameter.
+    eError FindMaskedInFiles(const unsigned char* lpPattern, const unsigned char* lpMask, uint32_t luLen, uint64_t luMaxMatches,
+                             std::vector<SFileMatch>& laMatches, uint64_t* lpTotal, std::vector<uint64_t>* lpFileCounts = nullptr);
     const modark::HeaderImage& Header() const { return mHeader; }
 
 private:
@@ -101,6 +108,9 @@ private:
     eError CheckEntriesInImage(uint64_t luImageSize) const;
     struct SearchSlot;
     struct SearchPass;
+    // FindInFiles (lpMask null) and FindMaskedInFiles.
+    eError FindOneInFiles(const unsigned char* lpPattern, const unsigned char* lpMask, uint32_t luLen, uint64_t luMaxMatches,
+                          std::vector<SFileMatch>& laMatches, uint64_t* lpTotal, std::vector<uint64_t>* lpFileCounts);
     eError SearchParts(const SearchPass& lPass, std::vector<uint64_t>& laFileCounts, std::vector<uint64_t>& laPatternCounts);
     struct PartTarget {
         int miFd = -1;             // part file open for writing

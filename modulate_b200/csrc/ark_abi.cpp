@@ -49,8 +49,9 @@ int mod_ark_unpack(const char* header_path, const char* part_dir, const char* ta
     });
 }
 
-int mod_ark_find(const char* header_path, const char* part_dir, const uint8_t* pattern, uint32_t len, int32_t body_key,
-                 uint64_t max_matches, uint32_t* out_file, uint32_t* out_offset, uint64_t* out_total)
+// The body of mod_ark_find and mod_ark_find_masked (mask null: the exact search).
+static int ArkFind(const char* header_path, const char* part_dir, const uint8_t* pattern, const uint8_t* mask, uint32_t len,
+                   int32_t body_key, uint64_t max_matches, uint32_t* out_file, uint32_t* out_offset, uint64_t* out_total)
 {
     return Guarded([&]() -> eError {
         if (!header_path || !pattern || !out_total || (max_matches && (!out_file || !out_offset)))
@@ -61,7 +62,8 @@ int mod_ark_find(const char* header_path, const char* part_dir, const uint8_t* p
         eError leError = lArkHeader.Load(header_path);
         SHOW_ERROR_AND_RETURN;
         std::vector<SFileMatch> laMatches;
-        leError = lArkHeader.FindInFiles(pattern, len, max_matches, laMatches, out_total);
+        leError = mask ? lArkHeader.FindMaskedInFiles(pattern, mask, len, max_matches, laMatches, out_total)
+                       : lArkHeader.FindInFiles(pattern, len, max_matches, laMatches, out_total);
         SHOW_ERROR_AND_RETURN;
         for (size_t ii = 0; ii < laMatches.size(); ++ii) {
             out_file[ii] = (uint32_t)laMatches[ii].file;
@@ -71,9 +73,24 @@ int mod_ark_find(const char* header_path, const char* part_dir, const uint8_t* p
     });
 }
 
-int mod_ark_find_set(const char* header_path, const char* part_dir, const uint8_t* bytes, const uint32_t* lens, uint32_t n,
-                     int32_t body_key, uint64_t max_matches, uint32_t* out_file, uint32_t* out_offset, uint32_t* out_pattern,
-                     uint64_t* out_total, uint64_t* out_pattern_counts)
+int mod_ark_find(const char* header_path, const char* part_dir, const uint8_t* pattern, uint32_t len, int32_t body_key,
+                 uint64_t max_matches, uint32_t* out_file, uint32_t* out_offset, uint64_t* out_total)
+{
+    return ArkFind(header_path, part_dir, pattern, nullptr, len, body_key, max_matches, out_file, out_offset, out_total);
+}
+
+int mod_ark_find_masked(const char* header_path, const char* part_dir, const uint8_t* pattern, const uint8_t* mask, uint32_t len,
+                        int32_t body_key, uint64_t max_matches, uint32_t* out_file, uint32_t* out_offset, uint64_t* out_total)
+{
+    if (!mask)
+        return eError_InvalidParameter;
+    return ArkFind(header_path, part_dir, pattern, mask, len, body_key, max_matches, out_file, out_offset, out_total);
+}
+
+// The body of mod_ark_find_set and mod_ark_find_set_nocase.
+static int ArkFindSet(const char* header_path, const char* part_dir, const uint8_t* bytes, const uint32_t* lens, uint32_t n,
+                      int32_t body_key, uint64_t max_matches, uint32_t* out_file, uint32_t* out_offset, uint32_t* out_pattern,
+                      uint64_t* out_total, uint64_t* out_pattern_counts, bool ignore_case)
 {
     return Guarded([&]() -> eError {
         if (!header_path || !bytes || !lens || !out_total || (max_matches && (!out_file || !out_offset || !out_pattern)))
@@ -91,7 +108,7 @@ int mod_ark_find_set(const char* header_path, const char* part_dir, const uint8_
         SHOW_ERROR_AND_RETURN;
         std::vector<SFileSetMatch> laMatches;
         std::vector<uint64_t> laPatternCounts;
-        leError = lArkHeader.FindSetInFiles(laPatterns, max_matches, laMatches, out_total, nullptr, &laPatternCounts);
+        leError = lArkHeader.FindSetInFiles(laPatterns, max_matches, laMatches, out_total, nullptr, &laPatternCounts, ignore_case);
         SHOW_ERROR_AND_RETURN;
         for (size_t ii = 0; ii < laMatches.size(); ++ii) {
             out_file[ii] = (uint32_t)laMatches[ii].file;
@@ -102,6 +119,22 @@ int mod_ark_find_set(const char* header_path, const char* part_dir, const uint8_
             std::copy(laPatternCounts.begin(), laPatternCounts.end(), out_pattern_counts);
         return eError_NoError;
     });
+}
+
+int mod_ark_find_set(const char* header_path, const char* part_dir, const uint8_t* bytes, const uint32_t* lens, uint32_t n,
+                     int32_t body_key, uint64_t max_matches, uint32_t* out_file, uint32_t* out_offset, uint32_t* out_pattern,
+                     uint64_t* out_total, uint64_t* out_pattern_counts)
+{
+    return ArkFindSet(header_path, part_dir, bytes, lens, n, body_key, max_matches, out_file, out_offset, out_pattern, out_total,
+                      out_pattern_counts, false);
+}
+
+int mod_ark_find_set_nocase(const char* header_path, const char* part_dir, const uint8_t* bytes, const uint32_t* lens, uint32_t n,
+                            int32_t body_key, uint64_t max_matches, uint32_t* out_file, uint32_t* out_offset,
+                            uint32_t* out_pattern, uint64_t* out_total, uint64_t* out_pattern_counts)
+{
+    return ArkFindSet(header_path, part_dir, bytes, lens, n, body_key, max_matches, out_file, out_offset, out_pattern, out_total,
+                      out_pattern_counts, true);
 }
 
 int mod_ark_pack(const char* reference_header_path, const char* input_dir, const char* output_dir, const char* header_name,

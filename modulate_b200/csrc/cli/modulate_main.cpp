@@ -7,7 +7,8 @@
 // Extensions: -bodykey K (cipher every entry body with key K, stream restarting per entry -- the
 // synthetic per-entry-key configurations), -device N (bind GPU N), -find TEXT / -findhex HEX (which
 // entries hold a byte pattern, searched on the GPU without unpacking), -findlist FILE / -findhexlist FILE
-// (the same for a list of patterns, all found in one pass).
+// (the same for a list of patterns, all found in one pass), -findi TEXT / -findilist FILE (ignoring ASCII
+// case) and -findwild HEX (hex with '?' nibbles that match anything).
 #include <algorithm>
 #include <cctype>
 #include <chrono>
@@ -115,16 +116,17 @@ eError Unpack(std::deque<std::string>& laParams)
     return eError_NoError;
 }
 
-// -find / -findhex: one line "<name>\t<offset>" per match in table order, then by offset, at most
-// kiMaxLines of them, and always the exact "<total> matches in <files> files".
-eError FindPattern(const std::string& lPattern)
+// -find / -findhex / -findi / -findwild: one line "<name>\t<offset>" per match in table order, then by offset, at
+// most kiMaxLines of them, and always the exact "<total> matches in <files> files".  lpMask (one byte per pattern
+// byte, see CArk::FindMaskedInFiles) or null for the exact search; lpHow is added to the header line.
+eError FindPattern(const std::string& lPattern, const std::string* lpMask = nullptr, const char* lpHow = "")
 {
     constexpr uint64_t kiMaxLines = 10000;
     if (lPattern.empty() || lPattern.size() > 64) {
         std::cout << "The pattern must be 1 to 64 bytes long\n";
         return eError_InvalidParameter;
     }
-    std::cout << "Searching " << HeaderName() << " for " << lPattern.size() << " bytes\n";
+    std::cout << "Searching " << HeaderName() << " for " << lPattern.size() << " bytes" << lpHow << "\n";
     CArk lArkHeader;
     lArkHeader.SetUniformEntryKey(giBodyKey);
     eError leError = lArkHeader.Load(HeaderName().c_str());
@@ -132,8 +134,12 @@ eError FindPattern(const std::string& lPattern)
     std::vector<SFileMatch> laMatches;
     std::vector<uint64_t> laFileCounts;
     uint64_t luTotal = 0;
-    leError = lArkHeader.FindInFiles((const unsigned char*)lPattern.data(), (uint32_t)lPattern.size(), kiMaxLines, laMatches,
-                                     &luTotal, &laFileCounts);
+    if (lpMask)
+        leError = lArkHeader.FindMaskedInFiles((const unsigned char*)lPattern.data(), (const unsigned char*)lpMask->data(),
+                                               (uint32_t)lPattern.size(), kiMaxLines, laMatches, &luTotal, &laFileCounts);
+    else
+        leError = lArkHeader.FindInFiles((const unsigned char*)lPattern.data(), (uint32_t)lPattern.size(), kiMaxLines, laMatches,
+                                         &luTotal, &laFileCounts);
     SHOW_ERROR_AND_RETURN;
     for (const SFileMatch& lMatch : laMatches)
         std::cout << lArkHeader.Header().maFiles[(size_t)lMatch.file].mName << "\t" << lMatch.offset << "\n";
@@ -151,6 +157,69 @@ eError Find(std::deque<std::string>& laParams)
     const std::string lText = laParams.front();
     laParams.pop_front();
     return FindPattern(lText);
+}
+
+// ASCII upper case: the folded form of a case-insensitive pattern ('a'..'z' -> 'A'..'Z', every other byte itself).
+std::string Folded(std::string lText)
+{
+    for (char& c : lText)
+        if (c >= 'a' && c <= 'z')
+            c = (char)(c - 0x20);
+    return lText;
+}
+
+// -findi: -find with every letter matching either case (pattern byte upper-cased, mask 0xDF; 0xFF elsewhere).
+eError FindIgnoreCase(std::deque<std::string>& laParams)
+{
+    if (laParams.empty())
+        return eError_InvalidParameter;
+    const std::string lText = Folded(laParams.front());
+    laParams.pop_front();
+    std::string lMask(lText.size(), (char)0xFF);
+    for (size_t ii = 0; ii < lText.size(); ++ii)
+        if (lText[ii] >= 'A' && lText[ii] <= 'Z')
+            lMask[ii] = (char)0xDF;
+    return FindPattern(lText, &lMask, ", ignoring case");
+}
+
+// -findwild: pairs of hex digits, whitespace ignored, in which any digit may be '?' (any nibble; "??" any byte).
+eError FindWild(std::deque<std::string>& laParams)
+{
+    if (laParams.empty())
+        return eError_InvalidParameter;
+    std::string lDigits;
+    for (char c : laParams.front())
+        if (!std::isspace((unsigned char)c))
+            lDigits += (char)std::tolower((unsigned char)c);
+    laParams.pop_front();
+    if (lDigits.size() % 2 != 0 || lDigits.find_first_not_of("0123456789abcdef?") != std::string::npos) {
+        std::cout << "-findwild takes pairs of hex digits, any of them ?\n";
+        return eError_InvalidParameter;
+    }
+    if (lDigits.empty() || lDigits.size() > 128) {
+        std::cout << "The pattern must be 1 to 64 bytes long\n";
+        return eError_InvalidParameter;
+    }
+    if (lDigits.find_first_not_of('?') == std::string::npos) {
+        std::cout << "-findwild: the pattern has no hex digit that is not ?\n";
+        return eError_InvalidParameter;
+    }
+    std::string lBytes, lMask;
+    for (size_t ii = 0; ii < lDigits.size(); ii += 2) {
+        uint32_t luValue = 0, luMask = 0;
+        for (size_t kk = 0; kk < 2; ++kk) {
+            const char c = lDigits[ii + kk];
+            luValue <<= 4;
+            luMask <<= 4;
+            if (c != '?') {
+                luValue |= (uint32_t)std::stoi(std::string(1, c), nullptr, 16);
+                luMask |= 0xFu;
+            }
+        }
+        lBytes += (char)luValue;
+        lMask += (char)luMask;
+    }
+    return FindPattern(lBytes, &lMask);
 }
 
 // Hex digit pairs, whitespace ignored (the -findhex syntax) -> lBytes; lpShown, when given, gets the digits
@@ -188,11 +257,12 @@ eError FindHex(std::deque<std::string>& laParams)
 // -findlist / -findhexlist: one pattern per line (a trailing '\r' stripped, empty lines skipped), all searched in one
 // pass.  One line "<name>\t<offset>\t<pattern>" per match in table order, then by offset, then list order, at most
 // kiMaxLines of them; then "<count>\t<pattern>" per pattern in list order, and the "<total> matches in <files>
-// files" of -find.  A hex pattern is shown as given, lowercased and without spaces.
-eError FindList(std::deque<std::string>& laParams, bool lbHex)
+// files" of -find.  A hex pattern is shown as given, lowercased and without spaces.  lbFold (-findilist): text
+// patterns whose letters match either case; two lines equal ignoring case are refused.
+eError FindList(std::deque<std::string>& laParams, bool lbHex, bool lbFold = false)
 {
     constexpr uint64_t kiMaxLines = 10000;
-    const char* lpWhat = lbHex ? "-findhexlist" : "-findlist";
+    const char* lpWhat = lbFold ? "-findilist" : lbHex ? "-findhexlist" : "-findlist";
     if (laParams.empty())
         return eError_InvalidParameter;
     const std::string lListPath = laParams.front();
@@ -219,9 +289,10 @@ eError FindList(std::deque<std::string>& laParams, bool lbHex)
             std::cout << lpWhat << ": line " << liLine << ": the pattern must be 1 to 64 bytes long\n";
             return eError_InvalidParameter;
         }
-        const auto lSeen = lLineOf.emplace(lBytes, liLine);
+        const auto lSeen = lLineOf.emplace(lbFold ? Folded(lBytes) : lBytes, liLine);
         if (!lSeen.second) {
-            std::cout << lpWhat << ": line " << liLine << " repeats the pattern of line " << lSeen.first->second << "\n";
+            std::cout << lpWhat << ": line " << liLine << " repeats the pattern of line " << lSeen.first->second
+                      << (lbFold ? " ignoring case" : "") << "\n";
             return eError_InvalidParameter;
         }
         if (laPatterns.size() == 256) {
@@ -235,7 +306,8 @@ eError FindList(std::deque<std::string>& laParams, bool lbHex)
         std::cout << lpWhat << ": " << lListPath << " holds no pattern\n";
         return eError_InvalidParameter;
     }
-    std::cout << "Searching " << HeaderName() << " for " << laPatterns.size() << " patterns\n";
+    std::cout << "Searching " << HeaderName() << " for " << laPatterns.size() << " patterns" << (lbFold ? ", ignoring case" : "")
+              << "\n";
     CArk lArkHeader;
     lArkHeader.SetUniformEntryKey(giBodyKey);
     eError leError = lArkHeader.Load(HeaderName().c_str());
@@ -243,7 +315,7 @@ eError FindList(std::deque<std::string>& laParams, bool lbHex)
     std::vector<SFileSetMatch> laMatches;
     std::vector<uint64_t> laFileCounts, laPatternCounts;
     uint64_t luTotal = 0;
-    leError = lArkHeader.FindSetInFiles(laPatterns, kiMaxLines, laMatches, &luTotal, &laFileCounts, &laPatternCounts);
+    leError = lArkHeader.FindSetInFiles(laPatterns, kiMaxLines, laMatches, &luTotal, &laFileCounts, &laPatternCounts, lbFold);
     SHOW_ERROR_AND_RETURN;
     for (const SFileSetMatch& lMatch : laMatches)
         std::cout << lArkHeader.Header().maFiles[(size_t)lMatch.file].mName << "\t" << lMatch.offset << "\t" << laShown[lMatch.pattern]
@@ -259,6 +331,7 @@ eError FindList(std::deque<std::string>& laParams, bool lbHex)
 
 eError FindListText(std::deque<std::string>& laParams) { return FindList(laParams, false); }
 eError FindListHex(std::deque<std::string>& laParams) { return FindList(laParams, true); }
+eError FindListIgnoreCase(std::deque<std::string>& laParams) { return FindList(laParams, false, true); }
 
 eError PackImpl(std::deque<std::string>& laParams)
 {
@@ -437,6 +510,9 @@ void PrintUsage()
               << "  -findhex <hex>              Same for a pattern given as hex bytes, e.g. 00ff1a\n"
               << "  -findlist <file>            Same for every pattern of <file> (one per line, up to 256), in one pass\n"
               << "  -findhexlist <file>         Same for a file of hex patterns, one per line\n"
+              << "  -findi <text>               -find ignoring the case of ASCII letters\n"
+              << "  -findilist <file>           -findlist ignoring the case of ASCII letters\n"
+              << "  -findwild <hex>             -findhex where any hex digit may be ?, e.g. 0a??00?f\n"
               << "  -listsongs <dir>            List the songs the DTA configs under <dir> define\n"
               << "  -dtaset <file> <key> <val>  Patch the value following symbol <key> in a binary DTA file\n"
               << "  -dtacopy <in> <out>         Load and re-save a binary DTA file\n";
@@ -468,6 +544,7 @@ int main(int argc, char* argv[])
         {"-pack_add", AddPack}, {"-decode", Decode},   {"-dtaset", DtaSet},          {"-dtacopy", DtaCopy},
         {"-listsongs", ListSongs}, {"-find", Find},     {"-findhex", FindHex},
         {"-findlist", FindListText}, {"-findhexlist", FindListHex},
+        {"-findi", FindIgnoreCase}, {"-findilist", FindListIgnoreCase}, {"-findwild", FindWild},
     };
 
     std::deque<std::string> laParams;

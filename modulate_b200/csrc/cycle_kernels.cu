@@ -740,11 +740,24 @@ __device__ __forceinline__ TileView decipher_tile(const TileRec* rec, const uint
     return TileView{src_rel, entry, head, end, halo};
 }
 
+// The masked instantiation (kMasked) differs in the filter and the compare only.  Its filter tests the anchor pair
+// (a, a + 1) -- the adjacent pattern bytes with the most mask bits, so that leading wildcards do not make every start
+// a candidate -- with the same SWAR test on (bytes ^ rep) & mrep; its compare masks the head word and every byte.
+//
+// Shared slack.  The masked filter of word w reads words w + a/4 and w + a/4 + 1, bytes up to 4w + a + 7.  A word is
+// tested only when 4w < p_end <= end + halo - L + 1, and a <= max(0, L - 2), halo <= min(rest, L - 1), so the
+// farthest byte is end + halo + 5 <= kTileBytes + kMaxPattern + 4 for L >= 2 (and end + 6 for L = 1, where
+// halo = 0).  s_w holds kTileBytes + 16 * kHaloChunks + 16 bytes.  Bytes past end + halo may be stale from an
+// earlier layout of the array; only the filter reads them, the compare stays below p + L <= end + halo.
+constexpr uint32_t kFindSlackWords = 4u;
+static_assert(kTileBytes + kMaxPattern + 4u < kTileBytes + 16u * kHaloChunks + 4u * kFindSlackWords,
+              "find_batch_kernel<true>: the masked filter reads past s_w");
+template <bool kMasked>
 __global__ void __launch_bounds__(kThreadsPerCta, MODK_MIN_CTAS_FIND) find_batch_kernel(const __grid_constant__ FindArgs f)
 {
     constexpr uint32_t T = (uint32_t)kThreadsPerCta;
-    // the tile, its halo, and one word of slack for the filter's second word
-    __shared__ __align__(16) uint32_t s_w[(kTileBytes + 16u * kHaloChunks) / 4u + 4u];
+    // the tile, its halo, and slack for the filter's second word (the masked filter's words past the anchor)
+    __shared__ __align__(16) uint32_t s_w[(kTileBytes + 16u * kHaloChunks) / 4u + kFindSlackWords];
     const uint32_t tid = threadIdx.x;
     uint32_t pw[kUnroll];
     load_chunk_pows<kUnroll>(pw, tid);
@@ -763,11 +776,24 @@ __global__ void __launch_bounds__(kThreadsPerCta, MODK_MIN_CTAS_FIND) find_batch
     const bool two_bytes = f.len > 1u;
     for (uint32_t w = (head >> 2) + tid; 4u * w < p_end; w += T) {
         const uint32_t x = s_w[w], y = s_w[w + 1u];
-        const uint32_t v0 = x ^ f.rep0;
-        uint32_t m = (v0 - 0x01010101u) & ~v0;
-        if (two_bytes) {
-            const uint32_t v1 = __funnelshift_r(x, y, 8u) ^ f.rep1;
-            m &= (v1 - 0x01010101u) & ~v1;
+        uint32_t m;
+        if constexpr (!kMasked) {
+            const uint32_t v0 = x ^ f.rep0;
+            m = (v0 - 0x01010101u) & ~v0;
+            if (two_bytes) {
+                const uint32_t v1 = __funnelshift_r(x, y, 8u) ^ f.rep1;
+                m &= (v1 - 0x01010101u) & ~v1;
+            }
+        } else {
+            // bytes p + a and p + a + 1 of starts p = 4w..4w+3; the clamped shift of a & 3 == 3 takes all of the second word
+            const uint32_t wa = w + (f.anchor >> 2u), sh = 8u * (f.anchor & 3u);
+            const uint32_t xa = s_w[wa], ya = s_w[wa + 1u];
+            const uint32_t v0 = (__funnelshift_r(xa, ya, sh) ^ f.rep0) & f.mrep0;
+            m = (v0 - 0x01010101u) & ~v0;
+            if (two_bytes) {
+                const uint32_t v1 = (__funnelshift_rc(xa, ya, sh + 8u) ^ f.rep1) & f.mrep1;
+                m &= (v1 - 0x01010101u) & ~v1;
+            }
         }
         if (__builtin_expect((m & 0x80808080u) == 0u, 1))
             continue;
@@ -778,7 +804,7 @@ __global__ void __launch_bounds__(kThreadsPerCta, MODK_MIN_CTAS_FIND) find_batch
                 continue;
             bool hit = true;
             for (uint32_t k = 4u; k < f.len && hit; ++k)
-                hit = sb[p + k] == f.pattern[k];
+                hit = kMasked ? ((sb[p + k] ^ f.pattern[k]) & f.mask[k]) == 0u : sb[p + k] == f.pattern[k];
             if (hit)
                 find_record(f, entry, src_rel, p);
         }
@@ -800,10 +826,13 @@ __global__ void __launch_bounds__(kThreadsPerCta, MODK_MIN_CTAS_FIND) find_batch
 // Every pattern of the set that starts at tile-local p, whose first two bytes passed the filter: the length-1
 // pattern of the first byte, then the patterns of the 2-byte key (binary search over the distinct keys), each
 // checked against `lim` (where the deciphered entry bytes end), its head word and then its remaining bytes.
-// `pos0` is the entry position of tile-local byte 0.
+// `pos0` is the entry position of tile-local byte 0.  A folded set (kFold) holds upper-cased patterns, so the
+// candidate's key, head word and bytes are folded before they are compared.
+template <bool kFold>
 __device__ __noinline__ void find_set_verify(const FindSetArgs& f, const uint8_t* sb, const uint16_t* s_keys, uint32_t p,
                                              uint32_t lim, uint32_t entry, int64_t pos0)
 {
+    auto at = [&](uint32_t i) -> uint32_t { return kFold ? fold_ascii(sb[i]) : sb[i]; };
     auto record = [&](uint32_t id) {
         atomicAdd(&f.counts[entry], 1u);
         atomicAdd(&f.pattern_counts[id], 1ull);
@@ -815,7 +844,7 @@ __device__ __noinline__ void find_set_verify(const FindSetArgs& f, const uint8_t
             m[2] = id;
         }
     };
-    const uint32_t b0 = sb[p], key = b0 | ((uint32_t)sb[p + 1] << 8);
+    const uint32_t b0 = at(p), key = b0 | (at(p + 1) << 8);
     const uint32_t one = __ldg(&f.set->one[b0]);
     if (one)
         record(one - 1u);
@@ -829,7 +858,7 @@ __device__ __noinline__ void find_set_verify(const FindSetArgs& f, const uint8_t
     }
     if (lo == f.n_keys || s_keys[lo] != key)
         return;
-    const uint32_t word = b0 | ((uint32_t)sb[p + 1] << 8) | ((uint32_t)sb[p + 2] << 16) | ((uint32_t)sb[p + 3] << 24);
+    const uint32_t word = b0 | (at(p + 1) << 8) | (at(p + 2) << 16) | (at(p + 3) << 24);
     const uint32_t r1 = __ldg(&f.set->group[lo + 1u]);
     for (uint32_t r = __ldg(&f.set->group[lo]); r < r1; ++r) {
         const uint4 sp = __ldg(reinterpret_cast<const uint4*>(&f.set->pat[r]));  // {id, len, head, mask}
@@ -837,12 +866,13 @@ __device__ __noinline__ void find_set_verify(const FindSetArgs& f, const uint8_t
             continue;
         bool hit = true;
         for (uint32_t k = 4u; k < sp.y && hit; ++k)
-            hit = sb[p + k] == __ldg(&f.set->bytes[r][k]);
+            hit = at(p + k) == __ldg(&f.set->bytes[r][k]);
         if (hit)
             record(sp.x);
     }
 }
 
+template <bool kFold>
 __global__ void __launch_bounds__(kThreadsPerCta, MODK_MIN_CTAS_FIND_SET) find_set_kernel(const __grid_constant__ FindSetArgs f)
 {
     constexpr uint32_t T = (uint32_t)kThreadsPerCta;
@@ -879,7 +909,7 @@ __global__ void __launch_bounds__(kThreadsPerCta, MODK_MIN_CTAS_FIND_SET) find_s
             for (uint32_t o = 0; o < 4u; ++o) {
                 const uint32_t p = 4u * w + o;
                 if ((bit(o) & 1u) != 0u && p >= v.head && p < pe)
-                    find_set_verify(f, sb, s_keys, p, lim, v.entry, pos0);
+                    find_set_verify<kFold>(f, sb, s_keys, p, lim, v.entry, pos0);
             }
         }
         __syncthreads();  // the tile is no longer read: the next one may overwrite it
@@ -955,14 +985,17 @@ cudaError_t launch_batch_inline(const BatchArgs& args, const InlineDescs& descs,
     return cudaGetLastError();
 }
 
-cudaError_t launch_find(const FindArgs& args, cudaStream_t stream)
+cudaError_t launch_find(const FindArgs& args, bool masked, cudaStream_t stream)
 {
     for (uint32_t t0 = 0; t0 < args.n_tiles;) {
         const uint32_t n = args.n_tiles - t0 < kMaxGrid ? args.n_tiles - t0 : kMaxGrid;
         FindArgs a = args;
         a.tiles = args.tiles + t0;
         a.n_tiles = n;
-        find_batch_kernel<<<n, kThreadsPerCta, 0, stream>>>(a);
+        if (masked)
+            find_batch_kernel<true><<<n, kThreadsPerCta, 0, stream>>>(a);
+        else
+            find_batch_kernel<false><<<n, kThreadsPerCta, 0, stream>>>(a);
         const cudaError_t err = cudaGetLastError();
         if (err != cudaSuccess)
             return err;
@@ -971,20 +1004,21 @@ cudaError_t launch_find(const FindArgs& args, cudaStream_t stream)
     return cudaSuccess;
 }
 
-cudaError_t launch_find_set(const FindSetArgs& args, cudaStream_t stream)
+cudaError_t launch_find_set(const FindSetArgs& args, bool fold, cudaStream_t stream)
 {
     if (args.n_tiles == 0)
         return cudaSuccess;
+    void (*kernel)(const FindSetArgs) = fold ? find_set_kernel<true> : find_set_kernel<false>;
     int dev = 0, sms = 0, per_sm = 0;
     cudaError_t err = cudaGetDevice(&dev);
     if (err == cudaSuccess)
         err = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     if (err == cudaSuccess)
-        err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, find_set_kernel, kThreadsPerCta, 0);
+        err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kThreadsPerCta, 0);
     if (err != cudaSuccess)
         return err;
     const uint32_t grid = (uint32_t)std::max(1, sms * per_sm);
-    find_set_kernel<<<std::min(grid, args.n_tiles), kThreadsPerCta, 0, stream>>>(args);
+    kernel<<<std::min(grid, args.n_tiles), kThreadsPerCta, 0, stream>>>(args);
     return cudaGetLastError();
 }
 

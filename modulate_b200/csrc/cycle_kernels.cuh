@@ -85,10 +85,16 @@ struct FindArgs {
     uint64_t cap;
     uint32_t len;        // pattern bytes, 1..kMaxPattern
     uint32_t head_word;  // first min(4, len) pattern bytes, little-endian
-    uint32_t head_mask;  // which bytes of head_word take part
-    uint32_t rep0, rep1; // pattern[0] and pattern[1] (0 if len == 1) in every byte: the search filter
+    uint32_t head_mask;  // which bytes of head_word take part (masked search: its first four mask bytes)
+    uint32_t rep0, rep1; // pattern[a] and pattern[a + 1] (0 if len == 1) in every byte: the search filter
     uint32_t two = 2;
     uint8_t pattern[kMaxPattern];
+    // Masked search only (find_batch_kernel<true>): byte t matches pattern byte k when ((t ^ pattern[k]) & mask[k])
+    // == 0, pattern[k] already AND-ed with mask[k].  The filter tests the anchor pair (a, a + 1), the adjacent pair
+    // with the most mask bits; the exact kernel's anchor is a = 0 and it reads none of these fields.
+    uint32_t anchor;             // a
+    uint32_t mrep0, mrep1;       // mask[a] and mask[a + 1] (0 if len == 1) in every byte
+    uint8_t mask[kMaxPattern];
 };
 
 // Pattern-set search (find_set_kernel): the decipher stage of find_batch_kernel, then every start tested against
@@ -101,6 +107,9 @@ struct __align__(16) SetPattern {  // read as one 16-byte load
     uint32_t head;  // first min(4, len) bytes, little-endian
     uint32_t mask;  // which bytes of head take part
 };
+// A case-folded set (mod_pattern_set_create_nocase) holds upper-cased keys, bytes and length-1 entries, and its
+// bitmap has a bit for every case variant of a pattern's first two bytes.
+__host__ __device__ inline uint32_t fold_ascii(uint32_t b) { return b - 0x61u < 26u ? b - 0x20u : b; }
 struct SetIndex {  // ~30 KB, one cudaMalloc
     uint32_t bitmap[65536 / 32];          // bit b0 | b1 << 8: some pattern starts with (b0, b1); length 1 sets (b0, *)
     uint16_t keys[kMaxSetPatterns];       // distinct 2-byte keys of the patterns of length >= 2, ascending
@@ -141,8 +150,9 @@ __host__ __device__ inline uint32_t tiles_for_entry(uint32_t h0, uint32_t len)
 cudaError_t upload_tables();  // jump tables -> __constant__ / global memory of the current device
 cudaError_t launch_batch(const BatchArgs& args, cudaStream_t stream);
 cudaError_t launch_batch_inline(const BatchArgs& args, const InlineDescs& descs, cudaStream_t stream);
-cudaError_t launch_find(const FindArgs& args, cudaStream_t stream);
-cudaError_t launch_find_set(const FindSetArgs& args, cudaStream_t stream);
+// `masked`: find_batch_kernel<true> (FindArgs' mask fields); `fold`: find_set_kernel<true> (a case-folded set).
+cudaError_t launch_find(const FindArgs& args, bool masked, cudaStream_t stream);
+cudaError_t launch_find_set(const FindSetArgs& args, bool fold, cudaStream_t stream);
 // Plan kernel: expands descriptors into per-tile records (binary search + jump-ahead per tile).
 cudaError_t launch_build_tiles(const DevDesc* descs, uint32_t n_descs, uint32_t dst_align, TileRec* tiles,
                                uint32_t n_tiles, cudaStream_t stream);

@@ -856,6 +856,7 @@ struct mod_pattern_set {
     uint32_t n = 0;
     uint32_t n_keys = 0;  // distinct 2-byte keys of the patterns of length >= 2
     uint32_t lmin = 0, lmax = 0;
+    bool fold = false;    // mod_pattern_set_create_nocase: upper-cased patterns, searched with find_set_kernel<true>
 };
 
 extern "C" {
@@ -1310,10 +1311,38 @@ static int find_window_check(const char* who, const mod_plan* plan, uint64_t til
     return MOD_OK;
 }
 
-// The launch shared by mod_plan_find and mod_plan_find_window; [lo16, hi16) are the granules that may be loaded whole.
+// The mask checks of the masked searches: a mask with a byte to anchor on, `len` within 1..kMaxPattern.
+static int masked_check(const char* who, const uint8_t* pattern, const uint8_t* mask, uint32_t len)
+{
+    if (!pattern || !mask || len == 0 || len > modk::kMaxPattern)
+        return fail(MOD_ERR_ARG, "%s: the pattern and its mask must be 1 to %u bytes", who, modk::kMaxPattern);
+    for (uint32_t k = 0; k < len; ++k)
+        if (mask[k])
+            return MOD_OK;
+    return fail(MOD_ERR_ARG, "%s: the mask is all zero (no byte to anchor on)", who);
+}
+
+// The anchor of a masked pattern: the adjacent pair (a, a + 1) with the most mask bits, the first of equals (0 if
+// len == 1).
+static uint32_t find_anchor(const uint8_t* mask, uint32_t len)
+{
+    uint32_t a = 0;
+    int best = -1;
+    for (uint32_t k = 0; k + 1 < len; ++k) {
+        const int bits = __builtin_popcount(mask[k]) + __builtin_popcount(mask[k + 1]);
+        if (bits > best) {
+            best = bits;
+            a = k;
+        }
+    }
+    return a;
+}
+
+// The launch shared by mod_plan_find*, mod_plan_find_masked*; [lo16, hi16) are the granules that may be loaded whole.
+// `mask` (len bytes, checked by masked_check) or nullptr: the exact search.  An all-0xFF mask is the exact search too.
 static int plan_find_launch(const char* who, const mod_plan* plan, uint64_t tile_begin, uint64_t tile_end,
-                            const uint8_t* src_base, uint64_t lo16, uint64_t hi16, const uint8_t* pattern, uint32_t len,
-                            uint32_t* d_counts, mod_match* d_matches, uint64_t cap, uint64_t* d_total, void* stream)
+                            const uint8_t* src_base, uint64_t lo16, uint64_t hi16, const uint8_t* pattern, const uint8_t* mask,
+                            uint32_t len, uint32_t* d_counts, mod_match* d_matches, uint64_t cap, uint64_t* d_total, void* stream)
 {
     if (!pattern || len == 0 || len > modk::kMaxPattern)
         return fail(MOD_ERR_ARG, "%s: the pattern must be 1 to %u bytes", who, modk::kMaxPattern);
@@ -1322,6 +1351,17 @@ static int plan_find_launch(const char* who, const mod_plan* plan, uint64_t tile
     int rc = find_check(who, plan, src_base, d_counts, d_total, cap, d_matches);
     if (rc != MOD_OK)
         return rc;
+    uint8_t v[modk::kMaxPattern];
+    if (mask) {
+        bool exact = true;
+        for (uint32_t k = 0; k < len; ++k) {
+            v[k] = pattern[k] & mask[k];
+            exact = exact && mask[k] == 0xFFu;
+        }
+        pattern = v;
+        if (exact)
+            mask = nullptr;
+    }
     modk::FindArgs f;
     f.src = src_base;
     f.tiles = plan->d_tiles + tile_begin;
@@ -1344,7 +1384,22 @@ static int plan_find_launch(const char* who, const mod_plan* plan, uint64_t tile
     f.rep1 = len > 1 ? 0x01010101u * pattern[1] : 0u;
     std::memset(f.pattern, 0, sizeof(f.pattern));
     std::memcpy(f.pattern, pattern, len);
-    CUDA_TRY(modk::launch_find(f, (cudaStream_t)stream));
+    f.anchor = 0;
+    f.mrep0 = f.mrep1 = 0;
+    std::memset(f.mask, 0, sizeof(f.mask));
+    if (mask) {
+        const uint32_t a = find_anchor(mask, len);
+        f.anchor = a;
+        f.head_mask = 0;
+        for (uint32_t k = 0; k < 4 && k < len; ++k)
+            f.head_mask |= (uint32_t)mask[k] << (8 * k);
+        f.rep0 = 0x01010101u * pattern[a];
+        f.mrep0 = 0x01010101u * mask[a];
+        f.rep1 = len > 1 ? 0x01010101u * pattern[a + 1] : 0u;
+        f.mrep1 = len > 1 ? 0x01010101u * mask[a + 1] : 0u;
+        std::memcpy(f.mask, mask, len);
+    }
+    CUDA_TRY(modk::launch_find(f, mask != nullptr, (cudaStream_t)stream));
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return MOD_OK;
 }
@@ -1358,7 +1413,21 @@ int mod_plan_find(const mod_plan* plan, const void* d_src, const uint8_t* patter
         return fail(MOD_ERR_ARG, "mod_plan_find: null buffer");
     return plan_find_launch("mod_plan_find", plan, 0, plan->n_tiles, (const uint8_t*)d_src,
                             ((uint64_t)(uintptr_t)d_src + 15u) & ~15ull, ((uint64_t)(uintptr_t)d_src + plan->src_bytes) & ~15ull,
-                            pattern, len, d_counts, d_matches, cap, d_total, stream);
+                            pattern, nullptr, len, d_counts, d_matches, cap, d_total, stream);
+}
+
+// The body of mod_plan_find_window and mod_plan_find_masked_window (mask: nullptr for the exact search).
+static int plan_find_window(const char* who, const mod_plan* plan, uint64_t tile_begin, uint64_t tile_end, const void* d_src_win,
+                            uint64_t src_win_off, uint64_t src_win_bytes, const uint8_t* pattern, const uint8_t* mask,
+                            uint32_t len, uint32_t* d_counts, mod_match* d_matches, uint64_t cap, uint64_t* d_total, void* stream)
+{
+    int rc = find_window_check(who, plan, tile_begin, tile_end, d_src_win, src_win_off, src_win_bytes, len - 1);
+    if (rc != MOD_OK)
+        return rc;
+    return plan_find_launch(who, plan, tile_begin, tile_end, (const uint8_t*)d_src_win - src_win_off,
+                            ((uint64_t)(uintptr_t)d_src_win + 15u) & ~15ull,
+                            ((uint64_t)(uintptr_t)d_src_win + src_win_bytes) & ~15ull, pattern, mask, len, d_counts, d_matches,
+                            cap, d_total, stream);
 }
 
 int mod_plan_find_window(const mod_plan* plan, uint64_t tile_begin, uint64_t tile_end, const void* d_src_win,
@@ -1369,13 +1438,37 @@ int mod_plan_find_window(const mod_plan* plan, uint64_t tile_begin, uint64_t til
         return fail(MOD_ERR_ARG, "mod_plan_find_window: null plan");
     if (!pattern || len == 0 || len > modk::kMaxPattern)
         return fail(MOD_ERR_ARG, "mod_plan_find_window: the pattern must be 1 to %u bytes", modk::kMaxPattern);
-    int rc = find_window_check("mod_plan_find_window", plan, tile_begin, tile_end, d_src_win, src_win_off, src_win_bytes, len - 1);
+    return plan_find_window("mod_plan_find_window", plan, tile_begin, tile_end, d_src_win, src_win_off, src_win_bytes, pattern,
+                            nullptr, len, d_counts, d_matches, cap, d_total, stream);
+}
+
+int mod_plan_find_masked(const mod_plan* plan, const void* d_src, const uint8_t* pattern, const uint8_t* mask, uint32_t len,
+                         uint32_t* d_counts, mod_match* d_matches, uint64_t cap, uint64_t* d_total, void* stream)
+{
+    if (!plan)
+        return fail(MOD_ERR_ARG, "mod_plan_find_masked: null plan");
+    if (!d_src && plan->n_tiles)
+        return fail(MOD_ERR_ARG, "mod_plan_find_masked: null buffer");
+    const int rc = masked_check("mod_plan_find_masked", pattern, mask, len);
     if (rc != MOD_OK)
         return rc;
-    return plan_find_launch("mod_plan_find_window", plan, tile_begin, tile_end, (const uint8_t*)d_src_win - src_win_off,
-                            ((uint64_t)(uintptr_t)d_src_win + 15u) & ~15ull,
-                            ((uint64_t)(uintptr_t)d_src_win + src_win_bytes) & ~15ull, pattern, len, d_counts, d_matches,
-                            cap, d_total, stream);
+    return plan_find_launch("mod_plan_find_masked", plan, 0, plan->n_tiles, (const uint8_t*)d_src,
+                            ((uint64_t)(uintptr_t)d_src + 15u) & ~15ull, ((uint64_t)(uintptr_t)d_src + plan->src_bytes) & ~15ull,
+                            pattern, mask, len, d_counts, d_matches, cap, d_total, stream);
+}
+
+int mod_plan_find_masked_window(const mod_plan* plan, uint64_t tile_begin, uint64_t tile_end, const void* d_src_win,
+                                uint64_t src_win_off, uint64_t src_win_bytes, const uint8_t* pattern, const uint8_t* mask,
+                                uint32_t len, uint32_t* d_counts, mod_match* d_matches, uint64_t cap, uint64_t* d_total,
+                                void* stream)
+{
+    if (!plan)
+        return fail(MOD_ERR_ARG, "mod_plan_find_masked_window: null plan");
+    const int rc = masked_check("mod_plan_find_masked_window", pattern, mask, len);
+    if (rc != MOD_OK)
+        return rc;
+    return plan_find_window("mod_plan_find_masked_window", plan, tile_begin, tile_end, d_src_win, src_win_off, src_win_bytes,
+                            pattern, mask, len, d_counts, d_matches, cap, d_total, stream);
 }
 
 // Plan + one search launch + destroy, synchronous: the body of mod_find_batch and mod_find_set_batch.  One device
@@ -1459,23 +1552,49 @@ int mod_find_batch(const mod_desc* descs, uint64_t n, const void* d_src, uint64_
     MOD_ABI_END("mod_find_batch")
 }
 
-/* ---- pattern sets ------------------------------------------------------------------------------ */
-
-int mod_pattern_set_create(const uint8_t* bytes, const uint32_t* lens, uint32_t n, mod_pattern_set** out)
+int mod_find_masked_batch(const mod_desc* descs, uint64_t n, const void* d_src, uint64_t src_bytes, const uint8_t* pattern,
+                          const uint8_t* mask, uint32_t len, uint32_t* counts_out, mod_match* matches_out, uint64_t cap,
+                          uint64_t* total_out)
 {
     MOD_ABI_BEGIN
+    int rc = masked_check("mod_find_masked_batch", pattern, mask, len);
+    if (rc != MOD_OK)
+        return rc;
+    rc = find_batch_run("mod_find_masked_batch", descs, n, d_src, src_bytes, counts_out, nullptr, 0, matches_out, 8, cap,
+                        total_out, [&](mod_plan* plan, uint32_t* d_counts, uint8_t*, uint8_t* d_list, uint64_t* d_total) {
+                            return mod_plan_find_masked(plan, d_src, pattern, mask, len, d_counts, (mod_match*)d_list, cap,
+                                                        d_total, nullptr);
+                        });
+    if (rc != MOD_OK)
+        return rc;
+    std::sort(matches_out, matches_out + std::min(*total_out, cap),
+              [](const mod_match& a, const mod_match& b) { return a.desc != b.desc ? a.desc < b.desc : a.pos < b.pos; });
+    return MOD_OK;
+    MOD_ABI_END("mod_find_masked_batch")
+}
+
+/* ---- pattern sets ------------------------------------------------------------------------------ */
+
+// The body of mod_pattern_set_create and mod_pattern_set_create_nocase.  A folded set (`fold`) keeps every pattern
+// upper-cased (modk::fold_ascii) and sets the filter bit of every case variant of its first two bytes.
+static int pattern_set_create(const char* who, const uint8_t* bytes, const uint32_t* lens, uint32_t n, bool fold,
+                              mod_pattern_set** out)
+{
     if (!out)
-        return fail(MOD_ERR_ARG, "mod_pattern_set_create: out is null");
+        return fail(MOD_ERR_ARG, "%s: out is null", who);
     *out = nullptr;
     if (!bytes || !lens || n == 0 || n > modk::kMaxSetPatterns)
-        return fail(MOD_ERR_ARG, "mod_pattern_set_create: a set holds 1 to %u patterns", modk::kMaxSetPatterns);
+        return fail(MOD_ERR_ARG, "%s: a set holds 1 to %u patterns", who, modk::kMaxSetPatterns);
     std::vector<std::string> pats(n);
     uint64_t at = 0;
     for (uint32_t j = 0; j < n; ++j) {
         if (lens[j] == 0 || lens[j] > modk::kMaxPattern)
-            return fail(MOD_ERR_ARG, "mod_pattern_set_create: pattern %u is %u bytes, not 1 to %u", j, lens[j], modk::kMaxPattern);
+            return fail(MOD_ERR_ARG, "%s: pattern %u is %u bytes, not 1 to %u", who, j, lens[j], modk::kMaxPattern);
         pats[j].assign((const char*)bytes + at, lens[j]);
         at += lens[j];
+        if (fold)
+            for (char& ch : pats[j])
+                ch = (char)modk::fold_ascii((uint8_t)ch);
     }
     std::vector<uint32_t> order(n);
     for (uint32_t j = 0; j < n; ++j)
@@ -1483,7 +1602,8 @@ int mod_pattern_set_create(const uint8_t* bytes, const uint32_t* lens, uint32_t 
     std::sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return pats[a] != pats[b] ? pats[a] < pats[b] : a < b; });
     for (uint32_t j = 1; j < n; ++j)
         if (pats[order[j]] == pats[order[j - 1]])
-            return fail(MOD_ERR_ARG, "mod_pattern_set_create: patterns %u and %u are the same", order[j - 1], order[j]);
+            return fail(MOD_ERR_ARG, fold ? "%s: patterns %u and %u are the same ignoring case" : "%s: patterns %u and %u are the same",
+                        who, order[j - 1], order[j]);
 
     // the index: filter bits, the length-1 table, and the longer patterns sorted by their 2-byte key
     std::unique_ptr<modk::SetIndex> idx(new modk::SetIndex());
@@ -1495,12 +1615,18 @@ int mod_pattern_set_create(const uint8_t* bytes, const uint32_t* lens, uint32_t 
         lmin = std::min(lmin, lens[j]);
         lmax = std::max(lmax, lens[j]);
         const uint32_t b0 = (uint8_t)pats[j][0];
+        // the case variants of a folded byte: itself, and its lower case if it is a letter
+        const uint32_t v0 = fold && b0 - 0x41u < 26u ? b0 | 0x20u : b0;
         if (lens[j] == 1) {
             idx->one[b0] = (uint16_t)(j + 1);
-            for (uint32_t b1 = 0; b1 < 256; ++b1)
+            for (uint32_t b1 = 0; b1 < 256; ++b1) {
                 idx->bitmap[(b0 | b1 << 8) >> 5] |= 1u << ((b0 | b1 << 8) & 31u);
+                idx->bitmap[(v0 | b1 << 8) >> 5] |= 1u << ((v0 | b1 << 8) & 31u);
+            }
         } else {
-            idx->bitmap[key_of(j) >> 5] |= 1u << (key_of(j) & 31u);
+            const uint32_t b1 = (uint8_t)pats[j][1], v1 = fold && b1 - 0x41u < 26u ? b1 | 0x20u : b1;
+            for (uint32_t k : {b0 | b1 << 8, v0 | b1 << 8, b0 | v1 << 8, v0 | v1 << 8})
+                idx->bitmap[k >> 5] |= 1u << (k & 31u);
             longer.push_back(j);
         }
     }
@@ -1534,7 +1660,7 @@ int mod_pattern_set_create(const uint8_t* bytes, const uint32_t* lens, uint32_t 
         e = cudaStreamSynchronize(nullptr);
     if (e != cudaSuccess) {
         cudaFree(d_idx);
-        return fail(MOD_ERR_CUDA, "mod_pattern_set_create: %s", cudaGetErrorString(e));
+        return fail(MOD_ERR_CUDA, "%s: %s", who, cudaGetErrorString(e));
     }
     mod_pattern_set* set = new mod_pattern_set();
     set->device = c->device;
@@ -1543,9 +1669,23 @@ int mod_pattern_set_create(const uint8_t* bytes, const uint32_t* lens, uint32_t 
     set->n_keys = n_keys;
     set->lmin = lmin;
     set->lmax = lmax;
+    set->fold = fold;
     *out = set;
     return MOD_OK;
+}
+
+int mod_pattern_set_create(const uint8_t* bytes, const uint32_t* lens, uint32_t n, mod_pattern_set** out)
+{
+    MOD_ABI_BEGIN
+    return pattern_set_create("mod_pattern_set_create", bytes, lens, n, false, out);
     MOD_ABI_END("mod_pattern_set_create")
+}
+
+int mod_pattern_set_create_nocase(const uint8_t* bytes, const uint32_t* lens, uint32_t n, mod_pattern_set** out)
+{
+    MOD_ABI_BEGIN
+    return pattern_set_create("mod_pattern_set_create_nocase", bytes, lens, n, true, out);
+    MOD_ABI_END("mod_pattern_set_create_nocase")
 }
 
 int mod_pattern_set_destroy(mod_pattern_set* set)
@@ -1594,7 +1734,7 @@ static int plan_find_set_launch(const char* who, const mod_plan* plan, uint64_t 
     f.matches = (uint32_t*)d_matches;
     f.total = (unsigned long long*)d_total;
     f.cap = cap;
-    CUDA_TRY(modk::launch_find_set(f, (cudaStream_t)stream));
+    CUDA_TRY(modk::launch_find_set(f, set->fold, (cudaStream_t)stream));
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return MOD_OK;
 }
