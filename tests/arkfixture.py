@@ -1,7 +1,9 @@
 """Synthetic HDR + ARK sets on disk for the facade / CLI tests (built with the oracle)."""
 from __future__ import annotations
 
+import json
 import os
+import subprocess
 from typing import List, Optional, Sequence
 
 import numpy as np
@@ -9,6 +11,13 @@ import numpy as np
 import oracle
 import synth
 from oracle import ark_oracle as ao
+
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+# the reference-generated archive fixtures (tests/golden/make_ark_golden.py): one case per key, and the song list
+# the reference derived from the two DTA configs under "songs"
+with open(os.path.join(GOLD, "ark", "manifest.json")) as _f:
+    MANIFEST = json.load(_f)
+CASES = sorted(k for k in MANIFEST if k != "songs")
 
 DIRS = ["ps4/config", "ps4/songs/credits", "ps4/songs/tut0", "ps4/songs/custom1", "ps4/ui", "ps4/ui/textures", "ps4"]
 EXTS = ["dta_dta_ps4", "mogg", "png_ps4", "bin", "moggsong"]
@@ -188,3 +197,25 @@ def song_config_tree():
                              ("tree", 16, 15, [sym("preview_start_ms"), ("int", 6, 30000)]),
                              ("tree", 17, 16, [sym("boss_level"), ("int", 0, -1), ("float", 1, struct.pack("<f", 0.5))])])
     return ("tree", 16, 1, [sym("songs"), song, ("tree", 16, 20, [sym("unlock_tokens"), ("int", 0, 3)])])
+
+
+def ref_header(case: str) -> bytes:
+    """The header bytes the reference's SaveArk wrote for fixture `case`."""
+    plat = MANIFEST[case]["platform"]
+    with open(os.path.join(GOLD, "ark", case, f"main_{plat}.hdr"), "rb") as f:
+        return f.read()
+
+
+# ---- running the CLI -----------------------------------------------------------------------------------------
+
+def run(cli, cwd, *args, expect=0):
+    """stdout of the CLI `cli` run in `cwd`; exit code 0, or the CLI's error exit when `expect` is not 0."""
+    out = subprocess.run([cli, *args], cwd=cwd, capture_output=True, text=True, timeout=300)
+    assert out.returncode == (expect if expect == 0 else 255), out.stdout + out.stderr
+    return out.stdout
+
+
+def check_unpacked(out_dir, hdr, payloads):
+    for e, p in zip(hdr.entries, payloads):
+        got = open(os.path.join(out_dir, e.name), "rb").read()
+        assert got == p, e.name

@@ -1,7 +1,7 @@
 // tests/cpp/mock_abi.cpp -- TEST INFRASTRUCTURE.  A stand-in for the CUDA library's C ABI that
 // answers the facade's calls with the CPU ORACLE (oracle/cycle_oracle.c), so the host-side C++
 // (CArk, ArkHeader, the CLI) can be exercised end to end on a box without a GPU.  It is linked only
-// into tests/_build/modulate_mock; the product library never contains it.
+// into the test binaries of tests/_build (tests/searchutil.py); the product library never contains it.
 //
 // "Device" memory is host memory, "streams" run synchronously at enqueue time, and a plan is the
 // descriptor list plus the same first-tile prefix the real library computes (8 KiB tiles of one
@@ -14,31 +14,8 @@
 // library's plan_check_device; a stream of another device is a CUDA error there).
 #include <cstdlib>
 #include <cstring>
-#include <vector>
 
-#include "../../include/modulate_b200.h"
-
-extern "C" {
-void oracle_cycle_at(unsigned char* data, uint64_t size, int32_t key, uint64_t pos);
-int32_t oracle_key_jump(int32_t key, uint64_t pos);
-struct oracle_desc {
-    uint64_t src_off, dst_off;
-    uint32_t len;
-    int32_t key;
-};
-void oracle_cycle_batch(const oracle_desc* d, uint64_t n, const unsigned char* src, unsigned char* dst);
-}
-
-struct mod_plan {
-    std::vector<mod_desc> descs;
-    std::vector<uint64_t> first_tile;  // n + 1
-    uint32_t dst_align = 0;
-    int device = 0;
-};
-
-struct mock_stream {
-    int device;
-};
+#include "mock_abi.h"
 
 static thread_local int tl_device = 0;
 

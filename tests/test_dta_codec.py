@@ -7,7 +7,14 @@ import numpy as np
 import pytest
 
 from oracle import dta_oracle as do
-from test_facade_host import cli, run  # noqa: F401  (fixture + helper)
+from arkfixture import run, song_config_tree  # song_config_tree: shared with bench.py's cfg5 workload
+from searchutil import mock_cli
+
+
+@pytest.fixture(scope="session")
+def cli():
+    """modulate CLI on the mock ABI, without the search entry points."""
+    return mock_cli(0)
 
 
 def random_tree(rng, depth=0, ttype=16):
@@ -28,9 +35,6 @@ def random_tree(rng, depth=0, ttype=16):
         else:
             children.append(("int", 0, 7))
     return ("tree", ttype, int(rng.integers(0, 3000)), children)
-
-
-from arkfixture import song_config_tree  # noqa: E402,F401  (shared with bench.py's cfg5 workload)
 
 
 def test_oracle_roundtrip_and_known_bytes():

@@ -1,7 +1,6 @@
 """CPU: the host-side C++ (CArk facade, ArkHeader codec, CLI) driven end to end through a MOCK of
 the C ABI that answers with the oracle (tests/cpp/mock_abi.cpp).  Same flows run on the GPU with
 the real library in tests/test_gpu_facade.py."""
-import glob
 import os
 import subprocess
 
@@ -12,38 +11,14 @@ import oracle
 import synth
 from oracle import ark_oracle as ao
 import arkfixture
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-CSRC = os.path.join(ROOT, "modulate_b200", "csrc")
-BUILD = os.path.join(ROOT, "tests", "_build")
-MOCK = os.path.join(BUILD, "modulate_mock")
+from arkfixture import check_unpacked, reconstruct_walk, run
+from searchutil import ROOT, link, mock_cli
 
 
 @pytest.fixture(scope="session")
 def cli():
-    """modulate CLI linked against the oracle-backed mock ABI (g++ only, no CUDA)."""
-    oracle.build()
-    os.makedirs(BUILD, exist_ok=True)
-    srcs = sorted(glob.glob(os.path.join(CSRC, "*.cpp"))) + [os.path.join(CSRC, "cli", "modulate_main.cpp"),
-                                                              os.path.join(ROOT, "tests", "cpp", "mock_abi.cpp")]
-    deps = srcs + glob.glob(os.path.join(CSRC, "*.h")) + [os.path.join(ROOT, "include", "modulate_b200.h")]
-    if not os.path.exists(MOCK) or any(os.path.getmtime(d) > os.path.getmtime(MOCK) for d in deps):
-        subprocess.check_call(["g++", "-O1", "-std=c++17", "-Wall", "-pthread", "-I", os.path.join(ROOT, "include"), "-o", MOCK,
-                               *srcs, "-L", os.path.join(ROOT, "oracle"), "-loracle",
-                               f"-Wl,-rpath,{os.path.join(ROOT, 'oracle')}"])
-    return MOCK
-
-
-def run(cli, cwd, *args, expect=0):
-    out = subprocess.run([cli, *args], cwd=cwd, capture_output=True, text=True, timeout=300)
-    assert out.returncode == (expect if expect == 0 else 255), out.stdout + out.stderr
-    return out.stdout
-
-
-def check_unpacked(out_dir, hdr, payloads):
-    for e, p in zip(hdr.entries, payloads):
-        got = open(os.path.join(out_dir, e.name), "rb").read()
-        assert got == p, e.name
+    """modulate CLI linked against the oracle-backed mock ABI, without the search entry points (g++ only, no CUDA)."""
+    return mock_cli(0)
 
 
 @pytest.mark.parametrize("ps4", [True, False])
@@ -131,9 +106,6 @@ def test_pack_roundtrip_offsets_parts_and_header_bytes(cli, tmp_path, ps4):
     os.replace(tmp_path / "repacked" / f"main_{plat}.hdr", tmp_path / "again" / f"main_{plat}.hdr")
     run(cli, tmp_path / "again", *pre, "-unpack", "out")
     check_unpacked(tmp_path / "again" / "out", hdr, payloads)
-
-
-reconstruct_walk = arkfixture.reconstruct_walk
 
 
 def test_pack_filters_unknown_files_and_songs(cli, tmp_path):
@@ -297,12 +269,7 @@ def test_header_fuzz_never_crashes(cli, tmp_path):
 
 def test_external_caller_compiles_against_facade_headers(cli, tmp_path):
     """A caller that only includes the facade headers (reference class names and signatures)."""
-    exe = os.path.join(BUILD, "facade_sample")
-    srcs = sorted(glob.glob(os.path.join(CSRC, "*.cpp"))) + [os.path.join(ROOT, "tests", "cpp", "facade_sample.cpp"),
-                                                              os.path.join(ROOT, "tests", "cpp", "mock_abi.cpp")]
-    subprocess.check_call(["g++", "-O1", "-std=c++17", "-Wall", "-pthread", "-I", CSRC, "-I", os.path.join(ROOT, "include"),
-                           "-o", exe, *srcs, "-L", os.path.join(ROOT, "oracle"), "-loracle",
-                           f"-Wl,-rpath,{os.path.join(ROOT, 'oracle')}"])
+    exe = link("facade_sample", os.path.join(ROOT, "tests", "cpp", "facade_sample.cpp"))
     hdr, payloads, _ = arkfixture.write_archive(str(tmp_path), n_files=25, n_parts=2, seed=41)
     out = subprocess.run([exe, "main_ps4.hdr", "out/"], cwd=tmp_path, capture_output=True, text=True, timeout=120)
     assert out.returncode == 0, out.stdout + out.stderr

@@ -1,138 +1,29 @@
 """CPU: the wildcard and case-insensitive searches (-findwild / -findi / -findilist, CArk::FindMaskedInFiles,
 CArk::FindSetInFiles with lbIgnoreCase) driven end to end through the oracle-backed mock of the C ABI
-(tests/cpp/mock_abi.cpp, mock_find_abi.cpp and mock_find_masked_abi.cpp, which also answers the set entry points with
-sets that may be folded).  Expected results come from numpy over the oracle-deciphered entries: every start compared
-under the mask, or after ASCII case folding."""
-import glob
+(tests/cpp/mock_abi.cpp, mock_find_abi.cpp).  Expected results come from the numpy reference of tests/searchutil.py
+over the oracle-deciphered entries: every start compared under the mask, or after ASCII case folding."""
 import os
 import re
 import subprocess
 
-import numpy as np
 import pytest
 
 import arkfixture
-import kernel_model_masked as kmm
-import oracle
-from test_facade_host import BUILD, CSRC, ROOT, run
-from test_find_host import PIECE_GROUP, SUMMARY, image_of, piece_cut_archive, planted_archive  # noqa: F401
-from test_ref_fixtures import CASES, MANIFEST, fixture_file_bytes, ref_header
-
-MOCK_FIND_MASKED = os.path.join(BUILD, "modulate_mock_find_masked")
-MOCK_NO_MASKED = os.path.join(BUILD, "modulate_mock_no_masked")
-FOLD = np.array([kmm.fold(b) for b in range(256)], np.uint8)
-
-
-def _link(out, mocks):
-    oracle.build()
-    os.makedirs(BUILD, exist_ok=True)
-    srcs = sorted(glob.glob(os.path.join(CSRC, "*.cpp"))) + [os.path.join(CSRC, "cli", "modulate_main.cpp")] + \
-        [os.path.join(ROOT, "tests", "cpp", f) for f in mocks]
-    deps = srcs + glob.glob(os.path.join(CSRC, "*.h")) + [os.path.join(ROOT, "include", "modulate_b200.h")]
-    if not os.path.exists(out) or any(os.path.getmtime(d) > os.path.getmtime(out) for d in deps):
-        subprocess.check_call(["g++", "-O1", "-std=c++17", "-Wall", "-pthread", "-I", os.path.join(ROOT, "include"), "-o",
-                               out, *srcs, "-L", os.path.join(ROOT, "oracle"), "-loracle",
-                               f"-Wl,-rpath,{os.path.join(ROOT, 'oracle')}"])
-    return out
+from arkfixture import MANIFEST, CASES, fixture_file_bytes, ref_header, run
+from searchutil import (SUMMARY, check_nocase, check_nocase_set, check_wild, expected_output, mock_cli, piece_cut_archive,
+                        planted_archive)
 
 
 @pytest.fixture(scope="session")
 def cli():
-    """modulate CLI linked against the mock ABI with every search entry point, the masked ones included
-    (mock_find_masked_abi.cpp takes the place of mock_find_set_abi.cpp)."""
-    return _link(MOCK_FIND_MASKED, ("mock_abi.cpp", "mock_find_abi.cpp", "mock_find_masked_abi.cpp"))
+    """modulate CLI on the mock ABI with every search entry point, the masked ones and folded sets included."""
+    return mock_cli(3)
 
 
 @pytest.fixture(scope="session")
 def old_cli():
-    """The same without mock_find_masked_abi.cpp: a library that predates the masked entry points."""
-    return _link(MOCK_NO_MASKED, ("mock_abi.cpp", "mock_find_abi.cpp", "mock_find_set_abi.cpp"))
-
-
-def wild_hex(value: bytes, mask: bytes) -> str:
-    """The -findwild text of (value, mask) with nibble masks only."""
-    out = []
-    for v, m in zip(value, mask):
-        out.append("".join("%x" % ((v >> s) & 15) if (m >> s) & 15 == 15 else "?" for s in (4, 0)))
-    return " ".join(out)
-
-
-def entries(root, plat, key):
-    hdr, _ = arkfixture.read_header(os.path.join(root, f"main_{plat}.hdr"))
-    image = image_of(root, hdr)
-    for e in hdr.entries:
-        yield e, (oracle.cycle(image[e.offset:e.offset + e.size], key) if key else image[e.offset:e.offset + e.size])
-
-
-def oracle_masked(root, plat, value, mask, key=0):
-    """(lines, total, files) the CLI must print for a masked search."""
-    lines, total, files = [], 0, 0
-    for e, data in entries(root, plat, key):
-        pos = kmm.masked_positions(data, value, mask)
-        total += len(pos)
-        files += bool(pos)
-        lines += [f"{e.name}\t{p}" for p in pos]
-    return lines, total, files
-
-
-def cli_out(cli, root, *args, env=None, expect=0):
-    out = subprocess.run([cli, *args], cwd=root, capture_output=True, timeout=600, env=env)
-    stdout = out.stdout.decode("latin-1")
-    assert out.returncode == (0 if expect == 0 else 255), stdout + out.stderr.decode("latin-1")
-    m = SUMMARY.search(stdout)
-    lines = [ln for ln in stdout.splitlines() if "\t" in ln]
-    return lines, int(m.group(1)) if m else None, int(m.group(2)) if m else None, stdout
-
-
-def _pre(plat, key):
-    return (["-ps3"] if plat == "ps3" else []) + (["-bodykey", str(key)] if key else [])
-
-
-def check_wild(cli, root, plat, value, mask, key=0, env=None):
-    got = cli_out(cli, root, *_pre(plat, key), "-findwild", wild_hex(value, mask), env=env)
-    want = oracle_masked(root, plat, bytes(v & m for v, m in zip(value, mask)), mask, key)
-    assert got[1:3] == want[1:], (value.hex(), mask.hex())
-    if want[1] <= 10000:
-        assert got[0] == want[0]
-    return got
-
-
-def check_nocase(cli, root, plat, text: bytes, key=0):
-    got = cli_out(cli, root, *_pre(plat, key), "-findi", text)
-    folded = bytes(FOLD[np.frombuffer(text, np.uint8)])
-    mask = bytes(0xDF if 0x41 <= b <= 0x5A else 0xFF for b in folded)
-    want = oracle_masked(root, plat, folded, mask, key)
-    assert got[1:3] == want[1:], text
-    if want[1] <= 10000:
-        assert got[0] == want[0]
-    assert f"for {len(text)} bytes, ignoring case" in got[3]
-    return got
-
-
-def oracle_nocase_set(root, plat, pats, key=0):
-    lines, counts, total, files = [], [0] * len(pats), 0, 0
-    for e, data in entries(root, plat, key):
-        fdata = FOLD[data]
-        hits = sorted((p, j) for j, pat in enumerate(pats)
-                      for p in kmm.masked_positions(fdata, bytes(FOLD[np.frombuffer(pat, np.uint8)]), b"\xff" * len(pat)))
-        for _, j in hits:
-            counts[j] += 1
-        total += len(hits)
-        files += bool(hits)
-        lines += [f"{e.name}\t{p}\t{pats[j].decode('latin-1')}" for p, j in hits]
-    return lines, [f"{c}\t{p.decode('latin-1')}" for c, p in zip(counts, pats)], total, files
-
-
-def check_nocase_set(cli, root, plat, pats, key=0):
-    (root / "ilist.txt").write_bytes(b"".join(p + b"\n" for p in pats))
-    lines, total, files, stdout = cli_out(cli, root, *_pre(plat, key), "-findilist", str(root / "ilist.txt"))
-    want_lines, want_counts, want_total, want_files = oracle_nocase_set(root, plat, pats, key)
-    assert (total, files) == (want_total, want_files)
-    assert [ln for ln in lines if ln.count("\t") == 1] == want_counts
-    if want_total <= 10000:
-        assert [ln for ln in lines if ln.count("\t") == 2] == want_lines
-    assert f"for {len(pats)} patterns, ignoring case" in stdout
-    return total
+    """The same on a library that predates the masked entry points (single-pattern and set search only)."""
+    return mock_cli(2)
 
 
 def _reference_archive(tmp_path, case):
@@ -224,9 +115,9 @@ def test_two_mock_devices(cli, tmp_path):
     out = subprocess.run([cli, "-bodykey", str(key), "-findwild", "17 ?a"], cwd=tmp_path, capture_output=True, timeout=600,
                          env=env)
     assert out.returncode == 0 and "on 2 GPU(s)" in out.stderr.decode()
-    want = oracle_masked(tmp_path, "ps4", b"\x17\x0a", b"\xff\x0f", key)
-    assert SUMMARY.search(out.stdout.decode("latin-1")).groups() == (str(want[1]), str(want[2]))
-    assert want[1] > 10000
+    _, _, want_total, want_files = expected_output(tmp_path, "ps4", [b"\x17\x0a"], [b"\xff\x0f"], key=key)
+    assert SUMMARY.search(out.stdout.decode("latin-1")).groups() == (str(want_total), str(want_files))
+    assert want_total > 10000
 
 
 def test_facade_without_the_masked_entry_points(old_cli, tmp_path):

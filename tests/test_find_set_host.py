@@ -1,8 +1,7 @@
 """CPU: the pattern-set search (-findlist / -findhexlist, CArk::FindSetInFiles, the owned-start bounds of the
 slot-ring GPU step) driven end to end through the oracle-backed mock of the C ABI (tests/cpp/mock_abi.cpp,
-mock_find_abi.cpp, mock_find_set_abi.cpp).  Expected results come from numpy over the oracle-deciphered entries:
-every start compared with every pattern, so overlapping matches and several patterns at one start all count."""
-import glob
+mock_find_abi.cpp).  Expected results come from numpy over the oracle-deciphered entries: every start compared with
+every pattern, so overlapping matches and several patterns at one start all count."""
 import os
 import re
 import subprocess
@@ -11,70 +10,20 @@ import numpy as np
 import pytest
 
 import arkfixture
-import oracle
-from test_facade_host import BUILD, CSRC, ROOT, run
-from test_find_host import MOCK_FIND, PIECE_GROUP, SUMMARY, cli as find_cli, image_of, planted_archive, positions  # noqa: F401
-from test_ref_fixtures import CASES, MANIFEST, fixture_file_bytes, ref_header
-
-MOCK_FIND_SET = os.path.join(BUILD, "modulate_mock_find_set")
+from arkfixture import CASES, MANIFEST, fixture_file_bytes, ref_header, run
+from searchutil import SUMMARY, check_set, cli_find_set, expected_output, mock_cli, owned_trap_archive, planted_archive
 
 
 @pytest.fixture(scope="session")
 def cli():
-    """modulate CLI linked against the oracle-backed mock ABI with its search and set-search entry points."""
-    oracle.build()
-    os.makedirs(BUILD, exist_ok=True)
-    srcs = sorted(glob.glob(os.path.join(CSRC, "*.cpp"))) + [os.path.join(CSRC, "cli", "modulate_main.cpp")] + \
-        [os.path.join(ROOT, "tests", "cpp", f) for f in ("mock_abi.cpp", "mock_find_abi.cpp", "mock_find_set_abi.cpp")]
-    deps = srcs + glob.glob(os.path.join(CSRC, "*.h")) + [os.path.join(ROOT, "include", "modulate_b200.h")]
-    if not os.path.exists(MOCK_FIND_SET) or any(os.path.getmtime(d) > os.path.getmtime(MOCK_FIND_SET) for d in deps):
-        subprocess.check_call(["g++", "-O1", "-std=c++17", "-Wall", "-pthread", "-I", os.path.join(ROOT, "include"), "-o",
-                               MOCK_FIND_SET, *srcs, "-L", os.path.join(ROOT, "oracle"), "-loracle",
-                               f"-Wl,-rpath,{os.path.join(ROOT, 'oracle')}"])
-    return MOCK_FIND_SET
+    """modulate CLI on the mock ABI of a library with the single-pattern and the set search."""
+    return mock_cli(2)
 
 
-def oracle_find_set(root, plat, pats, shown, key=0):
-    """(match lines, per-pattern lines, total, files) the CLI must print."""
-    hdr, _ = arkfixture.read_header(os.path.join(root, f"main_{plat}.hdr"))
-    image = image_of(root, hdr)
-    lines, counts, total, files = [], [0] * len(pats), 0, 0
-    for e in hdr.entries:
-        data = oracle.cycle(image[e.offset:e.offset + e.size], key) if key else image[e.offset:e.offset + e.size]
-        hits = sorted((p, j) for j, pat in enumerate(pats) for p in positions(data, pat))
-        for p, j in hits:
-            counts[j] += 1
-        total += len(hits)
-        files += bool(hits)
-        lines += [f"{e.name}\t{p}\t{shown[j]}" for p, j in hits]
-    return lines, [f"{c}\t{s}" for c, s in zip(counts, shown)], total, files
-
-
-def cli_find_set(cli, root, pats, *pre, env=None, hex_form=True, expect=0):
-    """Write the list, run the CLI -> (match lines, count lines, total, files, stdout)."""
-    path = os.path.join(root, "patterns.txt")
-    with open(path, "wb") as f:
-        f.write(b"".join((p.hex() if hex_form else p.decode("latin-1")).encode("latin-1") + b"\n" for p in pats))
-    out = subprocess.run([cli, *pre, "-findhexlist" if hex_form else "-findlist", path], cwd=root, capture_output=True,
-                         timeout=600, env=env)
-    stdout = out.stdout.decode("latin-1")
-    assert out.returncode == (0 if expect == 0 else 255), stdout + out.stderr.decode("latin-1")
-    rows = [ln for ln in stdout.splitlines() if "\t" in ln]
-    match_lines = [ln for ln in rows if ln.count("\t") == 2]
-    count_lines = [ln for ln in rows if ln.count("\t") == 1]
-    m = SUMMARY.search(stdout)
-    return match_lines, count_lines, int(m.group(1)) if m else None, int(m.group(2)) if m else None, stdout
-
-
-def check_set(cli, root, plat, pats, key=0, env=None, hex_form=True):
-    pre = (["-ps3"] if plat == "ps3" else []) + (["-bodykey", str(key)] if key else [])
-    shown = [p.hex() for p in pats] if hex_form else [p.decode("latin-1") for p in pats]
-    got = cli_find_set(cli, root, pats, *pre, env=env, hex_form=hex_form)
-    want = oracle_find_set(root, plat, pats, shown, key)
-    assert got[1:4] == want[1:], (got[1:4], want[1:])
-    if want[2] <= 10000:
-        assert got[0] == want[0]
-    return got
+@pytest.fixture(scope="session")
+def find_cli():
+    """The same on a library with the single-pattern search only."""
+    return mock_cli(1)
 
 
 @pytest.mark.parametrize("case", CASES)
@@ -145,7 +94,7 @@ def test_output_order_and_the_line_cut(cli, tmp_path):
     arkfixture.write_archive(str(tmp_path), n_files=len(sizes), n_parts=2, seed=5, sizes=sizes, contents=contents)
     pats = [b"AA", b"A", b"AAAA", b"B"]
     lines, counts, total, files, stdout = cli_find_set(cli, tmp_path, pats)
-    want_lines, want_counts, want_total, want_files = oracle_find_set(tmp_path, "ps4", pats, [p.hex() for p in pats])
+    want_lines, want_counts, want_total, want_files = expected_output(tmp_path, "ps4", pats, shown=[p.hex() for p in pats])
     assert (counts, total, files) == (want_counts, want_total, want_files)
     assert want_total > 10000 and lines == want_lines[:10000]
     assert f"... {want_total - 10000} more" in stdout
@@ -174,31 +123,12 @@ def test_two_mock_devices(cli, tmp_path):
     assert out.returncode == 0, out.stdout.decode("latin-1")
     assert "on 2 GPU(s)" in out.stderr.decode()
     stdout = out.stdout.decode("latin-1")
-    want_lines, want_counts, want_total, want_files = oracle_find_set(tmp_path, "ps4", pats, [p.hex() for p in pats], key)
+    want_lines, want_counts, want_total, want_files = expected_output(tmp_path, "ps4", pats, key=key,
+                                                                      shown=[p.hex() for p in pats])
     rows = [ln for ln in stdout.splitlines() if "\t" in ln]
     assert [ln for ln in rows if ln.count("\t") == 1] == want_counts
     assert SUMMARY.search(stdout).groups() == (str(want_total), str(want_files))
     assert want_total > 10000
-
-
-def owned_trap_archive(root, pats):
-    """Big entries that 1 MiB groups cut into pieces overlapping by Lmax - 1 = 63 bytes, with every pattern planted
-    in the 63 bytes after every cut: a piece that reported starts in its overlap would count them twice."""
-    G = PIECE_GROUP
-    key = 0x0BADC0DE
-    sizes = [3_500_000, 10, 2_200_001, 1_572_864, 70_000]
-    rng = np.random.default_rng(17)
-    contents = {}
-    for i, s in enumerate(sizes):
-        blob = bytearray(rng.integers(0, 256, size=s, dtype=np.uint8).tobytes())
-        for cut in range(G, s, G):
-            for start, pat in ((cut, pats[0]), (cut + 1, pats[1]), (cut + 30, pats[0]), (cut + 62, pats[0]),
-                               (cut + 20, pats[1]), (cut + 40, pats[1]), (cut - 64, pats[2]), (cut + 70, pats[2])):
-                if start + len(pat) <= s:
-                    blob[start:start + len(pat)] = pat
-        contents[i] = bytes(blob)
-    arkfixture.write_archive(str(root), n_files=len(sizes), n_parts=2, seed=23, body_key=key, sizes=sizes, contents=contents)
-    return key
 
 
 def test_owned_starts_at_every_piece_cut(cli, tmp_path):
@@ -215,7 +145,7 @@ def test_owned_starts_at_every_piece_cut(cli, tmp_path):
 
 def test_facade_without_the_set_search_entry_points(find_cli, tmp_path):
     """Linked against an ABI implementation with the single-pattern search but without the set entry points (the
-    mock without mock_find_set_abi.cpp), the facade still links, -find works and -findlist says what is missing."""
+    mock of generation 1), the facade still links, -find works and -findlist says what is missing."""
     arkfixture.write_archive(str(tmp_path), n_files=12, n_parts=2, seed=3)
     (tmp_path / "l.txt").write_bytes(b"abc\n")
     assert "has no set search" in run(find_cli, tmp_path, "-findlist", str(tmp_path / "l.txt"), expect=1)

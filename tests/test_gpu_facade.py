@@ -10,7 +10,7 @@ import oracle
 import synth
 from oracle import ark_oracle as ao
 import arkfixture
-from test_facade_host import check_unpacked, reconstruct_walk
+from arkfixture import check_unpacked, reconstruct_walk
 
 pytestmark = pytest.mark.gpu
 

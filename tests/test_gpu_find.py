@@ -12,39 +12,10 @@ import oracle
 import synth
 import arkfixture
 import modulate_b200 as mb
-from gpuutil import DeviceBuffer, sync
-from test_find_host import check, oracle_find, piece_cut_archive, SUMMARY
+from gpuutil import CLI, EDGE_KEYS, DeviceBuffer, build_source, shm_dir, sync
+from searchutil import MOD_ERR_ARG, SUMMARY, check, expected_output, piece_cut_archive, search_one
 
 pytestmark = pytest.mark.gpu
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-CLI = os.path.join(ROOT, "modulate_b200", "bin", "modulate")
-EDGE_KEYS = [0, 0x7FFFFFFF, -0x80000000, -1, 1]
-
-
-def plain_find(plain_entries, pat):
-    """Oracle matches (desc, pos) and counts of the wanted deciphered entries."""
-    out, counts = [], []
-    P = np.frombuffer(pat, np.uint8)
-    for i, e in enumerate(plain_entries):
-        n = 0
-        if e.size >= len(pat):
-            w = np.lib.stride_tricks.sliding_window_view(e, len(pat))
-            pos = np.nonzero((w == P).all(axis=1))[0]
-            out += [(i, int(p)) for p in pos]
-            n = len(pos)
-        counts.append(n)
-    return out, np.array(counts, np.uint32)
-
-
-def build_source(plain_entries, keys, phase):
-    """Byte-packed source whose entries decipher to `plain_entries` (Cycle is its own inverse)."""
-    sizes = np.array([e.size for e in plain_entries], np.int64)
-    src_off = synth.packed_offsets(sizes) + phase
-    src = np.zeros(int(phase + sizes.sum() + 64), np.uint8)
-    for e, o, k in zip(plain_entries, src_off, keys):
-        src[o:o + e.size] = oracle.cycle(e, k)
-    return mb.make_descs(src_off, src_off, sizes, keys), src
 
 
 def run_find(plain_entries, keys, pat, phase=0, cap=1 << 16):
@@ -85,7 +56,7 @@ def test_kernel_matches_oracle_planted(L):
         ents = planted_entries(L, pat, rng, phase)
         for keys in ([k for k in EDGE_KEYS for _ in range(3)][:len(ents)], synth.entry_keys(len(ents)).tolist()):
             counts, matches, total = run_find(ents, keys, pat, phase)
-            want, want_counts = plain_find(ents, pat)
+            want, want_counts = search_one(ents, pat)
             assert matches == want and total == len(want) and (counts == want_counts).all(), (L, phase)
             assert len(want) >= 5
 
@@ -114,7 +85,7 @@ def test_redo_branch_inside_the_tile_and_the_halo():
         canon = km.canonical_bytes(km.chunk_states(int(st), chunk))
         assert spec[trig[0]] != canon[trig[0]]  # the speculative keystream is wrong inside the match
         counts, matches, total = run_find([plain], [km.i32(key)], pat, phase=h0)
-        want, _ = plain_find([plain], pat)
+        want, _ = search_one([plain], pat)
         assert (0, s) in want and matches == want and total == len(want)
 
 
@@ -124,7 +95,7 @@ def test_cap_truncation_keeps_exact_counts():
     for e in ents:
         e[rng.integers(0, e.size, size=e.size // 3)] = 1
     keys = synth.entry_keys(len(ents)).tolist()
-    want, want_counts = plain_find(ents, b"\x00")
+    want, want_counts = search_one(ents, b"\x00")
     counts, matches, total = run_find(ents, keys, b"\x00", cap=1000)
     assert total == len(want) and (counts == want_counts).all()
     assert len(matches) == 1000 and set(matches) <= set(want) and matches == sorted(matches)
@@ -137,7 +108,7 @@ def test_find_window_over_a_slot_ring_equals_the_whole_plan():
     ents = [rng.integers(0, 256, size=s, dtype=np.uint8) for s in sizes]
     keys = synth.entry_keys(len(ents)).tolist()
     descs, src = build_source(ents, keys, 9)
-    want, want_counts = plain_find(ents, pat)
+    want, want_counts = search_one(ents, pat)
     whole = DeviceBuffer.from_numpy(src)
     plan = mb.Plan(descs, src.size, src.size, 0)
     cap = 1 << 16
@@ -178,7 +149,7 @@ def test_find_window_over_a_slot_ring_equals_the_whole_plan():
             mb.find_batch(descs, whole.ptr, bad, src_bytes=src.size)
         cnt, tot = np.zeros(len(ents), np.uint32), ctypes.c_uint64()
         assert lib.mod_find_batch(descs.ctypes.data, len(descs), whole.ptr, src.size, bad + b"\0", len(bad), cnt.ctypes.data,
-                                  None, 0, ctypes.byref(tot)) == -2  # MOD_ERR_ARG
+                                  None, 0, ctypes.byref(tot)) == MOD_ERR_ARG
     plan.close()
 
 
@@ -217,12 +188,6 @@ def test_one_gib_ten_thousand_entries_against_numpy():
     buf.free()
 
 
-def shm_dir(tmp_path):
-    base = "/dev/shm" if os.path.isdir("/dev/shm") and os.access("/dev/shm", os.W_OK) else str(tmp_path)
-    import tempfile
-    return tempfile.mkdtemp(prefix="modfind", dir=base)
-
-
 def test_facade_find_on_a_ciphered_1gib_archive(tmp_path):
     import shutil
     if not os.path.exists(CLI):
@@ -234,7 +199,7 @@ def test_facade_find_on_a_ciphered_1gib_archive(tmp_path):
         sizes = [int(x) for x in synth.entry_sizes_loguniform(10000, 1 << 30, seed=5)]
         arkfixture.write_archive(root, n_files=len(sizes), n_parts=4, seed=37, body_key=key, sizes=sizes)
         pat = b"\x5a\xa5\x0f"
-        want_lines, want_total, want_files = oracle_find(root, "ps4", pat, key)
+        want_lines, _, want_total, want_files = expected_output(root, "ps4", [pat], key=key)
         runs = [{}]
         if mb.device_count() >= 2:
             runs.append({"MOD_DEVICES": "0x3"})

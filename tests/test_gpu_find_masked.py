@@ -17,29 +17,11 @@ import oracle
 import synth
 import modulate_b200 as mb
 from modulate_b200 import _abi
-from gpuutil import DeviceBuffer, sync
-from test_find_masked_host import check_nocase, check_nocase_set, check_wild
-from test_find_host import piece_cut_archive
-from test_gpu_find import CLI, build_source, shm_dir
-from test_gpu_find_paths import Results, _buffer, _cases, _mdescs, _plain
-from test_gpu_find_set import as_list
+from gpuutil import (CLI, DeviceBuffer, Results, aligned_buffer, as_list, build_source, cases_by_cell, decipher_entries,
+                     model_descs, shm_dir, sync)
+from searchutil import FOLD, MOD_ERR_ARG, check_nocase, check_nocase_set, check_wild, piece_cut_archive, search, search_one
 
 pytestmark = pytest.mark.gpu
-
-MOD_ERR_ARG = -2
-FOLD = np.array([kmm.fold(b) for b in range(256)], np.uint8)
-
-
-def masked_find(plain_entries, value, mask):
-    """numpy: matches (desc, pos) and counts per entry."""
-    out = []
-    for i, e in enumerate(plain_entries):
-        out += [(i, p) for p in kmm.masked_positions(e, value, mask)]
-    return out, np.bincount([d for d, _ in out], minlength=len(plain_entries)).astype(np.uint32)
-
-
-def fold_mask(value: bytes) -> bytes:
-    return bytes(0xDF if 0x41 <= b <= 0x5A else 0xFF for b in value)
 
 
 def cell_masks(L):
@@ -54,18 +36,18 @@ def cell_masks(L):
 
 @pytest.mark.parametrize("cell", sorted(km.reachable_find_cells()), ids=lambda c: "-".join(c))
 def test_model_cases_through_the_masked_kernel(mb, cell):
-    case = _cases()[cell]
-    plain = _plain(case.descs, case.image)
+    case = cases_by_cell()[cell]
+    plain = decipher_entries(case.descs, case.image)
     mem = case.memory()
-    buf = _buffer(mem)
+    buf = aligned_buffer(mem)
     la, r = case.target_tile()
     base = km.TILE_BYTES * r.tin - r.h0
     try:
         for mask in cell_masks(case.L):
             value = bytes(v & m for v, m in zip(case.pattern, mask))
-            want, want_counts = masked_find(plain, value, mask)
+            want, want_counts = search_one(plain, value, mask)
             if case.kind == "batch":
-                counts, matches, total = mb.find_batch(_mdescs(case.descs), buf.ptr + case.src_ptr, value,
+                counts, matches, total = mb.find_batch(model_descs(case.descs), buf.ptr + case.src_ptr, value,
                                                        src_bytes=case.image_bytes, max_matches=1 << 16, mask=mask)
                 matches = [(int(a), int(b)) for a, b in zip(matches["desc"], matches["pos"])]
             else:
@@ -74,7 +56,7 @@ def test_model_cases_through_the_masked_kernel(mb, cell):
                 want = [(d, p) for d, p in want if d == case.target and lo <= p < hi]
                 want_counts = np.zeros(len(case.descs), np.uint32)
                 want_counts[case.target] = len(want)
-                plan = mb.Plan(_mdescs(case.descs), case.image_bytes, case.image_bytes, case.dst_align)
+                plan = mb.Plan(model_descs(case.descs), case.image_bytes, case.image_bytes, case.dst_align)
                 res = Results(len(case.descs), 1 << 12)
                 plan.find_window(t0, t1, buf.ptr + wp, wo, wb, value, res.counts, res.matches, res.cap, res.total, mask=mask)
                 sync()
@@ -156,7 +138,7 @@ def test_length_anchor_phase_matrix(mb, L, kind):
             counts, matches, total = mb.find_batch(descs, buf.ptr, value, src_bytes=src.size, max_matches=1 << 16, mask=mask)
         finally:
             buf.free()
-        want, want_counts = masked_find(ents, value, mask)
+        want, want_counts = search_one(ents, value, mask)
         got = [(int(d), int(p)) for d, p in zip(matches["desc"], matches["pos"])]
         assert total == len(want) and got == want and counts.tolist() == want_counts.tolist(), (L, a, phase, mask.hex())
         assert total >= 4
@@ -172,7 +154,7 @@ def test_fold_edge_bytes_do_not_fold(mb, pair):
     for b in (lo, hi):
         value, mask = mb.ignore_case_pattern(bytes([b, 0x61]))
         assert mask[0] == 0xFF
-        want, _ = masked_find(ents, value, mask)
+        want, _ = search_one(ents, value, mask)
         descs, src = build_source(ents, [0x1234], 3)
         buf = DeviceBuffer.from_numpy(src)
         _, matches, total = mb.find_batch(descs, buf.ptr, value, src_bytes=src.size, mask=mask)
@@ -203,7 +185,7 @@ def _one_entry_plan(rng):
 def test_cap_accumulation_and_windows(mb):
     rng = np.random.default_rng(9)
     ent, descs, src, value, mask = _one_entry_plan(rng)
-    want, _ = masked_find([ent], value, mask)
+    want, _ = search_one([ent], value, mask)
     n = len(want)
     buf = DeviceBuffer.from_numpy(src)
     plan = mb.Plan(descs, src.size, src.size, buf.ptr & 15)
@@ -267,16 +249,6 @@ def _mixed_case(p, rng):
     return bytes(b ^ 0x20 if (0x41 <= (b & 0xDF) <= 0x5A and rng.integers(2)) else b for b in p)
 
 
-def plain_find_set_nocase(ents, pats):
-    out = []
-    for i, e in enumerate(ents):
-        fe = FOLD[e]
-        for j, p in enumerate(pats):
-            out += [(i, q, j) for q in kmm.masked_positions(fe, bytes(FOLD[np.frombuffer(p, np.uint8)]), b"\xff" * len(p))]
-    out.sort()
-    return out
-
-
 @pytest.mark.parametrize("K", [1, 17, 256])
 def test_folded_sets_against_numpy(mb, K):
     rng = np.random.default_rng(K)
@@ -308,7 +280,7 @@ def test_folded_sets_against_numpy(mb, K):
             sync()
             total = res.read()[0]
             got = sorted(as_list(m.download().view(mb.SET_MATCH_DTYPE)[:total]))
-            want = plain_find_set_nocase(ents, pats)
+            want = search(ents, pats, fold=True)[0]
             assert total == len(want) and got == want, (K, phase)
             assert pc.download().view(np.uint64).tolist() == np.bincount([w[2] for w in want], minlength=K).tolist()
             for x in (plan, pset):
@@ -336,7 +308,7 @@ def test_folded_set_prefixes_letters_and_refusals(mb):
     plan.find_set(buf.ptr, pset, res.counts, pc.ptr, m.ptr, 1 << 14, res.total)
     sync()
     total = res.read()[0]
-    want = plain_find_set_nocase(ents, pats)
+    want = search(ents, pats, fold=True)[0]
     assert sorted(as_list(m.download().view(mb.SET_MATCH_DTYPE)[:total])) == want
     assert pc.download().view(np.uint64).tolist() == np.bincount([w[2] for w in want], minlength=4).tolist()
     assert sum(1 for w in want if w[0] == 0 and w[2] < 2) == 200  # aB1 AB1 / Ab2 ab2

@@ -7,72 +7,29 @@ where the tile has a second trigger, a false match that only a skipped redo repo
 decoy in the bytes the CTA deciphers but does not own -- chunk 0 before the entry, the last chunk after it, the
 zero-filled end of the halo, the next tile -- written in cipher space so that the tile holds the pattern there:
 the kernel must not count it."""
-import functools
-
 import numpy as np
 import pytest
 
 import kernel_model as km
 import oracle
 import modulate_b200 as mb
-from gpuutil import DeviceBuffer, sync
-from test_gpu_find import plain_find
+from gpuutil import DeviceBuffer, Results, aligned_buffer, cases_by_cell, decipher_entries, model_descs, sync
+from searchutil import MOD_ERR_ALIGN, MOD_ERR_ARG, search_one
 
 pytestmark = pytest.mark.gpu
-
-MOD_ERR_ARG, MOD_ERR_ALIGN = -2, -3
-
-
-@functools.lru_cache(maxsize=None)
-def _cases():
-    return {c.cell: c for c in km.find_cases()}
-
-
-def _buffer(a: np.ndarray) -> DeviceBuffer:
-    b = DeviceBuffer.from_numpy(a)
-    assert b.ptr % 16 == 0  # the model's addresses are offsets from 16-byte aligned bases
-    return b
-
-
-class Results:
-    """total (u64), counts (u32 per descriptor) and a list of `cap` matches in one device buffer; the list is
-    16-byte aligned, as mod_match stores need."""
-
-    def __init__(self, n: int, cap: int):
-        self.n, self.cap = n, cap
-        self.list_at = (16 + 4 * n + 15) & ~15
-        self.buf = DeviceBuffer(self.list_at + 8 * max(cap, 1))
-        self.buf.upload(np.zeros(self.buf.nbytes, np.uint8))
-        self.total, self.counts, self.matches = self.buf.ptr, self.buf.ptr + 16, self.buf.ptr + self.list_at
-
-    def read(self):
-        raw = self.buf.download()
-        total = int(raw[:8].view(np.uint64)[0])
-        counts = raw[16:16 + 4 * self.n].view(np.uint32).copy()
-        m = raw[self.list_at:].view(mb.MATCH_DTYPE)[:min(total, self.cap)]
-        return total, counts, [(int(a), int(b)) for a, b in zip(m["desc"], m["pos"])]
-
-
-def _plain(descs, image):
-    return [oracle.cycle(image[so:so + ln], key) for so, ln, key in descs]
-
-
-def _mdescs(descs):
-    so, ln, key = zip(*descs)
-    return mb.make_descs(list(so), list(so), list(ln), [k & 0xFFFFFFFF for k in key])
 
 
 @pytest.mark.parametrize("cell", sorted(km.reachable_find_cells()), ids=lambda c: "-".join(c))
 def test_find_path_cell(mb, cell):
-    case = _cases()[cell]
+    case = cases_by_cell()[cell]
     assert cell in case.cells()
     pat = case.pattern
-    want, want_counts = plain_find(_plain(case.descs, case.image), pat)
+    want, want_counts = search_one(decipher_entries(case.descs, case.image), pat)
     mem = case.memory()
-    buf = _buffer(mem)
+    buf = aligned_buffer(mem)
     try:
         if case.kind == "batch":
-            counts, matches, total = mb.find_batch(_mdescs(case.descs), buf.ptr + case.src_ptr, pat,
+            counts, matches, total = mb.find_batch(model_descs(case.descs), buf.ptr + case.src_ptr, pat,
                                                    src_bytes=case.image_bytes, max_matches=1 << 16)
             matches = [(int(a), int(b)) for a, b in zip(matches["desc"], matches["pos"])]
         else:
@@ -81,7 +38,7 @@ def test_find_path_cell(mb, cell):
             want = [(d, p) for d, p in want if d == case.target and lo <= p < hi]
             want_counts = np.zeros(len(case.descs), np.uint32)
             want_counts[case.target] = len(want)
-            plan = mb.Plan(_mdescs(case.descs), case.image_bytes, case.image_bytes, case.dst_align)
+            plan = mb.Plan(model_descs(case.descs), case.image_bytes, case.image_bytes, case.dst_align)
             res = Results(len(case.descs), 1 << 12)
             plan.find_window(t0, t1, buf.ptr + wp, wo, wb, pat, res.counts, res.matches, res.cap, res.total)
             sync()
@@ -165,9 +122,9 @@ def test_compare_and_filter_matrix(mb, L, kind):
     image = rng.integers(0, 256, size=off + 40, dtype=np.uint8)
     for (so, ln, key), p in zip(descs, plains):
         image[so:so + ln] = oracle.cycle(p, key)
-    want, want_counts = plain_find(plains, pat.tobytes())
-    buf = _buffer(np.concatenate([np.zeros(src_ptr, np.uint8), image]))
-    counts, matches, total = mb.find_batch(_mdescs(descs), buf.ptr + src_ptr, pat.tobytes(), src_bytes=image.size,
+    want, want_counts = search_one(plains, pat.tobytes())
+    buf = aligned_buffer(np.concatenate([np.zeros(src_ptr, np.uint8), image]))
+    counts, matches, total = mb.find_batch(model_descs(descs), buf.ptr + src_ptr, pat.tobytes(), src_bytes=image.size,
                                            max_matches=1 << 20)
     buf.free()
     got = [(int(a), int(b)) for a, b in zip(matches["desc"], matches["pos"])]
@@ -196,11 +153,11 @@ def many_matches():
 def test_cap_keeps_exact_counts_and_lists_true_matches(mb, many_matches, which):
     descs, image, plains = many_matches
     pat = b"\x01\x02\x03"
-    want, want_counts = plain_find(plains, pat)
+    want, want_counts = search_one(plains, pat)
     n = len(want)
     cap = {"0": 0, "1": 1, "n-1": n - 1, "n": n, "n+1": n + 1}[which]
-    buf = _buffer(image)
-    plan = mb.Plan(_mdescs(descs), image.size, image.size, 0)
+    buf = aligned_buffer(image)
+    plan = mb.Plan(model_descs(descs), image.size, image.size, 0)
     res = Results(len(descs), cap)
     plan.find(buf.ptr, pat, res.counts, res.matches if cap else 0, cap, res.total)
     sync()
@@ -234,7 +191,7 @@ def test_window_bounds_inside_an_entry(mb, L):
     dst_align = (h0 - so) & 15
     image = rng.integers(0, 256, size=so + ln + 500, dtype=np.uint8)
     image[so:so + ln] = oracle.cycle(plain, key)
-    plan = mb.Plan(_mdescs(descs), image.size, image.size, dst_align)
+    plan = mb.Plan(model_descs(descs), image.size, image.size, dst_align)
     t0, t1 = 1, 3
     b0 = so + km.TILE_BYTES - h0
     b1 = so + 3 * km.TILE_BYTES - h0 + L - 1
@@ -246,10 +203,10 @@ def test_window_bounds_inside_an_entry(mb, L):
         _, a, p_end = km.scan_bounds(r, L)
         starts |= {km.TILE_BYTES * r.tin - h0 + p for p in range(a, p_end)}
     assert starts == set(range(lo, 3 * km.TILE_BYTES - h0))
-    want = sorted((0, q) for _, q in plain_find([plain], pat.tobytes())[0] if q in starts)
+    want = sorted((0, q) for _, q in search_one([plain], pat.tobytes())[0] if q in starts)
     for w_lo, w_hi, ok in ((b0, b1, True), (b0 + 1, b1, False), (b0, b1 - 1, False)):
         win_ptr = (w_lo + dst_align) & 15
-        buf = _buffer(np.concatenate([np.zeros(win_ptr, np.uint8), image[w_lo:w_hi]]))
+        buf = aligned_buffer(np.concatenate([np.zeros(win_ptr, np.uint8), image[w_lo:w_hi]]))
         res = Results(1, 1 << 10)
         assert km.find_window_ok(descs, dst_align, t0, t1, w_lo, w_hi - w_lo, L) == ok
         if ok:
@@ -284,9 +241,9 @@ def test_plans_off_the_source_grid_are_refused(mb):
     for (so, ln, key), p in zip(descs, plains):
         image[so:so + ln] = oracle.cycle(p, key)
     pat = b"\x02\x03"
-    want, want_counts = plain_find(plains, pat)
+    want, want_counts = search_one(plains, pat)
     src_ptr = 3
-    buf = _buffer(np.concatenate([np.zeros(src_ptr, np.uint8), image]))
+    buf = aligned_buffer(np.concatenate([np.zeros(src_ptr, np.uint8), image]))
     so, ln, key = zip(*descs)
     key = [k & 0xFFFFFFFF for k in key]
 

@@ -15,32 +15,11 @@ import kernel_model as km
 import oracle
 import synth
 import modulate_b200 as mb
-from gpuutil import DeviceBuffer, sync
-from test_find_set_host import check_set, oracle_find_set, owned_trap_archive
-from test_gpu_find import CLI, EDGE_KEYS, build_source, shm_dir
-from test_gpu_find_paths import Results, _buffer, _cases, _mdescs, _plain
+from gpuutil import (CLI, EDGE_KEYS, DeviceBuffer, Results, aligned_buffer, as_list, build_source, cases_by_cell,
+                     decipher_entries, model_descs, shm_dir, sync)
+from searchutil import MOD_ERR_ALIGN, MOD_ERR_ARG, check_set, expected_output, owned_trap_archive, search
 
 pytestmark = pytest.mark.gpu
-
-MOD_ERR_ARG, MOD_ERR_ALIGN = -2, -3
-
-
-def plain_find_set(plain_entries, pats):
-    """Oracle matches (desc, pos, pattern) sorted, counts per descriptor and per pattern."""
-    out = []
-    for i, e in enumerate(plain_entries):
-        for j, pat in enumerate(pats):
-            if e.size >= len(pat):
-                w = np.lib.stride_tricks.sliding_window_view(e, len(pat))
-                out += [(i, int(p), j) for p in np.nonzero((w == np.frombuffer(pat, np.uint8)).all(axis=1))[0]]
-    out.sort()
-    counts = np.bincount([m[0] for m in out], minlength=len(plain_entries)).astype(np.uint32)
-    pcounts = np.bincount([m[2] for m in out], minlength=len(pats)).astype(np.uint64)
-    return out, counts, pcounts
-
-
-def as_list(matches):
-    return [(int(a), int(b), int(c)) for a, b, c in zip(matches["desc"], matches["pos"], matches["pattern"])]
 
 
 def run_set(plain_entries, keys, pats, phase=0, cap=1 << 18):
@@ -55,7 +34,7 @@ def run_set(plain_entries, keys, pats, phase=0, cap=1 << 18):
 
 def check_against_oracle(ents, keys, pats, phase=0):
     counts, pcounts, matches, total = run_set(ents, keys, pats, phase)
-    want, want_counts, want_p = plain_find_set(ents, pats)
+    want, want_counts, want_p = search(ents, pats)
     assert total == len(want) and matches == want, (phase, len(pats))
     assert counts.tolist() == want_counts.tolist() and pcounts.tolist() == want_p.tolist()
     return want
@@ -155,16 +134,16 @@ def test_model_cases_through_the_set_kernel(cell):
     """Every case the kernel model builds for find_batch_kernel (redo cells, halo cells, guard decoys) run through the
     set kernel with the case's pattern inside a set of other lengths: the case's pattern gives the oracle's counts.
     Window cases take only patterns up to the case's length, so that the case's minimal window still holds."""
-    case = _cases()[cell]
+    case = cases_by_cell()[cell]
     rng = np.random.default_rng(zlib.crc32("-".join(cell).encode()))
     pats = _companions(case.pattern, rng, 64 if case.kind == "batch" else case.L)
-    ents = _plain(case.descs, case.image)
-    want, want_counts, want_p = plain_find_set(ents, pats)
+    ents = decipher_entries(case.descs, case.image)
+    want, want_counts, want_p = search(ents, pats)
     mem = case.memory()
-    buf = _buffer(mem)
+    buf = aligned_buffer(mem)
     try:
         if case.kind == "batch":
-            counts, pcounts, matches, total = mb.find_set_batch(_mdescs(case.descs), buf.ptr + case.src_ptr, pats,
+            counts, pcounts, matches, total = mb.find_set_batch(model_descs(case.descs), buf.ptr + case.src_ptr, pats,
                                                                 src_bytes=case.image_bytes, max_matches=1 << 16)
             assert total == len(want) and as_list(matches) == want, cell
             assert counts.tolist() == want_counts.tolist() and pcounts.tolist() == want_p.tolist()
@@ -172,7 +151,7 @@ def test_model_cases_through_the_set_kernel(cell):
             t0, t1, wp, wo, wb = case.win
             lo, hi = case.entry_starts()
             want0 = [(d, p, 0) for d, p, j in want if j == 0 and d == case.target and lo <= p < hi]
-            plan = mb.Plan(_mdescs(case.descs), case.image_bytes, case.image_bytes, case.dst_align)
+            plan = mb.Plan(model_descs(case.descs), case.image_bytes, case.image_bytes, case.dst_align)
             pset = mb.PatternSet(pats)
             res = Results(len(case.descs), 1 << 12)
             pc = DeviceBuffer(8 * len(pats))
@@ -255,7 +234,7 @@ def test_cap_and_accumulation(which):
     for e in ents:
         e[rng.integers(0, e.size, size=e.size // 3)] = 1
     keys = synth.entry_keys(len(ents)).tolist()
-    want, want_counts, want_p = plain_find_set(ents, pats)
+    want, want_counts, want_p = search(ents, pats)
     n = len(want)
     cap = {"0": 0, "1": 1, "n": n, "n+1": n + 1}[which]
     descs, src, buf, plan, res, pc, m = _plan_and_buffers(ents, keys, pats, cap=cap)
@@ -299,7 +278,7 @@ def test_window_bounds_use_lmax():
     sync()
     total = int(res.buf.download()[:8].view(np.uint64)[0])
     got = sorted(as_list(m.download().view(mb.SET_MATCH_DTYPE)[:total]))
-    want, _, _ = plain_find_set([oracle.cycle(src[:ent.size], 0x1234567)], pats)
+    want, _, _ = search([oracle.cycle(src[:ent.size], 0x1234567)], pats)
     assert got == [x for x in want if lo <= x[1] < 8192 * t1 - h0] and (0, 3 * 8192 - 7, 2) in got
     for bad_lo, bad_hi in ((lo + 1, hi), (lo, hi - 1)):
         lib = mb._abi.load()
@@ -375,7 +354,7 @@ def test_facade_find_set_on_a_ciphered_1gib_archive_on_every_gpu(tmp_path):
         arkfixture.write_archive(root, n_files=len(sizes), n_parts=4, seed=37, body_key=key, sizes=sizes)
         pats = [b"\x5a\xa5\x0f", b"\x5a\xa5", b"\x01\x02\x03\x04\x05", b"\x33\x44\x55\x66"]
         shown = [p.hex() for p in pats]
-        want_lines, want_counts, want_total, want_files = oracle_find_set(root, "ps4", pats, shown, key)
+        want_lines, want_counts, want_total, want_files = expected_output(root, "ps4", pats, key=key, shown=shown)
         with open(os.path.join(root, "l.txt"), "w") as f:
             f.write("\n".join(shown) + "\n")
         all_gpus = hex((1 << mb.device_count()) - 1)

@@ -27,16 +27,18 @@ import oracle
 import synth
 from oracle import ark_oracle as ao
 from oracle import dta_oracle as do
-from arkfixture import fixture_file_bytes
-from test_facade_host import cli, run  # noqa: F401  (fixture + helper)
+from arkfixture import CASES, GOLD, MANIFEST, fixture_file_bytes, ref_header, run
+from searchutil import mock_cli
 
-GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-with open(os.path.join(GOLD, "ark", "manifest.json")) as _f:
-    MANIFEST = json.load(_f)
 with open(os.path.join(GOLD, "dtb", "index.json")) as _f:
     DTB_INDEX = json.load(_f)
-SONGS = MANIFEST.pop("songs")
-CASES = sorted(MANIFEST)
+SONGS = MANIFEST["songs"]
+
+
+@pytest.fixture(scope="session")
+def cli():
+    """modulate CLI on the mock ABI, without the search entry points."""
+    return mock_cli(0)
 
 
 def sha(b: bytes) -> str:
@@ -52,12 +54,6 @@ def masked(hdr: bytes) -> bytes:
 def decipher(raw: bytes) -> bytes:
     magic = int.from_bytes(raw[:4], "little")
     return raw[:4] + oracle.cycle(np.frombuffer(raw[4:], dtype=np.uint8), ao.platform_key(magic)).tobytes()
-
-
-def ref_header(case: str) -> bytes:
-    plat = MANIFEST[case]["platform"]
-    with open(os.path.join(GOLD, "ark", case, f"main_{plat}.hdr"), "rb") as f:
-        return f.read()
 
 
 def entries_of(table):
